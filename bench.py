@@ -3,7 +3,7 @@
 
 Metric (BASELINE.json): k=200 Murty problems/sec at 1/2/4/8 B200; permanent n=24 latency vs host CPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path -- cost matrix in, k-best lists + gains + nM x (nL+1)
 association weights out (SURVEY.md 8d) -- over one batch of 100 000 KITTI-shaped synthetic problems
@@ -15,11 +15,14 @@ collective; one max-reduction of the elapsed time).
   e2e     the same metric through the reference-facing call -- batched assignmentProb
           (pda_murty_batch_host): HOST cost matrices in, HOST weights out, copies inside the timed region
   roofline  HBM: algorithmic bytes of a pass / measured kernel time, against MEASURED_PEAKS.json
-  cpu_baseline  the reference's own CPU code (oracle/_ref, built from /root/reference) or, failing that,
+  cpu_baseline  the reference's own CPU code (oracle/_ref, built from the reference's sources) or, failing that,
           the oracle port, on this box's host cores over a bounded sample of the same workload
   extra.permanent_n24  latency of one dense 24x24 permanent, GPU vs the same CPU arm
 
 --impl reference times the reference's CPU implementation only (no GPU code on that path).
+
+--dump-outputs DIR writes what the last timed step returned (rank 0's batch) as DIR/<name>.npy, so that two builds
+can be compared output for output on identical seeded inputs: see dump_outputs().
 """
 from __future__ import annotations
 
@@ -137,6 +140,52 @@ def cpu_permanent_ms(chk, threads: int = 1):
     return sec * 1e3
 
 
+DUMP_PROBLEMS = 1024
+DUMP_BYTES = 64 << 20
+DUMP_SEED = 20260217
+
+
+def dump_outputs(plan, pb, out_dir):
+    """Writes the k-best pass's results for a fixed, seeded sample of problems (at most DUMP_PROBLEMS, at most DUMP_BYTES
+    in all), concatenated in sample order:
+      problems  the sampled problem indices                        n_found  nFound per problem
+      gain      [problems, k], NaN beyond nFound                   probs    the nM x (nL+1) weight table per problem
+      row4col   the k x nM list per problem, col4row  the k x (nL+nM) list per problem; -1 beyond nFound
+    Index lists are stored as float32 (exact for these small integers), everything else as float64.  Only the first
+    nFound hypotheses of a problem are defined, so the rest is masked to make runs comparable bit for bit."""
+    import torch
+    k = plan.k
+    nc = pb.nM.astype(np.int64)
+    nr = pb.num_row.astype(np.int64)
+    w = nc * (pb.nL.astype(np.int64) + 1)
+    order = np.random.default_rng(DUMP_SEED).permutation(len(pb))[:DUMP_PROBLEMS]
+    cost = np.cumsum(16 + 8 * k + 4 * k * (nc[order] + nr[order]) + 8 * w[order])
+    idx = np.sort(order[:int(np.searchsorted(cost, DUMP_BYTES, side="right"))])
+    nf = plan.n_found.cpu().numpy()[idx].astype(np.int64)
+
+    def gather(t, off, size):
+        """The segments [off[p], off[p] + size[p]) of device tensor t for the sampled p, and each element's position
+        inside its segment."""
+        start, size = off[idx], size[idx]
+        within = np.arange(int(size.sum())) - np.repeat(np.cumsum(size) - size, size)
+        pos = torch.from_numpy(np.repeat(start, size) + within).to(t.device)
+        return t[pos].cpu().numpy(), within, size
+
+    def lists(t, off, width):
+        v, within, size = gather(t, off, width * k)
+        hyp = within // np.repeat(width[idx], size)
+        return np.where(hyp < np.repeat(nf, size), v, -1).astype(np.float32)
+
+    gain = plan.gain.view(plan.n, k)[torch.from_numpy(idx).to(plan.gain.device)].cpu().numpy()
+    gain[np.arange(k)[None, :] >= nf[:, None]] = np.nan
+    out = {"problems": idx.astype(np.float64), "n_found": nf.astype(np.float64), "gain": gain,
+           "row4col": lists(plan.row4col, plan.r4c_off_h, nc), "col4row": lists(plan.col4row, plan.c4r_off_h, nr),
+           "probs": gather(plan.probs, plan.prob_off_h, w)[0]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_reference(args):
     """--impl reference: the reference's CPU implementation of the path, all host threads."""
     rank = int(os.environ.get("RANK", "0"))
@@ -178,7 +227,12 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--skip-config3", action="store_true", help="skip extra.config3_k1000_strong (profiling runs)")
     ap.add_argument("--skip-config4", action="store_true", help="skip extra.permanent_batch_sharded (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's results; --impl reference has none")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -230,6 +284,8 @@ def main():
     alg_bytes = plan.algorithmic_bytes()
     kernel_ms = statistics.mean(step_ms)
     fallback_problems = int(plan.workspace[8:12].view(torch.int32).item())  # problems the pruning kernel handed to the exact one
+    if args.dump_outputs and rank == 0:
+        dump_outputs(plan, pb, args.dump_outputs)
 
     # ---- end to end: host buffers through the C ABI (batched assignmentProb) ----------------------------
     nL32, nM32 = pb.nL.astype(np.int32), pb.nM.astype(np.int32)

@@ -37,6 +37,21 @@ def assert_kbest_equal(got, want, what=""):
     np.testing.assert_array_equal(bits(got[3][:n]), bits(want[3][:n]), err_msg=f"{what}: gain bits")
 
 
+def compmethods_dat_files(directory):
+    """Writes the .dat cost-matrix files that the compMethods-style driver reads in tests/test_gpu_dropin.py: ten gated
+    G2 frames (the wire format quantises to 6 decimals, so exact ties appear) and three small dense G1 frames.
+    Returns [(path, matrix before quantisation)]."""
+    from probabilisticsemslam_b200 import datfile, synth
+    files = []
+    for run_id, pb in (("o30_p0_k200_perm0_net1", synth.g2_gated(10, first=900)),
+                       ("small", synth.g1_dense(3, nL=9, nM=3, first=77))):
+        for p in range(len(pb)):
+            path = datfile.frame_path(directory, run_id, p + 1)
+            datfile.write_dat(path, pb.matrix(p))
+            files.append((path, pb.matrix(p)))
+    return files
+
+
 def rel_err(a, b):
     a, b = np.asarray(a, np.float64), np.asarray(b, np.float64)
     d = np.abs(a - b)
