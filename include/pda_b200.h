@@ -185,6 +185,39 @@ int pda_association_probs_batch_host(const double* costs, const int64_t* costOff
                                      int64_t nProblems, int32_t k, double* probs, const int64_t* probOff,
                                      int32_t device);
 
+/* The same body with usePerm == 1 (assignment.cpp:64: permanentProb(cond, condL, nM, 1) in place of assignmentProb),
+ * fused on the device: conditionCosts -> likelihoods -> every sub-permanent by one fused gather / condition / subset-DP
+ * kernel that keeps each sub-matrix in shared memory -> column sums, normalisation and the scatter through rowIdx.
+ * Tables are bit-identical to conditionCosts -> pda_permanent_prob_batch_host(.., 1) -> scatter.  Arguments as for
+ * pda_association_probs_batch; status[p] = 0, 1 where the reference throws (a sub-matrix with more than 32 kept rows),
+ * 2 where problem p exceeds maxNumRow / maxNumCol (not computed, table untouched -- the conditioning skips it too), 3
+ * where conditioning kept fewer rows than there are detections (condL = goodRows - nM < 0, where the reference's size_t
+ * subtraction underflows; table all zero).  A gated dummy row with goodRows >= nM is computed as the reference does.
+ * pda_association_perm_probs_batch takes problems with nM <= 11 only (maxNumCol > 11 -> PDA_ERR_UNSUPPORTED): every
+ *   sub-permanent then has a short side <= 10 and none can come out negative.  It enqueues four launches on `stream`
+ *   and never synchronises, so it can be captured in a CUDA graph.  Workspace: O(sum of nM*(nL+1)) doubles.
+ * pda_association_perm_probs_batch_host validates the whole batch on the host first; problems with 12+ detections take
+ *   the route above (conditionCosts, pda_permanent_prob_batch_host, scatter), so their results are that route's.
+ * pda_association_perm_from_moments_batch_host: pda_quadric_cost_batch followed by the pipeline (the usePerm form of
+ *   pda_association_from_moments_batch_host); probs and status per frame, frames back to back.
+ * The _multi forms cut the batch into contiguous slices, one per device (offsets must be non-decreasing). */
+int64_t pda_association_perm_workspace_bytes(int64_t nProblems, int64_t totalCostElems, int64_t totalRows,
+                                             int64_t totalProbElems, int32_t maxNumRow, int32_t maxNumCol);
+int pda_association_perm_probs_batch(const double* costs, const int64_t* costOff, const int32_t* nL, const int32_t* nM,
+                                     const int64_t* rowOff, int64_t nProblems, int64_t totalCostElems, int64_t totalRows,
+                                     int64_t totalProbElems, int32_t maxNumRow, int32_t maxNumCol,
+                                     double* probs, const int64_t* probOff, int32_t* status,
+                                     void* workspace, int64_t workspaceBytes, void* stream);
+int pda_association_perm_probs_batch_host(const double* costs, const int64_t* costOff, const int32_t* nL, const int32_t* nM,
+                                          int64_t nProblems, double* probs, const int64_t* probOff, int32_t* status,
+                                          int32_t device);
+int pda_association_probs_batch_host_multi(const double* costs, const int64_t* costOff, const int32_t* nL, const int32_t* nM,
+                                           int64_t nProblems, int32_t k, double* probs, const int64_t* probOff,
+                                           const int32_t* devices, int32_t nDevices);
+int pda_association_perm_probs_batch_host_multi(const double* costs, const int64_t* costOff, const int32_t* nL,
+                                                const int32_t* nM, int64_t nProblems, double* probs, const int64_t* probOff,
+                                                int32_t* status, const int32_t* devices, int32_t nDevices);
+
 /* ------------------------------------------------------------------------------------------
  * The step in front of the path: cost matrices from quadric moments, on the device.
  * pda_quadric_covs_batch: getCovs (assignment.cpp:693-703) -- quadrics = n 4x4 dual-quadric matrices (16 doubles
@@ -213,6 +246,10 @@ int pda_quadric_cost_batch_host(const double* landMean, const double* landCov, c
 int pda_association_from_moments_batch_host(const double* landMean, const double* landCov, const int64_t* landOff,
                                             const double* measMean, const double* measCov, const int64_t* measOff,
                                             int64_t nFrames, double nonassign, int32_t k, double* probs, int32_t device);
+int pda_association_perm_from_moments_batch_host(const double* landMean, const double* landCov, const int64_t* landOff,
+                                                 const double* measMean, const double* measCov, const int64_t* measOff,
+                                                 int64_t nFrames, double nonassign, double* probs, int32_t* status,
+                                                 int32_t device);
 
 /* ------------------------------------------------------------------------------------------
  * Stereo bounding-box association: asgnBB (assignment.h:21, assignment.cpp:724-775) with computeBBCostMatrix

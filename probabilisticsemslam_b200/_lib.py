@@ -40,11 +40,17 @@ SIGNATURES = {
     "pda_association_workspace_bytes": (i64, [i64, i64, i64, i64, i32, i32, i32]),
     "pda_association_probs_batch": (C.c_int, [ptr, ptr, ptr, ptr, ptr, i64, i64, i64, i64, i32, i32, i32, ptr, ptr, ptr, ptr, i64, ptr]),
     "pda_association_probs_batch_host": (C.c_int, [ptr, ptr, ptr, ptr, i64, i32, ptr, ptr, i32]),
+    "pda_association_perm_workspace_bytes": (i64, [i64, i64, i64, i64, i32, i32]),
+    "pda_association_perm_probs_batch": (C.c_int, [ptr, ptr, ptr, ptr, ptr, i64, i64, i64, i64, i32, i32, ptr, ptr, ptr, ptr, i64, ptr]),
+    "pda_association_perm_probs_batch_host": (C.c_int, [ptr, ptr, ptr, ptr, i64, ptr, ptr, ptr, i32]),
+    "pda_association_probs_batch_host_multi": (C.c_int, [ptr, ptr, ptr, ptr, i64, i32, ptr, ptr, ptr, i32]),
+    "pda_association_perm_probs_batch_host_multi": (C.c_int, [ptr, ptr, ptr, ptr, i64, ptr, ptr, ptr, ptr, i32]),
     "pda_quadric_covs_batch": (C.c_int, [ptr, i64, ptr, ptr]),
     "pda_quadric_covs_batch_host": (C.c_int, [ptr, i64, ptr, i32]),
     "pda_quadric_cost_batch": (C.c_int, [ptr, ptr, ptr, ptr, ptr, ptr, i64, dbl, ptr, ptr, ptr, ptr, ptr]),
     "pda_quadric_cost_batch_host": (C.c_int, [ptr, ptr, ptr, ptr, ptr, ptr, i64, dbl, ptr, i32]),
     "pda_association_from_moments_batch_host": (C.c_int, [ptr, ptr, ptr, ptr, ptr, ptr, i64, dbl, i32, ptr, i32]),
+    "pda_association_perm_from_moments_batch_host": (C.c_int, [ptr, ptr, ptr, ptr, ptr, ptr, i64, dbl, ptr, ptr, i32]),
     "pda_asgn_bb_batch_host": (C.c_int, [ptr, ptr, ptr, ptr, i64, dbl, ptr, i32]),
     "pda_permanent_workspace_bytes": (i64, [i64]),
     "pda_permanent_batch": (C.c_int, [ptr, ptr, ptr, ptr, i64, i32, ptr, ptr, ptr, i64, ptr]),

@@ -108,8 +108,12 @@ int launch_lap(const LapArgs& a, cudaStream_t stream);
 int launch_condition_costs(const double* costs, const int64_t* costOff, const int32_t* numRow,
                            const int32_t* numCol, int64_t nProblems, const int64_t* rowOff,
                            double* outCosts, int64_t* rowIdx, int32_t* goodRows, cudaStream_t stream,
-                           const int32_t* nLopt = nullptr, int32_t* condNL = nullptr);  // nLopt: numRow = nLopt + numCol
-int launch_to_probs(double* values, const int64_t* off, const int64_t* len, int64_t nVectors, cudaStream_t stream);
+                           const int32_t* nLopt = nullptr, int32_t* condNL = nullptr,  // nLopt: numRow = nLopt + numCol
+                           int32_t maxRow = INT32_MAX, int32_t maxCol = INT32_MAX);    // larger problems are skipped
+// rows / cols (device, optional): vector p is the rows[p] x cols[p] matrix at off[p] (len is not read) -- the
+// conditioned matrices, whose size only the device knows
+int launch_to_probs(double* values, const int64_t* off, const int64_t* len, int64_t nVectors, cudaStream_t stream,
+                    const int32_t* rows = nullptr, const int32_t* cols = nullptr);
 
 // ---- permanents (permanent_kernel.cu) ------------------------------------------------------------
 int launch_permanent_batch(const double* mats, const int64_t* matOff, const int32_t* rows, const int32_t* cols,

@@ -16,6 +16,7 @@
 // max(rows, cols), divide by (|rows - cols|)!.
 #include "pda_internal.h"
 #include "pda_host_stage.h"
+#include "perm_device.cuh"
 
 #include <algorithm>
 #include <vector>
@@ -483,33 +484,10 @@ __global__ void __launch_bounds__(PERM_THREADS, perm_min_blocks(NP)) perm_kernel
 __device__ __forceinline__ void perm_dp_warp(const PermArgs& a, const int64_t it, const int rows, const int cols,
                                              double* __restrict__ buf, double* __restrict__ out,
                                              int32_t* __restrict__ status, const int lane) {
-    const int m = rows < cols ? rows : cols, n = rows < cols ? cols : rows;
+    const int n = rows < cols ? cols : rows;
     if (n > PDA_MAX_PERM_DIM) { if (lane == 0) { out[it] = 0.0; if (status) status[it] = 1; } return; }  // nwPerm.cpp:327-330
-    const int cap = 1 << a.dpBits, states = 1 << m;
-    double* cur = buf;
-    double* nxt = cur + cap;
-    double* sb = cur + 2 * cap;
-    for (int S = lane; S < states; S += 32) cur[S] = (S == 0) ? 1.0 : 0.0;
-    const double* A = a.mats + a.matOff[it];
-    const bool shortRows = rows <= cols;
-    for (int j = 0; j < n; ++j) {
-        __syncwarp();
-        if (lane < m) sb[lane] = shortRows ? A[lane + (size_t)j * rows] : A[j + (size_t)lane * rows];
-        __syncwarp();
-        for (int S = lane; S < states; S += 32) {
-            double acc = cur[S];
-            unsigned bits = (unsigned)S;
-            while (bits) {
-                const int i = __ffs(bits) - 1;
-                bits &= bits - 1u;
-                acc = fma(sb[i], cur[S ^ (1 << i)], acc);
-            }
-            nxt[S] = acc;
-        }
-        double* t = cur; cur = nxt; nxt = t;
-    }
-    __syncwarp();
-    if (lane == 0) { out[it] = cur[states - 1]; if (status) status[it] = 0; }
+    const double r = perm_dp_subsets(a.mats + a.matOff[it], rows, cols, buf, 1 << a.dpBits, lane);
+    if (lane == 0) { out[it] = r; if (status) status[it] = 0; }
 }
 
 // One warp per matrix: sums the per-CTA partials (lane-strided, then a fixed shuffle tree -- the order depends

@@ -74,6 +74,14 @@ std::vector<std::vector<double> > permanentProb(std::vector<double> costMatrix, 
     return unflatten(probs, nM, nL + 1);
 }
 
+// status of the usePerm pipeline -> the reference's exceptions
+static void permStatusCheck(int32_t status) {
+    if (status == 1) throw std::runtime_error("Maximum matrix dimension limited to 32. Error inside permanentExactSquare().");
+    if (status)
+        throw std::runtime_error("getAssignmentProbs: conditionCosts kept fewer rows than there are detections, so condL "
+                                 "= goodRows - nM is negative (the reference's size_t subtraction underflows)");
+}
+
 std::vector<std::vector<double> > getAssignmentProbsFromCosts(const std::vector<double>& costMatrix, size_t nL, size_t nM,
                                                               size_t k, bool usePerm) {
     if (nM == 0) return std::vector<std::vector<double> >();
@@ -86,17 +94,15 @@ std::vector<std::vector<double> > getAssignmentProbsFromCosts(const std::vector<
                  "getAssignmentProbsFromCosts");
         return unflatten(probs, nM, nL + 1);
     }
-    if (nL == 0) return std::vector<std::vector<double> >(nM, std::vector<double>{1});
-    std::vector<ptrdiff_t> rowIdx;
-    std::vector<double> cond = conditionCosts(costMatrix, nL + nM, nM, rowIdx);
-    const size_t condL = (cond.size() / nM) - nM;
-    std::vector<std::vector<double> > cp = permanentProb(cond, condL, nM, 1);
-    std::vector<std::vector<double> > probs(nM, std::vector<double>(nL + 1, 0));
-    for (size_t m = 0; m < nM; m++) {
-        for (size_t l = 0; l < condL; l++) probs[m][size_t(rowIdx[l])] = cp[m][l];
-        probs[m][nL] = cp[m][condL];
-    }
-    return probs;
+    const int64_t costOff = 0, probOff = 0;  // usePerm: the fused permanent pipeline
+    const int32_t nl = int32_t(nL), nm = int32_t(nM);
+    int32_t status = 0;
+    std::vector<double> probs(nM * (nL + 1), 0.0);
+    pdaCheck(pda_association_perm_probs_batch_host(costMatrix.data(), &costOff, &nl, &nm, 1, probs.data(), &probOff, &status,
+                                                   pdaShimDevice()),
+             "getAssignmentProbsFromCosts");
+    permStatusCheck(status);
+    return unflatten(probs, nM, nL + 1);
 }
 
 std::vector<double> computeQuadricCostMatrixRaw(const std::vector<double>& landMeans, const std::vector<double>& landCovs,
@@ -125,6 +131,25 @@ std::vector<std::vector<double> > getAssignmentProbsFromMoments(const std::vecto
     pdaCheck(pda_association_from_moments_batch_host(landMeans.data(), landCovs.data(), offL, measMeans.data(), measCovs.data(), offM, 1,
                                                      nonassign, int32_t(k), probs.data(), pdaShimDevice()),
              "getAssignmentProbsFromMoments");
+    return unflatten(probs, nM, nL + 1);
+}
+
+std::vector<std::vector<double> > getAssignmentProbsFromMoments(const std::vector<double>& landMeans,
+                                                                const std::vector<double>& landCovs,
+                                                                const std::vector<double>& measMeans,
+                                                                const std::vector<double>& measCovs, double nonassign, size_t k,
+                                                                bool usePerm) {
+    if (!usePerm) return getAssignmentProbsFromMoments(landMeans, landCovs, measMeans, measCovs, nonassign, k);
+    const size_t nL = landMeans.size() / 3, nM = measMeans.size() / 3;
+    if (landCovs.size() != 9 * nL || measCovs.size() != 9 * nM) throw std::runtime_error("getAssignmentProbs: moment sizes disagree");
+    if (nM == 0) return std::vector<std::vector<double> >();
+    const int64_t offL[2] = {0, int64_t(nL)}, offM[2] = {0, int64_t(nM)};
+    std::vector<double> probs(nM * (nL + 1), 0.0);
+    int32_t status = 0;
+    pdaCheck(pda_association_perm_from_moments_batch_host(landMeans.data(), landCovs.data(), offL, measMeans.data(), measCovs.data(),
+                                                          offM, 1, nonassign, probs.data(), &status, pdaShimDevice()),
+             "getAssignmentProbsFromMoments");
+    permStatusCheck(status);
     return unflatten(probs, nM, nL + 1);
 }
 
@@ -269,6 +294,32 @@ std::vector<std::vector<std::vector<double> > > permanentProbBatch(const std::ve
                  "permanentProbBatch");
     for (size_t p = 0; p < n; p++)
         if (status[p]) throw std::runtime_error("permanentProbBatch: the reference throws for one of these problems (dimension > 32 or bad permOpt)");
+    return fb.tables(nL, nM);
+}
+
+std::vector<std::vector<std::vector<double> > > getAssignmentProbsBatch(const std::vector<std::vector<double> >& costs,
+                                                                        const std::vector<size_t>& nL,
+                                                                        const std::vector<size_t>& nM, size_t k, bool usePerm,
+                                                                        const std::vector<int>& devices) {
+    if (nL.size() != costs.size() || nM.size() != costs.size()) throw std::invalid_argument("getAssignmentProbsBatch: nL / nM sizes differ from costs");
+    FlatBatch fb(costs, nL, nM);
+    const size_t n = costs.size();
+    const std::vector<int32_t> dev = deviceList(devices);
+    if (n == 0) return fb.tables(nL, nM);
+    for (size_t p = 0; p < n; p++)
+        if (nM[p] == 0) throw std::invalid_argument("getAssignmentProbsBatch: a frame without detections");
+    if (!usePerm) {
+        pdaCheck(pda_association_probs_batch_host_multi(fb.flat.data(), fb.costOff.data(), fb.nl.data(), fb.nc.data(), int64_t(n), int32_t(k),
+                                                        fb.probs.data(), fb.probOff.data(), dev.data(), int32_t(dev.size())),
+                 "getAssignmentProbsBatch");
+        return fb.tables(nL, nM);
+    }
+    std::vector<int32_t> status(n, 0);
+    pdaCheck(pda_association_perm_probs_batch_host_multi(fb.flat.data(), fb.costOff.data(), fb.nl.data(), fb.nc.data(), int64_t(n),
+                                                         fb.probs.data(), fb.probOff.data(), status.data(), dev.data(),
+                                                         int32_t(dev.size())),
+             "getAssignmentProbsBatch");
+    for (size_t p = 0; p < n; p++) permStatusCheck(status[p]);
     return fb.tables(nL, nM);
 }
 

@@ -30,13 +30,17 @@ __global__ void condition_costs_kernel(const double* __restrict__ costs, const i
                                        const int64_t nProblems, const int64_t* __restrict__ rowOff,
                                        double* __restrict__ outCosts, int64_t* __restrict__ rowIdx,
                                        int32_t* __restrict__ goodRows, const int32_t* __restrict__ nLopt,
-                                       int32_t* __restrict__ condNL) {
+                                       int32_t* __restrict__ condNL, const int32_t maxRow, const int32_t maxCol) {
     __shared__ double colMinS[WARPS][PDA_MAX_DIM];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int64_t p = (int64_t)blockIdx.x * WARPS + warp;
     if (p >= nProblems) return;
     const int nC = numCol[p];
     const int nR = nLopt ? nLopt[p] + nC : numRow[p];  // the association pipeline passes nL and lets this kernel add
+    if (nC > maxCol || nR > maxRow) {  // outside the caller's scope: left alone (colMinS holds PDA_MAX_DIM columns)
+        if (lane == 0) { goodRows[p] = 0; if (condNL) condNL[p] = -1; }
+        return;
+    }
     const double* C = costs + costOff[p];
     double* colMin = colMinS[warp];
     for (int c = 0; c < nC; ++c) {
@@ -84,12 +88,13 @@ __global__ void condition_costs_kernel(const double* __restrict__ costs, const i
 }
 
 __global__ void to_probs_kernel(double* __restrict__ values, const int64_t* __restrict__ off,
-                                const int64_t* __restrict__ len, const int64_t nVectors) {
+                                const int64_t* __restrict__ len, const int64_t nVectors,
+                                const int32_t* __restrict__ rows, const int32_t* __restrict__ cols) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int64_t p = (int64_t)blockIdx.x * WARPS + warp;
     if (p >= nVectors) return;
     double* v = values + off[p];
-    const int64_t n = len[p];
+    const int64_t n = rows ? (int64_t)rows[p] * cols[p] : len[p];
     double lo = CUDART_INF;
     for (int64_t i = lane; i < n; i += 32) { const double x = v[i]; lo = (x < lo) ? x : lo; }
     lo = warp_min(lo);
@@ -104,17 +109,18 @@ __global__ void to_probs_kernel(double* __restrict__ values, const int64_t* __re
 int launch_condition_costs(const double* costs, const int64_t* costOff, const int32_t* numRow,
                            const int32_t* numCol, int64_t nProblems, const int64_t* rowOff,
                            double* outCosts, int64_t* rowIdx, int32_t* goodRows, cudaStream_t stream,
-                           const int32_t* nLopt, int32_t* condNL) {
+                           const int32_t* nLopt, int32_t* condNL, int32_t maxRow, int32_t maxCol) {
     const int64_t ctas = (nProblems + WARPS - 1) / WARPS;
     condition_costs_kernel<<<(unsigned)ctas, 32 * WARPS, 0, stream>>>(costs, costOff, numRow, numCol, nProblems, rowOff,
-                                                                      outCosts, rowIdx, goodRows, nLopt, condNL);
+                                                                      outCosts, rowIdx, goodRows, nLopt, condNL, maxRow, maxCol);
     PDA_CUDA_TRY(cudaGetLastError());
     return PDA_OK;
 }
 
-int launch_to_probs(double* values, const int64_t* off, const int64_t* len, int64_t nVectors, cudaStream_t stream) {
+int launch_to_probs(double* values, const int64_t* off, const int64_t* len, int64_t nVectors, cudaStream_t stream,
+                    const int32_t* rows, const int32_t* cols) {
     const int64_t ctas = (nVectors + WARPS - 1) / WARPS;
-    to_probs_kernel<<<(unsigned)ctas, 32 * WARPS, 0, stream>>>(values, off, len, nVectors);
+    to_probs_kernel<<<(unsigned)ctas, 32 * WARPS, 0, stream>>>(values, off, len, nVectors, rows, cols);
     PDA_CUDA_TRY(cudaGetLastError());
     return PDA_OK;
 }
