@@ -270,6 +270,11 @@ int pda_asgn_bb_batch_host(const double* boxesL, const int64_t* offL, const doub
  *   exactly as the reference does.  out[i] = permanent; status[i] = 0, or 1 where the
  *   reference throws (dimension > 32).  maxDim >= max(rows[i], cols[i]) over the batch
  *   (it selects the register tile; a batch is fastest when its matrices share one size).
+ *   This device-pointer form walks every matrix the reference's way (NW on the ones-padded
+ *   square), whatever its size; a matrix with max(rows, cols) above maxDim (but <= 32) is not
+ *   computed: out[i] = 0 and status[i] = 2.  Status 1 takes precedence.
+ * pda_permanent_batch_host sees the dimensions, so it sends matrices whose short side is <= 10
+ *   to a cancellation-free subset dynamic programme instead; it never reports status 2.
  * pda_permanent_range: partial NW sum of ONE n x n matrix over Gray indices [begin, end)
  *   (index 0 = the empty-subset seed term), as an unevaluated double-double partial[0] + partial[1];
  *   partial sums over disjoint ranges covering [0, 2^(n-1)) add up to p, and the permanent is

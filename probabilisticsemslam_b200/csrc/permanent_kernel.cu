@@ -369,6 +369,7 @@ __device__ __forceinline__ void perm_finish_warp(const PermArgs& a, const int64_
     const int rows = a.oneDim > 0 ? a.oneDim : a.rows[m], cols = a.oneDim > 0 ? a.oneDim : a.cols[m];
     const int n = rows > cols ? rows : cols;
     if (n > PDA_MAX_PERM_DIM) { out[m] = 0.0; if (status) status[m] = 1; return; }  // nwPerm.cpp:327-330 throws
+    if (n > a.maxN) { out[m] = 0.0; if (status) status[m] = 2; return; }  // above the call's maxDim: perm_kernel skipped it
     if (status) status[m] = 0;
     if (n == 0) { out[m] = 1.0; return; }  // nwPerm.cpp:261-264
     double p = (double)(4 * (n & 1) - 2) * (t.hi + t.lo);
@@ -570,11 +571,13 @@ int launch_permanent_batch(const double* mats, const int64_t* matOff, const int3
                            int64_t workspaceBytes, cudaStream_t stream, int32_t maxSmall, int32_t minSmall) {
     DeviceInfo dev;
     PDA_TRY(current_device_info(&dev));
-    const int effDim = std::max(1, std::min<int>(maxDim, PDA_MAX_PERM_DIM));
+    // 0 when maxDim is 0: every matrix with a side then ends as status 2 (perm_finish_warp)
+    const int effDim = std::max(0, std::min<int>(maxDim, PDA_MAX_PERM_DIM));
     // maxSmall / minSmall: bounds on min(rows, cols) over the batch when the caller knows them (else maxDim / 0)
     const int dpBits = std::min(PERM_DP_MAX, std::max(0, std::min<int>(maxSmall < 0 ? maxDim : maxSmall, maxDim)));
-    const bool allDp = (maxSmall >= 0 ? maxSmall : maxDim) <= dpBits;   // nothing for the NW walk
     const bool noneDp = minSmall > dpBits;
+    // nothing for the NW walk.  Never together with noneDp: the DP path then has no shared memory (dpSmem == 0)
+    const bool allDp = !noneDp && (maxSmall >= 0 ? maxSmall : maxDim) <= dpBits;
     const size_t dpSmem = noneDp ? 0 : (size_t)4 * (2 * ((size_t)1 << dpBits) + 16) * sizeof(double);  // 4 warps per finalize CTA
     if (dpSmem > 48 * 1024) PDA_CUDA_TRY(cudaFuncSetAttribute(perm_finalize_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dpSmem));
     if (allDp) {
@@ -655,8 +658,9 @@ int pda_permanent_batch(const double* mats, const int64_t* matOff, const int32_t
     if (!mats || !matOff || !rows || !cols || !out || !workspace) return fail(PDA_ERR_INVALID, "permanent: NULL argument");
     if (maxDim < 0) return fail(PDA_ERR_INVALID, "permanent: maxDim < 0");
     // the dimensions live on the device, so this entry cannot tell whether any matrix has a short side: it walks every
-    // matrix the reference's way (NW on the ones-padded square).  The *_host entries, which see the dimensions, send
-    // short-sided matrices to the cancellation-free subset programme (perm_dp_warp).
+    // matrix the reference's way (NW on the ones-padded square), tiles 2..32 alike (minSmall above every dpBits keeps
+    // perm_dp_warp out).  The *_host entries, which see the dimensions, send short-sided matrices to the
+    // cancellation-free subset programme (perm_dp_warp).  A matrix above maxDim ends as status 2 (perm_finish_warp).
     return launch_permanent_batch(mats, matOff, rows, cols, nMats, maxDim, out, status, workspace, workspaceBytes,
                                   reinterpret_cast<cudaStream_t>(stream), -1, PDA_MAX_DIM + 1);
 }
