@@ -108,6 +108,15 @@ std::vector<std::vector<std::vector<double> > > assignmentProbBatch(const std::v
                                                                     const std::vector<size_t>& nL,
                                                                     const std::vector<size_t>& nM, size_t k,
                                                                     const std::vector<int>& devices);
+/* assignmentProb for several k at once (compMethods' k = 1, 20, 1000, 100, 200, ... on one frame,
+ * comparison.cpp:194-222) from ONE enumeration to the largest k: returns probs[j][m][l], the table of ks[j], each
+ * bit-identical to assignmentProb(costMatrix, nL, nM, ks[j]).  ks: 1 to 16 values >= 1, any order, duplicates allowed.
+ * The Batch form takes problems as assignmentProbBatch does and returns probs[p][j][m][l]. */
+std::vector<std::vector<std::vector<double> > > assignmentProbLadder(const std::vector<double>& costMatrix, size_t nL, size_t nM,
+                                                                     const std::vector<size_t>& ks);
+std::vector<std::vector<std::vector<std::vector<double> > > > assignmentProbLadderBatch(
+    const std::vector<std::vector<double> >& costs, const std::vector<size_t>& nL, const std::vector<size_t>& nM,
+    const std::vector<size_t>& ks);
 /* permanentProb (assignment.cpp:145-290) for many problems, optionally over several GPUs (empty `devices` = the shim's
  * device).  Throws where the reference throws. */
 std::vector<std::vector<std::vector<double> > > permanentProbBatch(const std::vector<std::vector<double> >& costs,

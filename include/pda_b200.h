@@ -136,6 +136,32 @@ int pda_murty_batch_host_multi(const double* costs, const int64_t* costOff, cons
                                int32_t weightMode, double* probs, const int64_t* probOff, const int32_t* nL,
                                const int32_t* devices, int32_t nDevices);
 
+/* assignmentProb (assignment.cpp:547-683) for several k at once, from ONE Murty enumeration: the weight tables of
+ * every k in ks[0..nK) (any order, duplicates allowed, 1 <= nK <= 16, every k >= 1).  The enumeration runs to the
+ * largest k.  Exactness: kBest2DCutoff's k only bounds its sweep loop, so the list for k is the first min(k, nFound)
+ * entries of the list for any larger k, and assignmentProb adds the weights in list order and normalises at the end;
+ * each table is the running sum after its k-th hypothesis with that same normalisation.  Slot j is therefore
+ * bit-identical to a separate pda_murty_batch(k = ks[j], PDA_CUT_RELATIVE, cutoff 42, PDA_WEIGHTS_GATED) call, nFound
+ * included, on every kernel path.
+ *   probs     slot j of problem p: numCol[p] x (nL[p]+1) row-major at probs + probOff[p] + j*numCol[p]*(nL[p]+1)
+ *   nFound    slot j of problem p at nFound[p*nK + j]: min(ks[j], hypotheses found); 0 = infeasible (NaN tables);
+ *             -1 = malformed or above maxNumRow / maxNumCol (device-pointer form only; the _host form rejects such
+ *             batches up front)
+ *   ks        a HOST array, in both forms
+ * Workspace, kernel choice (pda_murty_set_path) and launch shape are those of pda_murty_batch at k = max(ks):
+ * size the workspace with pda_murty_workspace_bytes(n, max(ks), ...).  The device-pointer form enqueues on `stream`
+ * and does not synchronise.  The _host form stages as pda_murty_batch_host does, page-locked buffers from
+ * pda_host_alloc used in place.  PDA_ERR_INVALID: nK outside 1..16, a k < 1, NULL ks, or what pda_murty_batch rejects. */
+int pda_assignment_prob_ladder_batch(const double* costs, const int64_t* costOff, const int32_t* numRow,
+                                     const int32_t* numCol, const int32_t* nL, int64_t nProblems, int32_t maxNumRow,
+                                     int32_t maxNumCol, const int32_t* ks, int32_t nK, double* probs,
+                                     const int64_t* probOff, int32_t* nFound, void* workspace, int64_t workspaceBytes,
+                                     void* stream);
+int pda_assignment_prob_ladder_batch_host(const double* costs, const int64_t* costOff, const int32_t* numRow,
+                                          const int32_t* numCol, const int32_t* nL, int64_t nProblems, const int32_t* ks,
+                                          int32_t nK, double* probs, const int64_t* probOff, int32_t* nFound,
+                                          int32_t device);
+
 /* Single LAP on a rectangular matrix without padding: assign2D (shortestPathCPP.hpp:144-149) when
  * makeSafe != 0, shortestPathCPP (hpp:178-182) on an already-safe matrix otherwise.
  * Per problem p: col4row[rowOff.. +numRow], row4col[colOff.. +numCol], u[colOff..], v[rowOff..],

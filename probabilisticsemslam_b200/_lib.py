@@ -29,6 +29,8 @@ SIGNATURES = {
                                        ptr, ptr, ptr, ptr, ptr, ptr, i32, ptr, ptr, ptr, i32]),
     "pda_murty_batch_host_multi": (C.c_int, [ptr, ptr, ptr, ptr, i64, i32, i32, dbl, i32, i32,
                                              ptr, ptr, ptr, ptr, ptr, ptr, i32, ptr, ptr, ptr, ptr, i32]),
+    "pda_assignment_prob_ladder_batch": (C.c_int, [ptr, ptr, ptr, ptr, ptr, i64, i32, i32, ptr, i32, ptr, ptr, ptr, ptr, i64, ptr]),
+    "pda_assignment_prob_ladder_batch_host": (C.c_int, [ptr, ptr, ptr, ptr, ptr, i64, ptr, i32, ptr, ptr, ptr, i32]),
     "pda_lap_batch": (C.c_int, [ptr, ptr, ptr, ptr, ptr, i64, i32, i32, i32, i32, ptr, ptr,
                                 ptr, ptr, ptr, ptr, ptr, ptr, ptr, ptr]),
     "pda_lap_batch_host": (C.c_int, [ptr, ptr, ptr, ptr, ptr, i64, i32, i32, ptr, ptr,

@@ -104,6 +104,25 @@ def assignment_prob_batch(pb: ProblemBatch, k: int, device: int = 0) -> KBestRes
                        want_lists=False, device=device)
 
 
+def assignment_prob_ladder_batch(pb: ProblemBatch, ks, device: int = 0):
+    """assignmentProb for every problem and every k in ks, from one enumeration to max(ks);
+    pda_assignment_prob_ladder_batch_host.  Returns (one (nK, nM, nL+1) array per problem, nFound[n, nK]); slot j is
+    bit-identical to assignment_prob_batch(pb, ks[j])."""
+    n = len(pb)
+    ks = np.ascontiguousarray(ks, dtype=np.int32)
+    nk = int(ks.size)
+    num_row, num_col, nL = pb.num_row, pb.nM.astype(np.int32), pb.nL.astype(np.int32)
+    cells = num_col.astype(np.int64) * (nL.astype(np.int64) + 1)
+    prob_off = _prefix(cells * nk)
+    probs = np.zeros(max(int(cells.sum()) * nk, 1))
+    nf = np.zeros((n, max(nk, 1)), np.int32)
+    check(lib().pda_assignment_prob_ladder_batch_host(_p(pb.costs), _p(pb.cost_off), _p(num_row), _p(num_col), _p(nL), n,
+                                                      _p(ks), nk, _p(probs), _p(prob_off), _p(nf), device))
+    tabs = [probs[prob_off[p]:prob_off[p] + nk * int(cells[p])].reshape(nk, int(num_col[p]), int(nL[p]) + 1)
+            for p in range(n)]
+    return tabs, nf
+
+
 def lap_batch(pb: ProblemBatch, *, make_safe: bool = True, maximize: bool = False,
               num_col4gain: np.ndarray | None = None, device: int = 0):
     n = len(pb)
@@ -398,6 +417,12 @@ def assignmentProb(C: np.ndarray, nL: int, k: int, device: int = 0) -> np.ndarra
     """assignment.cpp:547-683 -> probs[nM, nL+1]."""
     pb = _one(C, nL)
     return assignment_prob_batch(pb, k, device).prob_table(pb, 0).copy()
+
+
+def assignmentProbLadder(C: np.ndarray, nL: int, ks, device: int = 0) -> np.ndarray:
+    """assignmentProb(C, nL, k) for every k in ks from one enumeration -> probs[nK, nM, nL+1]."""
+    tabs, _ = assignment_prob_ladder_batch(_one(C, nL), ks, device)
+    return tabs[0].copy()
 
 
 def brute_force_k(C: np.ndarray) -> int:

@@ -254,9 +254,11 @@ __device__ __forceinline__ void smem_pop(int4* top, const int lenBefore) {
 }
 
 // ---- warp 0: staging, single-detection shortcut, root LAP (shortestPathCPP.cpp:119-238) ---------------
-template <int R>
+template <int R, bool LADDER, class... Ladder>  // the ladder as in solve_problem_cta
 __device__ void root_phase(const MurtyArgs& a, const long long p, const CtaSmem& S, const WarpSmem& sm, const Heap& heap,
-                           const CtaArena& A, const int lane) {
+                           const CtaArena& A, const int lane, const Ladder*... ladder) {
+    const MurtyLadder* L = nullptr;
+    if constexpr (LADDER) ((L = ladder), ...);
     CtaCtl* ctl = S.ctl;
     const int n = a.numRow[p], nc = a.numCol[p];
     const int D = a.geo.nodeDim;
@@ -269,8 +271,12 @@ __device__ void root_phase(const MurtyArgs& a, const long long p, const CtaSmem&
         double norm = 0.0;
         for (int i = 0; i <= nL; ++i) if (Cg[i] < a.weightGate) norm += sm.acc[i];
         norm = 1.0 / norm;
-        double* out = a.probs + a.probOff[p];
-        for (int i = lane; i <= nL; i += 32) out[i] = sm.acc[i] * norm;
+        if constexpr (LADDER) {  // the same table for every k
+            for (int i = lane; i <= nL; i += 32) ladder_put(a, *L, p, 0, PDA_LADDER_MAX, nL + 1, i, sm.acc[i] * norm);
+        } else {
+            double* out = a.probs + a.probOff[p];
+            for (int i = lane; i <= nL; i += 32) out[i] = sm.acc[i] * norm;
+        }
         __syncwarp();
     }
     const bool maximize = a.maximize != 0;
@@ -287,10 +293,16 @@ __device__ void root_phase(const MurtyArgs& a, const long long p, const CtaSmem&
         const bool stuck = augment_from<R>(c, nc, n, sm, nd, allRows, 0u, lane);
         publish_cols<R>(sm, nd, lane);  // the next column starts from this solution
         if (stuck) {
-            if (lane == 0) { a.nFound[p] = 0; ctl->feasible = 0; ctl->done[0] = ctl->done[1] = 1; ctl->nFound = 0; ctl->nEmit = 0; }
+            if constexpr (LADDER) {
+                ladder_found(a, *L, p, 0, lane);
+                if (lane == 0) { ctl->feasible = 0; ctl->done[0] = ctl->done[1] = 1; ctl->nFound = 0; ctl->nEmit = 0; }
+            } else {
+                if (lane == 0) { a.nFound[p] = 0; ctl->feasible = 0; ctl->done[0] = ctl->done[1] = 1; ctl->nFound = 0; ctl->nEmit = 0; }
+            }
             if (wantW && nc > 1) {
                 double* out = a.probs + a.probOff[p];
-                for (int i = lane; i < nc * (nL + 1); i += 32) out[i] = CUDART_NAN;
+                const int len = (LADDER ? L->nSlots : 1) * nc * (nL + 1);  // ladder: the slots lie back to back
+                for (int i = lane; i < len; i += 32) out[i] = CUDART_NAN;
             }
             return;
         }
@@ -522,16 +534,23 @@ __device__ void run_task(const MurtyArgs& a, const CtaSmem& S, const WarpSmem& s
     __syncwarp();
 }
 
-template <int R>
+// LADDER: the k-ladder form (MurtyLadder): weights only, k = the largest rung, a table stored at every rung.  The ladder
+// comes in through the pack, which is empty for the plain kernel: its calls keep the signature they have without the
+// ladder, and with it the compiler's inlining decisions.
+template <int R, bool LADDER, class... Ladder>
 __device__ void solve_problem_cta(const MurtyArgs& a, const CtaGeometry& cg, const long long p, const CtaSmem& S,
-                                  unsigned char* arenaBase) {
+                                  unsigned char* arenaBase, const Ladder*... ladder) {
+    const MurtyLadder* L = nullptr;
+    if constexpr (LADDER) ((L = ladder), ...);
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int n = a.numRow[p], nc = a.numCol[p];
     const bool wantW = a.weightMode != PDA_WEIGHTS_NONE;
     const int nL = wantW ? a.nL[p] : 0;
     if (nc < 1 || nc > n || n > 32 * R || nc > PDA_CTA_MAX_COL || n > a.geo.nodeDim || n * nc > a.geo.cCap || nc > a.geo.maxCol ||
         (wantW && nL + nc != n)) {
-        if (threadIdx.x == 0) a.nFound[p] = -1;  // malformed or beyond the launch's maxima: not solved (0 would mean infeasible)
+        // malformed or beyond the launch's maxima: not solved (0 would mean infeasible)
+        if constexpr (LADDER) ladder_found(a, *L, p, -1, threadIdx.x);
+        else if (threadIdx.x == 0) a.nFound[p] = -1;
         return;
     }
     const WarpSmem sm = warp_view(S, cg, R, warp);
@@ -545,7 +564,7 @@ __device__ void solve_problem_cta(const MurtyArgs& a, const CtaGeometry& cg, con
 #ifdef PDA_CTA_PROFILE
     if (threadIdx.x == 0) { ctl->tCommit = ctl->tSelect = ctl->tTasks = ctl->tPop = ctl->tPush = 0; ctl->rounds = ctl->tasksTotal = ctl->commits = 0; ctl->t0 = PROF_T(); asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ctl->ns0)); }
 #endif
-    if (warp == 0) root_phase<R>(a, p, S, sm, heap, A, lane);
+    if (warp == 0) root_phase<R, LADDER>(a, p, S, sm, heap, A, lane, ladder...);
     __syncthreads();
 #ifdef PDA_CTA_PROFILE
     if (threadIdx.x == 0) ctl->tRoot = PROF_T() - ctl->t0;
@@ -595,7 +614,8 @@ __device__ void solve_problem_cta(const MurtyArgs& a, const CtaGeometry& cg, con
         if (lane < nc) A.hypRows[(size_t)i * PDA_CTA_MAX_COL + lane] = nb[D + lane];
         if (a.gainBest && lane == 0) a.gainBest[p * (long long)a.k + i] = A.orderGain[i];
     }
-    if (threadIdx.x == 0) a.nFound[p] = nFound;
+    if constexpr (LADDER) ladder_found(a, *L, p, nFound, threadIdx.x);
+    else if (threadIdx.x == 0) a.nFound[p] = nFound;
 
     // ---- weights (assignment.cpp:616-648, 910-945): every table entry adds its terms in hypothesis order ---
     if (wantW && nc > 1) {
@@ -610,14 +630,19 @@ __device__ void solve_problem_cta(const MurtyArgs& a, const CtaGeometry& cg, con
         for (int t = threadIdx.x; t < cells; t += blockDim.x) {
             const int c = t / (nL + 1), to = t - c * (nL + 1);
             double acc = 0.0, total = 0.0;
+            int rungAt = 0;  // ladder: the next rung to store (nFound <= its k for the last rung)
             for (int i = 0; i < nFound; ++i) {
                 const double w = A.orderW[i];
                 int r = (int)(signed char)A.hypRows[(size_t)i * PDA_CTA_MAX_COL + c];
                 r = r >= nL ? nL : r;
                 total += w;
                 if (r == to) acc += w;
+                if constexpr (LADDER) {
+                    if (i + 1 == L->rung[rungAt]) { ladder_put(a, *L, p, rungAt, rungAt, cells, t, acc * (1.0 / total)); ++rungAt; }
+                }
             }
-            a.probs[a.probOff[p] + t] = acc * (1.0 / total);
+            if constexpr (LADDER) ladder_put(a, *L, p, rungAt, PDA_LADDER_MAX, cells, t, acc * (1.0 / total));  // rungs past the end
+            else a.probs[a.probOff[p] + t] = acc * (1.0 / total);
         }
     }
 #ifdef PDA_CTA_PROFILE
@@ -632,6 +657,7 @@ __device__ void solve_problem_cta(const MurtyArgs& a, const CtaGeometry& cg, con
 #endif
 }
 
+#ifndef PDA_MURTY_LADDER_TU  // murty_ladder_kernel.cu compiles this file for the ladder kernels alone
 template <int R>
 __global__ void __launch_bounds__(32 * CTA_WARPS, 1) murty_cta_kernel(const MurtyArgs a, const CtaGeometry cg) {
     extern __shared__ __align__(16) unsigned char smemRaw[];
@@ -639,7 +665,7 @@ __global__ void __launch_bounds__(32 * CTA_WARPS, 1) murty_cta_kernel(const Murt
     const CtaSmem S = carve_cta(smemRaw, a.geo, cg);
     unsigned char* arena = a.arena + (size_t)blockIdx.x * cg.arenaStride;
     if (a.cursor == nullptr) {  // one CTA per problem and enough arenas for all of them: no work queue
-        solve_problem_cta<R>(a, cg, (long long)blockIdx.x, S, arena);
+        solve_problem_cta<R, false>(a, cg, (long long)blockIdx.x, S, arena);
         return;
     }
     for (;;) {
@@ -648,7 +674,7 @@ __global__ void __launch_bounds__(32 * CTA_WARPS, 1) murty_cta_kernel(const Murt
         __syncthreads();
         const long long p = S.ctl->problem;
         if (p >= a.nProblems) break;
-        solve_problem_cta<R>(a, cg, p, S, arena);
+        solve_problem_cta<R, false>(a, cg, p, S, arena);
     }
 }
 
@@ -696,10 +722,11 @@ static int launch_murty_cta_r(const MurtyArgs& a, const CtaGeometry& cg, cudaStr
     return PDA_OK;
 }
 
-int launch_murty_cta(const MurtyArgs& args, const CtaGeometry& cg, cudaStream_t stream) {
+int launch_murty_cta(const MurtyArgs& args, const CtaGeometry& cg, cudaStream_t stream, const MurtyLadder* ladder) {
     MurtyArgs a = args;
     if (a.nProblems <= a.nWarps) a.cursor = nullptr;  // every problem has its own CTA: skip the queue and its memset
     else PDA_CUDA_TRY(cudaMemsetAsync(a.cursor, 0, sizeof(unsigned long long), stream));
+    if (ladder) return launch_murty_cta_ladder(a, cg, *ladder, stream);
     switch (a.geo.R) {
         case 1: return launch_murty_cta_r<1>(a, cg, stream);
         case 2: return launch_murty_cta_r<2>(a, cg, stream);
@@ -707,6 +734,47 @@ int launch_murty_cta(const MurtyArgs& args, const CtaGeometry& cg, cudaStream_t 
     }
     return fail(PDA_ERR_UNSUPPORTED, "murty: unsupported row-slot count %d", a.geo.R);
 }
+
+#else
+// The k-ladder form (written out apart from murty_cta_kernel for the reason given at murty_ladder_kernel)
+template <int R>
+__global__ void __launch_bounds__(32 * CTA_WARPS, 1)
+    murty_cta_ladder_kernel(const MurtyArgs a, const CtaGeometry cg, const __grid_constant__ MurtyLadder L) {
+    extern __shared__ __align__(16) unsigned char smemRaw[];
+    if ((int)blockIdx.x >= a.nWarps) return;  // nWarps = arenas available = CTAs allowed to run
+    const CtaSmem S = carve_cta(smemRaw, a.geo, cg);
+    unsigned char* arena = a.arena + (size_t)blockIdx.x * cg.arenaStride;
+    if (a.cursor == nullptr) {
+        solve_problem_cta<R, true>(a, cg, (long long)blockIdx.x, S, arena, &L);
+        return;
+    }
+    for (;;) {
+        __syncthreads();  // the previous problem's readers of ctl are done
+        if (threadIdx.x == 0) S.ctl->problem = (long long)atomicAdd(a.cursor, 1ULL);
+        __syncthreads();
+        const long long p = S.ctl->problem;
+        if (p >= a.nProblems) break;
+        solve_problem_cta<R, true>(a, cg, p, S, arena, &L);
+    }
+}
+
+}  // namespace
+
+int launch_murty_cta_ladder(const MurtyArgs& a, const CtaGeometry& cg, const MurtyLadder& ladder, cudaStream_t stream) {
+    void (*k)(const MurtyArgs, const CtaGeometry, const MurtyLadder) = nullptr;
+    switch (a.geo.R) {
+        case 1: k = murty_cta_ladder_kernel<1>; break;
+        case 2: k = murty_cta_ladder_kernel<2>; break;
+        case 4: k = murty_cta_ladder_kernel<4>; break;
+        default: return fail(PDA_ERR_UNSUPPORTED, "murty: unsupported row-slot count %d", a.geo.R);
+    }
+    PDA_CUDA_TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, cg.smemBytes));
+    const int ctas = (int)(a.nProblems < a.nWarps ? a.nProblems : a.nWarps);
+    k<<<ctas, 32 * CTA_WARPS, cg.smemBytes, stream>>>(a, cg, ladder);
+    PDA_CUDA_TRY(cudaGetLastError());
+    return PDA_OK;
+}
+#endif  // PDA_MURTY_LADDER_TU
 
 }  // namespace pda
 

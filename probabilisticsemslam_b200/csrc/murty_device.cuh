@@ -750,6 +750,37 @@ __device__ __forceinline__ void add_weight(const MurtyArgs& a, const WarpSmem& s
     }
 }
 
+// ---- k ladder (MurtyLadder, pda_internal.h) -----------------------------------------------------------
+// nFound of every slot of problem p from the count reached by the enumeration to the largest rung; thread t < nSlots
+// writes slot t.  min(k, count) keeps -1 (malformed) and 0 (infeasible) as they are.
+__device__ __forceinline__ void ladder_found(const MurtyArgs& a, const MurtyLadder& L, const long long p, const int count,
+                                             const int t) {
+    if (t < L.nSlots) {
+        const int k = L.rung[L.slotRung[t]];
+        a.nFound[p * L.nSlots + t] = count < k ? count : k;
+    }
+}
+// v into cell `cell` of every slot of problem p whose rung lies in [rLo, rHi]
+__device__ __forceinline__ void ladder_put(const MurtyArgs& a, const MurtyLadder& L, const long long p, const int rLo,
+                                           const int rHi, const int cells, const int cell, const double v) {
+    double* out = a.probs + a.probOff[p] + cell;
+    for (int j = 0; j < L.nSlots; ++j)
+        if (L.slotRung[j] >= rLo && L.slotRung[j] <= rHi) out[(long long)j * cells] = v;
+}
+// Warp kernel: hypothesis h has just been added to the accumulators.  If it is the last one of rung `rungAt`
+// (rungK == h + 1), that rung's tables are stored with the end-of-problem expression and the next rung comes up.
+__device__ __forceinline__ void ladder_step(const MurtyArgs& a, const MurtyLadder& L, const long long p, const WarpSmem& sm,
+                                            const int h, const int cells, const double total, int& rungAt, int& rungK,
+                                            const int lane) {
+    if (h + 1 != rungK) return;
+    __syncwarp();  // lanes own different columns of acc
+    const double norm = 1.0 / total;
+    for (int i = lane; i < cells; i += 32) ladder_put(a, L, p, rungAt, rungAt, cells, i, sm.acc[i] * norm);
+    __syncwarp();  // read before the next hypothesis is added
+    ++rungAt;
+    rungK = rungAt < L.nRungs ? L.rung[rungAt] : 0;
+}
+
 }  // namespace
 }  // namespace pda
 #endif

@@ -49,9 +49,10 @@ __device__ unsigned long long g_fastStats[8];  // children, abandoned, dropped a
 #define PDA_STAT(i, v) do { } while (0)
 #endif
 
-template <int R, bool FAST>
+// LADDER: the k-ladder form (MurtyLadder): weights only, k = the largest rung, tables stored at every rung.
+template <int R, bool FAST, bool LADDER = false>
 __device__ void solve_problem(const MurtyArgs& a, const long long p, const WarpSmem& sm, const Heap& heap,
-                              const FastPQ& pq, unsigned char* nodes, const int lane) {
+                              const FastPQ& pq, unsigned char* nodes, const int lane, const MurtyLadder* L = nullptr) {
     const int n = a.numRow[p], nc = a.numCol[p];
     const int D = a.geo.nodeDim;
     const bool wantW = a.weightMode != PDA_WEIGHTS_NONE;
@@ -59,7 +60,8 @@ __device__ void solve_problem(const MurtyArgs& a, const long long p, const WarpS
     // malformed, or larger than the maxima this launch was sized for (shared-memory matrix, node slots, arena): not
     // solved; reported as -1, which no reference call can return (0 = infeasible)
     if (nc < 1 || nc > n || n > 32 * R || n > a.geo.nodeDim || n * nc > a.geo.cCap || nc > a.geo.maxCol || (wantW && nL + nc != n)) {
-        if (lane == 0) a.nFound[p] = -1;
+        if constexpr (LADDER) ladder_found(a, *L, p, -1, lane);
+        else if (lane == 0) a.nFound[p] = -1;
         return;
     }
     const double* Cg = a.costs + a.costOff[p];
@@ -71,8 +73,12 @@ __device__ void solve_problem(const MurtyArgs& a, const long long p, const WarpS
         double norm = 0.0;
         for (int i = 0; i <= nL; ++i) if (Cg[i] < a.weightGate) norm += sm.acc[i];
         norm = 1.0 / norm;
-        double* out = a.probs + a.probOff[p];
-        for (int i = lane; i <= nL; i += 32) out[i] = sm.acc[i] * norm;
+        if constexpr (LADDER) {  // the same table for every k
+            for (int i = lane; i <= nL; i += 32) ladder_put(a, *L, p, 0, PDA_LADDER_MAX, nL + 1, i, sm.acc[i] * norm);
+        } else {
+            double* out = a.probs + a.probOff[p];
+            for (int i = lane; i <= nL; i += 32) out[i] = sm.acc[i] * norm;
+        }
         __syncwarp();
     }
 
@@ -98,10 +104,12 @@ __device__ void solve_problem(const MurtyArgs& a, const long long p, const WarpS
         const bool stuck = augment_from<R, false, PDA_ROOT_FF != 0>(c, nc, n, sm, nd, allRows, 0u, lane);
         publish_cols<R>(sm, nd, lane);  // the next column starts from this solution
         if (stuck) {
-            if (lane == 0) a.nFound[p] = 0;
+            if constexpr (LADDER) ladder_found(a, *L, p, 0, lane);
+            else if (lane == 0) a.nFound[p] = 0;
             if (wantW && nc > 1) {  // the reference ends up scaling zeros by 1/0 here
                 double* out = a.probs + a.probOff[p];
-                for (int i = lane; i < nc * (nL + 1); i += 32) out[i] = CUDART_NAN;
+                const int len = (LADDER ? L->nSlots : 1) * nc * (nL + 1);  // ladder: the slots lie back to back
+                for (int i = lane; i < len; i += 32) out[i] = CUDART_NAN;
             }
             return;
         }
@@ -129,6 +137,11 @@ __device__ void solve_problem(const MurtyArgs& a, const long long p, const WarpS
     emit<R>(ep, 0, n, nc, nd, gain0Out, lane);
     double total = 0.0;
     if (wantW && nc > 1) add_weight<R>(a, sm, nd, nc, nL, gain0Out, gain0Out, total, lane);
+    int rungAt = 0, rungK = 0;  // ladder: the next rung to store and its k
+    if constexpr (LADDER) {
+        rungK = L->rung[0];
+        if (nc > 1) ladder_step(a, *L, p, sm, 0, nc * (nL + 1), total, rungAt, rungK, lane);
+    }
 
     int heapLen = FAST ? 0 : 1;   // exact: the root is the heap's only entry (its state is live in registers, slot 0 of
                                   // the arena stays unused); fast: slots in use, the root never enters the list
@@ -244,17 +257,25 @@ __device__ void solve_problem(const MurtyArgs& a, const long long p, const WarpS
         emit<R>(ep, sweep, n, nc, nd, gainOut, lane);
         if (stop) break;
         if (wantW && nc > 1) add_weight<R>(a, sm, nd, nc, nL, gain0Out, gainOut, total, lane);
+        if constexpr (LADDER) {
+            if (nc > 1) ladder_step(a, *L, p, sm, sweep, nc * (nL + 1), total, rungAt, rungK, lane);
+        }
     }
     if (FAST && bail) {  // not decidable without the reference's heap order (or the list is full): the exact kernel redoes it
         if (lane == 0) a.fallbackList[atomicAdd(a.fallbackCount, 1u)] = (int32_t)p;
         return;
     }
-    if (lane == 0) a.nFound[p] = sweep;
+    if constexpr (LADDER) ladder_found(a, *L, p, sweep, lane);
+    else if (lane == 0) a.nFound[p] = sweep;
     if (wantW && nc > 1) {
         __syncwarp();
         const double norm = 1.0 / total;
-        double* out = a.probs + a.probOff[p];
-        for (int i = lane; i < nc * (nL + 1); i += 32) out[i] = sm.acc[i] * norm;
+        if constexpr (LADDER) {  // the loop ended (cutoff, empty queue, k): every rung not stored yet gets the final table
+            for (int i = lane; i < nc * (nL + 1); i += 32) ladder_put(a, *L, p, rungAt, PDA_LADDER_MAX, nc * (nL + 1), i, sm.acc[i] * norm);
+        } else {
+            double* out = a.probs + a.probOff[p];
+            for (int i = lane; i < nc * (nL + 1); i += 32) out[i] = sm.acc[i] * norm;
+        }
         __syncwarp();
     }
 }
@@ -275,6 +296,7 @@ __device__ __forceinline__ WarpSmem carve(unsigned char* base, const MurtyGeomet
     return sm;
 }
 
+#ifndef PDA_MURTY_LADDER_TU  // murty_ladder_kernel.cu compiles this file for the ladder kernels alone
 template <int R, bool FAST>
 __global__ void __launch_bounds__(32 * PDA_MURTY_WPC, FAST ? PDA_FAST_MINB : PDA_MURTY_MINB) murty_kernel(const MurtyArgs a) {
     extern __shared__ __align__(16) unsigned char smemRaw[];
@@ -472,10 +494,11 @@ int murty_geometry(int32_t k, int32_t maxNumRow, int32_t maxNumCol, bool weights
 }
 
 template <int R, bool FAST>
-static int launch_murty_r(const MurtyArgs& a, cudaStream_t stream) {
+static int launch_murty_r(const MurtyArgs& a, cudaStream_t stream, const MurtyLadder* ladder) {
     const int wpc = FAST ? a.geo.fastWarpsPerCta : a.geo.warpsPerCta;
     const int threads = 32 * wpc;
     const int smem = wpc * (FAST ? a.geo.fastSmemPerWarp : a.geo.smemPerWarp);
+    if (ladder) return launch_murty_ladder(a, FAST, *ladder, wpc, smem, stream);
     PDA_CUDA_TRY(cudaFuncSetAttribute(murty_kernel<R, FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     const int ctas = (a.nWarps + wpc - 1) / wpc;
     murty_kernel<R, FAST><<<ctas, threads, smem, stream>>>(a);
@@ -484,11 +507,11 @@ static int launch_murty_r(const MurtyArgs& a, cudaStream_t stream) {
 }
 
 template <bool FAST>
-static int launch_murty_any(const MurtyArgs& a, cudaStream_t stream) {
+static int launch_murty_any(const MurtyArgs& a, cudaStream_t stream, const MurtyLadder* ladder) {
     switch (a.geo.R) {
-        case 1: return launch_murty_r<1, FAST>(a, stream);
-        case 2: return launch_murty_r<2, FAST>(a, stream);
-        case 4: return launch_murty_r<4, FAST>(a, stream);
+        case 1: return launch_murty_r<1, FAST>(a, stream, ladder);
+        case 2: return launch_murty_r<2, FAST>(a, stream, ladder);
+        case 4: return launch_murty_r<4, FAST>(a, stream, ladder);
     }
     return fail(PDA_ERR_UNSUPPORTED, "murty: unsupported row-slot count %d", a.geo.R);
 }
@@ -501,23 +524,24 @@ extern "C" void pda_debug_fast_stats(unsigned long long* out, int reset) {
 }
 #endif
 
-int launch_murty(const MurtyArgs& a, cudaStream_t stream) {
+int launch_murty(const MurtyArgs& a, cudaStream_t stream, const MurtyLadder* ladder) {
     // header of the workspace: cursor (8 B) | fallback count (4 B, +4 pad) | cursor of the fallback pass (8 B)
     PDA_CUDA_TRY(cudaMemsetAsync(a.cursor, 0, 32, stream));
     if (a.order) {
         order_by_cost_kernel<<<1, 1024, 0, stream>>>(a.numCol, a.nProblems, a.order);
         PDA_CUDA_TRY(cudaGetLastError());
     }
-    if (!a.useFast) return launch_murty_any<false>(a, stream);
-    int rc = launch_murty_any<true>(a, stream);
+    if (!a.useFast) return launch_murty_any<false>(a, stream, ladder);
+    int rc = launch_murty_any<true>(a, stream, ladder);
     if (rc) return rc;
-    // the exact kernel over whatever the fast one could not decide (usually nothing: it then finds a count of zero)
+    // the exact kernel over whatever the fast one could not decide (usually nothing: it then finds a count of zero); a
+    // ladder problem it redoes gets every rung rewritten, with the same bits where the fast kernel had stored one
     MurtyArgs b = a;
     b.useFast = 0;
     b.cursor = a.cursor2;
     b.order = a.fallbackList;
     b.nProblemsDev = a.fallbackCount;
-    return launch_murty_any<false>(b, stream);
+    return launch_murty_any<false>(b, stream, ladder);
 }
 
 template <int R>
@@ -546,5 +570,70 @@ int launch_lap(const LapArgs& a, cudaStream_t stream) {
     if (R == 2) return launch_lap_r<2>(a, stream, dev);
     return launch_lap_r<4>(a, stream, dev);
 }
+
+#else
+// The k-ladder form: same geometry, same launch shape, the same loop over problems as murty_kernel.  (The loop is
+// written out twice rather than shared through an inlined helper: with the helper, the code of murty_kernel<4, *> moves.)
+template <int R, bool FAST>
+__global__ void __launch_bounds__(32 * PDA_MURTY_WPC, FAST ? PDA_FAST_MINB : PDA_MURTY_MINB)
+    murty_ladder_kernel(const MurtyArgs a, const __grid_constant__ MurtyLadder L) {
+    extern __shared__ __align__(16) unsigned char smemRaw[];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int gw = blockIdx.x * (blockDim.x >> 5) + warp;
+    if (gw >= a.nWarps) return;
+    const int smemPerWarp = FAST ? a.geo.fastSmemPerWarp : a.geo.smemPerWarp;
+    unsigned char* mySmem = smemRaw + (size_t)warp * smemPerWarp;
+    const WarpSmem sm = carve<R>(mySmem, a.geo);
+    unsigned char* arena = a.arena + (size_t)gw * a.geo.arenaStride;
+    Heap heap;
+    heap.deep = reinterpret_cast<HeapEntry*>(arena);
+    heap.top = reinterpret_cast<HeapEntry*>(mySmem + a.geo.heapTopOff);
+    heap.topCap = a.geo.heapTopCap;
+    FastPQ pq;
+    pq.cap = a.geo.pqCap;
+    pq.gmin = reinterpret_cast<unsigned long long*>(mySmem + a.geo.heapTopOff);
+    if (a.geo.pqInSmem) {
+        pq.key = pq.gmin + (a.geo.pqCap >> 5);
+        pq.node = reinterpret_cast<int*>(pq.key + a.geo.pqCap);
+    } else {  // the arena's heap region is free in this kernel
+        pq.key = reinterpret_cast<unsigned long long*>(arena);
+        pq.node = reinterpret_cast<int*>(pq.key + a.geo.pqCap);
+    }
+    pq.hist = reinterpret_cast<unsigned*>(sm.spc);
+    unsigned char* nodes = arena + a.geo.heapBytes;
+    // the exact kernel, when it runs behind the fast one, takes its problem count from the fallback counter
+    const long long nProblems = a.nProblemsDev ? (long long)*a.nProblemsDev : a.nProblems;
+    for (;;) {
+        unsigned long long p = 0;
+        if (lane == 0) p = atomicAdd(a.cursor, 1ULL);
+        p = __shfl_sync(FULL, p, 0);
+        if ((long long)p >= nProblems) break;
+        if (a.order) p = (unsigned long long)a.order[p];  // most expensive problems first: a short tail
+        solve_problem<R, FAST, true>(a, (long long)p, sm, heap, pq, nodes, lane, &L);
+        __syncwarp();
+    }
+}
+
+}  // namespace
+
+int launch_murty_ladder(const MurtyArgs& a, const bool fast, const MurtyLadder& ladder, const int wpc, const int smem,
+                        cudaStream_t stream) {
+    const int ctas = (a.nWarps + wpc - 1) / wpc;
+    void (*k)(const MurtyArgs, const MurtyLadder) = nullptr;
+    switch (a.geo.R * 2 + (fast ? 1 : 0)) {
+        case 2: k = murty_ladder_kernel<1, false>; break;
+        case 3: k = murty_ladder_kernel<1, true>; break;
+        case 4: k = murty_ladder_kernel<2, false>; break;
+        case 5: k = murty_ladder_kernel<2, true>; break;
+        case 8: k = murty_ladder_kernel<4, false>; break;
+        case 9: k = murty_ladder_kernel<4, true>; break;
+        default: return fail(PDA_ERR_UNSUPPORTED, "murty: unsupported row-slot count %d", a.geo.R);
+    }
+    PDA_CUDA_TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    k<<<ctas, 32 * wpc, smem, stream>>>(a, ladder);
+    PDA_CUDA_TRY(cudaGetLastError());
+    return PDA_OK;
+}
+#endif  // PDA_MURTY_LADDER_TU
 
 }  // namespace pda

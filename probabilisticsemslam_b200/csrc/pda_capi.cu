@@ -194,14 +194,18 @@ int pda_murty_set_path(int32_t path) {
     return g_murtyPath.exchange(path);
 }
 
-int pda_murty_batch(const double* costs, const int64_t* costOff, const int32_t* numRow, const int32_t* numCol,
-                    int64_t nProblems, int32_t maxNumRow, int32_t maxNumCol,
-                    int32_t k, int32_t cutMode, double cutoff, int32_t maximize, int32_t cutMaximize,
-                    int64_t* row4colBest, const int64_t* r4cOff,
-                    int64_t* col4rowBest, const int64_t* c4rOff,
-                    double* gainBest, int32_t* nFound,
-                    int32_t weightMode, double* probs, const int64_t* probOff, const int32_t* nL,
-                    void* workspace, int64_t workspaceBytes, void* stream) {
+}  // extern "C"
+
+// pda_murty_batch, and with `ladder` the k-ladder form behind pda_assignment_prob_ladder_batch (k = its largest rung;
+// nFound and the weight tables then have ladder->nSlots entries per problem).  Path choice and geometry are the same.
+static int murty_batch_dev(const double* costs, const int64_t* costOff, const int32_t* numRow, const int32_t* numCol,
+                           int64_t nProblems, int32_t maxNumRow, int32_t maxNumCol,
+                           int32_t k, int32_t cutMode, double cutoff, int32_t maximize, int32_t cutMaximize,
+                           int64_t* row4colBest, const int64_t* r4cOff,
+                           int64_t* col4rowBest, const int64_t* c4rOff,
+                           double* gainBest, int32_t* nFound,
+                           int32_t weightMode, double* probs, const int64_t* probOff, const int32_t* nL,
+                           void* workspace, int64_t workspaceBytes, void* stream, const MurtyLadder* ladder) {
     if (nProblems < 0) return fail(PDA_ERR_INVALID, "murty: nProblems < 0");
     if (nProblems == 0) return PDA_OK;
     if (!costs || !costOff || !numRow || !numCol || !nFound) return fail(PDA_ERR_INVALID, "murty: NULL input");
@@ -232,7 +236,7 @@ int pda_murty_batch(const double* costs, const int64_t* costOff, const int32_t* 
         const int64_t ctas = rc ? 0 : std::min<int64_t>(std::min<int64_t>(nProblems, dev.smCount), (workspaceBytes - 256) / cg.arenaStride);
         if (rc == PDA_OK && ctas >= 1) {
             a.nWarps = (int32_t)ctas;  // arenas == CTAs allowed to run
-            return launch_murty_cta(a, cg, reinterpret_cast<cudaStream_t>(stream));
+            return launch_murty_cta(a, cg, reinterpret_cast<cudaStream_t>(stream), ladder);
         }
         if (forced) return rc ? rc : fail(PDA_ERR_WORKSPACE, "murty (CTA path): workspace of %lld B holds no arena (%lld B each)",
                                           (long long)workspaceBytes, (long long)cg.arenaStride);
@@ -255,17 +259,20 @@ int pda_murty_batch(const double* costs, const int64_t* costOff, const int32_t* 
         a.useFast = 1;
         a.fallbackList = reinterpret_cast<int32_t*>(reinterpret_cast<unsigned char*>(workspace) + used);
     }  // else (k <= 2, a list too long for shared-memory group minima, a tight workspace): the exact kernel alone
-    return launch_murty(a, reinterpret_cast<cudaStream_t>(stream));
+    return launch_murty(a, reinterpret_cast<cudaStream_t>(stream), ladder);
 }
 
-int pda_murty_batch_host(const double* costs, const int64_t* costOff, const int32_t* numRow, const int32_t* numCol,
-                         int64_t nProblems, int32_t k, int32_t cutMode, double cutoff, int32_t maximize,
-                         int32_t cutMaximize,
-                         int64_t* row4colBest, const int64_t* r4cOff,
-                         int64_t* col4rowBest, const int64_t* c4rOff,
-                         double* gainBest, int32_t* nFound,
-                         int32_t weightMode, double* probs, const int64_t* probOff, const int32_t* nL,
-                         int32_t device) {
+// pda_murty_batch_host, and with `ladder` the staging of pda_assignment_prob_ladder_batch_host (S = ladder->nSlots
+// tables and counts per problem).
+static int murty_batch_host(const double* costs, const int64_t* costOff, const int32_t* numRow, const int32_t* numCol,
+                            int64_t nProblems, int32_t k, int32_t cutMode, double cutoff, int32_t maximize,
+                            int32_t cutMaximize,
+                            int64_t* row4colBest, const int64_t* r4cOff,
+                            int64_t* col4rowBest, const int64_t* c4rOff,
+                            double* gainBest, int32_t* nFound,
+                            int32_t weightMode, double* probs, const int64_t* probOff, const int32_t* nL,
+                            int32_t device, const MurtyLadder* ladder) {
+    const size_t S = ladder ? (size_t)ladder->nSlots : 1;
     if (nProblems < 0) return fail(PDA_ERR_INVALID, "murty: nProblems < 0");
     if (nProblems == 0) return PDA_OK;
     if (!costs || !costOff || !numRow || !numCol || !nFound) return fail(PDA_ERR_INVALID, "murty: NULL input");
@@ -288,14 +295,14 @@ int pda_murty_batch_host(const double* costs, const int64_t* costOff, const int3
             if (costOff[p] < costOff[p - 1] + (int64_t)pr * pc) contiguous = false;
             if (row4colBest && r4cOff[p] < r4cOff[p - 1] + (int64_t)k * pc) contiguous = false;
             if (col4rowBest && c4rOff[p] < c4rOff[p - 1] + (int64_t)k * pr) contiguous = false;
-            if (weightMode && probOff[p] < probOff[p - 1] + (int64_t)pc * (nL[p - 1] + 1)) contiguous = false;
+            if (weightMode && probOff[p] < probOff[p - 1] + (int64_t)S * pc * (nL[p - 1] + 1)) contiguous = false;
         }
         rCost.add((size_t)costOff[p], (size_t)r * c);
         if (row4colBest) rR4c.add((size_t)r4cOff[p], (size_t)k * c);
         if (col4rowBest) rC4r.add((size_t)c4rOff[p], (size_t)k * r);
         if (weightMode) {
             if (nL[p] + c != r) return fail(PDA_ERR_INVALID, "murty: problem %lld has nL + numCol != numRow", (long long)p);
-            rProb.add((size_t)probOff[p], (size_t)c * (nL[p] + 1));
+            rProb.add((size_t)probOff[p], S * c * (nL[p] + 1));
         }
     }
     const size_t nCost = rCost.len(), nR4c = rR4c.len(), nC4r = rC4r.len(), nProb = rProb.len();
@@ -305,14 +312,14 @@ int pda_murty_batch_host(const double* costs, const int64_t* costOff, const int3
     int64_t wsBytes = pda_murty_workspace_bytes(nProblems, k, maxR, maxC);
     if (wsBytes < 0) return (int)wsBytes;
     const size_t n = (size_t)nProblems;
-    const size_t ioBytes = 8 * (nCost + nR4c + nC4r + nProb + (gainBest ? n * (size_t)k : 0) + 4 * n) + 16 * n;
+    const size_t ioBytes = 8 * (nCost + nR4c + nC4r + nProb + (gainBest ? n * (size_t)k : 0) + 4 * n) + 16 * n + 4 * n * (S - 1);
     if (ioBytes <= PDA_PACKED_LIMIT) {  // small call: one pinned copy each way
         Stage st(device);
         PackedIO io(st);
         const size_t oCost = io.in(costs + loCost, nCost * 8), oCostOff = io.in(costOff, n * 8), oNR = io.in(numRow, n * 4), oNC = io.in(numCol, n * 4);
         const size_t oR4cOff = io.in(row4colBest ? r4cOff : nullptr, n * 8), oC4rOff = io.in(col4rowBest ? c4rOff : nullptr, n * 8);
         const size_t oProbOff = io.in(weightMode ? probOff : nullptr, n * 8), oNL = io.in(weightMode ? nL : nullptr, n * 4);
-        const size_t oFound = io.out(nFound, n * 4), oGain = io.out(gainBest, gainBest ? n * (size_t)k * 8 : 0);
+        const size_t oFound = io.out(nFound, n * 4 * S), oGain = io.out(gainBest, gainBest ? n * (size_t)k * 8 : 0);
         const size_t oProb = io.out(weightMode ? probs + loProb : nullptr, nProb * 8);
         const size_t oR4c = io.out(row4colBest ? row4colBest + loR4c : nullptr, nR4c * 8), oC4r = io.out(col4rowBest ? col4rowBest + loC4r : nullptr, nC4r * 8);
         const size_t oWs = st.reserve((size_t)wsBytes);
@@ -320,13 +327,13 @@ int pda_murty_batch_host(const double* costs, const int64_t* costOff, const int3
         HostStreams* hs = nullptr;
         PDA_TRY(host_streams(device, &hs));
         PDA_TRY(io.upload(hs->run));
-        PDA_TRY(pda_murty_batch(st.at<double>(oCost) - loCost, st.at<int64_t>(oCostOff), st.at<int32_t>(oNR), st.at<int32_t>(oNC), nProblems,
+        PDA_TRY(murty_batch_dev(st.at<double>(oCost) - loCost, st.at<int64_t>(oCostOff), st.at<int32_t>(oNR), st.at<int32_t>(oNC), nProblems,
                                 maxR, maxC, k, cutMode, cutoff, maximize, cutMaximize,
                                 row4colBest ? st.at<int64_t>(oR4c) - loR4c : nullptr, st.at<int64_t>(oR4cOff),
                                 col4rowBest ? st.at<int64_t>(oC4r) - loC4r : nullptr, st.at<int64_t>(oC4rOff),
                                 gainBest ? st.at<double>(oGain) : nullptr, st.at<int32_t>(oFound),
                                 weightMode, weightMode ? st.at<double>(oProb) - loProb : nullptr, st.at<int64_t>(oProbOff),
-                                st.at<int32_t>(oNL), st.at<unsigned char>(oWs), wsBytes, hs->run));
+                                st.at<int32_t>(oNL), st.at<unsigned char>(oWs), wsBytes, hs->run, ladder));
         return io.download(hs->run);
     }
     // Page-locked caller buffers are used in place: a warp reads its 2.4 KB cost matrix over PCIe once when it takes
@@ -337,7 +344,7 @@ int pda_murty_batch_host(const double* costs, const int64_t* costOff, const int3
     Stage st(device);
     const size_t oCost = st.reserve(costsDev ? 0 : nCost * 8), oCostOff = st.reserve(n * 8), oNR = st.reserve(n * 4), oNC = st.reserve(n * 4);
     const size_t oR4c = st.reserve(nR4c * 8), oR4cOff = st.reserve(n * 8), oC4r = st.reserve(nC4r * 8), oC4rOff = st.reserve(n * 8);
-    const size_t oGain = st.reserve(gainBest ? n * k * 8 : 0), oFound = st.reserve(n * 4);
+    const size_t oGain = st.reserve(gainBest ? n * k * 8 : 0), oFound = st.reserve(n * 4 * S);
     const size_t oProb = st.reserve(probsDev ? 0 : nProb * 8), oProbOff = st.reserve(n * 8), oNL = st.reserve(n * 4);
     const size_t oWs = st.reserve((size_t)wsBytes);
     PDA_TRY(st.commit());
@@ -382,12 +389,12 @@ int pda_murty_batch_host(const double* costs, const int64_t* costOff, const int3
             PDA_CUDA_TRY(cudaEventRecord(evIn[c], sIn));
             // run
             PDA_CUDA_TRY(cudaStreamWaitEvent(sRun, evIn[c], 0));
-            PDA_TRY(pda_murty_batch(dCost, st.at<int64_t>(oCostOff) + p0, st.at<int32_t>(oNR) + p0,
+            PDA_TRY(murty_batch_dev(dCost, st.at<int64_t>(oCostOff) + p0, st.at<int32_t>(oNR) + p0,
                                     st.at<int32_t>(oNC) + p0, (int64_t)m, maxR, maxC, k, cutMode, cutoff, maximize, cutMaximize,
                                     dR4c, st.at<int64_t>(oR4cOff) + p0, dC4r, st.at<int64_t>(oC4rOff) + p0,
-                                    gainBest ? st.at<double>(oGain) + p0 * (size_t)k : nullptr, st.at<int32_t>(oFound) + p0,
+                                    gainBest ? st.at<double>(oGain) + p0 * (size_t)k : nullptr, st.at<int32_t>(oFound) + p0 * S,
                                     weightMode, dProb, st.at<int64_t>(oProbOff) + p0, st.at<int32_t>(oNL) + p0,
-                                    st.at<unsigned char>(oWs), wsBytes, sRun));
+                                    st.at<unsigned char>(oWs), wsBytes, sRun, ladder));
             PDA_CUDA_TRY(cudaEventRecord(evRun[c], sRun));
             // copy out: this chunk's results
             PDA_CUDA_TRY(cudaStreamWaitEvent(sOut, evRun[c], 0));
@@ -400,7 +407,7 @@ int pda_murty_batch_host(const double* costs, const int64_t* costOff, const int3
                 PDA_TRY(d2h(col4rowBest + a0, dC4r + a0, a1 - a0, sOut));
             }
             if (gainBest) PDA_TRY(d2h(gainBest + p0 * (size_t)k, st.at<double>(oGain) + p0 * (size_t)k, m * (size_t)k, sOut));
-            PDA_TRY(d2h(nFound + p0, st.at<int32_t>(oFound) + p0, m, sOut));
+            PDA_TRY(d2h(nFound + p0 * S, st.at<int32_t>(oFound) + p0 * S, m * S, sOut));
             if (weightMode && !probsDev) {
                 const size_t a0 = nChunks == 1 ? rProb.lo : (size_t)probOff[p0], a1 = (nChunks == 1 || last) ? rProb.hi : (size_t)probOff[p1];
                 PDA_TRY(d2h(probs + a0, dProb + a0, a1 - a0, sOut));
@@ -415,6 +422,72 @@ int pda_murty_batch_host(const double* costs, const int64_t* costOff, const int3
     if (rc != PDA_OK) { cudaStreamSynchronize(sIn); cudaStreamSynchronize(sRun); cudaStreamSynchronize(sOut); (void)cudaGetLastError(); }
     for (size_t c = 0; c < nChunks; ++c) { cudaEventDestroy(evIn[c]); cudaEventDestroy(evRun[c]); }
     return rc;
+}
+
+// ks (host) -> the ladder: rungs = the sorted distinct ks, slot j -> the rung equal to ks[j]
+static int make_ladder(const int32_t* ks, int32_t nK, MurtyLadder* L) {
+    if (!ks) return fail(PDA_ERR_INVALID, "ladder: NULL ks");
+    if (nK < 1 || nK > PDA_LADDER_MAX) return fail(PDA_ERR_INVALID, "ladder: need 1 <= nK <= %d (got %d)", PDA_LADDER_MAX, nK);
+    for (int j = 0; j < nK; ++j)
+        if (ks[j] < 1) return fail(PDA_ERR_INVALID, "ladder: ks[%d] = %d (need k >= 1)", j, ks[j]);
+    std::vector<int32_t> r(ks, ks + nK);
+    std::sort(r.begin(), r.end());
+    r.erase(std::unique(r.begin(), r.end()), r.end());
+    memset(L, 0, sizeof(*L));
+    L->nRungs = (int32_t)r.size();
+    L->nSlots = nK;
+    for (size_t i = 0; i < r.size(); ++i) L->rung[i] = r[i];
+    for (int j = 0; j < nK; ++j) L->slotRung[j] = (int32_t)(std::lower_bound(r.begin(), r.end(), ks[j]) - r.begin());
+    return PDA_OK;
+}
+
+extern "C" {
+
+int pda_murty_batch(const double* costs, const int64_t* costOff, const int32_t* numRow, const int32_t* numCol,
+                    int64_t nProblems, int32_t maxNumRow, int32_t maxNumCol,
+                    int32_t k, int32_t cutMode, double cutoff, int32_t maximize, int32_t cutMaximize,
+                    int64_t* row4colBest, const int64_t* r4cOff,
+                    int64_t* col4rowBest, const int64_t* c4rOff,
+                    double* gainBest, int32_t* nFound,
+                    int32_t weightMode, double* probs, const int64_t* probOff, const int32_t* nL,
+                    void* workspace, int64_t workspaceBytes, void* stream) {
+    return murty_batch_dev(costs, costOff, numRow, numCol, nProblems, maxNumRow, maxNumCol, k, cutMode, cutoff, maximize,
+                           cutMaximize, row4colBest, r4cOff, col4rowBest, c4rOff, gainBest, nFound, weightMode, probs, probOff,
+                           nL, workspace, workspaceBytes, stream, nullptr);
+}
+
+int pda_murty_batch_host(const double* costs, const int64_t* costOff, const int32_t* numRow, const int32_t* numCol,
+                         int64_t nProblems, int32_t k, int32_t cutMode, double cutoff, int32_t maximize,
+                         int32_t cutMaximize,
+                         int64_t* row4colBest, const int64_t* r4cOff,
+                         int64_t* col4rowBest, const int64_t* c4rOff,
+                         double* gainBest, int32_t* nFound,
+                         int32_t weightMode, double* probs, const int64_t* probOff, const int32_t* nL,
+                         int32_t device) {
+    return murty_batch_host(costs, costOff, numRow, numCol, nProblems, k, cutMode, cutoff, maximize, cutMaximize, row4colBest,
+                            r4cOff, col4rowBest, c4rOff, gainBest, nFound, weightMode, probs, probOff, nL, device, nullptr);
+}
+
+// assignmentProb's settings (assignment.cpp:547-683, as in the assignmentProb shim): kBest2DCutoff with cutoff 42, gated
+// weights, no lists
+int pda_assignment_prob_ladder_batch(const double* costs, const int64_t* costOff, const int32_t* numRow, const int32_t* numCol,
+                                     const int32_t* nL, int64_t nProblems, int32_t maxNumRow, int32_t maxNumCol,
+                                     const int32_t* ks, int32_t nK, double* probs, const int64_t* probOff, int32_t* nFound,
+                                     void* workspace, int64_t workspaceBytes, void* stream) {
+    MurtyLadder L;
+    PDA_TRY(make_ladder(ks, nK, &L));
+    return murty_batch_dev(costs, costOff, numRow, numCol, nProblems, maxNumRow, maxNumCol, L.rung[L.nRungs - 1], PDA_CUT_RELATIVE,
+                           42.0, 0, 0, nullptr, nullptr, nullptr, nullptr, nullptr, nFound, PDA_WEIGHTS_GATED, probs, probOff, nL,
+                           workspace, workspaceBytes, stream, &L);
+}
+
+int pda_assignment_prob_ladder_batch_host(const double* costs, const int64_t* costOff, const int32_t* numRow,
+                                          const int32_t* numCol, const int32_t* nL, int64_t nProblems, const int32_t* ks,
+                                          int32_t nK, double* probs, const int64_t* probOff, int32_t* nFound, int32_t device) {
+    MurtyLadder L;
+    PDA_TRY(make_ladder(ks, nK, &L));
+    return murty_batch_host(costs, costOff, numRow, numCol, nProblems, L.rung[L.nRungs - 1], PDA_CUT_RELATIVE, 42.0, 0, 0,
+                            nullptr, nullptr, nullptr, nullptr, nullptr, nFound, PDA_WEIGHTS_GATED, probs, probOff, nL, device, &L);
 }
 
 // One host thread per device, each running the single-device call on a contiguous slice of the batch (SURVEY.md 8e:

@@ -75,7 +75,21 @@ struct MurtyArgs {
     unsigned long long* cursor2;       // work cursor of the fallback pass
     int32_t useFast;
 };
-int launch_murty(const MurtyArgs& a, cudaStream_t stream);
+// The k ladder of pda_assignment_prob_ladder_batch: ONE enumeration to k = rung[nRungs - 1] gives the weight tables of
+// every rung.  The list for k is the first min(k, nFound) entries of the list for any larger k (k only bounds the sweep
+// loop), and the tables add their terms in list order, so the table of rung r is the running sum after hypothesis
+// rung[r] - 1 with the end-of-problem normalisation.  Slot j of problem p -- the numCol x (nL+1) table at
+// probs + probOff[p] + j*numCol*(nL+1) and nFound[p*nSlots + j] -- takes rung slotRung[j].  The ladder kernels are
+// separate instantiations; the plain ones do not see this struct.
+#define PDA_LADDER_MAX 16
+struct MurtyLadder {
+    int32_t nRungs, nSlots;
+    int32_t rung[PDA_LADDER_MAX];      // ascending, distinct, >= 1
+    int32_t slotRung[PDA_LADDER_MAX];  // rung of each requested slot
+};
+int launch_murty(const MurtyArgs& a, cudaStream_t stream, const MurtyLadder* ladder = nullptr);
+// the ladder launches, compiled apart in murty_ladder_kernel.cu (wpc, smem: the launch shape launch_murty chose)
+int launch_murty_ladder(const MurtyArgs& a, bool fast, const MurtyLadder& ladder, int wpc, int smem, cudaStream_t stream);
 
 // ---- Murty k-best, one CTA per problem (murty_cta_kernel.cu): the latency path for small batches ----
 #define PDA_CTA_MAX_COL 16  // detections per problem the CTA path takes (children per split record)
@@ -90,7 +104,8 @@ struct CtaGeometry {
 };
 int murty_cta_geometry(int32_t k, int32_t maxNumRow, int32_t maxNumCol, bool weights, const DeviceInfo& dev,
                        MurtyGeometry* g, CtaGeometry* cg);
-int launch_murty_cta(const MurtyArgs& a, const CtaGeometry& cg, cudaStream_t stream);
+int launch_murty_cta(const MurtyArgs& a, const CtaGeometry& cg, cudaStream_t stream, const MurtyLadder* ladder = nullptr);
+int launch_murty_cta_ladder(const MurtyArgs& a, const CtaGeometry& cg, const MurtyLadder& ladder, cudaStream_t stream);
 
 struct LapArgs {
     const double* costs; const int64_t* costOff; const int32_t* numRow; const int32_t* numCol;

@@ -280,6 +280,45 @@ std::vector<std::vector<std::vector<double> > > assignmentProbBatch(const std::v
     return assignmentProbBatch(costs, nL, nM, k, std::vector<int>());
 }
 
+std::vector<std::vector<std::vector<std::vector<double> > > > assignmentProbLadderBatch(
+    const std::vector<std::vector<double> >& costs, const std::vector<size_t>& nL, const std::vector<size_t>& nM,
+    const std::vector<size_t>& ks) {
+    if (nL.size() != costs.size() || nM.size() != costs.size()) throw std::invalid_argument("assignmentProbLadder: nL / nM sizes differ from costs");
+    if (ks.empty() || ks.size() > 16) throw std::invalid_argument("assignmentProbLadder: need 1 to 16 values of k");
+    std::vector<int32_t> k32(ks.size());
+    for (size_t j = 0; j < ks.size(); j++) {
+        if (ks[j] < 1 || ks[j] > size_t(INT32_MAX)) throw std::invalid_argument("assignmentProbLadder: k out of range");
+        k32[j] = int32_t(ks[j]);
+    }
+    const size_t n = costs.size(), nK = ks.size();
+    FlatBatch fb(costs, nL, nM);
+    std::vector<int64_t> probOff(n);
+    size_t nProb = 0;
+    for (size_t p = 0; p < n; p++) { probOff[p] = int64_t(nProb); nProb += nK * nM[p] * (nL[p] + 1); }
+    std::vector<double> probs(nProb ? nProb : 1);
+    std::vector<int32_t> found(n * nK + 1);
+    if (n)
+        pdaCheck(pda_assignment_prob_ladder_batch_host(fb.flat.data(), fb.costOff.data(), fb.nr.data(), fb.nc.data(), fb.nl.data(),
+                                                       int64_t(n), k32.data(), int32_t(nK), probs.data(), probOff.data(),
+                                                       found.data(), pdaShimDevice()),
+                 "assignmentProbLadder");
+    std::vector<std::vector<std::vector<std::vector<double> > > > out(n);
+    for (size_t p = 0; p < n; p++) {
+        const size_t cells = nM[p] * (nL[p] + 1);
+        for (size_t j = 0; j < nK; j++) {
+            const std::vector<double> slice(probs.begin() + probOff[p] + j * cells, probs.begin() + probOff[p] + (j + 1) * cells);
+            out[p].push_back(unflatten(slice, nM[p], nL[p] + 1));
+        }
+    }
+    return out;
+}
+
+std::vector<std::vector<std::vector<double> > > assignmentProbLadder(const std::vector<double>& costMatrix, size_t nL, size_t nM,
+                                                                     const std::vector<size_t>& ks) {
+    return assignmentProbLadderBatch(std::vector<std::vector<double> >(1, costMatrix), std::vector<size_t>(1, nL),
+                                     std::vector<size_t>(1, nM), ks)[0];
+}
+
 std::vector<std::vector<std::vector<double> > > permanentProbBatch(const std::vector<std::vector<double> >& costs,
                                                                    const std::vector<size_t>& nL,
                                                                    const std::vector<size_t>& nM, int permOpt,
