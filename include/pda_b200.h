@@ -357,6 +357,41 @@ int pda_permanent_prob_batch_host(const double* costs, const int64_t* costOff, c
                                   const int32_t* nM, int64_t nProblems, int32_t permOpt,
                                   double* probs, const int64_t* probOff, int32_t* status, int32_t device);
 
+/* Device-pointer forms of pda_conditioned_permanent_batch_host and pda_permanent_prob_batch_host: every array is a device
+ * pointer, the host reads none of it, and the call is enqueued on `stream` without a synchronisation or a copy between
+ * host and device, so it can follow a device producer and be captured in a CUDA graph.  Tables, results and statuses
+ * are bit-identical to the _host forms on any batch the _host form runs as one chunk (up to 65 536 sub-permanents;
+ * every conditioned_permanent batch), for every permOpt:
+ *   - a sub-matrix whose short side is <= 10 runs the subset programme in shared memory, straight out of the input;
+ *   - a short side of 11..31 is walked by the NW kernel with the launch shape the _host form takes for the batch (its
+ *     sub-permanent count and largest dimension, counted over all problems), and an item that comes out negative is
+ *     walked again untransposed with the shape of a one-matrix launch (assignment.cpp:409-419), all on the device;
+ *   - permOpt == 0 runs Huber's approximation (300 trials) with the seed of pda_set_approx_seed.  Its draws are keyed by
+ *     item index: for permanent_prob, the sub-permanents of the call counted from its first problem, nM * (nL+1) per
+ *     problem with nM > 1, (m, l) in m-major order; for conditioned_permanent, the matrix index.
+ * Status per problem / matrix: 0 computed; 1 where the reference throws (a sub-matrix keeps more than 32 rows, or
+ * permOpt outside 0..2 for a problem with nM > 1 / any matrix); 2 above the call's maxNumRow / maxNumCol (maxDim), or
+ * with nL < 0, nM < 1 or a negative dimension: not computed, its table (out[i]) is left untouched.  The nM * (nL+1)
+ * tables must not overlap: the sub-permanents of the call must fit in totalProbElems, a problem beyond that is status 2.
+ *
+ * Workspace (pda_*_workspace_bytes, for the current device): a copy of the costs, per problem 12 B, and per item
+ * (totalProbElems, or nMats) 20 B.  Calls that may materialise items -- permOpt == 0, or sub-matrices with a short side
+ * of 11 or more (maxNumCol >= 12 and maxNumRow >= 12; maxDim >= 11) -- add per item the scaled sub-matrix, 8 B times
+ * min(32, maxNumRow - 1) * min(32, maxNumCol - 1) (min(32, maxDim)^2), and 32 B of descriptors; calls that may walk
+ * (permOpt 1 or 2 with such sub-matrices) add 16 B per CTA a matrix may take (twice the SM count) plus 4 B per item.
+ * A smaller workspace is PDA_ERR_WORKSPACE; nothing beyond workspaceBytes is written. */
+int64_t pda_permanent_prob_workspace_bytes(int64_t nProblems, int64_t totalCostElems, int64_t totalProbElems,
+                                           int32_t maxNumRow, int32_t maxNumCol, int32_t permOpt);
+int pda_permanent_prob_batch(const double* costs, const int64_t* costOff, const int32_t* nL, const int32_t* nM,
+                             int64_t nProblems, int64_t totalCostElems, int64_t totalProbElems,
+                             int32_t maxNumRow, int32_t maxNumCol, int32_t permOpt,
+                             double* probs, const int64_t* probOff, int32_t* status,
+                             void* workspace, int64_t workspaceBytes, void* stream);
+int64_t pda_conditioned_permanent_workspace_bytes(int64_t nMats, int32_t maxDim, int32_t permOpt);
+int pda_conditioned_permanent_batch(const double* mats, const int64_t* matOff, const int32_t* rows, const int32_t* cols,
+                                    int64_t nMats, int32_t maxDim, int32_t permOpt, double* out, int32_t* status,
+                                    void* workspace, int64_t workspaceBytes, void* stream);
+
 /* The same over several devices: contiguous slices of problems, one per device (the (nL+1) * nM sub-permanents of a
  * problem stay together; assignment.cpp:213-246). */
 int pda_permanent_prob_batch_host_multi(const double* costs, const int64_t* costOff, const int32_t* nL,

@@ -67,6 +67,10 @@ SIGNATURES = {
     "pda_conditioned_permanent_batch_host": (C.c_int, [ptr, ptr, ptr, ptr, i64, i32, ptr, ptr, i32]),
     "pda_permanent_prob_batch_host": (C.c_int, [ptr, ptr, ptr, ptr, i64, i32, ptr, ptr, ptr, i32]),
     "pda_permanent_prob_batch_host_multi": (C.c_int, [ptr, ptr, ptr, ptr, i64, i32, ptr, ptr, ptr, ptr, i32]),
+    "pda_permanent_prob_workspace_bytes": (i64, [i64, i64, i64, i32, i32, i32]),
+    "pda_permanent_prob_batch": (C.c_int, [ptr, ptr, ptr, ptr, i64, i64, i64, i32, i32, i32, ptr, ptr, ptr, ptr, i64, ptr]),
+    "pda_conditioned_permanent_workspace_bytes": (i64, [i64, i32, i32]),
+    "pda_conditioned_permanent_batch": (C.c_int, [ptr, ptr, ptr, ptr, i64, i32, i32, ptr, ptr, ptr, i64, ptr]),
 }
 
 

@@ -218,6 +218,58 @@ def permanent_prob_batch(pb: ProblemBatch, perm_opt: int = 1, device: int = 0):
     return tabs, st
 
 
+def _device_call_args(tensors, what):
+    import torch
+    for name, t in tensors.items():
+        if not (isinstance(t, torch.Tensor) and t.is_cuda and t.is_contiguous()):
+            raise ValueError(f"{what}: {name} must be a contiguous CUDA tensor")
+    return torch.cuda.current_stream().cuda_stream
+
+
+def permanent_prob_batch_device(costs, cost_off, nL, nM, prob_off, total_prob_elems: int, max_num_row: int, max_num_col: int,
+                                perm_opt: int = 1, probs=None, status=None, workspace=None):
+    """pda_permanent_prob_batch on CUDA tensors, enqueued on the current stream (no synchronisation): costs float64,
+    cost_off / prob_off int64, nL / nM int32.  The nM x (nL+1) tables go to probs (float64, total_prob_elems; allocated
+    when None) at prob_off; status (int32) as in include/pda_b200.h.  Returns (probs, status)."""
+    import torch
+    dev = costs.device
+    probs = torch.zeros(max(int(total_prob_elems), 1), dtype=torch.float64, device=dev) if probs is None else probs
+    status = torch.empty(nL.shape[0], dtype=torch.int32, device=dev) if status is None else status
+    n = int(nL.shape[0])
+    if workspace is None:
+        ws = int(lib().pda_permanent_prob_workspace_bytes(n, int(costs.numel()), int(total_prob_elems), max_num_row, max_num_col, perm_opt))
+        check(min(ws, 0))
+        workspace = torch.empty(ws, dtype=torch.uint8, device=dev)
+    stream = _device_call_args(dict(costs=costs, cost_off=cost_off, nL=nL, nM=nM, prob_off=prob_off, probs=probs,
+                                    status=status, workspace=workspace), "permanent_prob_batch_device")
+    check(lib().pda_permanent_prob_batch(costs.data_ptr(), cost_off.data_ptr(), nL.data_ptr(), nM.data_ptr(), n,
+                                         int(costs.numel()), int(total_prob_elems), max_num_row, max_num_col, perm_opt,
+                                         probs.data_ptr(), prob_off.data_ptr(), status.data_ptr(), workspace.data_ptr(),
+                                         int(workspace.numel()), stream))
+    return probs, status
+
+
+def conditioned_permanent_batch_device(mats, mat_off, rows, cols, max_dim: int, perm_opt: int = 1, out=None, status=None,
+                                       workspace=None):
+    """pda_conditioned_permanent_batch on CUDA tensors (mats float64 column-major at mat_off int64, rows / cols int32),
+    enqueued on the current stream.  Returns (out float64, status int32)."""
+    import torch
+    dev = mats.device
+    n = int(rows.shape[0])
+    out = torch.zeros(n, dtype=torch.float64, device=dev) if out is None else out
+    status = torch.empty(n, dtype=torch.int32, device=dev) if status is None else status
+    if workspace is None:
+        ws = int(lib().pda_conditioned_permanent_workspace_bytes(n, max_dim, perm_opt))
+        check(min(ws, 0))
+        workspace = torch.empty(ws, dtype=torch.uint8, device=dev)
+    stream = _device_call_args(dict(mats=mats, mat_off=mat_off, rows=rows, cols=cols, out=out, status=status,
+                                    workspace=workspace), "conditioned_permanent_batch_device")
+    check(lib().pda_conditioned_permanent_batch(mats.data_ptr(), mat_off.data_ptr(), rows.data_ptr(), cols.data_ptr(), n,
+                                                max_dim, perm_opt, out.data_ptr(), status.data_ptr(), workspace.data_ptr(),
+                                                int(workspace.numel()), stream))
+    return out, status
+
+
 def association_probs_batch(pb: ProblemBatch, k: int, device: int = 0) -> list[np.ndarray]:
     """getAssignmentProbs from the cost matrices on (assignment.cpp:57-74, usePerm = 0), fused on the device:
     conditionCosts -> assignmentProb -> scatter back through rowIdx.  Returns one (nM, nL+1) table per problem."""

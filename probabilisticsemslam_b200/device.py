@@ -144,6 +144,69 @@ class PermanentPlan:
         return float(self.n) * 3.0 * self.dim * 2.0 ** (self.dim - 1)
 
 
+class PermanentProbPlan:
+    """permanentProb of a ProblemBatch, resident on the current CUDA device: run() enqueues pda_permanent_prob_batch on
+    the current stream, result() copies the tables back."""
+
+    def __init__(self, pb: ProblemBatch, perm_opt: int = 1, *, max_num_row: int | None = None, max_num_col: int | None = None):
+        assert torch.cuda.is_available(), "PermanentProbPlan needs a CUDA device (there is no CPU fallback)"
+        dev = torch.device("cuda", torch.cuda.current_device())
+        self.n, self.perm_opt = len(pb), int(perm_opt)
+        self.nL_h, self.nM_h = pb.nL.astype(np.int32), pb.nM.astype(np.int32)
+        sizes = self.nM_h.astype(np.int64) * (self.nL_h.astype(np.int64) + 1)
+        self.prob_off_h = api._prefix(sizes)
+        self.total_prob = int(sizes.sum())
+        self.max_row = int((self.nL_h + self.nM_h).max()) if max_num_row is None else int(max_num_row)
+        self.max_col = int(self.nM_h.max()) if max_num_col is None else int(max_num_col)
+        up = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(dev)
+        self.costs = up(pb.costs if pb.costs.size else np.zeros(1))
+        self.cost_off, self.nL, self.nM, self.prob_off = up(pb.cost_off.astype(np.int64)), up(self.nL_h), up(self.nM_h), up(self.prob_off_h)
+        self.probs = torch.zeros(max(self.total_prob, 1), dtype=torch.float64, device=dev)
+        self.status = torch.empty(self.n, dtype=torch.int32, device=dev)
+        ws = int(lib().pda_permanent_prob_workspace_bytes(self.n, int(self.costs.numel()), self.total_prob, self.max_row,
+                                                          self.max_col, self.perm_opt))
+        check(min(ws, 0))
+        self.workspace = torch.empty(ws, dtype=torch.uint8, device=dev)
+
+    def run(self):
+        api.permanent_prob_batch_device(self.costs, self.cost_off, self.nL, self.nM, self.prob_off, self.total_prob,
+                                        self.max_row, self.max_col, self.perm_opt, self.probs, self.status, self.workspace)
+
+    def result(self):
+        """(list of (nM, nL+1) tables, status), as api.permanent_prob_batch returns them."""
+        probs, st = self.probs.cpu().numpy(), self.status.cpu().numpy()
+        o, L, M = self.prob_off_h, self.nL_h, self.nM_h
+        return [probs[o[p]:o[p] + int(M[p]) * (int(L[p]) + 1)].reshape(int(M[p]), int(L[p]) + 1) for p in range(self.n)], st
+
+
+class ConditionedPermanentPlan:
+    """conditionedPermanent of a list of matrices, resident on the current CUDA device (pda_conditioned_permanent_batch)."""
+
+    def __init__(self, mats: list[np.ndarray], perm_opt: int = 1, *, max_dim: int | None = None):
+        assert torch.cuda.is_available(), "ConditionedPermanentPlan needs a CUDA device (there is no CPU fallback)"
+        dev = torch.device("cuda", torch.cuda.current_device())
+        self.n, self.perm_opt = len(mats), int(perm_opt)
+        rows = np.asarray([m.shape[0] for m in mats], np.int32)
+        cols = np.asarray([m.shape[1] for m in mats], np.int32)
+        flat = np.concatenate([np.asarray(m, np.float64).reshape(-1, order="F") for m in mats] + [np.zeros(1)])
+        self.max_dim = int(max(rows.max(), cols.max())) if max_dim is None else int(max_dim)
+        up = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(dev)
+        self.mats, self.mat_off = up(flat), up(api._prefix(rows.astype(np.int64) * cols))
+        self.rows, self.cols = up(rows), up(cols)
+        self.out = torch.zeros(self.n, dtype=torch.float64, device=dev)
+        self.status = torch.empty(self.n, dtype=torch.int32, device=dev)
+        ws = int(lib().pda_conditioned_permanent_workspace_bytes(self.n, self.max_dim, self.perm_opt))
+        check(min(ws, 0))
+        self.workspace = torch.empty(ws, dtype=torch.uint8, device=dev)
+
+    def run(self):
+        api.conditioned_permanent_batch_device(self.mats, self.mat_off, self.rows, self.cols, self.max_dim, self.perm_opt,
+                                               self.out, self.status, self.workspace)
+
+    def result(self):
+        return self.out.cpu().numpy(), self.status.cpu().numpy()
+
+
 class PermanentRangePlan:
     """One large permanent: this rank's share of the Gray-code range, as a double-double partial."""
 
