@@ -133,7 +133,7 @@ int launch_to_probs(double* values, const int64_t* off, const int64_t* len, int6
 // ---- permanents (permanent_kernel.cu) ------------------------------------------------------------
 int launch_permanent_batch(const double* mats, const int64_t* matOff, const int32_t* rows, const int32_t* cols,
                            int64_t nMats, int32_t maxDim, double* out, int32_t* status, void* workspace,
-                           int64_t workspaceBytes, cudaStream_t stream, int32_t maxSmall = -1, int32_t minSmall = 0);
+                           int64_t workspaceBytes, cudaStream_t stream, int32_t maxSmall, int32_t minSmall);
 int launch_permanent_range(const double* A, int32_t n, uint64_t begin, uint64_t end, double* partial,
                            void* workspace, int64_t workspaceBytes, cudaStream_t stream);
 

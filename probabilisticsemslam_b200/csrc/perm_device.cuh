@@ -1,6 +1,6 @@
-// perm_device.cuh -- device pieces of permanentProb shared by the materialising item path (permprob_kernel.cu,
-// permanent_kernel.cu) and the fused conditioned-permanent pipeline (association_perm_kernel.cu).  Both paths run the
-// SAME code here, so their results agree bit for bit.
+// perm_device.cuh -- device pieces of permanentProb shared by permanentProb / conditionedPermanent
+// (permprob_device_kernel.cu), the permanent kernel's subset DP (permanent_kernel.cu) and the fused conditioned-permanent
+// pipeline (association_perm_kernel.cu).  All of them run the SAME code here, so their results agree bit for bit.
 #ifndef PDA_PERM_DEVICE_CUH
 #define PDA_PERM_DEVICE_CUH
 

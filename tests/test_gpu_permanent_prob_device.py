@@ -1,12 +1,16 @@
-"""Device-pointer forms of permanentProb and conditionedPermanent (pda_permanent_prob_batch,
-pda_conditioned_permanent_batch).
+"""permanentProb and conditionedPermanent: the device-pointer forms (pda_permanent_prob_batch,
+pda_conditioned_permanent_batch) and the host forms, which stage their inputs and run the device form per chunk.
 
-Tables, results and statuses must equal the host forms' bit for bit: sub-matrices with a short side of at most 10 through
-the fused subset programme, larger ones through the NW walk with the host form's launch shape, negative results through
-the retry on the device, and permOpt 0 with the same draws.  The device form must also run on device inputs only: one call
-captured in a CUDA graph and replayed on new inputs gives the bits of direct calls.  The CPU tests at the bottom check the
-argument handling, which runs before any device work."""
+Tables, results and statuses of both forms must equal the bits pinned in tests/golden/permprob_host_bits.npz
+(tests/golden/make_golden_permprob.py): the host forms' results from when they ran a separate materialising pipeline
+(commit aa4e759).  That covers sub-matrices with a short side of at most 10 through the fused subset programme, larger
+ones through the NW walk with its launch shape, negative results through the retry on the device, and permOpt 0 with the
+same draws.  The device form must also run on device inputs only: one call captured in a CUDA graph and replayed on new
+inputs gives the bits of direct calls.  The CPU tests at the bottom check the argument handling, which runs before any
+device work."""
 import ctypes
+import functools
+import hashlib
 import os
 import subprocess
 
@@ -55,6 +59,46 @@ def run_device_mats(mats, perm_opt, max_dim=None):
     return plan.result()
 
 
+@functools.cache
+def _pinned():
+    return golden("permprob_host_bits")
+
+
+def pinned(key, walked):
+    """(status, bits) of one pinned host call.  Sub-permanents the NW walk takes follow the launch shape, which follows
+    the SM count: such cases run only on a device with the SM count the bits were pinned on."""
+    z = _pinned()
+    if walked:
+        import torch
+        sm, want = torch.cuda.get_device_properties(0).multi_processor_count, int(z["sm_count"])
+        if sm != want:
+            pytest.skip(f"NW-walked bits pinned on {z['device']} with {want} SMs; this device has {sm}")
+    return z[key + ".status"], z[key + ".bits"]
+
+
+def digests(tabs):
+    """SHA-256 of each table's bits, as the pinned file stores them."""
+    return np.array([np.frombuffer(hashlib.sha256(bits(t).tobytes()).digest(), np.uint8) for t in tabs]).reshape(-1, 32)
+
+
+def assert_pinned_tables(got, key, what, skip=(), walked=False):
+    want_st, want_dg = pinned(key, walked)
+    tabs, st = got
+    assert len(tabs) == len(want_st), what
+    dg = digests(tabs)
+    for p in range(len(want_st)):
+        if p in skip:
+            continue
+        assert st[p] == want_st[p], f"{what}: status of problem {p}: {st[p]} != pinned {want_st[p]}"
+        assert np.array_equal(dg[p], want_dg[p]), f"{what}: problem {p} (status {st[p]}) differs from the pinned bits"
+
+
+def assert_pinned_mats(got, key, what, walked=False):
+    want_st, want_bits = pinned(key, walked)
+    np.testing.assert_array_equal(got[1], want_st, err_msg=f"{what}: status")
+    np.testing.assert_array_equal(bits(got[0]), want_bits, err_msg=f"{what}: values")
+
+
 def assert_tables(got, want, what, skip=()):
     (gt, gs), (wt, ws) = got, want
     for p in range(len(wt)):
@@ -72,6 +116,11 @@ def assert_mats(got, want, what):
 def golden_problems():
     z1, za = golden("probs_config1"), golden("probs_appendixA")
     return synth.pack([z1["C"], za["C"]], [int(z1["nL"]), int(za["nL"])])
+
+
+def golden_mats():
+    z = golden("conditioned_permanent")
+    return [z[f"A{i}"] for i in range(int(z["n"]))]
 
 
 def g1_mixed():
@@ -94,6 +143,11 @@ def nw_problems():
     return mats, nls
 
 
+def nw_mats():
+    """Square matrices of the NW sizes, as conditioned matrices."""
+    return [np.abs(np.sin(np.arange(k * k, dtype=np.float64).reshape(k, k) + k)) for k in (11, 12, 15, 16, 20)]
+
+
 def ragged(api):
     """nM = 1, nL = 0, the NW sizes, a sub-matrix with more than 32 kept rows (status 1) and, last, two problems above
     maxNumRow = 44 / maxNumCol = 16 (status 2)."""
@@ -109,22 +163,46 @@ def ragged(api):
     return synth.pack(mats, nls)
 
 
-# ---- bit identity with the host forms ----------------------------------------------------------------------------
+def invalid_opt_mats():
+    return [np.eye(3) + 0.5, np.ones((2, 4))]
+
+
+def approx_problems():
+    return synth.pack([synth.g1_dense(20, nM=m, first=300 * m).matrix(p) for m in (2, 4, 6) for p in range(20)], [30] * 60)
+
+
+def approx_mats():
+    return [np.abs(np.cos(np.arange(r * c, dtype=np.float64).reshape(r, c))) + 0.05 for r, c in ((4, 4), (6, 5), (8, 8), (12, 12))]
+
+
+def edge_mats():
+    """Shapes at the edges of conditionedPermanent, with a matrix the NW walk takes among them: 0x0, 1xn, nx1, 1x40 and
+    36x3 (more than 32 kept rows or columns: status 1) and 130x4 (a side above PDA_MAX_DIM: status 1)."""
+    rng = np.random.default_rng(SEED)
+    return [rng.uniform(0.1, 1.0, s) for s in ((4, 4), (0, 0), (1, 5), (5, 1), (1, 40), (36, 3), (130, 4), (12, 14))]
+
+
+def chunked_problems():
+    return synth.g1_dense(600, first=50)
+
+
+# ---- bit identity with the pinned host results -------------------------------------------------------------------
 @gpu
 @pytest.mark.parametrize("perm_opt", [1, 2])
 def test_golden_inputs(papi, perm_opt):
-    pb = golden_problems()
-    assert_tables(run_device(pb, perm_opt), papi.permanent_prob_batch(pb, perm_opt), "probs golden")
-    z = golden("conditioned_permanent")
-    mats = [z[f"A{i}"] for i in range(int(z["n"]))]
-    assert_mats(run_device_mats(mats, perm_opt), papi.conditioned_permanent_batch(mats, perm_opt), "conditioned golden")
+    pb, mats = golden_problems(), golden_mats()
+    assert_pinned_tables(run_device(pb, perm_opt), f"golden.{perm_opt}", "probs golden, device")
+    assert_pinned_tables(papi.permanent_prob_batch(pb, perm_opt), f"golden.{perm_opt}", "probs golden, host")
+    assert_pinned_mats(run_device_mats(mats, perm_opt), f"golden_mats.{perm_opt}", "conditioned golden, device")
+    assert_pinned_mats(papi.conditioned_permanent_batch(mats, perm_opt), f"golden_mats.{perm_opt}", "conditioned golden, host")
 
 
 @gpu
 @pytest.mark.parametrize("perm_opt", [1, 2])
 def test_g1_and_conditioned_g2(papi, perm_opt):
     for what, pb in (("g1", g1_mixed()), ("g2", g2_conditioned(papi))):
-        assert_tables(run_device(pb, perm_opt), papi.permanent_prob_batch(pb, perm_opt), what)
+        assert_pinned_tables(run_device(pb, perm_opt), f"{what}.{perm_opt}", f"{what}, device")
+        assert_pinned_tables(papi.permanent_prob_batch(pb, perm_opt), f"{what}.{perm_opt}", f"{what}, host")
 
 
 @gpu
@@ -134,24 +212,36 @@ def test_ragged_batch_with_nw_items_and_statuses(papi, perm_opt):
     n = len(pb)
     got = run_device(pb, perm_opt, max_row=44, max_col=16, fill=-7.0)
     want = papi.permanent_prob_batch(pb, perm_opt)
-    assert_tables(got, want, "ragged", skip=(n - 2, n - 1))
+    assert_pinned_tables(got, f"ragged.{perm_opt}", "ragged, device", skip=(n - 2, n - 1), walked=True)
+    assert_pinned_tables(want, f"ragged.{perm_opt}", "ragged, host", walked=True)
     assert want[1][n - 3] == 1 and got[1][n - 3] == 1
     assert list(got[1][n - 2:]) == [2, 2]
     for p in (n - 2, n - 1):
         assert np.all(got[0][p] == -7.0), "a status-2 table must be left untouched"
     # the same problems one by one as conditioned matrices, NW sizes included
-    mats = [np.abs(np.sin(np.arange(k * k, dtype=np.float64).reshape(k, k) + k)) for k in (11, 12, 15, 16, 20)]
-    assert_mats(run_device_mats(mats, perm_opt), papi.conditioned_permanent_batch(mats, perm_opt), "conditioned NW")
+    mats = nw_mats()
+    assert_pinned_mats(run_device_mats(mats, perm_opt), f"nw_mats.{perm_opt}", "conditioned NW, device", walked=True)
+    assert_pinned_mats(papi.conditioned_permanent_batch(mats, perm_opt), f"nw_mats.{perm_opt}", "conditioned NW, host",
+                       walked=True)
 
 
 @gpu
 def test_invalid_perm_opt_matches_host(papi):
     pb = ragged(papi)
     n = len(pb)
-    got, want = run_device(pb, 5, max_row=44, max_col=16), papi.permanent_prob_batch(pb, 5)
-    assert_tables(got, want, "permOpt 5", skip=(n - 2, n - 1))
-    mats = [np.eye(3) + 0.5, np.ones((2, 4))]
-    assert_mats(run_device_mats(mats, -1), papi.conditioned_permanent_batch(mats, -1), "conditioned permOpt -1")
+    assert_pinned_tables(run_device(pb, 5, max_row=44, max_col=16), "ragged.5", "permOpt 5, device", skip=(n - 2, n - 1))
+    assert_pinned_tables(papi.permanent_prob_batch(pb, 5), "ragged.5", "permOpt 5, host")
+    mats = invalid_opt_mats()
+    assert_pinned_mats(run_device_mats(mats, -1), "invalid_opt_mats.-1", "conditioned permOpt -1, device")
+    assert_pinned_mats(papi.conditioned_permanent_batch(mats, -1), "invalid_opt_mats.-1", "conditioned permOpt -1, host")
+
+
+@gpu
+@pytest.mark.parametrize("perm_opt", [0, 1, 2])
+def test_host_edge_shapes(papi, perm_opt):
+    got = papi.conditioned_permanent_batch(edge_mats(), perm_opt)
+    assert_pinned_mats(got, f"edges.{perm_opt}", f"edge shapes, permOpt {perm_opt}", walked=perm_opt != 0)
+    assert list(got[1][4:7]) == [1, 1, 1]
 
 
 # ---- the negative-permanent retry -------------------------------------------------------------------------------
@@ -186,8 +276,10 @@ def test_retry_of_negative_permanents(papi):
     negative = [i for i in range(len(mats)) if first[i] < 0]
     assert negative, "no seeded input reaches the retry"
     for perm_opt in (1, 2):
-        got, want = run_device_mats(mats, perm_opt), papi.conditioned_permanent_batch(mats, perm_opt)
-        assert_mats(got, want, f"retry permOpt {perm_opt}")
+        got = run_device_mats(mats, perm_opt)
+        assert_pinned_mats(got, f"retry.{perm_opt}", f"retry permOpt {perm_opt}, device", walked=True)
+        assert_pinned_mats(papi.conditioned_permanent_batch(mats, perm_opt), f"retry.{perm_opt}",
+                           f"retry permOpt {perm_opt}, host", walked=True)
         # the retried values are the untransposed walk's, not the negative first attempt's
         assert all(bits(np.array([got[0][i]]))[0] != bits(np.array([first[i]]))[0] for i in negative)
 
@@ -196,11 +288,13 @@ def test_retry_of_negative_permanents(papi):
 @gpu
 def test_approximation_same_draws_as_host(papi):
     from truth import perm_injective
-    pb = synth.pack([synth.g1_dense(20, nM=m, first=300 * m).matrix(p) for m in (2, 4, 6) for p in range(20)], [30] * 60)
-    assert_tables(run_device(pb, 0), papi.permanent_prob_batch(pb, 0), "permOpt 0")
-    mats = [np.abs(np.cos(np.arange(r * c, dtype=np.float64).reshape(r, c))) + 0.05 for r, c in ((4, 4), (6, 5), (8, 8), (12, 12))]
+    pb = approx_problems()
+    assert_pinned_tables(run_device(pb, 0), "approx.0", "permOpt 0, device")
+    assert_pinned_tables(papi.permanent_prob_batch(pb, 0), "approx.0", "permOpt 0, host")
+    mats = approx_mats()
     got = run_device_mats(mats, 0)
-    assert_mats(got, papi.conditioned_permanent_batch(mats, 0), "conditioned permOpt 0")
+    assert_pinned_mats(got, "approx_mats.0", "conditioned permOpt 0, device")
+    assert_pinned_mats(papi.conditioned_permanent_batch(mats, 0), "approx_mats.0", "conditioned permOpt 0, host")
     for A, est in zip(mats, got[0]):  # 300 trials: the estimator's spread, far inside a factor of two
         exact = perm_injective(A)
         assert abs(est / exact - 1.0) < 0.5, (A.shape, est, exact)
@@ -267,9 +361,11 @@ def host_chunks(pb):
 
 @gpu
 def test_beyond_one_host_chunk(papi):
-    pb = synth.g1_dense(600, first=50)
+    pb = chunked_problems()
     assert int((pb.nM.astype(np.int64) * (pb.nL + 1)).sum()) > HOST_CHUNK
     tabs, st = run_device(pb, 1)
+    assert_pinned_tables((tabs, st), "chunks.1", "600 problems, device")
+    assert_pinned_tables(papi.permanent_prob_batch(pb, 1), "chunks.1", "600 problems, host")
     chunks = host_chunks(pb)
     assert len(chunks) > 1
     for lo, hi in chunks:
@@ -282,6 +378,8 @@ def test_smallest_workspace(papi):
     from probabilisticsemslam_b200._lib import PdaError
     pb = synth.pack(*nw_problems())
     small = run_device(pb, 1)
+    assert_pinned_tables(small, "nw.1", "NW problems, smallest workspace", walked=True)
+    assert_pinned_tables(papi.permanent_prob_batch(pb, 1), "nw.1", "NW problems, host", walked=True)
     assert_tables(run_device(pb, 1, ws_extra=1 << 20), small, "full workspace")
     with pytest.raises(PdaError, match="error -4"):
         run_device(pb, 1, ws_delta=-1)
@@ -346,6 +444,31 @@ def test_argument_errors():
     rc, msg = mcall(a10=16)
     assert rc == -4 and "workspace" in msg
     assert L.pda_conditioned_permanent_workspace_bytes(-1, 8, 1) == -1
+
+
+def test_host_argument_errors():
+    L = _lib()
+    buf = ctypes.create_string_buffer(1 << 16)
+    p = ctypes.cast(buf, ctypes.c_void_p).value
+    # permOpt outside 0..2, where the reference throws: 0 and status 1, without a device
+    out, st = np.full(3, 5.0), np.zeros(3, np.int32)
+    assert L.pda_conditioned_permanent_batch_host(p, p, p, p, 3, 7, out.ctypes.data, st.ctypes.data, 0) == 0
+    assert list(out) == [0.0] * 3 and list(st) == [1] * 3
+    # NULL arguments and negative counts fail before any device call (without a device that would be -2)
+    for i in range(6):
+        args = [p, p, p, p, 2, 1, p, p, 0]
+        args[i if i < 4 else i + 2] = None
+        assert L.pda_conditioned_permanent_batch_host(*args) == -1
+        assert L.pda_last_error().decode() == "conditioned_permanent: NULL argument"
+    assert L.pda_conditioned_permanent_batch_host(p, p, p, p, -1, 1, p, p, 0) == -1
+    assert L.pda_last_error().decode() == "conditioned_permanent: nMats < 0"
+    for i in (0, 1, 2, 3, 6, 7, 8):
+        args = [p, p, p, p, 3, 1, p, p, p, 0]
+        args[i] = None
+        assert L.pda_permanent_prob_batch_host(*args) == -1
+        assert L.pda_last_error().decode() == "permanent_prob: NULL argument"
+    assert L.pda_permanent_prob_batch_host(p, p, p, p, -1, 1, p, p, p, 0) == -1
+    assert L.pda_last_error().decode() == "permanent_prob: nProblems < 0"
 
 
 def test_no_device_is_a_cuda_error():
