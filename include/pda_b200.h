@@ -277,6 +277,49 @@ int pda_association_perm_from_moments_batch_host(const double* landMean, const d
                                                  int64_t nFrames, double nonassign, double* probs, int32_t* status,
                                                  int32_t device);
 
+/* Device-pointer forms of the two moments entries above, with the frame shapes read on the device: every pointer is a
+ * device pointer, the host reads only the scalar arguments, and the call enqueues on `stream` without a
+ * synchronisation, an allocation or a copy between host and device.  One CUDA graph captured with fixed bounds
+ * therefore serves frames of any shape within them (the per-frame call of the SLAM loop).
+ *   maxNL, maxNM          the caller's per-frame bounds (host scalars); maxNL >= 0, maxNM >= 1
+ *   landCapacity          landmarks the landMean / landCov arrays hold; measCapacity likewise for detections
+ *   probs, probCapacity   the tables and the number of doubles probs holds
+ *   probOff               nFrames + 1 entries, written: probOff[0] = 0, probOff[f+1] = probOff[f] + nM*(nL+1) for a
+ *                         frame that passes the checks below, + 0 for one that does not
+ *   status[f]             2: not computed and no table entry written -- offsets negative or descending, reaching past
+ *                         landCapacity / measCapacity, nL > maxNL or nM > maxNM (all of these add nothing to probOff),
+ *                         or a non-empty table that would end past probCapacity (that frame keeps its span in probOff,
+ *                         so every later non-empty frame is status 2 too).  Otherwise the status of the _host form: 0,
+ *                         and in the usePerm form 1 and 3 as in pda_association_perm_probs_batch.
+ *   nFound[f]             (k-best form; may be NULL) as pda_association_probs_batch reports it; -1 for status 2 or nM == 0
+ * Tables of frames with status 0 are bit-identical to the _host form's on the same frames, for any bounds at or above
+ * the batch's real maxima.  The usePerm form takes maxNM <= 11 (PDA_ERR_UNSUPPORTED above): its _host form sends
+ * frames with 12+ detections down a separate host-driven route, which this form does not have.
+ * Errors: PDA_ERR_INVALID for a NULL pointer (other than nFound), nFrames < 0, maxNL < 0, maxNM < 1, a negative capacity
+ * or k < 1; PDA_ERR_UNSUPPORTED for maxNL + maxNM > PDA_MAX_DIM; PDA_ERR_WORKSPACE below *_workspace_bytes.
+ * Workspace (for the current device): per frame the (maxNL+maxNM) x maxNM cost matrix and 44 B of shapes, plus the
+ * chained pipeline's workspace (pda_association_workspace_bytes / pda_association_perm_workspace_bytes at
+ * nFrames * (maxNL+maxNM) * maxNM cost elements, nFrames * (maxNL+maxNM) rows and probCapacity table elements). */
+int64_t pda_association_from_moments_workspace_bytes(int64_t nFrames, int32_t maxNL, int32_t maxNM, int64_t probCapacity,
+                                                     int32_t k);
+int pda_association_from_moments_batch(const double* landMean, const double* landCov, const int64_t* landOff,
+                                       int64_t landCapacity,
+                                       const double* measMean, const double* measCov, const int64_t* measOff,
+                                       int64_t measCapacity, int64_t nFrames, int32_t maxNL, int32_t maxNM,
+                                       double nonassign, int32_t k,
+                                       double* probs, int64_t probCapacity, int64_t* probOff,
+                                       int32_t* status, int32_t* nFound,
+                                       void* workspace, int64_t workspaceBytes, void* stream);
+int64_t pda_association_perm_from_moments_workspace_bytes(int64_t nFrames, int32_t maxNL, int32_t maxNM,
+                                                          int64_t probCapacity);
+int pda_association_perm_from_moments_batch(const double* landMean, const double* landCov, const int64_t* landOff,
+                                            int64_t landCapacity,
+                                            const double* measMean, const double* measCov, const int64_t* measOff,
+                                            int64_t measCapacity, int64_t nFrames, int32_t maxNL, int32_t maxNM,
+                                            double nonassign,
+                                            double* probs, int64_t probCapacity, int64_t* probOff, int32_t* status,
+                                            void* workspace, int64_t workspaceBytes, void* stream);
+
 /* ------------------------------------------------------------------------------------------
  * Stereo bounding-box association: asgnBB (assignment.h:21, assignment.cpp:724-775) with computeBBCostMatrix
  * (:777-797) and boundBox::IoU (boundBox.h:62-75), for a batch of frames.  A box is five doubles

@@ -53,6 +53,12 @@ SIGNATURES = {
     "pda_quadric_cost_batch_host": (C.c_int, [ptr, ptr, ptr, ptr, ptr, ptr, i64, dbl, ptr, i32]),
     "pda_association_from_moments_batch_host": (C.c_int, [ptr, ptr, ptr, ptr, ptr, ptr, i64, dbl, i32, ptr, i32]),
     "pda_association_perm_from_moments_batch_host": (C.c_int, [ptr, ptr, ptr, ptr, ptr, ptr, i64, dbl, ptr, ptr, i32]),
+    "pda_association_from_moments_workspace_bytes": (i64, [i64, i32, i32, i64, i32]),
+    "pda_association_from_moments_batch": (C.c_int, [ptr, ptr, ptr, i64, ptr, ptr, ptr, i64, i64, i32, i32, dbl, i32,
+                                                     ptr, i64, ptr, ptr, ptr, ptr, i64, ptr]),
+    "pda_association_perm_from_moments_workspace_bytes": (i64, [i64, i32, i32, i64]),
+    "pda_association_perm_from_moments_batch": (C.c_int, [ptr, ptr, ptr, i64, ptr, ptr, ptr, i64, i64, i32, i32, dbl,
+                                                          ptr, i64, ptr, ptr, ptr, i64, ptr]),
     "pda_asgn_bb_batch_host": (C.c_int, [ptr, ptr, ptr, ptr, i64, dbl, ptr, i32]),
     "pda_permanent_workspace_bytes": (i64, [i64]),
     "pda_permanent_batch": (C.c_int, [ptr, ptr, ptr, ptr, i64, i32, ptr, ptr, ptr, i64, ptr]),

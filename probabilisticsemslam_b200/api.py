@@ -347,6 +347,82 @@ def association_perm_from_moments_batch(frames, nonassign: float, device: int = 
     return [out[off[f]:off[f + 1]].reshape(int(nM[f]), int(nL[f]) + 1) for f in range(len(frames))], st
 
 
+def _moments_device_call(name, land_mean, land_cov, land_off, meas_mean, meas_cov, meas_off, max_nL, max_nM, prob_capacity,
+                         probs, prob_off, status, workspace, ws_args, extra_out):
+    """Shared body of the two *_from_moments_batch_device calls: outputs and workspace allocated where None, no host read
+    of device memory.  A moments array with no rows goes in as a one-element stand-in, since its pointer may not be NULL."""
+    import torch
+    dev = land_off.device
+    n = int(land_off.shape[0]) - 1
+    land_cap = min(land_mean.numel() // 3, land_cov.numel() // 9)
+    meas_cap = min(meas_mean.numel() // 3, meas_cov.numel() // 9)
+    stand_in = lambda t: t if t.numel() else torch.zeros(1, dtype=torch.float64, device=dev)
+    land_mean, land_cov, meas_mean, meas_cov = map(stand_in, (land_mean, land_cov, meas_mean, meas_cov))
+    if prob_capacity is None:
+        prob_capacity = probs.numel() if probs is not None else n * max_nM * (max_nL + 1)
+    probs = torch.zeros(max(int(prob_capacity), 1), dtype=torch.float64, device=dev) if probs is None else probs
+    prob_off = torch.empty(n + 1, dtype=torch.int64, device=dev) if prob_off is None else prob_off
+    status = torch.empty(max(n, 1), dtype=torch.int32, device=dev) if status is None else status
+    if workspace is None:
+        ws = int(getattr(lib(), name + "_workspace_bytes")(n, max_nL, max_nM, int(prob_capacity), *ws_args))
+        check(min(ws, 0))
+        workspace = torch.empty(ws, dtype=torch.uint8, device=dev)
+    tensors = dict(land_mean=land_mean, land_cov=land_cov, land_off=land_off, meas_mean=meas_mean, meas_cov=meas_cov,
+                   meas_off=meas_off, probs=probs, prob_off=prob_off, status=status, workspace=workspace)
+    tensors.update({k: v for k, v in extra_out.items() if v is not None})
+    stream = _device_call_args(tensors, name)
+    return dict(land_cap=land_cap, meas_cap=meas_cap, prob_capacity=int(prob_capacity), probs=probs, prob_off=prob_off,
+                status=status, workspace=workspace, stream=stream, means=(land_mean, land_cov, meas_mean, meas_cov))
+
+
+def association_from_moments_batch_device(land_mean, land_cov, land_off, meas_mean, meas_cov, meas_off, max_nL: int,
+                                          max_nM: int, nonassign: float, k: int, prob_capacity: int | None = None,
+                                          probs=None, prob_off=None, status=None, n_found=None, workspace=None):
+    """pda_association_from_moments_batch on CUDA tensors, enqueued on the current stream (no synchronisation, so it can
+    be captured in a CUDA graph): moments float64 (means 3, covariances 9 column-major per row), land_off / meas_off
+    int64 with nFrames+1 entries, frame shapes read on the device against the bounds max_nL / max_nM.  probs holds
+    prob_capacity doubles (default: probs.numel(), or nFrames * max_nM * (max_nL+1) when probs is None).
+    Returns (probs, prob_off, status, n_found); status 2 marks a frame that was not computed (include/pda_b200.h)."""
+    import torch
+    n = int(land_off.shape[0]) - 1
+    n_found = torch.empty(max(n, 1), dtype=torch.int32, device=land_off.device) if n_found is None else n_found
+    a = _moments_device_call("pda_association_from_moments", land_mean, land_cov, land_off, meas_mean, meas_cov, meas_off,
+                             max_nL, max_nM, prob_capacity, probs, prob_off, status, workspace, (int(k),), dict(n_found=n_found))
+    lm, lc, mm, mc = a["means"]
+    check(lib().pda_association_from_moments_batch(
+        lm.data_ptr(), lc.data_ptr(), land_off.data_ptr(), a["land_cap"], mm.data_ptr(), mc.data_ptr(), meas_off.data_ptr(),
+        a["meas_cap"], n, max_nL, max_nM, float(nonassign), int(k), a["probs"].data_ptr(), a["prob_capacity"],
+        a["prob_off"].data_ptr(), a["status"].data_ptr(), n_found.data_ptr(), a["workspace"].data_ptr(),
+        int(a["workspace"].numel()), a["stream"]))
+    return a["probs"], a["prob_off"], a["status"], n_found
+
+
+def association_perm_from_moments_batch_device(land_mean, land_cov, land_off, meas_mean, meas_cov, meas_off, max_nL: int,
+                                               max_nM: int, nonassign: float, prob_capacity: int | None = None, probs=None,
+                                               prob_off=None, status=None, workspace=None):
+    """pda_association_perm_from_moments_batch (usePerm, max_nM <= 11) on CUDA tensors, as
+    association_from_moments_batch_device.  Returns (probs, prob_off, status)."""
+    n = int(land_off.shape[0]) - 1
+    a = _moments_device_call("pda_association_perm_from_moments", land_mean, land_cov, land_off, meas_mean, meas_cov,
+                             meas_off, max_nL, max_nM, prob_capacity, probs, prob_off, status, workspace, (), {})
+    lm, lc, mm, mc = a["means"]
+    check(lib().pda_association_perm_from_moments_batch(
+        lm.data_ptr(), lc.data_ptr(), land_off.data_ptr(), a["land_cap"], mm.data_ptr(), mc.data_ptr(), meas_off.data_ptr(),
+        a["meas_cap"], n, max_nL, max_nM, float(nonassign), a["probs"].data_ptr(), a["prob_capacity"],
+        a["prob_off"].data_ptr(), a["status"].data_ptr(), a["workspace"].data_ptr(), int(a["workspace"].numel()),
+        a["stream"]))
+    return a["probs"], a["prob_off"], a["status"]
+
+
+def moments_to_device(frames, device="cuda"):
+    """_pack_moments on CUDA tensors: (land_mean, land_cov, land_off, meas_mean, meas_cov, meas_off), the argument order
+    of the *_from_moments_batch_device calls."""
+    import torch
+    lm, lc, lo, mm, mc, mo = _pack_moments(frames)
+    t = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(device)
+    return t(lm), t(lc), t(lo), t(mm), t(mc), t(mo)
+
+
 def computeQuadricCostMatrix(land_mean, land_cov, meas_mean, meas_cov, nonassign: float, device: int = 0) -> np.ndarray:
     return quadric_cost_batch([(land_mean, land_cov, meas_mean, meas_cov)], nonassign, device)[0]
 

@@ -6,6 +6,8 @@
 // getCovs (:693-703) takes the 3x3 shape matrix out of a 4x4 dual quadric.  Built on the device so that a batch of
 // frames x window frames never ships cost matrices over PCIe: moments in, association weights out
 // (pda_association_from_moments_batch_host = this kernel -> conditionCosts -> k-best weights -> un-compaction).
+// The device-pointer forms pda_association_{,perm_}from_moments_batch read the frame shapes on the device instead
+// (moment_shapes_kernel), so a CUDA graph captured once with fixed bounds serves frames of any shape (DESIGN.md 3.8b).
 //
 // Eigen is not installed in this image, so the factorisation below restates Eigen 3.4's published algorithm
 // (Cholesky/LDLT.h, ldlt_inplace<Lower>::unblocked: diagonal pivoting with first-maximum ties, unit-lower L, then
@@ -119,6 +121,126 @@ __global__ void quadric_cost_kernel(const double* __restrict__ landMean, const d
         else if (row == nL + col) v = nonassign;
         C[e] = v;
     }
+}
+
+// ---- device-pointer moments entries: frame shapes are read on the device, never on the host ----
+constexpr unsigned FULL = 0xffffffffu;
+constexpr int SHAPE_THREADS = 1024;  // one CTA; 32 warps, so the warp totals are scanned by one warp
+
+struct MomentShapes {
+    int32_t* nL; int32_t* nM;            // sanitised counts: 0 / 0 for a rejected frame
+    int64_t* landStart; int64_t* measStart;
+    int64_t* costOff; int64_t* rowOff;   // fixed strides: f * (maxNL+maxNM) * maxNM and f * (maxNL+maxNM)
+    int32_t* innerStatus;                // the usePerm pipeline's status, merged into the caller's afterwards
+    double* costs;
+    unsigned char* inner;                // workspace of the chained pipeline
+    size_t bytes;                        // everything up to `inner`
+};
+
+size_t align256(size_t x) { return (x + 255) / 256 * 256; }
+
+MomentShapes carve_shapes(void* workspace, int64_t nFrames, int32_t maxNL, int32_t maxNM) {
+    const size_t n = (size_t)std::max<int64_t>(nFrames, 1), rows = (size_t)(maxNL + maxNM);
+    unsigned char* w = reinterpret_cast<unsigned char*>(workspace);
+    MomentShapes s;
+    size_t o = 0;
+    s.nL = reinterpret_cast<int32_t*>(w + o); o += align256(n * 4);
+    s.nM = reinterpret_cast<int32_t*>(w + o); o += align256(n * 4);
+    s.innerStatus = reinterpret_cast<int32_t*>(w + o); o += align256(n * 4);
+    s.landStart = reinterpret_cast<int64_t*>(w + o); o += align256(n * 8);
+    s.measStart = reinterpret_cast<int64_t*>(w + o); o += align256(n * 8);
+    s.costOff = reinterpret_cast<int64_t*>(w + o); o += align256(n * 8);
+    s.rowOff = reinterpret_cast<int64_t*>(w + o); o += align256(n * 8);
+    s.costs = reinterpret_cast<double*>(w + o); o += align256(n * rows * (size_t)maxNM * 8);
+    s.inner = w + o;
+    s.bytes = o;
+    return s;
+}
+
+// One CTA walks the frames in blocks of SHAPE_THREADS.  A frame passes when its offsets are non-negative and ascending,
+// lie within landCap / measCap, and its counts are within maxNL / maxNM; probOff is the running sum of nM * (nL+1) over
+// passing frames.  A passing non-empty frame whose span ends past probCap keeps its span but is not computed (status
+// 2), so probOff stays a plain prefix sum.  Rejected frames go on as 0 x 0: the chained pipelines then touch nothing of
+// theirs.
+__global__ void __launch_bounds__(SHAPE_THREADS) moment_shapes_kernel(
+    const int64_t* __restrict__ landOff, const int64_t landCap, const int64_t* __restrict__ measOff, const int64_t measCap,
+    const long long nFrames, const int32_t maxNL, const int32_t maxNM, const int64_t probCap, const MomentShapes s,
+    int64_t* __restrict__ probOff, int32_t* __restrict__ status) {
+    __shared__ long long warpSum[SHAPE_THREADS / 32];
+    __shared__ long long carry;
+    const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+    const long long rows = maxNL + maxNM;
+    if (t == 0) { carry = 0; probOff[0] = 0; }
+    for (long long base = 0; base < nFrames; base += SHAPE_THREADS) {
+        const long long f = base + t;
+        int L = 0, M = 0;
+        long long l0 = 0, m0 = 0;
+        bool ok = false;
+        if (f < nFrames) {
+            l0 = landOff[f]; m0 = measOff[f];
+            const long long l1 = landOff[f + 1], m1 = measOff[f + 1];
+            ok = l0 >= 0 && m0 >= 0 && l1 >= l0 && m1 >= m0 && l1 <= landCap && m1 <= measCap && l1 - l0 <= maxNL &&
+                 m1 - m0 <= maxNM;
+            if (ok) { L = (int)(l1 - l0); M = (int)(m1 - m0); }
+        }
+        const long long span = (long long)M * (L + 1);
+        long long x = span;  // inclusive scan: warp, then the warp totals, then the carry of earlier blocks
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const long long y = __shfl_up_sync(FULL, x, o);
+            if (lane >= o) x += y;
+        }
+        if (lane == 31) warpSum[warp] = x;
+        __syncthreads();
+        if (warp == 0) {
+            long long w = warpSum[lane];
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const long long y = __shfl_up_sync(FULL, w, o);
+                if (lane >= o) w += y;
+            }
+            warpSum[lane] = w;
+        }
+        __syncthreads();
+        const long long end = carry + (warp ? warpSum[warp - 1] : 0) + x;
+        if (f < nFrames) {
+            if (span > 0 && end > probCap) { ok = false; L = M = 0; }
+            s.nL[f] = L; s.nM[f] = M;
+            s.landStart[f] = ok ? l0 : 0; s.measStart[f] = ok ? m0 : 0;
+            s.costOff[f] = f * rows * maxNM; s.rowOff[f] = f * rows;
+            probOff[f + 1] = end;
+            status[f] = ok ? 0 : 2;
+        }
+        __syncthreads();  // every thread has read carry and warpSum
+        if (t == SHAPE_THREADS - 1) carry = end;
+    }
+}
+
+// quadric_cost_kernel on the sanitised shapes: frame f's (nL+nM) x nM matrix at f * slot, which holds the bounds' largest
+__global__ void quadric_cost_shaped_kernel(const double* __restrict__ landMean, const double* __restrict__ landCov,
+                                           const double* __restrict__ measMean, const double* __restrict__ measCov,
+                                           const MomentShapes s, const long long nFrames, const long long slot,
+                                           const double nonassign) {
+    const int lane = threadIdx.x & 31;
+    const long long f = (long long)blockIdx.x * QWARPS + (threadIdx.x >> 5);
+    if (f >= nFrames) return;
+    const long long l0 = s.landStart[f], m0 = s.measStart[f];
+    const int nL = s.nL[f], nM = s.nM[f];
+    const int nRows = nL + nM;
+    double* C = s.costs + f * slot;
+    for (int e = lane; e < nRows * nM; e += 32) {
+        const int col = e / nRows, row = e - col * nRows;
+        double v = CUDART_INF;
+        if (row < nL) v = mahalanobis3(landMean + 3 * (l0 + row), landCov + 9 * (l0 + row), measMean + 3 * (m0 + col), measCov + 9 * (m0 + col));
+        else if (row == nL + col) v = nonassign;
+        C[e] = v;
+    }
+}
+
+// status 2 from the shape scan stands; every other frame takes the usePerm pipeline's status
+__global__ void merge_status_kernel(const int32_t* __restrict__ inner, const long long nFrames, int32_t* __restrict__ status) {
+    const long long f = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (f < nFrames && status[f] != 2) status[f] = inner[f];
 }
 
 // getCovs (assignment.cpp:693-703): Q is a 4x4 dual quadric, 16 doubles (symmetric, so either storage order)
@@ -268,6 +390,109 @@ int pda_association_from_moments_batch_host(const double* landMean, const double
                                         st.at<int64_t>(oRO), nFrames, (int64_t)nCost, (int64_t)nRows, (int64_t)nProb, maxR, maxC, k,
                                         st.at<double>(oP), st.at<int64_t>(oPO), nullptr, st.at<unsigned char>(oWs), wsBytes, s));
     return io.download(s);
+}
+
+}  // extern "C"
+
+// argument checks shared by the device-pointer moments entries
+static int moments_args(const char* who, int64_t nFrames, int32_t maxNL, int32_t maxNM, int64_t probCapacity) {
+    if (nFrames < 0 || maxNL < 0 || maxNM < 1 || probCapacity < 0)
+        return fail(PDA_ERR_INVALID, "%s: nFrames %lld, maxNL %d, maxNM %d, probCapacity %lld", who, (long long)nFrames, maxNL,
+                    maxNM, (long long)probCapacity);
+    if ((int64_t)maxNL + maxNM > PDA_MAX_DIM)
+        return fail(PDA_ERR_UNSUPPORTED, "%s: maxNL + maxNM = %lld above %d", who, (long long)maxNL + maxNM, PDA_MAX_DIM);
+    return PDA_OK;
+}
+
+// the shape scan and the cost matrices in front of either pipeline
+static int launch_moment_costs(const double* landMean, const double* landCov, const int64_t* landOff, int64_t landCapacity,
+                               const double* measMean, const double* measCov, const int64_t* measOff, int64_t measCapacity,
+                               int64_t nFrames, int32_t maxNL, int32_t maxNM, double nonassign, int64_t probCapacity,
+                               const MomentShapes& sh, int64_t* probOff, int32_t* status, cudaStream_t s) {
+    moment_shapes_kernel<<<1, SHAPE_THREADS, 0, s>>>(landOff, landCapacity, measOff, measCapacity, nFrames, maxNL, maxNM,
+                                                    probCapacity, sh, probOff, status);
+    PDA_CUDA_TRY(cudaGetLastError());
+    if (nFrames == 0) return PDA_OK;
+    quadric_cost_shaped_kernel<<<(unsigned)((nFrames + QWARPS - 1) / QWARPS), 32 * QWARPS, 0, s>>>(
+        landMean, landCov, measMean, measCov, sh, nFrames, (long long)(maxNL + maxNM) * maxNM, nonassign);
+    PDA_CUDA_TRY(cudaGetLastError());
+    return PDA_OK;
+}
+
+extern "C" {
+
+int64_t pda_association_from_moments_workspace_bytes(int64_t nFrames, int32_t maxNL, int32_t maxNM, int64_t probCapacity,
+                                                     int32_t k) {
+    PDA_TRY(moments_args("association_from_moments", nFrames, maxNL, maxNM, probCapacity));
+    if (k < 1) return fail(PDA_ERR_INVALID, "association_from_moments: k < 1");
+    const int64_t n = std::max<int64_t>(nFrames, 1), rows = maxNL + maxNM;
+    const int64_t inner = pda_association_workspace_bytes(n, n * rows * maxNM, n * rows, probCapacity, k, (int32_t)rows, maxNM);
+    if (inner < 0) return inner;
+    return (int64_t)carve_shapes(nullptr, nFrames, maxNL, maxNM).bytes + inner;
+}
+
+int pda_association_from_moments_batch(const double* landMean, const double* landCov, const int64_t* landOff,
+                                       int64_t landCapacity,
+                                       const double* measMean, const double* measCov, const int64_t* measOff,
+                                       int64_t measCapacity, int64_t nFrames, int32_t maxNL, int32_t maxNM,
+                                       double nonassign, int32_t k,
+                                       double* probs, int64_t probCapacity, int64_t* probOff,
+                                       int32_t* status, int32_t* nFound,
+                                       void* workspace, int64_t workspaceBytes, void* stream) {
+    if (!landMean || !landCov || !landOff || !measMean || !measCov || !measOff || !probs || !probOff || !status || !workspace)
+        return fail(PDA_ERR_INVALID, "association_from_moments: NULL argument");
+    if (landCapacity < 0 || measCapacity < 0) return fail(PDA_ERR_INVALID, "association_from_moments: negative capacity");
+    const int64_t wsBytes = pda_association_from_moments_workspace_bytes(nFrames, maxNL, maxNM, probCapacity, k);
+    if (wsBytes < 0) return (int)wsBytes;
+    if (workspaceBytes < wsBytes)
+        return fail(PDA_ERR_WORKSPACE, "association_from_moments: workspace of %lld B, %lld B needed", (long long)workspaceBytes,
+                    (long long)wsBytes);
+    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+    const MomentShapes sh = carve_shapes(workspace, nFrames, maxNL, maxNM);
+    PDA_TRY(launch_moment_costs(landMean, landCov, landOff, landCapacity, measMean, measCov, measOff, measCapacity, nFrames, maxNL,
+                                maxNM, nonassign, probCapacity, sh, probOff, status, s));
+    if (nFrames == 0) return PDA_OK;
+    const int64_t rows = maxNL + maxNM;
+    return pda_association_probs_batch(sh.costs, sh.costOff, sh.nL, sh.nM, sh.rowOff, nFrames, nFrames * rows * maxNM, nFrames * rows,
+                                       probCapacity, (int32_t)rows, maxNM, k, probs, probOff, nFound, sh.inner,
+                                       workspaceBytes - (int64_t)sh.bytes, stream);
+}
+
+int64_t pda_association_perm_from_moments_workspace_bytes(int64_t nFrames, int32_t maxNL, int32_t maxNM, int64_t probCapacity) {
+    PDA_TRY(moments_args("association_perm_from_moments", nFrames, maxNL, maxNM, probCapacity));
+    const int64_t n = std::max<int64_t>(nFrames, 1), rows = maxNL + maxNM;
+    const int64_t inner = pda_association_perm_workspace_bytes(n, n * rows * maxNM, n * rows, probCapacity, (int32_t)rows, maxNM);
+    if (inner < 0) return inner;
+    return (int64_t)carve_shapes(nullptr, nFrames, maxNL, maxNM).bytes + inner;
+}
+
+int pda_association_perm_from_moments_batch(const double* landMean, const double* landCov, const int64_t* landOff,
+                                            int64_t landCapacity,
+                                            const double* measMean, const double* measCov, const int64_t* measOff,
+                                            int64_t measCapacity, int64_t nFrames, int32_t maxNL, int32_t maxNM,
+                                            double nonassign,
+                                            double* probs, int64_t probCapacity, int64_t* probOff, int32_t* status,
+                                            void* workspace, int64_t workspaceBytes, void* stream) {
+    if (!landMean || !landCov || !landOff || !measMean || !measCov || !measOff || !probs || !probOff || !status || !workspace)
+        return fail(PDA_ERR_INVALID, "association_perm_from_moments: NULL argument");
+    if (landCapacity < 0 || measCapacity < 0) return fail(PDA_ERR_INVALID, "association_perm_from_moments: negative capacity");
+    const int64_t wsBytes = pda_association_perm_from_moments_workspace_bytes(nFrames, maxNL, maxNM, probCapacity);
+    if (wsBytes < 0) return (int)wsBytes;
+    if (workspaceBytes < wsBytes)
+        return fail(PDA_ERR_WORKSPACE, "association_perm_from_moments: workspace of %lld B, %lld B needed",
+                    (long long)workspaceBytes, (long long)wsBytes);
+    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+    const MomentShapes sh = carve_shapes(workspace, nFrames, maxNL, maxNM);
+    PDA_TRY(launch_moment_costs(landMean, landCov, landOff, landCapacity, measMean, measCov, measOff, measCapacity, nFrames, maxNL,
+                                maxNM, nonassign, probCapacity, sh, probOff, status, s));
+    if (nFrames == 0) return PDA_OK;
+    const int64_t rows = maxNL + maxNM;
+    PDA_TRY(pda_association_perm_probs_batch(sh.costs, sh.costOff, sh.nL, sh.nM, sh.rowOff, nFrames, nFrames * rows * maxNM,
+                                             nFrames * rows, probCapacity, (int32_t)rows, maxNM, probs, probOff, sh.innerStatus,
+                                             sh.inner, workspaceBytes - (int64_t)sh.bytes, stream));
+    merge_status_kernel<<<(unsigned)((nFrames + 255) / 256), 256, 0, s>>>(sh.innerStatus, nFrames, status);
+    PDA_CUDA_TRY(cudaGetLastError());
+    return PDA_OK;
 }
 
 }  // extern "C"
