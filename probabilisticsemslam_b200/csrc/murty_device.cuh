@@ -372,14 +372,28 @@ __device__ __forceinline__ double path_gain(const WarpSmem& sm, const int ld, co
     for (int c = 0; c < numColGain; ++c) g = g + sm.C[c * ld + sm.r4c[c]];
     return g;
 }
+// More than 32 columns: column lane + 32 s pays the cost in row nd.r4c[s]; the terms in ascending column order.
+template <int R>
+__device__ __forceinline__ double path_gain_wide(const WarpSmem& sm, const Node<R>& nd, const int ld, const int numColGain,
+                                                 const int lane) {
+    double g = 0.0;
+#pragma unroll
+    for (int s = 0; s < R; ++s) {
+        const int c = lane + 32 * s;
+        const double x = (c < numColGain) ? sm.C[c * ld + nd.r4c[s]] : 0.0;
+        for (int j = 0; j < 32 && 32 * s + j < numColGain; ++j) g = g + __shfl_sync(FULL, x, j);
+    }
+    return g;
+}
 // The same sum from the working node's registers: lane c fetches the one cost its column pays, then the terms are
 // added in the reference's order.  Lanes past the last column contribute +0.0, and g + 0.0 == g (g is a sum of
 // entries of the shifted matrix, never -0.0), so the chain runs over a fixed eight columns at a time with no
-// per-column branch: ~3 instructions per column instead of a dependent shared-memory walk by every lane.
+// per-column branch: ~3 instructions per column instead of a dependent shared-memory walk by every lane.  (Not
+// path_gain: sm.r4c mirrors the node the search started from, not the child it produced.)
 template <int R>
 __device__ __forceinline__ double path_gain_reg(const WarpSmem& sm, const Node<R>& nd, const int ld, const int numColGain,
                                                 const int lane) {
-    if (numColGain > 32) return path_gain(sm, ld, numColGain);
+    if (numColGain > 32) return path_gain_wide<R>(sm, nd, ld, numColGain, lane);
     double x = 0.0;
     if (lane < numColGain) x = sm.C[lane * ld + nd.r4c[0]];
     double g = 0.0;

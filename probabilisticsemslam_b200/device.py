@@ -29,7 +29,9 @@ class MurtyPlan:
     def __init__(self, pb: ProblemBatch, k: int, *, weights: bool = False, weight_mode: int | None = None,
                  cut_mode: int = api.CUT_RELATIVE, cutoff: float = api.GATE, maximize: bool = False,
                  cut_maximize: bool = False, want_lists: bool = True, max_arenas: int | None = None,
-                 pinned_inputs: bool = False):
+                 pinned_inputs: bool = False, max_num_row: int | None = None, max_num_col: int | None = None):
+        """max_num_row / max_num_col: the bounds the call declares (default: the batch's own maxima).  Looser bounds
+        size the kernel geometry as a graph captured for larger frames would; the results do not change."""
         assert torch.cuda.is_available(), "MurtyPlan needs a CUDA device (there is no CPU fallback)"
         self.k, self.n = int(k), len(pb)
         self.cut_mode, self.cutoff, self.maximize, self.cut_maximize = cut_mode, float(cutoff), bool(maximize), bool(cut_maximize)
@@ -37,7 +39,8 @@ class MurtyPlan:
         dev = torch.device("cuda", torch.cuda.current_device())
         self.dev = dev
         num_row, num_col = pb.num_row, pb.nM.astype(np.int32)
-        self.max_row, self.max_col = int(num_row.max()), int(num_col.max())
+        self.max_row = int(num_row.max()) if max_num_row is None else int(max_num_row)
+        self.max_col = int(num_col.max()) if max_num_col is None else int(max_num_col)
         self.cost_off_h = pb.cost_off.astype(np.int64)
         self.r4c_off_h = api._prefix(num_col.astype(np.int64) * k)
         self.c4r_off_h = api._prefix(num_row.astype(np.int64) * k)
