@@ -166,7 +166,9 @@ int pda_assignment_prob_ladder_batch_host(const double* costs, const int64_t* co
  * makeSafe != 0, shortestPathCPP (hpp:178-182) on an already-safe matrix otherwise.
  * Per problem p: col4row[rowOff.. +numRow], row4col[colOff.. +numCol], u[colOff..], v[rowOff..],
  * forbidden[rowOff..] (bytes), gain[p], feasible[p] (1 solved, 0 infeasible).
- * rowOff/colOff are prefix sums of numRow/numCol.  Any output pointer may be NULL. */
+ * rowOff/colOff are prefix sums of numRow/numCol.  Any output pointer may be NULL.
+ * An n x 0 problem is feasible with gain 0.0, every col4row -1 and forbidden all 0.  In the device-pointer form a
+ * problem above maxNumRow x maxNumCol (or with numCol > numRow) is not solved: feasible[p] = 0, nothing else written. */
 int pda_lap_batch(const double* costs, const int64_t* costOff, const int32_t* numRow, const int32_t* numCol,
                   const int32_t* numCol4Gain, int64_t nProblems, int32_t maxNumRow, int32_t maxNumCol,
                   int32_t makeSafe, int32_t maximize,
@@ -183,6 +185,8 @@ int pda_lap_batch_host(const double* costs, const int64_t* costOff, const int32_
  * Cost conditioning and element-wise likelihoods.
  * conditionCosts (assignment.cpp:439-525): outCosts at costOff[p] (compacted goodRows[p] x numCol[p]),
  * rowIdx at rowOff[p] (first goodRows[p] entries valid).  toProbs (assignment.cpp:527-542) in place.
+ * numCol is at most PDA_MAX_DIM: the _host form rejects a larger problem (PDA_ERR_UNSUPPORTED); the device-pointer
+ * form skips it (goodRows[p] = 0, its outCosts and rowIdx not written) and conditions the rest of the batch.
  */
 int pda_condition_costs_batch(const double* costs, const int64_t* costOff, const int32_t* numRow,
                               const int32_t* numCol, int64_t nProblems, const int64_t* rowOff,
@@ -199,6 +203,9 @@ int pda_to_probs_batch_host(double* values, const int64_t* off, const int64_t* l
  * landmark indices through rowIdx.  In: the raw (nL+nM) x nM cost matrices (what computeQuadricCostMatrix,
  * assignment.cpp:705-722, produces).  Out: probs[p] = nM x (nL+1) row-major at probOff[p]; nL == 0 gives {1}
  * per detection (:51-53).  rowOff = prefix sums of (nL+nM); the total* arguments size the intermediates.
+ * The bounds must satisfy 1 <= maxNumCol <= maxNumRow <= PDA_MAX_DIM (else PDA_ERR_INVALID / PDA_ERR_UNSUPPORTED before
+ * anything is launched); a problem with nL+nM > maxNumRow or nM > maxNumCol is skipped: nFound[p] = -1 and its table
+ * is zeros (ones where nL == 0).
  */
 int64_t pda_association_workspace_bytes(int64_t nProblems, int64_t totalCostElems, int64_t totalRows,
                                         int64_t totalProbElems, int32_t k, int32_t maxNumRow, int32_t maxNumCol);

@@ -66,6 +66,12 @@ int pda_association_probs_batch(const double* costs, const int64_t* costOff, con
     if (nProblems == 0) return PDA_OK;
     if (!costs || !costOff || !nL || !nM || !rowOff || !probs || !probOff || !workspace)
         return fail(PDA_ERR_INVALID, "association: NULL argument");
+    // checked before the first launch: the conditioning kernel skips the problems beyond these bounds (the k-best
+    // kernel then reports nFound = -1 for them), which keeps its per-column minima inside shared memory
+    if (maxNumCol < 1 || maxNumCol > maxNumRow)
+        return fail(PDA_ERR_INVALID, "association: need 1 <= maxNumCol <= maxNumRow (got %d x %d)", maxNumRow, maxNumCol);
+    if (maxNumRow > PDA_MAX_DIM)
+        return fail(PDA_ERR_UNSUPPORTED, "association: maxNumRow %d exceeds PDA_MAX_DIM %d", maxNumRow, PDA_MAX_DIM);
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     const size_t n = (size_t)nProblems;
     unsigned char* w = reinterpret_cast<unsigned char*>(workspace);
@@ -80,7 +86,8 @@ int pda_association_probs_batch(const double* costs, const int64_t* costOff, con
     if ((int64_t)o + 256 > workspaceBytes) return fail(PDA_ERR_WORKSPACE, "association: workspace too small");
     // (numRow = nL + nM and condL = goodRows - nM are formed inside the conditioning kernel: two launches fewer)
     (void)numRow;
-    PDA_TRY(launch_condition_costs(costs, costOff, nullptr, nM, nProblems, rowOff, condCosts, rowIdx, goodRows, s, nL, condNL));
+    PDA_TRY(launch_condition_costs(costs, costOff, nullptr, nM, nProblems, rowOff, condCosts, rowIdx, goodRows, s, nL, condNL,
+                                   maxNumRow, maxNumCol));
     // conditioned problems live at the original cost offsets (they only shrink) and use the original probability offsets
     PDA_TRY(pda_murty_batch(condCosts, costOff, goodRows, nM, nProblems, maxNumRow, maxNumCol, k, PDA_CUT_RELATIVE, 42.0, 0, 0,
                             nullptr, nullptr, nullptr, nullptr, nullptr, nFound ? nFound : found, PDA_WEIGHTS_GATED, condProbs,

@@ -373,9 +373,13 @@ __global__ void lap_kernel(const LapArgs a, const int smemPerWarp, const int cCa
     const WarpSmem sm = carve<R>(smemRaw + (size_t)warp * smemPerWarp, g);
     const int n = a.numRow[p], nc = a.numCol[p];
     const int ncGain = a.numCol4Gain ? a.numCol4Gain[p] : nc;
-    if (nc < 0 || nc > n || n > 32 * R || n * nc > cCap) { if (lane == 0 && a.feasible) a.feasible[p] = 0; return; }  // malformed or beyond the declared maxima
+    if (nc < 0 || nc > n || n > a.maxNumRow || nc > a.maxNumCol || n > 32 * R || n * nc > cCap) {  // malformed or beyond the declared maxima
+        if (lane == 0 && a.feasible) a.feasible[p] = 0;
+        return;
+    }
     double CDelta = stage_safe_matrix(a.costs + a.costOff[p], sm.C, n * nc, a.maximize != 0, a.makeSafe != 0, lane);
-    CDelta = CDelta * (double)nc;
+    // n x 0: the extremum of no entries is +-inf, and inf * 0 would turn the gain (a sum of no terms) into NaN
+    CDelta = nc > 0 ? CDelta * (double)nc : 0.0;
     Node<R> nd;
 #pragma unroll
     for (int s = 0; s < R; ++s) { nd.v[s] = 0.0; nd.u[s] = 0.0; nd.c4r[s] = -1; nd.r4c[s] = -1; }

@@ -138,8 +138,10 @@ int pda_condition_costs_batch(const double* costs, const int64_t* costOff, const
     if (nProblems == 0) return PDA_OK;
     if (!costs || !costOff || !numRow || !numCol || !rowOff || !outCosts || !rowIdx || !goodRows)
         return fail(PDA_ERR_INVALID, "condition_costs: NULL argument");
+    // the kernel keeps one column minimum per column in shared memory: a problem with more than PDA_MAX_DIM columns
+    // is skipped (goodRows = 0, nothing else written), as the host form rejects it
     return launch_condition_costs(costs, costOff, numRow, numCol, nProblems, rowOff, outCosts, rowIdx, goodRows,
-                                  reinterpret_cast<cudaStream_t>(stream));
+                                  reinterpret_cast<cudaStream_t>(stream), nullptr, nullptr, INT32_MAX, PDA_MAX_DIM);
 }
 
 int pda_condition_costs_batch_host(const double* costs, const int64_t* costOff, const int32_t* numRow,
