@@ -122,38 +122,18 @@ int pda_association_probs_batch_host(const double* costs, const int64_t* costOff
     PDA_TRY(scope.enter(device));
     const int64_t wsBytes = pda_association_workspace_bytes(nProblems, (int64_t)nCost, (int64_t)nRows, (int64_t)nProb, k, maxR, maxC);
     if (wsBytes < 0) return (int)wsBytes;
-    if (8 * (nCost + nProb + 3 * n) + 8 * n <= PDA_PACKED_LIMIT) {  // small call (the per-frame SLAM shape): one pinned copy each way
-        Stage st(device);
-        PackedIO io(st);
-        const size_t oC = io.in(costs, nCost * 8), oCO = io.in(costOff, n * 8), oL = io.in(nL, n * 4), oM = io.in(nM, n * 4);
-        const size_t oRO = io.in(rowOff.data(), n * 8), oPO = io.in(probOff, n * 8);
-        const size_t oP = io.out(probs, nProb * 8), oWs = st.reserve((size_t)wsBytes);
-        PDA_TRY(st.commit());
-        HostStreams* hs = nullptr;
-        PDA_TRY(host_streams(device, &hs));
-        PDA_TRY(io.upload(hs->run));
-        PDA_TRY(pda_association_probs_batch(st.at<double>(oC), st.at<int64_t>(oCO), st.at<int32_t>(oL), st.at<int32_t>(oM),
-                                            st.at<int64_t>(oRO), nProblems, (int64_t)nCost, (int64_t)nRows, (int64_t)nProb, maxR, maxC, k,
-                                            st.at<double>(oP), st.at<int64_t>(oPO), nullptr, st.at<unsigned char>(oWs), wsBytes, hs->run));
-        return io.download(hs->run);
-    }
     Stage st(device);
-    const size_t oC = st.reserve(nCost * 8), oCO = st.reserve(n * 8), oL = st.reserve(n * 4), oM = st.reserve(n * 4);
-    const size_t oRO = st.reserve(n * 8), oP = st.reserve(nProb * 8), oPO = st.reserve(n * 8), oWs = st.reserve((size_t)wsBytes);
-    PDA_TRY(st.commit());
-    cudaStream_t s = 0;
-    PDA_TRY(h2d(st.at<double>(oC), costs, nCost, s));
-    PDA_TRY(h2d(st.at<int64_t>(oCO), costOff, n, s));
-    PDA_TRY(h2d(st.at<int32_t>(oL), nL, n, s));
-    PDA_TRY(h2d(st.at<int32_t>(oM), nM, n, s));
-    PDA_TRY(h2d(st.at<int64_t>(oRO), rowOff.data(), n, s));
-    PDA_TRY(h2d(st.at<int64_t>(oPO), probOff, n, s));
+    HostIO io(st);
+    const size_t oC = io.in(costs, nCost * 8), oCO = io.in(costOff, n * 8), oL = io.in(nL, n * 4), oM = io.in(nM, n * 4);
+    const size_t oRO = io.in(rowOff.data(), n * 8), oPO = io.in(probOff, n * 8);
+    const size_t oP = io.out(probs, nProb * 8), oWs = st.reserve((size_t)wsBytes);
+    PDA_TRY(io.commit());
+    PDA_TRY(io.upload());
     PDA_TRY(pda_association_probs_batch(st.at<double>(oC), st.at<int64_t>(oCO), st.at<int32_t>(oL), st.at<int32_t>(oM),
                                         st.at<int64_t>(oRO), nProblems, (int64_t)nCost, (int64_t)nRows, (int64_t)nProb, maxR, maxC, k,
-                                        st.at<double>(oP), st.at<int64_t>(oPO), nullptr, st.at<unsigned char>(oWs), wsBytes, s));
-    PDA_TRY(d2h(probs, st.at<double>(oP), nProb, s));
-    PDA_CUDA_TRY(cudaStreamSynchronize(s));
-    return PDA_OK;
+                                        st.at<double>(oP), st.at<int64_t>(oPO), nullptr, st.at<unsigned char>(oWs), wsBytes,
+                                        io.stream()));
+    return io.download();
 }
 
 }  // extern "C"

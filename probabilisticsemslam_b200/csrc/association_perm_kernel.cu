@@ -343,40 +343,17 @@ int pda_association_perm_probs_batch_host(const double* costs, const int64_t* co
         const int64_t wsBytes = pda_association_perm_workspace_bytes(nProblems, (int64_t)nCost, (int64_t)nRows, (int64_t)nProb, maxR, maxC);
         if (wsBytes < 0) return (int)wsBytes;
         Stage st(device);
-        if (8 * (nCost + nProb + 3 * n) + 12 * n <= PDA_PACKED_LIMIT) {  // small call (the per-frame SLAM shape): one pinned copy each way
-            PackedIO io(st);
-            const size_t oC = io.in(costs, nCost * 8), oCO = io.in(costOff, n * 8), oL = io.in(nL, n * 4), oM = io.in(nM, n * 4);
-            const size_t oRO = io.in(rowOff.data(), n * 8), oPO = io.in(probOff, n * 8);
-            const size_t oP = io.out(probs, nProb * 8), oS = io.out(status, n * 4), oWs = st.reserve((size_t)wsBytes);
-            PDA_TRY(st.commit());
-            HostStreams* hs = nullptr;
-            PDA_TRY(host_streams(device, &hs));
-            PDA_TRY(io.upload(hs->run));
-            PDA_TRY(pda_association_perm_probs_batch(st.at<double>(oC), st.at<int64_t>(oCO), st.at<int32_t>(oL), st.at<int32_t>(oM),
-                                                     st.at<int64_t>(oRO), nProblems, (int64_t)nCost, (int64_t)nRows, (int64_t)nProb, maxR,
-                                                     maxC, st.at<double>(oP), st.at<int64_t>(oPO), st.at<int32_t>(oS),
-                                                     st.at<unsigned char>(oWs), wsBytes, hs->run));
-            PDA_TRY(io.download(hs->run));
-        } else {
-            const size_t oC = st.reserve(nCost * 8), oCO = st.reserve(n * 8), oL = st.reserve(n * 4), oM = st.reserve(n * 4);
-            const size_t oRO = st.reserve(n * 8), oP = st.reserve(nProb * 8), oPO = st.reserve(n * 8), oS = st.reserve(n * 4);
-            const size_t oWs = st.reserve((size_t)wsBytes);
-            PDA_TRY(st.commit());
-            cudaStream_t s = 0;
-            PDA_TRY(h2d(st.at<double>(oC), costs, nCost, s));
-            PDA_TRY(h2d(st.at<int64_t>(oCO), costOff, n, s));
-            PDA_TRY(h2d(st.at<int32_t>(oL), nL, n, s));
-            PDA_TRY(h2d(st.at<int32_t>(oM), nM, n, s));
-            PDA_TRY(h2d(st.at<int64_t>(oRO), rowOff.data(), n, s));
-            PDA_TRY(h2d(st.at<int64_t>(oPO), probOff, n, s));
-            PDA_TRY(pda_association_perm_probs_batch(st.at<double>(oC), st.at<int64_t>(oCO), st.at<int32_t>(oL), st.at<int32_t>(oM),
-                                                     st.at<int64_t>(oRO), nProblems, (int64_t)nCost, (int64_t)nRows, (int64_t)nProb, maxR,
-                                                     maxC, st.at<double>(oP), st.at<int64_t>(oPO), st.at<int32_t>(oS),
-                                                     st.at<unsigned char>(oWs), wsBytes, s));
-            PDA_TRY(d2h(probs, st.at<double>(oP), nProb, s));
-            PDA_TRY(d2h(status, st.at<int32_t>(oS), n, s));
-            PDA_CUDA_TRY(cudaStreamSynchronize(s));
-        }
+        HostIO io(st);
+        const size_t oC = io.in(costs, nCost * 8), oCO = io.in(costOff, n * 8), oL = io.in(nL, n * 4), oM = io.in(nM, n * 4);
+        const size_t oRO = io.in(rowOff.data(), n * 8), oPO = io.in(probOff, n * 8);
+        const size_t oP = io.out(probs, nProb * 8), oS = io.out(status, n * 4), oWs = st.reserve((size_t)wsBytes);
+        PDA_TRY(io.commit());
+        PDA_TRY(io.upload());
+        PDA_TRY(pda_association_perm_probs_batch(st.at<double>(oC), st.at<int64_t>(oCO), st.at<int32_t>(oL), st.at<int32_t>(oM),
+                                                 st.at<int64_t>(oRO), nProblems, (int64_t)nCost, (int64_t)nRows, (int64_t)nProb, maxR,
+                                                 maxC, st.at<double>(oP), st.at<int64_t>(oPO), st.at<int32_t>(oS),
+                                                 st.at<unsigned char>(oWs), wsBytes, io.stream()));
+        PDA_TRY(io.download());
     }
     if (large.empty()) return PDA_OK;
     std::vector<std::vector<double> > lc(large.size());
@@ -426,17 +403,15 @@ int pda_association_perm_from_moments_batch_host(const double* landMean, const d
         const int64_t wsBytes = pda_association_perm_workspace_bytes(nFrames, (int64_t)nCost, (int64_t)nRows, (int64_t)nProb, maxR, maxC);
         if (wsBytes < 0) return (int)wsBytes;
         Stage st(device);
-        PackedIO io(st);
+        HostIO io(st);
         const size_t oLM = io.in(landMean, nLand * 24), oLC = io.in(landCov, nLand * 72), oLO = io.in(landOff, (n + 1) * 8);
         const size_t oMM = io.in(measMean, nMeas * 24), oMC = io.in(measCov, nMeas * 72), oMO = io.in(measOff, (n + 1) * 8);
         const size_t oCO = io.in(costOff.data(), n * 8), oPO = io.in(probOff.data(), n * 8), oRO = io.in(rowOff.data(), n * 8);
         const size_t oP = io.out(probs, nProb * 8), oS = io.out(status, n * 4);
         const size_t oC = st.reserve(nCost * 8), oNL = st.reserve(n * 4), oNM = st.reserve(n * 4), oWs = st.reserve((size_t)wsBytes);
-        PDA_TRY(st.commit());
-        HostStreams* hs = nullptr;
-        PDA_TRY(host_streams(device, &hs));
-        cudaStream_t s = hs->run;
-        PDA_TRY(io.upload(s));
+        PDA_TRY(io.commit());
+        const cudaStream_t s = io.stream();
+        PDA_TRY(io.upload());
         PDA_TRY(pda_quadric_cost_batch(st.at<double>(oLM), st.at<double>(oLC), st.at<int64_t>(oLO), st.at<double>(oMM), st.at<double>(oMC),
                                        st.at<int64_t>(oMO), nFrames, nonassign, st.at<double>(oC), st.at<int64_t>(oCO),
                                        st.at<int32_t>(oNL), st.at<int32_t>(oNM), s));
@@ -444,7 +419,7 @@ int pda_association_perm_from_moments_batch_host(const double* landMean, const d
                                                  st.at<int64_t>(oRO), nFrames, (int64_t)nCost, (int64_t)nRows, (int64_t)nProb, maxR, maxC,
                                                  st.at<double>(oP), st.at<int64_t>(oPO), st.at<int32_t>(oS), st.at<unsigned char>(oWs),
                                                  wsBytes, s));
-        PDA_TRY(io.download(s));
+        PDA_TRY(io.download());
     }
     if (large.empty()) return PDA_OK;
     // frames with 12+ detections: their cost matrices, then today's route

@@ -109,21 +109,15 @@ extern "C" int pda_asgn_bb_batch_host(const double* boxesL, const int64_t* offL,
     const int64_t wsBytes = pda_murty_workspace_bytes((int64_t)n, 1, maxR, maxC);
     if (wsBytes < 0) return (int)wsBytes;
     Stage st(device);
-    const size_t oBL = st.reserve((size_t)totalL * 40), oBR = st.reserve((size_t)totalR * 40);
-    const size_t oFL = st.reserve(n * 8), oFR = st.reserve(n * 8), oNR = st.reserve(n * 4), oNC = st.reserve(n * 4);
-    const size_t oCO = st.reserve(n * 8), oRO = st.reserve(n * 8), oC = st.reserve(nCost * 8), oR4c = st.reserve(nR4c * 8);
-    const size_t oFound = st.reserve(n * 4), oAsg = st.reserve((size_t)totalL * 4), oWs = st.reserve((size_t)wsBytes);
-    PDA_TRY(st.commit());
-    cudaStream_t s = 0;
-    PDA_TRY(h2d(st.at<double>(oBL), boxesL, (size_t)totalL * 5, s));
-    PDA_TRY(h2d(st.at<double>(oBR), boxesR, (size_t)totalR * 5, s));
-    PDA_TRY(h2d(st.at<int64_t>(oFL), firstL.data(), n, s));
-    PDA_TRY(h2d(st.at<int64_t>(oFR), firstR.data(), n, s));
-    PDA_TRY(h2d(st.at<int32_t>(oNR), numRow.data(), n, s));
-    PDA_TRY(h2d(st.at<int32_t>(oNC), numCol.data(), n, s));
-    PDA_TRY(h2d(st.at<int64_t>(oCO), costOff.data(), n, s));
-    PDA_TRY(h2d(st.at<int64_t>(oRO), r4cOff.data(), n, s));
-    PDA_TRY(h2d(st.at<int32_t>(oAsg), assignment, (size_t)totalL, s));
+    HostIO io(st);
+    const size_t oBL = io.in(boxesL, (size_t)totalL * 40), oBR = io.in(boxesR, (size_t)totalR * 40);
+    const size_t oFL = io.in(firstL.data(), n * 8), oFR = io.in(firstR.data(), n * 8), oNR = io.in(numRow.data(), n * 4);
+    const size_t oNC = io.in(numCol.data(), n * 4), oCO = io.in(costOff.data(), n * 8), oRO = io.in(r4cOff.data(), n * 8);
+    const size_t oAsg = io.inout(assignment, (size_t)totalL * 4);
+    const size_t oC = st.reserve(nCost * 8), oR4c = st.reserve(nR4c * 8), oFound = st.reserve(n * 4), oWs = st.reserve((size_t)wsBytes);
+    PDA_TRY(io.commit());
+    const cudaStream_t s = io.stream();
+    PDA_TRY(io.upload());
     const unsigned blocks = (unsigned)((n + WARPS - 1) / WARPS);
     bb_costs_kernel<<<blocks, 32 * WARPS, 0, s>>>(st.at<double>(oBL), st.at<double>(oBR), st.at<int64_t>(oFL), st.at<int64_t>(oFR),
                                                   st.at<int32_t>(oNR), st.at<int32_t>(oNC), st.at<int64_t>(oCO), (int64_t)n, nonassign,
@@ -136,7 +130,5 @@ extern "C" int pda_asgn_bb_batch_host(const double* boxesL, const int64_t* offL,
     bb_finish_kernel<<<blocks, 32 * WARPS, 0, s>>>(st.at<int64_t>(oR4c), st.at<int64_t>(oRO), st.at<int32_t>(oFound), st.at<int32_t>(oNR),
                                                    st.at<int32_t>(oNC), st.at<int64_t>(oFL), (int64_t)n, st.at<int32_t>(oAsg));
     PDA_CUDA_TRY(cudaGetLastError());
-    PDA_TRY(d2h(assignment, st.at<int32_t>(oAsg), (size_t)totalL, s));
-    PDA_CUDA_TRY(cudaStreamSynchronize(s));
-    return PDA_OK;
+    return io.download();
 }

@@ -312,29 +312,28 @@ static int murty_batch_host(const double* costs, const int64_t* costOff, const i
     int64_t wsBytes = pda_murty_workspace_bytes(nProblems, k, maxR, maxC);
     if (wsBytes < 0) return (int)wsBytes;
     const size_t n = (size_t)nProblems;
-    const size_t ioBytes = 8 * (nCost + nR4c + nC4r + nProb + (gainBest ? n * (size_t)k : 0) + 4 * n) + 16 * n + 4 * n * (S - 1);
-    if (ioBytes <= PDA_PACKED_LIMIT) {  // small call: one pinned copy each way
+    {
         Stage st(device);
-        PackedIO io(st);
+        HostIO io(st);
         const size_t oCost = io.in(costs + loCost, nCost * 8), oCostOff = io.in(costOff, n * 8), oNR = io.in(numRow, n * 4), oNC = io.in(numCol, n * 4);
         const size_t oR4cOff = io.in(row4colBest ? r4cOff : nullptr, n * 8), oC4rOff = io.in(col4rowBest ? c4rOff : nullptr, n * 8);
         const size_t oProbOff = io.in(weightMode ? probOff : nullptr, n * 8), oNL = io.in(weightMode ? nL : nullptr, n * 4);
         const size_t oFound = io.out(nFound, n * 4 * S), oGain = io.out(gainBest, gainBest ? n * (size_t)k * 8 : 0);
         const size_t oProb = io.out(weightMode ? probs + loProb : nullptr, nProb * 8);
         const size_t oR4c = io.out(row4colBest ? row4colBest + loR4c : nullptr, nR4c * 8), oC4r = io.out(col4rowBest ? col4rowBest + loC4r : nullptr, nC4r * 8);
-        const size_t oWs = st.reserve((size_t)wsBytes);
-        PDA_TRY(st.commit());
-        HostStreams* hs = nullptr;
-        PDA_TRY(host_streams(device, &hs));
-        PDA_TRY(io.upload(hs->run));
-        PDA_TRY(murty_batch_dev(st.at<double>(oCost) - loCost, st.at<int64_t>(oCostOff), st.at<int32_t>(oNR), st.at<int32_t>(oNC), nProblems,
-                                maxR, maxC, k, cutMode, cutoff, maximize, cutMaximize,
-                                row4colBest ? st.at<int64_t>(oR4c) - loR4c : nullptr, st.at<int64_t>(oR4cOff),
-                                col4rowBest ? st.at<int64_t>(oC4r) - loC4r : nullptr, st.at<int64_t>(oC4rOff),
-                                gainBest ? st.at<double>(oGain) : nullptr, st.at<int32_t>(oFound),
-                                weightMode, weightMode ? st.at<double>(oProb) - loProb : nullptr, st.at<int64_t>(oProbOff),
-                                st.at<int32_t>(oNL), st.at<unsigned char>(oWs), wsBytes, hs->run, ladder));
-        return io.download(hs->run);
+        if (io.packed()) {  // small call: one pinned copy each way
+            const size_t oWs = st.reserve((size_t)wsBytes);
+            PDA_TRY(io.commit());
+            PDA_TRY(io.upload());
+            PDA_TRY(murty_batch_dev(st.at<double>(oCost) - loCost, st.at<int64_t>(oCostOff), st.at<int32_t>(oNR), st.at<int32_t>(oNC), nProblems,
+                                    maxR, maxC, k, cutMode, cutoff, maximize, cutMaximize,
+                                    row4colBest ? st.at<int64_t>(oR4c) - loR4c : nullptr, st.at<int64_t>(oR4cOff),
+                                    col4rowBest ? st.at<int64_t>(oC4r) - loC4r : nullptr, st.at<int64_t>(oC4rOff),
+                                    gainBest ? st.at<double>(oGain) : nullptr, st.at<int32_t>(oFound),
+                                    weightMode, weightMode ? st.at<double>(oProb) - loProb : nullptr, st.at<int64_t>(oProbOff),
+                                    st.at<int32_t>(oNL), st.at<unsigned char>(oWs), wsBytes, io.stream(), ladder));
+            return io.download();
+        }
     }
     // Page-locked caller buffers are used in place: a warp reads its 2.4 KB cost matrix over PCIe once when it takes
     // the problem and writes the weight table when it is done, so both transfers hide under ~1.6 ms of computing per
@@ -550,33 +549,19 @@ int pda_lap_batch_host(const double* costs, const int64_t* costOff, const int32_
     PDA_TRY(scope.enter(device));
     const size_t n = (size_t)nProblems;
     Stage st(device);
-    const size_t oCost = st.reserve(nCost * 8), oCostOff = st.reserve(n * 8), oNR = st.reserve(n * 4), oNC = st.reserve(n * 4);
-    const size_t oNG = st.reserve(n * 4), oRO = st.reserve(n * 8), oCO = st.reserve(n * 8);
-    const size_t oC4r = st.reserve(nRows * 8), oR4c = st.reserve(nCols * 8), oU = st.reserve(nCols * 8), oV = st.reserve(nRows * 8);
-    const size_t oF = st.reserve(nRows), oG = st.reserve(n * 8), oFe = st.reserve(n * 4);
-    PDA_TRY(st.commit());
-    cudaStream_t s = 0;
-    PDA_TRY(h2d(st.at<double>(oCost), costs, nCost, s));
-    PDA_TRY(h2d(st.at<int64_t>(oCostOff), costOff, n, s));
-    PDA_TRY(h2d(st.at<int32_t>(oNR), numRow, n, s));
-    PDA_TRY(h2d(st.at<int32_t>(oNC), numCol, n, s));
-    if (numCol4Gain) PDA_TRY(h2d(st.at<int32_t>(oNG), numCol4Gain, n, s));
-    PDA_TRY(h2d(st.at<int64_t>(oRO), rowOff, n, s));
-    PDA_TRY(h2d(st.at<int64_t>(oCO), colOff, n, s));
+    HostIO io(st);
+    const size_t oCost = io.in(costs, nCost * 8), oCostOff = io.in(costOff, n * 8), oNR = io.in(numRow, n * 4), oNC = io.in(numCol, n * 4);
+    const size_t oNG = io.in(numCol4Gain, n * 4), oRO = io.in(rowOff, n * 8), oCO = io.in(colOff, n * 8);
+    const size_t oC4r = io.out(col4row, nRows * 8), oR4c = io.out(row4col, nCols * 8), oU = io.out(u, nCols * 8), oV = io.out(v, nRows * 8);
+    const size_t oF = io.out(forbidden, nRows), oG = io.out(gain, n * 8), oFe = io.out(feasible, n * 4);
+    PDA_TRY(io.commit());
+    PDA_TRY(io.upload());
     PDA_TRY(pda_lap_batch(st.at<double>(oCost), st.at<int64_t>(oCostOff), st.at<int32_t>(oNR), st.at<int32_t>(oNC),
                           numCol4Gain ? st.at<int32_t>(oNG) : nullptr, nProblems, maxR, maxC, makeSafe, maximize,
                           st.at<int64_t>(oRO), st.at<int64_t>(oCO), st.at<int64_t>(oC4r), st.at<int64_t>(oR4c),
                           st.at<double>(oU), st.at<double>(oV), st.at<uint8_t>(oF), st.at<double>(oG),
-                          st.at<int32_t>(oFe), s));
-    PDA_TRY(d2h(col4row, st.at<int64_t>(oC4r), nRows, s));
-    PDA_TRY(d2h(row4col, st.at<int64_t>(oR4c), nCols, s));
-    PDA_TRY(d2h(u, st.at<double>(oU), nCols, s));
-    PDA_TRY(d2h(v, st.at<double>(oV), nRows, s));
-    PDA_TRY(d2h(forbidden, st.at<uint8_t>(oF), nRows, s));
-    PDA_TRY(d2h(gain, st.at<double>(oG), n, s));
-    PDA_TRY(d2h(feasible, st.at<int32_t>(oFe), n, s));
-    PDA_CUDA_TRY(cudaStreamSynchronize(s));
-    return PDA_OK;
+                          st.at<int32_t>(oFe), io.stream()));
+    return io.download();
 }
 
 }  // extern "C"

@@ -147,29 +147,39 @@ inline int run_sharded(int64_t n, const int32_t* devices, int32_t nDevices, F&& 
     return PDA_OK;
 }
 
-// Small calls (a batch of one from the C++ shims, a handful of window frames) are dominated by the fixed cost of each
-// cudaMemcpy from pageable memory (~10 us apiece, a dozen per call).  PackedIO lays all inputs out contiguously in the
-// device arena, then all outputs, mirrors that layout in ONE pinned host buffer, and moves each side with a single
-// asynchronous copy: reserve in()s, then out()s, then (after Stage::commit) upload() -> launches -> download().
-constexpr size_t PDA_PACKED_LIMIT = 8u << 20;  // bytes of inputs + outputs below which a *_host call takes this path
+// The host <-> device copies of a single-device *_host call, all on the device's `run` stream.  The call declares its
+// arrays once -- in()s, then inout()s, then out()s, each returning its offset in the arena (a NULL pointer or 0 bytes
+// reserves without copying) -- then reserves its scratch on the Stage and runs commit() -> upload() -> launches on
+// stream() -> download(), which synchronises.
+// Calls of at most PDA_PACKED_LIMIT bytes of declared arrays (a batch of one from the C++ shims, a handful of window
+// frames) would be dominated by the fixed cost of each cudaMemcpy from pageable memory (~10 us apiece, a dozen per
+// call): their arrays lie contiguously in the arena (in | inout | out), mirrored in ONE pinned host buffer, and each
+// direction is a single copy.  Larger calls copy each array straight from and to the caller's memory, so the pinned
+// buffer never grows beyond the limit's size.
+constexpr size_t PDA_PACKED_LIMIT = 8u << 20;
 
-class PackedIO {
+class HostIO {
 public:
-    explicit PackedIO(Stage& st) : st_(st), begin_(st.used()), inEnd_(st.used()), end_(st.used()) {}
-    size_t in(const void* src, size_t bytes) {
-        const size_t o = st_.reserve(bytes);
-        if (src && bytes) items_.push_back({o, const_cast<void*>(src), bytes, true});
-        inEnd_ = end_ = st_.used();
-        return o;
+    explicit HostIO(Stage& st) : st_(st), begin_(st.used()), inEnd_(begin_), ioEnd_(begin_), end_(begin_) {}
+    size_t in(const void* src, size_t bytes) { const size_t o = add(const_cast<void*>(src), bytes, IN); inEnd_ = ioEnd_ = end_; return o; }
+    size_t inout(void* p, size_t bytes) { const size_t o = add(p, bytes, INOUT); ioEnd_ = end_; return o; }
+    size_t out(void* dst, size_t bytes) { return add(dst, bytes, OUT); }
+    bool packed() const { return end_ - begin_ <= PDA_PACKED_LIMIT; }
+    int commit() {
+        PDA_TRY(st_.commit());
+        HostStreams* hs = nullptr;
+        PDA_TRY(host_streams(st_.device(), &hs));
+        s_ = hs->run;
+        return PDA_OK;
     }
-    size_t out(void* dst, size_t bytes) {
-        const size_t o = st_.reserve(bytes);
-        if (dst && bytes) items_.push_back({o, dst, bytes, false});
-        end_ = st_.used();
-        return o;
-    }
-    size_t bytes() const { return end_ - begin_; }
-    int upload(cudaStream_t s) {
+    cudaStream_t stream() const { return s_; }
+    int upload() {
+        if (!packed()) {
+            for (const Item& it : items_)
+                if (it.dir != OUT)
+                    PDA_CUDA_TRY(cudaMemcpyAsync(st_.at<unsigned char>(it.off), it.host, it.bytes, cudaMemcpyHostToDevice, s_));
+            return PDA_OK;
+        }
         const size_t need = end_ - begin_;
         DeviceCtx& c = g_dev[st_.device()];
         if (c.pinnedCap < need) {
@@ -181,25 +191,40 @@ public:
         }
         pin_ = c.pinned;
         for (const Item& it : items_)
-            if (it.input) memcpy(pin_ + (it.off - begin_), it.host, it.bytes);
-        if (inEnd_ > begin_)
-            PDA_CUDA_TRY(cudaMemcpyAsync(st_.at<unsigned char>(begin_), pin_, inEnd_ - begin_, cudaMemcpyHostToDevice, s));
+            if (it.dir != OUT) memcpy(pin_ + (it.off - begin_), it.host, it.bytes);
+        if (ioEnd_ > begin_)
+            PDA_CUDA_TRY(cudaMemcpyAsync(st_.at<unsigned char>(begin_), pin_, ioEnd_ - begin_, cudaMemcpyHostToDevice, s_));
         return PDA_OK;
     }
-    int download(cudaStream_t s) {
+    int download() {
+        if (!packed()) {
+            for (const Item& it : items_)
+                if (it.dir != IN)
+                    PDA_CUDA_TRY(cudaMemcpyAsync(it.host, st_.at<unsigned char>(it.off), it.bytes, cudaMemcpyDeviceToHost, s_));
+            PDA_CUDA_TRY(cudaStreamSynchronize(s_));
+            return PDA_OK;
+        }
         if (end_ > inEnd_)
             PDA_CUDA_TRY(cudaMemcpyAsync(pin_ + (inEnd_ - begin_), st_.at<unsigned char>(inEnd_), end_ - inEnd_,
-                                         cudaMemcpyDeviceToHost, s));
-        PDA_CUDA_TRY(cudaStreamSynchronize(s));
+                                         cudaMemcpyDeviceToHost, s_));
+        PDA_CUDA_TRY(cudaStreamSynchronize(s_));
         for (const Item& it : items_)
-            if (!it.input) memcpy(it.host, pin_ + (it.off - begin_), it.bytes);
+            if (it.dir != IN) memcpy(it.host, pin_ + (it.off - begin_), it.bytes);
         return PDA_OK;
     }
 private:
-    struct Item { size_t off; void* host; size_t bytes; bool input; };
+    enum Dir { IN, INOUT, OUT };
+    struct Item { size_t off; void* host; size_t bytes; Dir dir; };
+    size_t add(void* host, size_t bytes, Dir dir) {
+        const size_t o = st_.reserve(bytes);
+        if (host && bytes) items_.push_back({o, host, bytes, dir});
+        end_ = st_.used();
+        return o;
+    }
     Stage& st_;
+    cudaStream_t s_ = nullptr;
     unsigned char* pin_ = nullptr;
-    size_t begin_, inEnd_, end_;
+    size_t begin_, inEnd_, ioEnd_, end_;
     std::vector<Item> items_;
 };
 

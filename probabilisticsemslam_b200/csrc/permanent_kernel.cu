@@ -373,14 +373,11 @@ int pda_permanent_batch_host(const double* mats, const int64_t* matOff, const in
     const size_t n = (size_t)nMats;
     const size_t wsBytes = (size_t)pda_permanent_workspace_bytes(nMats);
     Stage st(device);
-    const size_t oM = st.reserve((nEl - loEl) * 8), oOff = st.reserve(n * 8), oR = st.reserve(n * 4), oC = st.reserve(n * 4);
-    const size_t oOut = st.reserve(n * 8), oSt = st.reserve(n * 4), oWs = st.reserve(wsBytes);
-    PDA_TRY(st.commit());
-    cudaStream_t s = 0;
-    PDA_TRY(h2d(st.at<double>(oM), mats + loEl, nEl - loEl, s));
-    PDA_TRY(h2d(st.at<int64_t>(oOff), matOff, n, s));
-    PDA_TRY(h2d(st.at<int32_t>(oR), rows, n, s));
-    PDA_TRY(h2d(st.at<int32_t>(oC), cols, n, s));
+    HostIO io(st);
+    const size_t oM = io.in(mats + loEl, (nEl - loEl) * 8), oOff = io.in(matOff, n * 8), oR = io.in(rows, n * 4), oC = io.in(cols, n * 4);
+    const size_t oOut = io.out(out, n * 8), oSt = io.out(status, n * 4), oWs = st.reserve(wsBytes);
+    PDA_TRY(io.commit());
+    PDA_TRY(io.upload());
     int maxSmall = 0, minSmall = PDA_MAX_DIM;
     for (int64_t i = 0; i < nMats; ++i) {
         const int sm = std::min(rows[i], cols[i]);
@@ -388,11 +385,8 @@ int pda_permanent_batch_host(const double* mats, const int64_t* matOff, const in
     }
     PDA_TRY(launch_permanent_batch(st.at<double>(oM) - loEl, st.at<int64_t>(oOff), st.at<int32_t>(oR), st.at<int32_t>(oC), nMats,
                                    maxDim, st.at<double>(oOut), st.at<int32_t>(oSt), st.at<unsigned char>(oWs),
-                                   (int64_t)wsBytes, s, maxSmall, minSmall));
-    PDA_TRY(d2h(out, st.at<double>(oOut), n, s));
-    PDA_TRY(d2h(status, st.at<int32_t>(oSt), n, s));
-    PDA_CUDA_TRY(cudaStreamSynchronize(s));
-    return PDA_OK;
+                                   (int64_t)wsBytes, io.stream(), maxSmall, minSmall));
+    return io.download();
 }
 
 int pda_permanent_range(const double* A, int32_t n, uint64_t begin, uint64_t end, double* partial,
@@ -416,14 +410,13 @@ int pda_permanent_range_host(const double* A, int32_t n, uint64_t begin, uint64_
     PDA_TRY(current_device_info(&dev));
     const size_t wsBytes = 64 + (size_t)16 * 8192;
     Stage st(device);
-    const size_t oA = st.reserve((size_t)n * n * 8), oP = st.reserve(16), oWs = st.reserve(wsBytes);
-    PDA_TRY(st.commit());
-    cudaStream_t s = 0;
-    PDA_TRY(h2d(st.at<double>(oA), A, (size_t)n * n, s));
-    PDA_TRY(pda_permanent_range(st.at<double>(oA), n, begin, end, st.at<double>(oP), st.at<unsigned char>(oWs), (int64_t)wsBytes, s));
-    PDA_TRY(d2h(partial, st.at<double>(oP), 2, s));
-    PDA_CUDA_TRY(cudaStreamSynchronize(s));
-    return PDA_OK;
+    HostIO io(st);
+    const size_t oA = io.in(A, (size_t)n * n * 8), oP = io.out(partial, 16), oWs = st.reserve(wsBytes);
+    PDA_TRY(io.commit());
+    PDA_TRY(io.upload());
+    PDA_TRY(pda_permanent_range(st.at<double>(oA), n, begin, end, st.at<double>(oP), st.at<unsigned char>(oWs), (int64_t)wsBytes,
+                                io.stream()));
+    return io.download();
 }
 
 // ---- multi-device forms (SURVEY.md 8e): one host thread per device, no data-path collective except for the single

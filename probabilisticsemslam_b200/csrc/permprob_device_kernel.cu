@@ -676,20 +676,15 @@ int pda_conditioned_permanent_batch_host(const double* mats, const int64_t* matO
     PDA_TRY(current_device_info(&dev));
     const size_t wsBytes = carve(nullptr, 1, nMats, 0, nMats, maxDim, maxDim, permOpt, dev.smCount).bytes;
     Stage st(device);
-    const size_t oA = st.reserve(nEl * 8), oOff = st.reserve(n * 8), oR = st.reserve(n * 4), oC = st.reserve(n * 4);
-    const size_t oOut = st.reserve(n * 8), oSt = st.reserve(n * 4), oWs = st.reserve(wsBytes);
-    PDA_TRY(st.commit());
-    cudaStream_t s = 0;
-    PDA_TRY(h2d(st.at<double>(oA), mats, nEl, s));
-    PDA_TRY(h2d(st.at<int64_t>(oOff), matOff, n, s));
-    PDA_TRY(h2d(st.at<int32_t>(oR), r.data(), n, s));
-    PDA_TRY(h2d(st.at<int32_t>(oC), c.data(), n, s));
+    HostIO io(st);
+    const size_t oA = io.in(mats, nEl * 8), oOff = io.in(matOff, n * 8), oR = io.in(r.data(), n * 4), oC = io.in(c.data(), n * 4);
+    const size_t oOut = io.out(out, n * 8), oSt = io.out(status, n * 4), oWs = st.reserve(wsBytes);
+    PDA_TRY(io.commit());
+    PDA_TRY(io.upload());
     PDA_TRY(pda_conditioned_permanent_batch(st.at<double>(oA), st.at<int64_t>(oOff), st.at<int32_t>(oR), st.at<int32_t>(oC), nMats,
                                             maxDim, permOpt, st.at<double>(oOut), st.at<int32_t>(oSt), st.at<unsigned char>(oWs),
-                                            (int64_t)wsBytes, s));
-    PDA_TRY(d2h(out, st.at<double>(oOut), n, s));
-    PDA_TRY(d2h(status, st.at<int32_t>(oSt), n, s));
-    PDA_CUDA_TRY(cudaStreamSynchronize(s));
+                                            (int64_t)wsBytes, io.stream()));
+    PDA_TRY(io.download());
     for (size_t i = 0; i < n; ++i)
         if (std::max(rows[i], cols[i]) > PDA_MAX_DIM) status[i] = 1;
     return PDA_OK;
@@ -736,24 +731,20 @@ int pda_permanent_prob_batch_host(const double* costs, const int64_t* costOff, c
         // the capacity is the chunk's item count: callers may leave gaps between their tables
         const size_t wsBytes = carve(nullptr, 0, (int64_t)n, (int64_t)nCost, items, maxRow, maxCol, permOpt, dev.smCount).bytes;
         Stage st(device);
-        const size_t oP = st.reserve(nCost * 8), oOff = st.reserve(n * 8), oL = st.reserve(n * 4), oM = st.reserve(n * 4);
-        const size_t oProbs = st.reserve(nProb * 8), oProbOff = st.reserve(n * 8), oStatus = st.reserve(n * 4), oWs = st.reserve(wsBytes);
-        PDA_TRY(st.commit());
-        cudaStream_t s = 0;
-        PDA_TRY(h2d(st.at<double>(oP), costs + c0, nCost, s));
-        PDA_TRY(h2d(st.at<int64_t>(oOff), locCostOff.data(), n, s));
-        PDA_TRY(h2d(st.at<int32_t>(oL), nL + p0, n, s));
-        PDA_TRY(h2d(st.at<int32_t>(oM), nM + p0, n, s));
-        PDA_TRY(h2d(st.at<int64_t>(oProbOff), locProbOff.data(), n, s));
+        HostIO io(st);
+        const size_t oP = io.in(costs + c0, nCost * 8), oOff = io.in(locCostOff.data(), n * 8), oL = io.in(nL + p0, n * 4);
+        const size_t oM = io.in(nM + p0, n * 4), oProbOff = io.in(locProbOff.data(), n * 8);
+        const size_t oStatus = io.out(status + p0, n * 4), oProbs = io.out(probs + pr0, nProb * 8), oWs = st.reserve(wsBytes);
+        PDA_TRY(io.commit());
+        const cudaStream_t s = io.stream();
+        PDA_TRY(io.upload());
         // the whole staged range goes back: gaps between the caller's tables come back as zeros
         PDA_CUDA_TRY(cudaMemsetAsync(st.at<double>(oProbs), 0, nProb * 8, s));
         PDA_TRY(pda_permanent_prob_batch(st.at<double>(oP), st.at<int64_t>(oOff), st.at<int32_t>(oL), st.at<int32_t>(oM), (int64_t)n,
                                          (int64_t)nCost, items, maxRow, maxCol, permOpt, st.at<double>(oProbs),
                                          st.at<int64_t>(oProbOff), st.at<int32_t>(oStatus), st.at<unsigned char>(oWs),
                                          (int64_t)wsBytes, s));
-        PDA_TRY(d2h(status + p0, st.at<int32_t>(oStatus), n, s));
-        PDA_TRY(d2h(probs + pr0, st.at<double>(oProbs), nProb, s));
-        PDA_CUDA_TRY(cudaStreamSynchronize(s));
+        PDA_TRY(io.download());
         p0 = p1;
     }
     return PDA_OK;

@@ -280,14 +280,12 @@ int pda_quadric_covs_batch_host(const double* quadrics, int64_t n, double* covs,
     DeviceScope scope;
     PDA_TRY(scope.enter(device));
     Stage st(device);
-    const size_t oQ = st.reserve((size_t)n * 16 * 8), oC = st.reserve((size_t)n * 9 * 8);
-    PDA_TRY(st.commit());
-    cudaStream_t s = 0;
-    PDA_TRY(h2d(st.at<double>(oQ), quadrics, (size_t)n * 16, s));
-    PDA_TRY(pda_quadric_covs_batch(st.at<double>(oQ), n, st.at<double>(oC), s));
-    PDA_TRY(d2h(covs, st.at<double>(oC), (size_t)n * 9, s));
-    PDA_CUDA_TRY(cudaStreamSynchronize(s));
-    return PDA_OK;
+    HostIO io(st);
+    const size_t oQ = io.in(quadrics, (size_t)n * 16 * 8), oC = io.out(covs, (size_t)n * 9 * 8);
+    PDA_TRY(io.commit());
+    PDA_TRY(io.upload());
+    PDA_TRY(pda_quadric_covs_batch(st.at<double>(oQ), n, st.at<double>(oC), io.stream()));
+    return io.download();
 }
 
 int pda_quadric_cost_batch(const double* landMean, const double* landCov, const int64_t* landOff,
@@ -336,18 +334,17 @@ int pda_quadric_cost_batch_host(const double* landMean, const double* landCov, c
     DeviceScope scope;
     PDA_TRY(scope.enter(device));
     Stage st(device);
-    PackedIO io(st);
+    HostIO io(st);
     const size_t oLM = io.in(landMean, nLand * 24), oLC = io.in(landCov, nLand * 72), oLO = io.in(landOff, (n + 1) * 8);
     const size_t oMM = io.in(measMean, nMeas * 24), oMC = io.in(measCov, nMeas * 72), oMO = io.in(measOff, (n + 1) * 8);
     const size_t oCO = io.in(costOff.data(), n * 8);
     const size_t oC = io.out(costs, nCost * 8);
-    PDA_TRY(st.commit());
-    HostStreams* hs = nullptr;
-    PDA_TRY(host_streams(device, &hs));
-    PDA_TRY(io.upload(hs->run));
+    PDA_TRY(io.commit());
+    PDA_TRY(io.upload());
     PDA_TRY(pda_quadric_cost_batch(st.at<double>(oLM), st.at<double>(oLC), st.at<int64_t>(oLO), st.at<double>(oMM), st.at<double>(oMC),
-                                   st.at<int64_t>(oMO), nFrames, nonassign, st.at<double>(oC), st.at<int64_t>(oCO), nullptr, nullptr, hs->run));
-    return io.download(hs->run);
+                                   st.at<int64_t>(oMO), nFrames, nonassign, st.at<double>(oC), st.at<int64_t>(oCO), nullptr, nullptr,
+                                   io.stream()));
+    return io.download();
 }
 
 // getAssignmentProbs (assignment.cpp:38-74, usePerm == 0) from the quadric moments on, one stream, no host round trip:
@@ -372,24 +369,22 @@ int pda_association_from_moments_batch_host(const double* landMean, const double
     const int64_t wsBytes = pda_association_workspace_bytes(nFrames, (int64_t)nCost, (int64_t)nRows, (int64_t)nProb, k, maxR, maxC);
     if (wsBytes < 0) return (int)wsBytes;
     Stage st(device);
-    PackedIO io(st);
+    HostIO io(st);
     const size_t oLM = io.in(landMean, nLand * 24), oLC = io.in(landCov, nLand * 72), oLO = io.in(landOff, (n + 1) * 8);
     const size_t oMM = io.in(measMean, nMeas * 24), oMC = io.in(measCov, nMeas * 72), oMO = io.in(measOff, (n + 1) * 8);
     const size_t oCO = io.in(costOff.data(), n * 8), oPO = io.in(probOff.data(), n * 8), oRO = io.in(rowOff.data(), n * 8);
     const size_t oP = io.out(probs, nProb * 8);
     const size_t oC = st.reserve(nCost * 8), oNL = st.reserve(n * 4), oNM = st.reserve(n * 4), oWs = st.reserve((size_t)wsBytes);
-    PDA_TRY(st.commit());
-    HostStreams* hs = nullptr;
-    PDA_TRY(host_streams(device, &hs));
-    cudaStream_t s = hs->run;
-    PDA_TRY(io.upload(s));
+    PDA_TRY(io.commit());
+    const cudaStream_t s = io.stream();
+    PDA_TRY(io.upload());
     PDA_TRY(pda_quadric_cost_batch(st.at<double>(oLM), st.at<double>(oLC), st.at<int64_t>(oLO), st.at<double>(oMM), st.at<double>(oMC),
                                    st.at<int64_t>(oMO), nFrames, nonassign, st.at<double>(oC), st.at<int64_t>(oCO),
                                    st.at<int32_t>(oNL), st.at<int32_t>(oNM), s));
     PDA_TRY(pda_association_probs_batch(st.at<double>(oC), st.at<int64_t>(oCO), st.at<int32_t>(oNL), st.at<int32_t>(oNM),
                                         st.at<int64_t>(oRO), nFrames, (int64_t)nCost, (int64_t)nRows, (int64_t)nProb, maxR, maxC, k,
                                         st.at<double>(oP), st.at<int64_t>(oPO), nullptr, st.at<unsigned char>(oWs), wsBytes, s));
-    return io.download(s);
+    return io.download();
 }
 
 }  // extern "C"

@@ -162,23 +162,16 @@ int pda_condition_costs_batch_host(const double* costs, const int64_t* costOff, 
     PDA_TRY(scope.enter(device));
     const size_t n = (size_t)nProblems;
     Stage st(device);
-    const size_t oC = st.reserve(nCost * 8), oCO = st.reserve(n * 8), oNR = st.reserve(n * 4), oNC = st.reserve(n * 4);
-    const size_t oRO = st.reserve(n * 8), oOut = st.reserve(nCost * 8), oIdx = st.reserve(nRows * 8), oG = st.reserve(n * 4);
-    PDA_TRY(st.commit());
-    cudaStream_t s = 0;
-    PDA_TRY(h2d(st.at<double>(oC), costs, nCost, s));
-    PDA_TRY(h2d(st.at<int64_t>(oCO), costOff, n, s));
-    PDA_TRY(h2d(st.at<int32_t>(oNR), numRow, n, s));
-    PDA_TRY(h2d(st.at<int32_t>(oNC), numCol, n, s));
-    PDA_TRY(h2d(st.at<int64_t>(oRO), rowOff, n, s));
+    HostIO io(st);
+    const size_t oC = io.in(costs, nCost * 8), oCO = io.in(costOff, n * 8), oNR = io.in(numRow, n * 4), oNC = io.in(numCol, n * 4);
+    const size_t oRO = io.in(rowOff, n * 8);
+    const size_t oOut = io.out(outCosts, nCost * 8), oIdx = io.out(rowIdx, nRows * 8), oG = io.out(goodRows, n * 4);
+    PDA_TRY(io.commit());
+    PDA_TRY(io.upload());
     PDA_TRY(launch_condition_costs(st.at<double>(oC), st.at<int64_t>(oCO), st.at<int32_t>(oNR), st.at<int32_t>(oNC),
                                    nProblems, st.at<int64_t>(oRO), st.at<double>(oOut), st.at<int64_t>(oIdx),
-                                   st.at<int32_t>(oG), s));
-    PDA_TRY(d2h(outCosts, st.at<double>(oOut), nCost, s));
-    PDA_TRY(d2h(rowIdx, st.at<int64_t>(oIdx), nRows, s));
-    PDA_TRY(d2h(goodRows, st.at<int32_t>(oG), n, s));
-    PDA_CUDA_TRY(cudaStreamSynchronize(s));
-    return PDA_OK;
+                                   st.at<int32_t>(oG), io.stream()));
+    return io.download();
 }
 
 int pda_to_probs_batch(double* values, const int64_t* off, const int64_t* len, int64_t nVectors, void* stream) {
@@ -198,16 +191,12 @@ int pda_to_probs_batch_host(double* values, const int64_t* off, const int64_t* l
     PDA_TRY(scope.enter(device));
     const size_t n = (size_t)nVectors;
     Stage st(device);
-    const size_t oV = st.reserve(total * 8), oO = st.reserve(n * 8), oL = st.reserve(n * 8);
-    PDA_TRY(st.commit());
-    cudaStream_t s = 0;
-    PDA_TRY(h2d(st.at<double>(oV), values, total, s));
-    PDA_TRY(h2d(st.at<int64_t>(oO), off, n, s));
-    PDA_TRY(h2d(st.at<int64_t>(oL), len, n, s));
-    PDA_TRY(launch_to_probs(st.at<double>(oV), st.at<int64_t>(oO), st.at<int64_t>(oL), nVectors, s));
-    PDA_TRY(d2h(values, st.at<double>(oV), total, s));
-    PDA_CUDA_TRY(cudaStreamSynchronize(s));
-    return PDA_OK;
+    HostIO io(st);
+    const size_t oO = io.in(off, n * 8), oL = io.in(len, n * 8), oV = io.inout(values, total * 8);
+    PDA_TRY(io.commit());
+    PDA_TRY(io.upload());
+    PDA_TRY(launch_to_probs(st.at<double>(oV), st.at<int64_t>(oO), st.at<int64_t>(oL), nVectors, io.stream()));
+    return io.download();
 }
 
 }  // extern "C"
