@@ -79,9 +79,11 @@ double pda_diag_dfma_tflops(void);
  */
 int64_t pda_murty_workspace_bytes(int64_t nProblems, int32_t k, int32_t maxNumRow, int32_t maxNumCol);
 
-/* Page-locked host buffers for the *_host entry points.  A *_host call that finds its large arrays (cost matrices in,
- * weight tables out) page-locked uses them IN PLACE: every warp reads its cost matrix and writes its weight table over
- * the bus itself, so the transfers hide under the computing instead of standing in front of and behind the kernel.
+/* Page-locked host buffers for the k-best *_host entry points (pda_murty_batch_host, pda_assignment_prob_ladder_batch_host
+ * and their shards in pda_murty_batch_host_multi).  Such a call whose declared arrays exceed 8 MB, and which finds its
+ * cost matrices (in) or weight tables (out) page-locked, uses them IN PLACE: every warp reads its cost matrix and writes
+ * its weight table over the bus itself, so the transfers hide under the computing instead of standing in front of and
+ * behind the kernel.  Smaller calls, every other array and every other *_host entry copy, from any kind of memory.
  * Buffers from pda_host_alloc are portable: every device of the process may use them in place (the multi-device
  * entry points below).  Memory the caller pinned itself (cudaHostAlloc / cudaHostRegister) is used in place only by the
  * device whose context pinned it; pageable memory is copied.  Returns NULL on failure (pda_last_error). */
@@ -124,7 +126,7 @@ int pda_murty_batch_host(const double* costs, const int64_t* costOff, const int3
 
 /* The same over SEVERAL devices of one process (SURVEY.md 8e: "single process drives all GPUs"): the batch is cut into
  * one contiguous slice per entry of `devices`, every slice runs pda_murty_batch_host on its own host thread and device
- * (own lock, staging arena and streams), and the results land directly in the caller's arrays -- problems are
+ * (own lock, staging arena and stream), and the results land directly in the caller's arrays -- problems are
  * independent, so there is no data-path collective.  Offsets stay absolute: pass the arrays of the whole batch.
  * What a frames x probWin window batch of the SLAM loop (slidingWindow.cpp:260-339, system.cpp:268) would call. */
 int pda_murty_batch_host_multi(const double* costs, const int64_t* costOff, const int32_t* numRow, const int32_t* numCol,

@@ -122,16 +122,15 @@ int pda_association_probs_batch_host(const double* costs, const int64_t* costOff
     PDA_TRY(scope.enter(device));
     const int64_t wsBytes = pda_association_workspace_bytes(nProblems, (int64_t)nCost, (int64_t)nRows, (int64_t)nProb, k, maxR, maxC);
     if (wsBytes < 0) return (int)wsBytes;
-    Stage st(device);
-    HostIO io(st);
+    HostIO io(device);
     const size_t oC = io.in(costs, nCost * 8), oCO = io.in(costOff, n * 8), oL = io.in(nL, n * 4), oM = io.in(nM, n * 4);
     const size_t oRO = io.in(rowOff.data(), n * 8), oPO = io.in(probOff, n * 8);
-    const size_t oP = io.out(probs, nProb * 8), oWs = st.reserve((size_t)wsBytes);
+    const size_t oP = io.out(probs, nProb * 8), oWs = io.scratch((size_t)wsBytes);
     PDA_TRY(io.commit());
     PDA_TRY(io.upload());
-    PDA_TRY(pda_association_probs_batch(st.at<double>(oC), st.at<int64_t>(oCO), st.at<int32_t>(oL), st.at<int32_t>(oM),
-                                        st.at<int64_t>(oRO), nProblems, (int64_t)nCost, (int64_t)nRows, (int64_t)nProb, maxR, maxC, k,
-                                        st.at<double>(oP), st.at<int64_t>(oPO), nullptr, st.at<unsigned char>(oWs), wsBytes,
+    PDA_TRY(pda_association_probs_batch(io.at<double>(oC), io.at<int64_t>(oCO), io.at<int32_t>(oL), io.at<int32_t>(oM),
+                                        io.at<int64_t>(oRO), nProblems, (int64_t)nCost, (int64_t)nRows, (int64_t)nProb, maxR, maxC, k,
+                                        io.at<double>(oP), io.at<int64_t>(oPO), nullptr, io.at<unsigned char>(oWs), wsBytes,
                                         io.stream()));
     return io.download();
 }

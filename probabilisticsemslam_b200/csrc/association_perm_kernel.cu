@@ -342,17 +342,16 @@ int pda_association_perm_probs_batch_host(const double* costs, const int64_t* co
         PDA_TRY(scope.enter(device));
         const int64_t wsBytes = pda_association_perm_workspace_bytes(nProblems, (int64_t)nCost, (int64_t)nRows, (int64_t)nProb, maxR, maxC);
         if (wsBytes < 0) return (int)wsBytes;
-        Stage st(device);
-        HostIO io(st);
+        HostIO io(device);
         const size_t oC = io.in(costs, nCost * 8), oCO = io.in(costOff, n * 8), oL = io.in(nL, n * 4), oM = io.in(nM, n * 4);
         const size_t oRO = io.in(rowOff.data(), n * 8), oPO = io.in(probOff, n * 8);
-        const size_t oP = io.out(probs, nProb * 8), oS = io.out(status, n * 4), oWs = st.reserve((size_t)wsBytes);
+        const size_t oP = io.out(probs, nProb * 8), oS = io.out(status, n * 4), oWs = io.scratch((size_t)wsBytes);
         PDA_TRY(io.commit());
         PDA_TRY(io.upload());
-        PDA_TRY(pda_association_perm_probs_batch(st.at<double>(oC), st.at<int64_t>(oCO), st.at<int32_t>(oL), st.at<int32_t>(oM),
-                                                 st.at<int64_t>(oRO), nProblems, (int64_t)nCost, (int64_t)nRows, (int64_t)nProb, maxR,
-                                                 maxC, st.at<double>(oP), st.at<int64_t>(oPO), st.at<int32_t>(oS),
-                                                 st.at<unsigned char>(oWs), wsBytes, io.stream()));
+        PDA_TRY(pda_association_perm_probs_batch(io.at<double>(oC), io.at<int64_t>(oCO), io.at<int32_t>(oL), io.at<int32_t>(oM),
+                                                 io.at<int64_t>(oRO), nProblems, (int64_t)nCost, (int64_t)nRows, (int64_t)nProb, maxR,
+                                                 maxC, io.at<double>(oP), io.at<int64_t>(oPO), io.at<int32_t>(oS),
+                                                 io.at<unsigned char>(oWs), wsBytes, io.stream()));
         PDA_TRY(io.download());
     }
     if (large.empty()) return PDA_OK;
@@ -402,22 +401,21 @@ int pda_association_perm_from_moments_batch_host(const double* landMean, const d
         PDA_TRY(scope.enter(device));
         const int64_t wsBytes = pda_association_perm_workspace_bytes(nFrames, (int64_t)nCost, (int64_t)nRows, (int64_t)nProb, maxR, maxC);
         if (wsBytes < 0) return (int)wsBytes;
-        Stage st(device);
-        HostIO io(st);
+        HostIO io(device);
         const size_t oLM = io.in(landMean, nLand * 24), oLC = io.in(landCov, nLand * 72), oLO = io.in(landOff, (n + 1) * 8);
         const size_t oMM = io.in(measMean, nMeas * 24), oMC = io.in(measCov, nMeas * 72), oMO = io.in(measOff, (n + 1) * 8);
         const size_t oCO = io.in(costOff.data(), n * 8), oPO = io.in(probOff.data(), n * 8), oRO = io.in(rowOff.data(), n * 8);
         const size_t oP = io.out(probs, nProb * 8), oS = io.out(status, n * 4);
-        const size_t oC = st.reserve(nCost * 8), oNL = st.reserve(n * 4), oNM = st.reserve(n * 4), oWs = st.reserve((size_t)wsBytes);
+        const size_t oC = io.scratch(nCost * 8), oNL = io.scratch(n * 4), oNM = io.scratch(n * 4), oWs = io.scratch((size_t)wsBytes);
         PDA_TRY(io.commit());
         const cudaStream_t s = io.stream();
         PDA_TRY(io.upload());
-        PDA_TRY(pda_quadric_cost_batch(st.at<double>(oLM), st.at<double>(oLC), st.at<int64_t>(oLO), st.at<double>(oMM), st.at<double>(oMC),
-                                       st.at<int64_t>(oMO), nFrames, nonassign, st.at<double>(oC), st.at<int64_t>(oCO),
-                                       st.at<int32_t>(oNL), st.at<int32_t>(oNM), s));
-        PDA_TRY(pda_association_perm_probs_batch(st.at<double>(oC), st.at<int64_t>(oCO), st.at<int32_t>(oNL), st.at<int32_t>(oNM),
-                                                 st.at<int64_t>(oRO), nFrames, (int64_t)nCost, (int64_t)nRows, (int64_t)nProb, maxR, maxC,
-                                                 st.at<double>(oP), st.at<int64_t>(oPO), st.at<int32_t>(oS), st.at<unsigned char>(oWs),
+        PDA_TRY(pda_quadric_cost_batch(io.at<double>(oLM), io.at<double>(oLC), io.at<int64_t>(oLO), io.at<double>(oMM), io.at<double>(oMC),
+                                       io.at<int64_t>(oMO), nFrames, nonassign, io.at<double>(oC), io.at<int64_t>(oCO),
+                                       io.at<int32_t>(oNL), io.at<int32_t>(oNM), s));
+        PDA_TRY(pda_association_perm_probs_batch(io.at<double>(oC), io.at<int64_t>(oCO), io.at<int32_t>(oNL), io.at<int32_t>(oNM),
+                                                 io.at<int64_t>(oRO), nFrames, (int64_t)nCost, (int64_t)nRows, (int64_t)nProb, maxR, maxC,
+                                                 io.at<double>(oP), io.at<int64_t>(oPO), io.at<int32_t>(oS), io.at<unsigned char>(oWs),
                                                  wsBytes, s));
         PDA_TRY(io.download());
     }

@@ -108,27 +108,26 @@ extern "C" int pda_asgn_bb_batch_host(const double* boxesL, const int64_t* offL,
     PDA_TRY(scope.enter(device));
     const int64_t wsBytes = pda_murty_workspace_bytes((int64_t)n, 1, maxR, maxC);
     if (wsBytes < 0) return (int)wsBytes;
-    Stage st(device);
-    HostIO io(st);
+    HostIO io(device);
     const size_t oBL = io.in(boxesL, (size_t)totalL * 40), oBR = io.in(boxesR, (size_t)totalR * 40);
     const size_t oFL = io.in(firstL.data(), n * 8), oFR = io.in(firstR.data(), n * 8), oNR = io.in(numRow.data(), n * 4);
     const size_t oNC = io.in(numCol.data(), n * 4), oCO = io.in(costOff.data(), n * 8), oRO = io.in(r4cOff.data(), n * 8);
     const size_t oAsg = io.inout(assignment, (size_t)totalL * 4);
-    const size_t oC = st.reserve(nCost * 8), oR4c = st.reserve(nR4c * 8), oFound = st.reserve(n * 4), oWs = st.reserve((size_t)wsBytes);
+    const size_t oC = io.scratch(nCost * 8), oR4c = io.scratch(nR4c * 8), oFound = io.scratch(n * 4), oWs = io.scratch((size_t)wsBytes);
     PDA_TRY(io.commit());
     const cudaStream_t s = io.stream();
     PDA_TRY(io.upload());
     const unsigned blocks = (unsigned)((n + WARPS - 1) / WARPS);
-    bb_costs_kernel<<<blocks, 32 * WARPS, 0, s>>>(st.at<double>(oBL), st.at<double>(oBR), st.at<int64_t>(oFL), st.at<int64_t>(oFR),
-                                                  st.at<int32_t>(oNR), st.at<int32_t>(oNC), st.at<int64_t>(oCO), (int64_t)n, nonassign,
-                                                  st.at<double>(oC));
+    bb_costs_kernel<<<blocks, 32 * WARPS, 0, s>>>(io.at<double>(oBL), io.at<double>(oBR), io.at<int64_t>(oFL), io.at<int64_t>(oFR),
+                                                  io.at<int32_t>(oNR), io.at<int32_t>(oNC), io.at<int64_t>(oCO), (int64_t)n, nonassign,
+                                                  io.at<double>(oC));
     PDA_CUDA_TRY(cudaGetLastError());
-    PDA_TRY(pda_murty_batch(st.at<double>(oC), st.at<int64_t>(oCO), st.at<int32_t>(oNR), st.at<int32_t>(oNC), (int64_t)n, maxR, maxC,
-                            1, PDA_CUT_NONE, 0.0, 1 /* maximize */, 0, st.at<int64_t>(oR4c), st.at<int64_t>(oRO), nullptr, nullptr,
-                            nullptr, st.at<int32_t>(oFound), PDA_WEIGHTS_NONE, nullptr, nullptr, nullptr,
-                            st.at<unsigned char>(oWs), wsBytes, s));
-    bb_finish_kernel<<<blocks, 32 * WARPS, 0, s>>>(st.at<int64_t>(oR4c), st.at<int64_t>(oRO), st.at<int32_t>(oFound), st.at<int32_t>(oNR),
-                                                   st.at<int32_t>(oNC), st.at<int64_t>(oFL), (int64_t)n, st.at<int32_t>(oAsg));
+    PDA_TRY(pda_murty_batch(io.at<double>(oC), io.at<int64_t>(oCO), io.at<int32_t>(oNR), io.at<int32_t>(oNC), (int64_t)n, maxR, maxC,
+                            1, PDA_CUT_NONE, 0.0, 1 /* maximize */, 0, io.at<int64_t>(oR4c), io.at<int64_t>(oRO), nullptr, nullptr,
+                            nullptr, io.at<int32_t>(oFound), PDA_WEIGHTS_NONE, nullptr, nullptr, nullptr,
+                            io.at<unsigned char>(oWs), wsBytes, s));
+    bb_finish_kernel<<<blocks, 32 * WARPS, 0, s>>>(io.at<int64_t>(oR4c), io.at<int64_t>(oRO), io.at<int32_t>(oFound), io.at<int32_t>(oNR),
+                                                   io.at<int32_t>(oNC), io.at<int64_t>(oFL), (int64_t)n, io.at<int32_t>(oAsg));
     PDA_CUDA_TRY(cudaGetLastError());
     return io.download();
 }

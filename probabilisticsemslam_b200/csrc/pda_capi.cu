@@ -57,6 +57,15 @@ uint64_t approx_seed() { return g_approxSeed.load(); }
 
 DeviceCtx g_dev[PDA_MAX_DEVICES];
 
+static std::mutex g_pinMu;
+static std::vector<std::pair<const unsigned char*, size_t> > g_pinRanges;  // pda_host_alloc's buffers
+bool in_portable_range(const void* p) {
+    std::lock_guard<std::mutex> lk(g_pinMu);
+    for (const auto& r : g_pinRanges)
+        if ((const unsigned char*)p >= r.first && (const unsigned char*)p < r.first + r.second) return true;
+    return false;
+}
+
 }  // namespace pda
 
 using namespace pda;
@@ -110,16 +119,6 @@ int pda_device_count(void) {
     return n;
 }
 
-// Page-locked buffers handed out by pda_host_alloc: allocated portable + mapped, so EVERY device may use them in place.
-static std::mutex g_pinMu;
-static std::vector<std::pair<const unsigned char*, size_t> > g_pinRanges;
-static bool in_portable_range(const void* p) {
-    std::lock_guard<std::mutex> lk(g_pinMu);
-    for (const auto& r : g_pinRanges)
-        if ((const unsigned char*)p >= r.first && (const unsigned char*)p < r.first + r.second) return true;
-    return false;
-}
-
 void* pda_host_alloc(int64_t bytes) {
     if (bytes <= 0) { fail(PDA_ERR_INVALID, "pda_host_alloc: bytes <= 0"); return nullptr; }
     void* p = nullptr;
@@ -137,18 +136,6 @@ void pda_host_free(void* p) {
             if (g_pinRanges[i].first == (const unsigned char*)p) { g_pinRanges.erase(g_pinRanges.begin() + (long)i); break; }
     }
     cudaFreeHost(p);
-}
-
-// If `p` is page-locked host memory that the device can address (cudaHostAlloc / cudaHostRegister under unified
-// addressing), returns the device-side alias, else NULL.
-static void* mapped_alias(const void* p, int device) {
-    if (!p) return nullptr;
-    cudaPointerAttributes at;
-    if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { (void)cudaGetLastError(); return nullptr; }
-    // page-locked by a context of THIS device, or handed out by pda_host_alloc (portable).  Memory pinned for another
-    // device's context by somebody else is only guaranteed to be addressable there: take the copying path for it.
-    if (at.type != cudaMemoryTypeHost) return nullptr;
-    return (at.device == device || in_portable_range(p)) ? at.devicePointer : nullptr;
 }
 
 // ---------------------------------------------------------------------------------------- Murty
@@ -283,20 +270,12 @@ static int murty_batch_host(const double* costs, const int64_t* costOff, const i
     int maxR = 0, maxC = 0;
     struct Range { size_t lo = ~(size_t)0, hi = 0; void add(size_t o, size_t n) { lo = std::min(lo, o); hi = std::max(hi, o + n); } size_t len() const { return hi > lo ? hi - lo : 0; } };
     Range rCost, rR4c, rC4r, rProb;
-    bool contiguous = true;  // problem p+1 starts at or after the end of problem p in every array: chunks are ranges
     for (int64_t p = 0; p < nProblems; ++p) {
         const int r = numRow[p], c = numCol[p];
         if (r < 1 || c < 1 || c > r) return fail(PDA_ERR_INVALID, "murty: problem %lld is %d x %d (need numRow >= numCol >= 1)", (long long)p, r, c);
         if (costOff[p] < 0 || (row4colBest && r4cOff[p] < 0) || (col4rowBest && c4rOff[p] < 0) || (weightMode && probOff[p] < 0))
             return fail(PDA_ERR_INVALID, "murty: negative offset at problem %lld", (long long)p);
         maxR = std::max(maxR, r); maxC = std::max(maxC, c);
-        if (p > 0) {
-            const int pr = numRow[p - 1], pc = numCol[p - 1];
-            if (costOff[p] < costOff[p - 1] + (int64_t)pr * pc) contiguous = false;
-            if (row4colBest && r4cOff[p] < r4cOff[p - 1] + (int64_t)k * pc) contiguous = false;
-            if (col4rowBest && c4rOff[p] < c4rOff[p - 1] + (int64_t)k * pr) contiguous = false;
-            if (weightMode && probOff[p] < probOff[p - 1] + (int64_t)S * pc * (nL[p - 1] + 1)) contiguous = false;
-        }
         rCost.add((size_t)costOff[p], (size_t)r * c);
         if (row4colBest) rR4c.add((size_t)r4cOff[p], (size_t)k * c);
         if (col4rowBest) rC4r.add((size_t)c4rOff[p], (size_t)k * r);
@@ -309,118 +288,33 @@ static int murty_batch_host(const double* costs, const int64_t* costOff, const i
     const size_t loCost = rCost.lo, loR4c = nR4c ? rR4c.lo : 0, loC4r = nC4r ? rC4r.lo : 0, loProb = nProb ? rProb.lo : 0;
     DeviceScope scope;
     PDA_TRY(scope.enter(device));
-    int64_t wsBytes = pda_murty_workspace_bytes(nProblems, k, maxR, maxC);
+    const int64_t wsBytes = pda_murty_workspace_bytes(nProblems, k, maxR, maxC);
     if (wsBytes < 0) return (int)wsBytes;
     const size_t n = (size_t)nProblems;
-    {
-        Stage st(device);
-        HostIO io(st);
-        const size_t oCost = io.in(costs + loCost, nCost * 8), oCostOff = io.in(costOff, n * 8), oNR = io.in(numRow, n * 4), oNC = io.in(numCol, n * 4);
-        const size_t oR4cOff = io.in(row4colBest ? r4cOff : nullptr, n * 8), oC4rOff = io.in(col4rowBest ? c4rOff : nullptr, n * 8);
-        const size_t oProbOff = io.in(weightMode ? probOff : nullptr, n * 8), oNL = io.in(weightMode ? nL : nullptr, n * 4);
-        const size_t oFound = io.out(nFound, n * 4 * S), oGain = io.out(gainBest, gainBest ? n * (size_t)k * 8 : 0);
-        const size_t oProb = io.out(weightMode ? probs + loProb : nullptr, nProb * 8);
-        const size_t oR4c = io.out(row4colBest ? row4colBest + loR4c : nullptr, nR4c * 8), oC4r = io.out(col4rowBest ? col4rowBest + loC4r : nullptr, nC4r * 8);
-        if (io.packed()) {  // small call: one pinned copy each way
-            const size_t oWs = st.reserve((size_t)wsBytes);
-            PDA_TRY(io.commit());
-            PDA_TRY(io.upload());
-            PDA_TRY(murty_batch_dev(st.at<double>(oCost) - loCost, st.at<int64_t>(oCostOff), st.at<int32_t>(oNR), st.at<int32_t>(oNC), nProblems,
-                                    maxR, maxC, k, cutMode, cutoff, maximize, cutMaximize,
-                                    row4colBest ? st.at<int64_t>(oR4c) - loR4c : nullptr, st.at<int64_t>(oR4cOff),
-                                    col4rowBest ? st.at<int64_t>(oC4r) - loC4r : nullptr, st.at<int64_t>(oC4rOff),
-                                    gainBest ? st.at<double>(oGain) : nullptr, st.at<int32_t>(oFound),
-                                    weightMode, weightMode ? st.at<double>(oProb) - loProb : nullptr, st.at<int64_t>(oProbOff),
-                                    st.at<int32_t>(oNL), st.at<unsigned char>(oWs), wsBytes, io.stream(), ladder));
-            return io.download();
-        }
-    }
-    // Page-locked caller buffers are used in place: a warp reads its 2.4 KB cost matrix over PCIe once when it takes
-    // the problem and writes the weight table when it is done, so both transfers hide under ~1.6 ms of computing per
-    // problem instead of standing in front of and behind the kernel (161 MB in + 136 MB out per 100 000 problems).
-    double* const costsDev = static_cast<double*>(mapped_alias(costs, device));
-    double* const probsDev = weightMode ? static_cast<double*>(mapped_alias(probs, device)) : nullptr;
-    Stage st(device);
-    const size_t oCost = st.reserve(costsDev ? 0 : nCost * 8), oCostOff = st.reserve(n * 8), oNR = st.reserve(n * 4), oNC = st.reserve(n * 4);
-    const size_t oR4c = st.reserve(nR4c * 8), oR4cOff = st.reserve(n * 8), oC4r = st.reserve(nC4r * 8), oC4rOff = st.reserve(n * 8);
-    const size_t oGain = st.reserve(gainBest ? n * k * 8 : 0), oFound = st.reserve(n * 4 * S);
-    const size_t oProb = st.reserve(probsDev ? 0 : nProb * 8), oProbOff = st.reserve(n * 8), oNL = st.reserve(n * 4);
-    const size_t oWs = st.reserve((size_t)wsBytes);
-    PDA_TRY(st.commit());
+    // The cost matrices and the weight tables may be used in place (beyond the packed limit, from page-locked memory): a
+    // warp reads its 2.4 KB cost matrix over PCIe once when it takes the problem and writes the weight table when it is
+    // done, so both transfers hide under ~1.6 ms of computing per problem instead of standing in front of and behind the
+    // kernel (161 MB in + 136 MB out per 100 000 problems).
+    HostIO io(device);
+    const size_t oCost = io.in(costs + loCost, nCost * 8, HostIO::IN_PLACE), oCostOff = io.in(costOff, n * 8);
+    const size_t oNR = io.in(numRow, n * 4), oNC = io.in(numCol, n * 4);
+    const size_t oR4cOff = io.in(row4colBest ? r4cOff : nullptr, n * 8), oC4rOff = io.in(col4rowBest ? c4rOff : nullptr, n * 8);
+    const size_t oProbOff = io.in(weightMode ? probOff : nullptr, n * 8), oNL = io.in(weightMode ? nL : nullptr, n * 4);
+    const size_t oFound = io.out(nFound, n * 4 * S), oGain = io.out(gainBest, gainBest ? n * (size_t)k * 8 : 0);
+    const size_t oProb = io.out(weightMode ? probs + loProb : nullptr, nProb * 8, HostIO::IN_PLACE);
+    const size_t oR4c = io.out(row4colBest ? row4colBest + loR4c : nullptr, nR4c * 8), oC4r = io.out(col4rowBest ? col4rowBest + loC4r : nullptr, nC4r * 8);
+    const size_t oWs = io.scratch((size_t)wsBytes);
+    PDA_TRY(io.commit());
+    PDA_TRY(io.upload());
     // device-side bases such that base + offset[p] lands inside the staged range
-    double* const dCost = costsDev ? costsDev : st.at<double>(oCost) - loCost;
-    int64_t* const dR4c = row4colBest ? st.at<int64_t>(oR4c) - loR4c : nullptr;
-    int64_t* const dC4r = col4rowBest ? st.at<int64_t>(oC4r) - loC4r : nullptr;
-    double* const dProb = weightMode ? (probsDev ? probsDev : st.at<double>(oProb) - loProb) : nullptr;
-
-    // Large batches are cut into chunks that flow through three streams (copy in / run / copy out), so the PCIe
-    // transfers of one chunk overlap the kernel of another.  That needs the problems to lie one after the other in
-    // every array (then a chunk's inputs and outputs are contiguous ranges); otherwise, and for small batches, one chunk.
-    // A chunk must stay large (>= 64k problems, ~18 per resident warp): every launch ends with a tail in which the
-    // persistent warps run dry one by one, and at 12.5k problems per chunk that cost more than the overlap gained
-    // (measured: 100k problems in 8 chunks, e2e 1.70 M/s vs 1.92 M/s unchunked).
-    const size_t nChunks = contiguous ? std::max<size_t>(1, std::min<size_t>(8, n / 65536)) : 1;
-    HostStreams* hs = nullptr;
-    PDA_TRY(host_streams(device, &hs));
-    cudaStream_t sIn = hs->in, sRun = hs->run, sOut = hs->out;
-    std::vector<cudaEvent_t> evIn(nChunks), evRun(nChunks);
-    for (size_t c = 0; c < nChunks; ++c) {
-        PDA_CUDA_TRY(cudaEventCreateWithFlags(&evIn[c], cudaEventDisableTiming));
-        PDA_CUDA_TRY(cudaEventCreateWithFlags(&evRun[c], cudaEventDisableTiming));
-    }
-    int rc = PDA_OK;
-    auto body = [&]() -> int {
-        PDA_TRY(h2d(st.at<int64_t>(oCostOff), costOff, n, sIn));
-        PDA_TRY(h2d(st.at<int32_t>(oNR), numRow, n, sIn));
-        PDA_TRY(h2d(st.at<int32_t>(oNC), numCol, n, sIn));
-        if (row4colBest) PDA_TRY(h2d(st.at<int64_t>(oR4cOff), r4cOff, n, sIn));
-        if (col4rowBest) PDA_TRY(h2d(st.at<int64_t>(oC4rOff), c4rOff, n, sIn));
-        if (weightMode) {
-            PDA_TRY(h2d(st.at<int64_t>(oProbOff), probOff, n, sIn));
-            PDA_TRY(h2d(st.at<int32_t>(oNL), nL, n, sIn));
-        }
-        for (size_t c = 0; c < nChunks; ++c) {
-            const size_t p0 = n * c / nChunks, p1 = n * (c + 1) / nChunks, m = p1 - p0;
-            const bool last = (p1 == n);
-            // copy in: this chunk's cost matrices
-            const size_t c0 = nChunks == 1 ? rCost.lo : (size_t)costOff[p0], c1 = (nChunks == 1 || last) ? rCost.hi : (size_t)costOff[p1];
-            if (!costsDev) PDA_TRY(h2d(dCost + c0, costs + c0, c1 - c0, sIn));
-            PDA_CUDA_TRY(cudaEventRecord(evIn[c], sIn));
-            // run
-            PDA_CUDA_TRY(cudaStreamWaitEvent(sRun, evIn[c], 0));
-            PDA_TRY(murty_batch_dev(dCost, st.at<int64_t>(oCostOff) + p0, st.at<int32_t>(oNR) + p0,
-                                    st.at<int32_t>(oNC) + p0, (int64_t)m, maxR, maxC, k, cutMode, cutoff, maximize, cutMaximize,
-                                    dR4c, st.at<int64_t>(oR4cOff) + p0, dC4r, st.at<int64_t>(oC4rOff) + p0,
-                                    gainBest ? st.at<double>(oGain) + p0 * (size_t)k : nullptr, st.at<int32_t>(oFound) + p0 * S,
-                                    weightMode, dProb, st.at<int64_t>(oProbOff) + p0, st.at<int32_t>(oNL) + p0,
-                                    st.at<unsigned char>(oWs), wsBytes, sRun, ladder));
-            PDA_CUDA_TRY(cudaEventRecord(evRun[c], sRun));
-            // copy out: this chunk's results
-            PDA_CUDA_TRY(cudaStreamWaitEvent(sOut, evRun[c], 0));
-            if (row4colBest) {
-                const size_t a0 = nChunks == 1 ? rR4c.lo : (size_t)r4cOff[p0], a1 = (nChunks == 1 || last) ? rR4c.hi : (size_t)r4cOff[p1];
-                PDA_TRY(d2h(row4colBest + a0, dR4c + a0, a1 - a0, sOut));
-            }
-            if (col4rowBest) {
-                const size_t a0 = nChunks == 1 ? rC4r.lo : (size_t)c4rOff[p0], a1 = (nChunks == 1 || last) ? rC4r.hi : (size_t)c4rOff[p1];
-                PDA_TRY(d2h(col4rowBest + a0, dC4r + a0, a1 - a0, sOut));
-            }
-            if (gainBest) PDA_TRY(d2h(gainBest + p0 * (size_t)k, st.at<double>(oGain) + p0 * (size_t)k, m * (size_t)k, sOut));
-            PDA_TRY(d2h(nFound + p0 * S, st.at<int32_t>(oFound) + p0 * S, m * S, sOut));
-            if (weightMode && !probsDev) {
-                const size_t a0 = nChunks == 1 ? rProb.lo : (size_t)probOff[p0], a1 = (nChunks == 1 || last) ? rProb.hi : (size_t)probOff[p1];
-                PDA_TRY(d2h(probs + a0, dProb + a0, a1 - a0, sOut));
-            }
-        }
-        PDA_CUDA_TRY(cudaStreamSynchronize(sOut));
-        PDA_CUDA_TRY(cudaStreamSynchronize(sRun));
-        PDA_CUDA_TRY(cudaStreamSynchronize(sIn));
-        return PDA_OK;
-    };
-    rc = body();
-    if (rc != PDA_OK) { cudaStreamSynchronize(sIn); cudaStreamSynchronize(sRun); cudaStreamSynchronize(sOut); (void)cudaGetLastError(); }
-    for (size_t c = 0; c < nChunks; ++c) { cudaEventDestroy(evIn[c]); cudaEventDestroy(evRun[c]); }
-    return rc;
+    PDA_TRY(murty_batch_dev(io.at<double>(oCost) - loCost, io.at<int64_t>(oCostOff), io.at<int32_t>(oNR), io.at<int32_t>(oNC), nProblems,
+                            maxR, maxC, k, cutMode, cutoff, maximize, cutMaximize,
+                            row4colBest ? io.at<int64_t>(oR4c) - loR4c : nullptr, io.at<int64_t>(oR4cOff),
+                            col4rowBest ? io.at<int64_t>(oC4r) - loC4r : nullptr, io.at<int64_t>(oC4rOff),
+                            gainBest ? io.at<double>(oGain) : nullptr, io.at<int32_t>(oFound),
+                            weightMode, weightMode ? io.at<double>(oProb) - loProb : nullptr, io.at<int64_t>(oProbOff),
+                            io.at<int32_t>(oNL), io.at<unsigned char>(oWs), wsBytes, io.stream(), ladder));
+    return io.download();
 }
 
 // ks (host) -> the ladder: rungs = the sorted distinct ks, slot j -> the rung equal to ks[j]
@@ -548,19 +442,18 @@ int pda_lap_batch_host(const double* costs, const int64_t* costOff, const int32_
     DeviceScope scope;
     PDA_TRY(scope.enter(device));
     const size_t n = (size_t)nProblems;
-    Stage st(device);
-    HostIO io(st);
+    HostIO io(device);
     const size_t oCost = io.in(costs, nCost * 8), oCostOff = io.in(costOff, n * 8), oNR = io.in(numRow, n * 4), oNC = io.in(numCol, n * 4);
     const size_t oNG = io.in(numCol4Gain, n * 4), oRO = io.in(rowOff, n * 8), oCO = io.in(colOff, n * 8);
     const size_t oC4r = io.out(col4row, nRows * 8), oR4c = io.out(row4col, nCols * 8), oU = io.out(u, nCols * 8), oV = io.out(v, nRows * 8);
     const size_t oF = io.out(forbidden, nRows), oG = io.out(gain, n * 8), oFe = io.out(feasible, n * 4);
     PDA_TRY(io.commit());
     PDA_TRY(io.upload());
-    PDA_TRY(pda_lap_batch(st.at<double>(oCost), st.at<int64_t>(oCostOff), st.at<int32_t>(oNR), st.at<int32_t>(oNC),
-                          numCol4Gain ? st.at<int32_t>(oNG) : nullptr, nProblems, maxR, maxC, makeSafe, maximize,
-                          st.at<int64_t>(oRO), st.at<int64_t>(oCO), st.at<int64_t>(oC4r), st.at<int64_t>(oR4c),
-                          st.at<double>(oU), st.at<double>(oV), st.at<uint8_t>(oF), st.at<double>(oG),
-                          st.at<int32_t>(oFe), io.stream()));
+    PDA_TRY(pda_lap_batch(io.at<double>(oCost), io.at<int64_t>(oCostOff), io.at<int32_t>(oNR), io.at<int32_t>(oNC),
+                          numCol4Gain ? io.at<int32_t>(oNG) : nullptr, nProblems, maxR, maxC, makeSafe, maximize,
+                          io.at<int64_t>(oRO), io.at<int64_t>(oCO), io.at<int64_t>(oC4r), io.at<int64_t>(oR4c),
+                          io.at<double>(oU), io.at<double>(oV), io.at<uint8_t>(oF), io.at<double>(oG),
+                          io.at<int32_t>(oFe), io.stream()));
     return io.download();
 }
 

@@ -214,14 +214,13 @@ int pda_permanent_approx_batch_host(const double* mats, const int64_t* matOff, c
     DeviceScope scope;
     PDA_TRY(scope.enter(device));
     const size_t n = (size_t)nMats;
-    Stage st(device);
-    HostIO io(st);
+    HostIO io(device);
     const size_t oM = io.in(mats, nEl * 8), oOff = io.in(matOff, n * 8), oR = io.in(rows, n * 4), oC = io.in(cols, n * 4);
     const size_t oOut = io.out(out, n * 8), oSt = io.out(status, n * 4);
     PDA_TRY(io.commit());
     PDA_TRY(io.upload());
-    PDA_TRY(launch_permanent_approx_batch(st.at<double>(oM), st.at<int64_t>(oOff), st.at<int32_t>(oR), st.at<int32_t>(oC), nMats,
-                                          iterations, seed, st.at<double>(oOut), st.at<int32_t>(oSt), io.stream()));
+    PDA_TRY(launch_permanent_approx_batch(io.at<double>(oM), io.at<int64_t>(oOff), io.at<int32_t>(oR), io.at<int32_t>(oC), nMats,
+                                          iterations, seed, io.at<double>(oOut), io.at<int32_t>(oSt), io.stream()));
     return io.download();
 }
 

@@ -372,10 +372,9 @@ int pda_permanent_batch_host(const double* mats, const int64_t* matOff, const in
     PDA_TRY(current_device_info(&dev));
     const size_t n = (size_t)nMats;
     const size_t wsBytes = (size_t)pda_permanent_workspace_bytes(nMats);
-    Stage st(device);
-    HostIO io(st);
+    HostIO io(device);
     const size_t oM = io.in(mats + loEl, (nEl - loEl) * 8), oOff = io.in(matOff, n * 8), oR = io.in(rows, n * 4), oC = io.in(cols, n * 4);
-    const size_t oOut = io.out(out, n * 8), oSt = io.out(status, n * 4), oWs = st.reserve(wsBytes);
+    const size_t oOut = io.out(out, n * 8), oSt = io.out(status, n * 4), oWs = io.scratch(wsBytes);
     PDA_TRY(io.commit());
     PDA_TRY(io.upload());
     int maxSmall = 0, minSmall = PDA_MAX_DIM;
@@ -383,8 +382,8 @@ int pda_permanent_batch_host(const double* mats, const int64_t* matOff, const in
         const int sm = std::min(rows[i], cols[i]);
         maxSmall = std::max(maxSmall, sm); minSmall = std::min(minSmall, sm);
     }
-    PDA_TRY(launch_permanent_batch(st.at<double>(oM) - loEl, st.at<int64_t>(oOff), st.at<int32_t>(oR), st.at<int32_t>(oC), nMats,
-                                   maxDim, st.at<double>(oOut), st.at<int32_t>(oSt), st.at<unsigned char>(oWs),
+    PDA_TRY(launch_permanent_batch(io.at<double>(oM) - loEl, io.at<int64_t>(oOff), io.at<int32_t>(oR), io.at<int32_t>(oC), nMats,
+                                   maxDim, io.at<double>(oOut), io.at<int32_t>(oSt), io.at<unsigned char>(oWs),
                                    (int64_t)wsBytes, io.stream(), maxSmall, minSmall));
     return io.download();
 }
@@ -409,12 +408,11 @@ int pda_permanent_range_host(const double* A, int32_t n, uint64_t begin, uint64_
     DeviceInfo dev;
     PDA_TRY(current_device_info(&dev));
     const size_t wsBytes = 64 + (size_t)16 * 8192;
-    Stage st(device);
-    HostIO io(st);
-    const size_t oA = io.in(A, (size_t)n * n * 8), oP = io.out(partial, 16), oWs = st.reserve(wsBytes);
+    HostIO io(device);
+    const size_t oA = io.in(A, (size_t)n * n * 8), oP = io.out(partial, 16), oWs = io.scratch(wsBytes);
     PDA_TRY(io.commit());
     PDA_TRY(io.upload());
-    PDA_TRY(pda_permanent_range(st.at<double>(oA), n, begin, end, st.at<double>(oP), st.at<unsigned char>(oWs), (int64_t)wsBytes,
+    PDA_TRY(pda_permanent_range(io.at<double>(oA), n, begin, end, io.at<double>(oP), io.at<unsigned char>(oWs), (int64_t)wsBytes,
                                 io.stream()));
     return io.download();
 }

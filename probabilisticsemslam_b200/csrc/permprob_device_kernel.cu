@@ -675,14 +675,13 @@ int pda_conditioned_permanent_batch_host(const double* mats, const int64_t* matO
     DeviceInfo dev;
     PDA_TRY(current_device_info(&dev));
     const size_t wsBytes = carve(nullptr, 1, nMats, 0, nMats, maxDim, maxDim, permOpt, dev.smCount).bytes;
-    Stage st(device);
-    HostIO io(st);
+    HostIO io(device);
     const size_t oA = io.in(mats, nEl * 8), oOff = io.in(matOff, n * 8), oR = io.in(r.data(), n * 4), oC = io.in(c.data(), n * 4);
-    const size_t oOut = io.out(out, n * 8), oSt = io.out(status, n * 4), oWs = st.reserve(wsBytes);
+    const size_t oOut = io.out(out, n * 8), oSt = io.out(status, n * 4), oWs = io.scratch(wsBytes);
     PDA_TRY(io.commit());
     PDA_TRY(io.upload());
-    PDA_TRY(pda_conditioned_permanent_batch(st.at<double>(oA), st.at<int64_t>(oOff), st.at<int32_t>(oR), st.at<int32_t>(oC), nMats,
-                                            maxDim, permOpt, st.at<double>(oOut), st.at<int32_t>(oSt), st.at<unsigned char>(oWs),
+    PDA_TRY(pda_conditioned_permanent_batch(io.at<double>(oA), io.at<int64_t>(oOff), io.at<int32_t>(oR), io.at<int32_t>(oC), nMats,
+                                            maxDim, permOpt, io.at<double>(oOut), io.at<int32_t>(oSt), io.at<unsigned char>(oWs),
                                             (int64_t)wsBytes, io.stream()));
     PDA_TRY(io.download());
     for (size_t i = 0; i < n; ++i)
@@ -730,19 +729,18 @@ int pda_permanent_prob_batch_host(const double* costs, const int64_t* costOff, c
         const size_t n = (size_t)(p1 - p0);
         // the capacity is the chunk's item count: callers may leave gaps between their tables
         const size_t wsBytes = carve(nullptr, 0, (int64_t)n, (int64_t)nCost, items, maxRow, maxCol, permOpt, dev.smCount).bytes;
-        Stage st(device);
-        HostIO io(st);
+        HostIO io(device);
         const size_t oP = io.in(costs + c0, nCost * 8), oOff = io.in(locCostOff.data(), n * 8), oL = io.in(nL + p0, n * 4);
         const size_t oM = io.in(nM + p0, n * 4), oProbOff = io.in(locProbOff.data(), n * 8);
-        const size_t oStatus = io.out(status + p0, n * 4), oProbs = io.out(probs + pr0, nProb * 8), oWs = st.reserve(wsBytes);
+        const size_t oStatus = io.out(status + p0, n * 4), oProbs = io.out(probs + pr0, nProb * 8), oWs = io.scratch(wsBytes);
         PDA_TRY(io.commit());
         const cudaStream_t s = io.stream();
         PDA_TRY(io.upload());
         // the whole staged range goes back: gaps between the caller's tables come back as zeros
-        PDA_CUDA_TRY(cudaMemsetAsync(st.at<double>(oProbs), 0, nProb * 8, s));
-        PDA_TRY(pda_permanent_prob_batch(st.at<double>(oP), st.at<int64_t>(oOff), st.at<int32_t>(oL), st.at<int32_t>(oM), (int64_t)n,
-                                         (int64_t)nCost, items, maxRow, maxCol, permOpt, st.at<double>(oProbs),
-                                         st.at<int64_t>(oProbOff), st.at<int32_t>(oStatus), st.at<unsigned char>(oWs),
+        PDA_CUDA_TRY(cudaMemsetAsync(io.at<double>(oProbs), 0, nProb * 8, s));
+        PDA_TRY(pda_permanent_prob_batch(io.at<double>(oP), io.at<int64_t>(oOff), io.at<int32_t>(oL), io.at<int32_t>(oM), (int64_t)n,
+                                         (int64_t)nCost, items, maxRow, maxCol, permOpt, io.at<double>(oProbs),
+                                         io.at<int64_t>(oProbOff), io.at<int32_t>(oStatus), io.at<unsigned char>(oWs),
                                          (int64_t)wsBytes, s));
         PDA_TRY(io.download());
         p0 = p1;

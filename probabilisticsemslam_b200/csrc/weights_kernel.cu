@@ -161,16 +161,15 @@ int pda_condition_costs_batch_host(const double* costs, const int64_t* costOff, 
     DeviceScope scope;
     PDA_TRY(scope.enter(device));
     const size_t n = (size_t)nProblems;
-    Stage st(device);
-    HostIO io(st);
+    HostIO io(device);
     const size_t oC = io.in(costs, nCost * 8), oCO = io.in(costOff, n * 8), oNR = io.in(numRow, n * 4), oNC = io.in(numCol, n * 4);
     const size_t oRO = io.in(rowOff, n * 8);
     const size_t oOut = io.out(outCosts, nCost * 8), oIdx = io.out(rowIdx, nRows * 8), oG = io.out(goodRows, n * 4);
     PDA_TRY(io.commit());
     PDA_TRY(io.upload());
-    PDA_TRY(launch_condition_costs(st.at<double>(oC), st.at<int64_t>(oCO), st.at<int32_t>(oNR), st.at<int32_t>(oNC),
-                                   nProblems, st.at<int64_t>(oRO), st.at<double>(oOut), st.at<int64_t>(oIdx),
-                                   st.at<int32_t>(oG), io.stream()));
+    PDA_TRY(launch_condition_costs(io.at<double>(oC), io.at<int64_t>(oCO), io.at<int32_t>(oNR), io.at<int32_t>(oNC),
+                                   nProblems, io.at<int64_t>(oRO), io.at<double>(oOut), io.at<int64_t>(oIdx),
+                                   io.at<int32_t>(oG), io.stream()));
     return io.download();
 }
 
@@ -190,12 +189,11 @@ int pda_to_probs_batch_host(double* values, const int64_t* off, const int64_t* l
     DeviceScope scope;
     PDA_TRY(scope.enter(device));
     const size_t n = (size_t)nVectors;
-    Stage st(device);
-    HostIO io(st);
+    HostIO io(device);
     const size_t oO = io.in(off, n * 8), oL = io.in(len, n * 8), oV = io.inout(values, total * 8);
     PDA_TRY(io.commit());
     PDA_TRY(io.upload());
-    PDA_TRY(launch_to_probs(st.at<double>(oV), st.at<int64_t>(oO), st.at<int64_t>(oL), nVectors, io.stream()));
+    PDA_TRY(launch_to_probs(io.at<double>(oV), io.at<int64_t>(oO), io.at<int64_t>(oL), nVectors, io.stream()));
     return io.download();
 }
 

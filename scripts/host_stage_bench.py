@@ -1,15 +1,19 @@
-"""Times the single-device *_host entries at a batch of one and at about 50 MB of inputs + outputs, for one or more
-builds of libpda_b200.so, and states whether every build returned the same bytes.
+"""Times the single-device *_host entries at a batch of one and at about 50 MB of inputs + outputs, and
+pda_murty_batch_host at 140 000 and 262 144 problems (pageable and page-locked at k = 200, page-locked with every k-best
+list returned at k = 20), for one or more builds of libpda_b200.so, and states whether every build returned the same
+bytes.
 
     python scripts/host_stage_bench.py --libs OLD.so NEW.so [--rounds 3] [--out results.json]
 
 Each build runs in its own process (PDA_B200_LIB), and the builds take turns, round after round, so that drift on a
 shared machine falls on all of them.  A time is the median host-clock time of one call, which ends in a device
-synchronise; the output digest is a SHA-256 over every output array of the last call.
+synchronise; the output digest is a SHA-256 over every output array of the last call (of a k-best list, over the
+nFound hypotheses the call defines).
 """
 from __future__ import annotations
 
 import argparse
+import ctypes
 import hashlib
 import json
 import os
@@ -134,23 +138,76 @@ def cases(lib, big):
     return out
 
 
+def kbest_cases(lib, n, allocs):
+    """pda_murty_batch_host on n G1 problems: pageable and page-locked (pda_host_alloc) at k = 200, and page-locked with
+    every k-best list returned at k = 20.  Page-locked buffers are appended to `allocs`."""
+    from probabilisticsemslam_b200 import api, synth
+    pk = synth.g1_dense(n, first=50)
+    nr, nc, nl = pk.num_row, pk.nM.astype(np.int32), pk.nL.astype(np.int32)
+    cells = nc.astype(np.int64) * (nl + 1)
+    poff = _prefix(cells)
+
+    def pinned(a):
+        p = lib.pda_host_alloc(max(a.nbytes, 8))
+        assert p, "pda_host_alloc failed"
+        allocs.append(p)
+        v = np.ctypeslib.as_array((ctypes.c_uint8 * a.nbytes).from_address(p)).view(a.dtype)
+        v[:] = a
+        return v
+
+    def call(costs, found, probs, k, r4c=None, r4o=None, c4r=None, c4o=None, gain=None):
+        return lambda: lib.pda_murty_batch_host(_p(costs), _p(pk.cost_off), _p(nr), _p(nc), n, k, api.CUT_RELATIVE, 42.0, 0, 0,
+                                                _p(r4c), _p(r4o), _p(c4r), _p(c4o), _p(gain), _p(found), api.WEIGHTS_GATED,
+                                                _p(probs), _p(poff), _p(nl), 0)
+    ins = [pk.costs, pk.cost_off, nr, nc, nl, poff]
+    mb = lambda arrays: sum(a.nbytes for a in arrays)
+    found, probs = np.zeros(n, np.int32), np.zeros(int(cells.sum()))
+    out = {f"murty_k200_pageable/{n}": (call(pk.costs, found, probs, 200), [found, probs], mb(ins + [found, probs]))}
+    pc, pf, pp = pinned(pk.costs), pinned(found), pinned(probs)
+    out[f"murty_k200_pinned/{n}"] = (call(pc, pf, pp, 200), [pf, pp], mb(ins + [pf, pp]))
+    k = 20
+    r4o, c4o = _prefix(nc.astype(np.int64) * k), _prefix(nr.astype(np.int64) * k)
+    lf, lp = pinned(found), pinned(probs)
+    r4c, c4r, gain = pinned(np.zeros(int(nc.sum()) * k, np.int64)), pinned(np.zeros(int(nr.sum()) * k, np.int64)), pinned(np.zeros(n * k))
+
+    def defined():  # only the first nFound hypotheses of a problem are defined
+        f = lf.astype(np.int64)
+        lists = [gain[(np.arange(k)[None, :] < f[:, None]).reshape(-1)]]
+        lists += [r4c[o:o + x * c] for o, x, c in zip(r4o, f, nc)] + [c4r[o:o + x * r] for o, x, r in zip(c4o, f, nr)]
+        return [lf, lp] + lists
+    out[f"murty_k20_lists_pinned/{n}"] = (call(pc, lf, lp, k, r4c, r4o, c4r, c4o, gain), defined,
+                                          mb(ins + [r4o, c4o, lf, lp, r4c, c4r, gain]))
+    return out
+
+
 def worker(reps_small, reps_big):
     from probabilisticsemslam_b200 import _lib
     lib = _lib.lib()
     res = {}
+
+    def run(key, call, outs, nbytes, reps):
+        times = []
+        for i in range(2 + reps):
+            t0 = time.perf_counter()
+            _lib.check(call())
+            if i >= 2:
+                times.append(time.perf_counter() - t0)
+        h = hashlib.sha256()
+        for a in (outs() if callable(outs) else outs):
+            h.update(np.ascontiguousarray(a).tobytes())
+        res[key] = dict(ms=float(np.median(times)) * 1e3, mb=nbytes / 2**20, digest=h.hexdigest()[:16])
+
     for big in (False, True):
-        for name, (call, outs, nbytes) in cases(lib, big).items():
-            times = []
-            for i in range(2 + (reps_big if big else reps_small)):
-                t0 = time.perf_counter()
-                _lib.check(call())
-                if i >= 2:
-                    times.append(time.perf_counter() - t0)
-            h = hashlib.sha256()
-            for a in outs:
-                h.update(np.ascontiguousarray(a).tobytes())
-            res[f"{name}/{'50MB' if big else 'one'}"] = dict(ms=float(np.median(times)) * 1e3, mb=nbytes / 2**20,
-                                                             digest=h.hexdigest()[:16])
+        for name, case in cases(lib, big).items():
+            run(f"{name}/{'50MB' if big else 'one'}", *case, reps_big if big else reps_small)
+    for n in (140_000, 262_144):
+        allocs = []
+        try:
+            for name, case in kbest_cases(lib, n, allocs).items():
+                run(name, *case, reps_big)
+        finally:
+            for p in allocs:
+                lib.pda_host_free(p)
     print(json.dumps(res))
 
 

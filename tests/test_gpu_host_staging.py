@@ -1,8 +1,10 @@
 """Both transports of the single-device *_host entries (HostIO, pda_host_stage.h): a call whose declared arrays total at
 most PDA_PACKED_LIMIT (8 MB) moves them with one pinned copy each way, a larger one copies each array straight from and
-to the caller's memory.  Every entry runs once on each side of that limit, and its results -- statuses and counts
-included -- must be bit-identical to its device-pointer form run on the same inputs from CUDA tensors (asgnBB, which
-has no device-pointer form, against the CPU oracle)."""
+to the caller's memory -- except, for the k-best entries, cost matrices and weight tables in page-locked memory this
+device can address, which the kernel uses in place.  Every entry runs once on each side of that limit (the k-best ones
+with pageable, torch-pinned and pda_host_alloc buffers), and its results -- statuses and counts included -- must be
+bit-identical to its device-pointer form run on the same inputs from CUDA tensors (asgnBB, which has no device-pointer
+form, against the CPU oracle)."""
 from __future__ import annotations
 
 import numpy as np
@@ -356,6 +358,129 @@ def test_permanent_prob_with_gaps(gpu_api, large):
     for o, c in zip(prob_off, cells):
         gaps[o:o + c] = False
     assert gaps.sum() == 3 * (n - 1) and np.all(probs[gaps] == 0.0)
+
+
+# ---- k-best enumeration (pda_murty_batch_host, pda_assignment_prob_ladder_batch_host) --------------------------------------
+class _HostMemory:
+    """Copies of host arrays in one kind of memory: pageable numpy, torch.pin_memory() (page-locked by this device's
+    context) or pda_host_alloc (portable).  Beyond the limit the k-best entries use the last two in place."""
+
+    def __init__(self, kind):
+        self.kind, self.held, self.allocs = kind, [], []
+
+    def __call__(self, a):
+        import ctypes
+        import torch
+        a = np.ascontiguousarray(a)
+        if self.kind == "pageable":
+            return a.copy()
+        if self.kind == "torch_pinned":
+            t = torch.from_numpy(a.copy()).pin_memory()
+            self.held.append(t)
+            return t.numpy()
+        p = _lib().lib().pda_host_alloc(max(a.nbytes, 8))
+        assert p
+        self.allocs.append(p)
+        v = np.ctypeslib.as_array((ctypes.c_uint8 * a.nbytes).from_address(p)).view(a.dtype)
+        v[:] = a
+        return v
+
+    def free(self):
+        for p in self.allocs:
+            _lib().lib().pda_host_free(p)
+
+
+KINDS = ["pageable", "torch_pinned", "host_alloc"]
+
+
+def _kbest_inputs(large):
+    pb = _problems(large, 700)
+    nr, nc, nL = pb.num_row, pb.nM.astype(np.int32), pb.nL.astype(np.int32)
+    return pb, nr, nc, nL, nc.astype(np.int64) * (nL + 1)
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("kind", KINDS)
+@pytest.mark.parametrize("large", SIDES)
+def test_murty_lists_and_weights(gpu_api, large, kind):
+    import torch
+    from probabilisticsemslam_b200 import api
+    k = 5
+    pb, nr, nc, nL, cells = _kbest_inputs(large)
+    n = len(pb)
+    r4o, c4o, poff = _prefix(nc.astype(np.int64) * k), _prefix(nr.astype(np.int64) * k), _prefix(cells)
+    lib = _lib().lib()
+    mem = _HostMemory(kind)
+    try:
+        costs, off, hnr, hnc, hnl, hr4o, hc4o, hpoff = [mem(a) for a in (pb.costs, pb.cost_off, nr, nc, nL, r4o, c4o, poff)]
+        r4c, c4r = mem(np.full(int(nc.sum()) * k, -7, np.int64)), mem(np.full(int(nr.sum()) * k, -7, np.int64))
+        gain, found, probs = mem(np.zeros(n * k)), mem(np.full(n, -7, np.int32)), mem(np.full(int(cells.sum()), 7.5))
+        _side([costs, off, hnr, hnc, hnl, hr4o, hc4o, hpoff, r4c, c4r, gain, found, probs], large)
+        _call(lib.pda_murty_batch_host(costs.ctypes.data, off.ctypes.data, hnr.ctypes.data, hnc.ctypes.data, n, k,
+                                       api.CUT_RELATIVE, 42.0, 0, 0, r4c.ctypes.data, hr4o.ctypes.data, c4r.ctypes.data,
+                                       hc4o.ctypes.data, gain.ctypes.data, found.ctypes.data, api.WEIGHTS_GATED,
+                                       probs.ctypes.data, hpoff.ctypes.data, hnl.ctypes.data, 0))
+        got = [np.array(a) for a in (found, gain, r4c, c4r, probs)]
+    finally:
+        mem.free()
+    d = [_t(a) for a in (pb.costs, pb.cost_off, nr, nc, r4o, c4o, poff, nL)]
+    d_r4c = torch.full((got[2].size,), -7, dtype=torch.int64, device="cuda")
+    d_c4r = torch.full((got[3].size,), -7, dtype=torch.int64, device="cuda")
+    d_gain, d_found = torch.zeros(n * k, dtype=torch.float64, device="cuda"), torch.full((n,), -7, dtype=torch.int32, device="cuda")
+    d_probs = torch.full((got[4].size,), 7.5, dtype=torch.float64, device="cuda")
+    max_r, max_c = int(nr.max()), int(nc.max())
+    ws_bytes = int(lib.pda_murty_workspace_bytes(n, k, max_r, max_c))
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device="cuda")
+    _call(lib.pda_murty_batch(*[x.data_ptr() for x in d[:4]], n, max_r, max_c, k, api.CUT_RELATIVE, 42.0, 0, 0,
+                              d_r4c.data_ptr(), d[4].data_ptr(), d_c4r.data_ptr(), d[5].data_ptr(), d_gain.data_ptr(),
+                              d_found.data_ptr(), api.WEIGHTS_GATED, d_probs.data_ptr(), d[6].data_ptr(), d[7].data_ptr(),
+                              ws.data_ptr(), ws_bytes, None))
+    want = [_np(t) for t in (d_found, d_gain, d_r4c, d_c4r, d_probs)]
+    _same(got[0], want[0], "nFound")
+    _same(got[4], want[4], "weight tables")
+    assert want[0].min() >= 1
+    for p in range(n):  # only the first nFound hypotheses of a problem are defined
+        f = int(want[0][p])
+        _same(got[1][p * k:p * k + f], want[1][p * k:p * k + f], f"gains of problem {p}")
+        a, b = int(r4o[p]), int(r4o[p]) + f * int(nc[p])
+        _same(got[2][a:b], want[2][a:b], f"row4col of problem {p}")
+        a, b = int(c4o[p]), int(c4o[p]) + f * int(nr[p])
+        _same(got[3][a:b], want[3][a:b], f"col4row of problem {p}")
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("kind", KINDS)
+@pytest.mark.parametrize("large", SIDES)
+def test_assignment_prob_ladder(gpu_api, large, kind):
+    import torch
+    ks = np.asarray([3, 1, 5], np.int32)
+    nk = len(ks)
+    pb, nr, nc, nL, cells = _kbest_inputs(large)
+    n = len(pb)
+    poff = _prefix(cells * nk)
+    lib = _lib().lib()
+    mem = _HostMemory(kind)
+    try:
+        costs, off, hnr, hnc, hnl, hpoff = [mem(a) for a in (pb.costs, pb.cost_off, nr, nc, nL, poff)]
+        found, probs = mem(np.full(n * nk, -7, np.int32)), mem(np.full(int(cells.sum()) * nk, 7.5))
+        _side([costs, off, hnr, hnc, hnl, hpoff, found, probs], large)
+        _call(lib.pda_assignment_prob_ladder_batch_host(costs.ctypes.data, off.ctypes.data, hnr.ctypes.data, hnc.ctypes.data,
+                                                        hnl.ctypes.data, n, ks.ctypes.data, nk, probs.ctypes.data,
+                                                        hpoff.ctypes.data, found.ctypes.data, 0))
+        got = [np.array(a) for a in (found, probs)]
+    finally:
+        mem.free()
+    d = [_t(a) for a in (pb.costs, pb.cost_off, nr, nc, nL, poff)]
+    d_found = torch.full((n * nk,), -7, dtype=torch.int32, device="cuda")
+    d_probs = torch.full((got[1].size,), 7.5, dtype=torch.float64, device="cuda")
+    max_r, max_c = int(nr.max()), int(nc.max())
+    ws_bytes = int(lib.pda_murty_workspace_bytes(n, int(ks.max()), max_r, max_c))
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device="cuda")
+    _call(lib.pda_assignment_prob_ladder_batch(*[x.data_ptr() for x in d[:5]], n, max_r, max_c, ks.ctypes.data, nk,
+                                               d_probs.data_ptr(), d[5].data_ptr(), d_found.data_ptr(), ws.data_ptr(),
+                                               ws_bytes, None))
+    _same(got[0], _np(d_found), "nFound")
+    _same(got[1], _np(d_probs), "weight tables")
 
 
 # ---- asgnBB ------------------------------------------------------------------------------------------------------------

@@ -1,4 +1,4 @@
-"""Multi-device entry points of the C ABI (SURVEY.md 8e, "single process drives all GPUs") and the chunked host path.
+"""Multi-device entry points of the C ABI (SURVEY.md 8e, "single process drives all GPUs") and large host batches.
 
 On a one-GPU box the device list names device 0 several times: the slices then queue on that device's lock, which
 exercises the sharding, the offset handling and the result placement exactly as several devices would.  On a multi-GPU
@@ -128,10 +128,10 @@ def test_cpp_caller_drives_several_devices():
 
 
 @pytest.mark.parametrize("pinned", [False, True])
-def test_chunked_host_path(pinned):
-    """>= 131072 problems take the three-stream chunked branch of pda_murty_batch_host (copy in / run / copy out of
-    different chunks overlap).  Its results must equal the unchunked ones, with pageable and with page-locked buffers; a
-    batch whose problems SHARE one cost matrix (equal offsets) must not be chunked at all."""
+def test_large_host_batch(pinned):
+    """140 000 problems in ONE pda_murty_batch_host call must give what two half-size calls give, with pageable and with
+    page-locked buffers (lists and weights returned), and a batch whose problems all SHARE one cost matrix (equal
+    offsets) must give every problem that matrix's table."""
     import torch
     lib = _lib.lib()
     n, k = 140000, 4
@@ -167,7 +167,7 @@ def test_chunked_host_path(pinned):
     assert np.array_equal(got[3].reshape(n, k, 5)[np.arange(k)[None, :] < nf[:, None]], want[3].reshape(n, k, 5)[np.arange(k)[None, :] < nf[:, None]])
     assert np.array_equal(got[0].view(np.int64), want[0].view(np.int64))
     if not pinned:
-        # every problem reads the SAME matrix: offsets are equal, so a chunk's inputs are not a range of their own
+        # every problem reads the SAME matrix: the staged cost range is one matrix long
         one = synth.g1_dense(1, nL=3, nM=2, first=77)
         nr = np.full(n, 5, np.int32); nc = np.full(n, 2, np.int32); nl = np.full(n, 3, np.int32)
         off0 = np.zeros(n, np.int64)
