@@ -88,6 +88,11 @@ inline std::vector<double> computeQuadricCostMatrix(const std::vector<Eigen::Mat
  * (xmin, ymin, xmax, ymax, xOffset), nonassign = runConsts.NONASSIGN_BOUNDBOX.  Returns, per left box, the index of
  * the right box it is paired with or -1.  A boundBox-typed asgnBB is a three-line wrapper over this (INTEGRATION.md). */
 std::vector<int> asgnBBRaw(const std::vector<double>& boxesL, const std::vector<double>& boxesR, double nonassign);
+/* asgnBBRaw for many frames at once (boxesL[f] / boxesR[f] are frame f's boxes), optionally over several GPUs
+ * (contiguous slices, empty `devices` = the shim's device).  Returns, per frame, what asgnBBRaw returns for it. */
+std::vector<std::vector<int> > asgnBBRawBatch(const std::vector<std::vector<double> >& boxesL,
+                                              const std::vector<std::vector<double> >& boxesR, double nonassign,
+                                              const std::vector<int>& devices = std::vector<int>());
 
 /* raw form of conditionedPermanent: A is rows x cols, column-major */
 double conditionedPermanentRaw(const double* A, size_t rows, size_t cols, int permOpt);

@@ -335,9 +335,41 @@ int pda_association_perm_from_moments_batch(const double* landMean, const double
  * (xmin, ymin, xmax, ymax, xOffset); frame f owns left boxes [offL[f], offL[f+1]) and right boxes
  * [offR[f], offR[f+1]) (offL/offR have nFrames+1 entries).  assignment[i] = index (within its frame) of the right
  * box paired with left box i, or -1.  nonassign = NONASSIGN_BOUNDBOX.
+ * pda_asgn_bb_batch_host reads, stages and writes only [offL[0], offL[nFrames]) of boxesL / assignment and
+ * [offR[0], offR[nFrames]) of boxesR, so the entries of a larger batch outside that slice are left as they were.
+ * pda_asgn_bb_batch_host_multi cuts the frames into contiguous slices, one per device, each run by the _host form on
+ * its own host thread; the arrays are those of the whole batch.
  */
 int pda_asgn_bb_batch_host(const double* boxesL, const int64_t* offL, const double* boxesR, const int64_t* offR,
                            int64_t nFrames, double nonassign, int32_t* assignment, int32_t device);
+int pda_asgn_bb_batch_host_multi(const double* boxesL, const int64_t* offL, const double* boxesR, const int64_t* offR,
+                                 int64_t nFrames, double nonassign, int32_t* assignment,
+                                 const int32_t* devices, int32_t nDevices);
+
+/* Device-pointer form of pda_asgn_bb_batch_host, with the frame shapes read on the device: every pointer is a device
+ * pointer, the host reads only the scalar arguments, and the call enqueues on `stream` without a synchronisation, an
+ * allocation or a copy between host and device.  One CUDA graph captured with fixed bounds therefore serves frames of
+ * any shape within them (the per-frame stereo match of the SLAM loop, dataframe.cpp:306).
+ *   maxNL, maxBoxes   the caller's per-frame bounds (host scalars): left boxes nL <= maxNL, and nL + nR <= maxBoxes
+ *   capL, capR        boxes boxesL / boxesR hold; assignment holds capL entries.  boxesL (boxesR) may be NULL when capL
+ *                     (capR) is 0
+ *   status[f]         0: computed -- every left box of the frame gets its partner or -1 (all -1 without right boxes),
+ *                     bit-identical to the _host form for any bounds at or above the batch's maxima;
+ *                     2: not computed, nothing written.  A frame is status 2 when a range is negative, descending or
+ *                     past capL / capR, when nL > maxNL or nL + nR > maxBoxes, or when offL[f] is below an earlier
+ *                     offL[g] (g < f): then an earlier frame may own some of its left entries, and results are
+ *                     addressed by offL directly.  Entries outside every computed frame are left untouched.
+ * Errors: PDA_ERR_INVALID for a NULL pointer, nFrames < 0, a negative capacity, maxNL < 1 or maxBoxes < maxNL;
+ * PDA_ERR_UNSUPPORTED for maxBoxes > PDA_MAX_DIM (or what pda_murty_workspace_bytes refuses at these bounds);
+ * PDA_ERR_WORKSPACE below pda_asgn_bb_workspace_bytes.
+ * Workspace (for the current device and Murty path): per frame a maxBoxes x maxNL cost matrix, maxNL row4col entries
+ * and 48 B of shapes, plus pda_murty_workspace_bytes(nFrames, 1, maxBoxes, maxNL). */
+int64_t pda_asgn_bb_workspace_bytes(int64_t nFrames, int32_t maxNL, int32_t maxBoxes);
+int pda_asgn_bb_batch(const double* boxesL, const int64_t* offL, int64_t capL,
+                      const double* boxesR, const int64_t* offR, int64_t capR,
+                      int64_t nFrames, int32_t maxNL, int32_t maxBoxes, double nonassign,
+                      int32_t* assignment, int32_t* status,
+                      void* workspace, int64_t workspaceBytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Matrix permanent, Nijenhuis-Wilf / Ryser over Gray-code column subsets.

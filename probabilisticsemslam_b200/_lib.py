@@ -60,6 +60,9 @@ SIGNATURES = {
     "pda_association_perm_from_moments_batch": (C.c_int, [ptr, ptr, ptr, i64, ptr, ptr, ptr, i64, i64, i32, i32, dbl,
                                                           ptr, i64, ptr, ptr, ptr, i64, ptr]),
     "pda_asgn_bb_batch_host": (C.c_int, [ptr, ptr, ptr, ptr, i64, dbl, ptr, i32]),
+    "pda_asgn_bb_batch_host_multi": (C.c_int, [ptr, ptr, ptr, ptr, i64, dbl, ptr, ptr, i32]),
+    "pda_asgn_bb_workspace_bytes": (i64, [i64, i32, i32]),
+    "pda_asgn_bb_batch": (C.c_int, [ptr, ptr, i64, ptr, ptr, i64, i64, i32, i32, dbl, ptr, ptr, ptr, i64, ptr]),
     "pda_permanent_workspace_bytes": (i64, [i64]),
     "pda_permanent_batch": (C.c_int, [ptr, ptr, ptr, ptr, i64, i32, ptr, ptr, ptr, i64, ptr]),
     "pda_permanent_batch_host": (C.c_int, [ptr, ptr, ptr, ptr, i64, ptr, ptr, i32]),

@@ -448,9 +448,11 @@ def getAssignmentProbs(land_mean, land_cov, meas_mean, meas_cov, nonassign: floa
     return tabs[0]
 
 
-def asgn_bb_batch(boxes_l: list[np.ndarray], boxes_r: list[np.ndarray], nonassign: float, device: int = 0) -> list[np.ndarray]:
+def asgn_bb_batch(boxes_l: list[np.ndarray], boxes_r: list[np.ndarray], nonassign: float, device: int = 0,
+                  devices=None) -> list[np.ndarray]:
     """asgnBB (assignment.cpp:724-775) for a batch of frames; boxes are [count, 5] = xmin, ymin, xmax, ymax, xOffset.
-    Returns per frame the right-box index paired with each left box (-1 = none)."""
+    Returns per frame the right-box index paired with each left box (-1 = none).  devices: a list of CUDA device
+    ordinals spreads the frames over them (pda_asgn_bb_batch_host_multi, one contiguous slice each) instead of `device`."""
     n = len(boxes_l)
     cl = np.asarray([len(b) for b in boxes_l], np.int64)
     cr = np.asarray([len(b) for b in boxes_r], np.int64)
@@ -459,9 +461,39 @@ def asgn_bb_batch(boxes_l: list[np.ndarray], boxes_r: list[np.ndarray], nonassig
     flat_l = np.ascontiguousarray(np.concatenate([np.asarray(b, np.float64).reshape(-1, 5) for b in boxes_l] + [np.zeros((0, 5))]))
     flat_r = np.ascontiguousarray(np.concatenate([np.asarray(b, np.float64).reshape(-1, 5) for b in boxes_r] + [np.zeros((0, 5))]))
     out = np.full(max(int(off_l[-1]), 1), -7, np.int32)
-    check(lib().pda_asgn_bb_batch_host(_p(flat_l) if flat_l.size else None, _p(off_l), _p(flat_r) if flat_r.size else None,
-                                       _p(off_r), n, float(nonassign), _p(out), device))
+    pl, pr = _p(flat_l) if flat_l.size else None, _p(flat_r) if flat_r.size else None
+    if devices is None:
+        check(lib().pda_asgn_bb_batch_host(pl, _p(off_l), pr, _p(off_r), n, float(nonassign), _p(out), device))
+    else:
+        d = np.ascontiguousarray(devices, np.int32)
+        check(lib().pda_asgn_bb_batch_host_multi(pl, _p(off_l), pr, _p(off_r), n, float(nonassign), _p(out), _p(d), len(d)))
     return [out[off_l[f]:off_l[f + 1]].copy() for f in range(n)]
+
+
+def asgn_bb_batch_device(boxes_l, off_l, boxes_r, off_r, max_nL: int, max_boxes: int, nonassign: float, assignment=None,
+                         status=None, workspace=None):
+    """pda_asgn_bb_batch on CUDA tensors, enqueued on the current stream (no synchronisation, so it can be captured in a
+    CUDA graph): boxes float64 (5 per box), off_l / off_r int64 with nFrames+1 entries, frame shapes read on the device
+    against the bounds max_nL (left boxes) and max_boxes (left + right boxes).  assignment (int32, one entry per left
+    box the boxes_l tensor holds) is allocated filled with -1 when None.  Returns (assignment, status); status 2 marks a
+    frame that was not computed (include/pda_b200.h)."""
+    import torch
+    dev = off_l.device
+    n = int(off_l.shape[0]) - 1
+    cap_l, cap_r = boxes_l.numel() // 5, boxes_r.numel() // 5
+    assignment = torch.full((max(cap_l, 1),), -1, dtype=torch.int32, device=dev) if assignment is None else assignment
+    status = torch.empty(max(n, 1), dtype=torch.int32, device=dev) if status is None else status
+    if workspace is None:
+        ws = int(lib().pda_asgn_bb_workspace_bytes(n, max_nL, max_boxes))
+        check(min(ws, 0))
+        workspace = torch.empty(ws, dtype=torch.uint8, device=dev)
+    stream = _device_call_args(dict(boxes_l=boxes_l, off_l=off_l, boxes_r=boxes_r, off_r=off_r, assignment=assignment,
+                                    status=status, workspace=workspace), "asgn_bb_batch_device")
+    ptr = lambda t: t.data_ptr() if t.numel() else None
+    check(lib().pda_asgn_bb_batch(ptr(boxes_l), off_l.data_ptr(), cap_l, ptr(boxes_r), off_r.data_ptr(), cap_r, n, int(max_nL),
+                                  int(max_boxes), float(nonassign), assignment.data_ptr(), status.data_ptr(),
+                                  workspace.data_ptr(), int(workspace.numel()), stream))
+    return assignment, status
 
 
 def asgnBB(bbL: np.ndarray, bbR: np.ndarray, nonassign: float, device: int = 0) -> np.ndarray:

@@ -5,12 +5,15 @@
 //   asgnBB               assignment.cpp:724-775   kBest2D(k = 1, maximize = true); dummy pairing -> -1
 // Pipeline on one stream: bb_costs_kernel (one warp per frame) -> murty_kernel (k = 1, maximise) -> bb_finish_kernel.
 // A box is five doubles: xmin, ymin, xmax, ymax, xOffset.
+// The device-pointer form pda_asgn_bb_batch reads the frame shapes on the device (bb_shapes_kernel) instead of on the
+// host, so a CUDA graph captured once with fixed bounds serves frames of any shape (DESIGN.md 3.6b).
 #include "pda_internal.h"
 #include "pda_host_stage.h"
 
 #include <math_constants.h>
 
 #include <algorithm>
+#include <climits>
 #include <vector>
 
 namespace pda {
@@ -56,14 +59,16 @@ __global__ void bb_costs_kernel(const double* __restrict__ boxesL, const double*
     }
 }
 
+// nLeft[p] left boxes of problem p get their partner or -1: numCol[p] of them, or all of a frame that went to the
+// solver as 0 x 0 because it has no right box (the solver then reports nFound -1)
 __global__ void bb_finish_kernel(const int64_t* __restrict__ row4col, const int64_t* __restrict__ r4cOff,
                                  const int32_t* __restrict__ nFound, const int32_t* __restrict__ numRow,
-                                 const int32_t* __restrict__ numCol, const int64_t* __restrict__ firstL,
-                                 const int64_t nProblems, int32_t* __restrict__ assignment) {
+                                 const int32_t* __restrict__ numCol, const int32_t* __restrict__ nLeft,
+                                 const int64_t* __restrict__ firstL, const int64_t nProblems, int32_t* __restrict__ assignment) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int64_t p = (int64_t)blockIdx.x * WARPS + warp;
     if (p >= nProblems) return;
-    const int nL = numCol[p], nR = numRow[p] - nL;
+    const int nL = nLeft[p], nR = numRow[p] - numCol[p];
     for (int c = lane; c < nL; c += 32) {
         int a = -1;
         if (nFound[p] > 0) {
@@ -74,18 +79,115 @@ __global__ void bb_finish_kernel(const int64_t* __restrict__ row4col, const int6
     }
 }
 
+// ---- device-pointer form: frame shapes are read on the device, never on the host ----
+constexpr unsigned FULL = 0xffffffffu;
+constexpr int SHAPE_THREADS = 1024;  // one CTA; 32 warps, so the warp maxima are scanned by one warp
+
+struct BBShapes {
+    int32_t* numRow; int32_t* numCol;  // nL + nR and nL; 0 x 0 for a frame with an empty side or a rejected one
+    int32_t* nLeft;                    // left boxes the finish step writes: nL of a computed frame, else 0
+    int32_t* nFound;
+    int64_t* firstL; int64_t* firstR;
+    int64_t* costOff; int64_t* r4cOff;  // fixed strides: f * maxBoxes * maxNL and f * maxNL
+    double* costs;
+    int64_t* r4c;
+    unsigned char* murty;              // workspace of pda_murty_batch
+    size_t bytes;                      // everything up to `murty`
+};
+
+size_t align256(size_t x) { return (x + 255) / 256 * 256; }
+
+BBShapes carve_bb(void* workspace, int64_t nFrames, int32_t maxNL, int32_t maxBoxes) {
+    const size_t n = (size_t)std::max<int64_t>(nFrames, 1);
+    unsigned char* w = reinterpret_cast<unsigned char*>(workspace);
+    BBShapes s;
+    size_t o = 0;
+    s.numRow = reinterpret_cast<int32_t*>(w + o); o += align256(n * 4);
+    s.numCol = reinterpret_cast<int32_t*>(w + o); o += align256(n * 4);
+    s.nLeft = reinterpret_cast<int32_t*>(w + o); o += align256(n * 4);
+    s.nFound = reinterpret_cast<int32_t*>(w + o); o += align256(n * 4);
+    s.firstL = reinterpret_cast<int64_t*>(w + o); o += align256(n * 8);
+    s.firstR = reinterpret_cast<int64_t*>(w + o); o += align256(n * 8);
+    s.costOff = reinterpret_cast<int64_t*>(w + o); o += align256(n * 8);
+    s.r4cOff = reinterpret_cast<int64_t*>(w + o); o += align256(n * 8);
+    s.costs = reinterpret_cast<double*>(w + o); o += align256(n * (size_t)maxBoxes * (size_t)maxNL * 8);
+    s.r4c = reinterpret_cast<int64_t*>(w + o); o += align256(n * (size_t)maxNL * 8);
+    s.murty = w + o;
+    s.bytes = o;
+    return s;
+}
+
+// One CTA walks the frames in blocks of SHAPE_THREADS.  Results are addressed by offL directly, so a frame is computed
+// only if no other computed frame can write its left entries: offL[f] must be the largest of offL[0..f] (a running
+// maximum carried across blocks) and its own ranges must ascend.  Then every earlier frame ends at some offL[g+1] <=
+// offL[f] and every later computed frame starts at or after offL[f+1].  Both ranges must also lie within capL / capR,
+// and nL <= maxNL, nL + nR <= maxBoxes.  Right boxes are only read, so they need the bounds checks alone.  Frames with
+// an empty side go on as 0 x 0 (the solver reports nFound -1 and touches nothing), with their nL left boxes still
+// written -1 by the finish step when computed; status 2 frames write nothing.
+__global__ void __launch_bounds__(SHAPE_THREADS) bb_shapes_kernel(
+    const int64_t* __restrict__ offL, const int64_t capL, const int64_t* __restrict__ offR, const int64_t capR,
+    const long long nFrames, const int32_t maxNL, const int32_t maxBoxes, const BBShapes s, int32_t* __restrict__ status) {
+    __shared__ long long warpMax[SHAPE_THREADS / 32];
+    __shared__ long long carry;
+    const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+    if (t == 0) carry = LLONG_MIN;
+    __syncthreads();
+    for (long long base = 0; base < nFrames; base += SHAPE_THREADS) {
+        const long long f = base + t;
+        const long long l0 = f < nFrames ? offL[f] : LLONG_MIN;
+        long long x = l0;  // inclusive max-scan: warp, then the warp maxima, then the carry of earlier blocks
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const long long y = __shfl_up_sync(FULL, x, o);
+            if (lane >= o) x = max(x, y);
+        }
+        if (lane == 31) warpMax[warp] = x;
+        __syncthreads();
+        if (warp == 0) {
+            long long w = warpMax[lane];
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const long long y = __shfl_up_sync(FULL, w, o);
+                if (lane >= o) w = max(w, y);
+            }
+            warpMax[lane] = w;
+        }
+        __syncthreads();
+        const long long runMax = max(carry, max(warp ? warpMax[warp - 1] : LLONG_MIN, x));
+        if (f < nFrames) {
+            const long long l1 = offL[f + 1], r0 = offR[f], r1 = offR[f + 1];
+            const bool ok = l0 == runMax && l0 >= 0 && l1 >= l0 && l1 <= capL && r0 >= 0 && r1 >= r0 && r1 <= capR &&
+                            l1 - l0 <= maxNL && (l1 - l0) + (r1 - r0) <= maxBoxes;
+            const int nL = ok ? (int)(l1 - l0) : 0, nR = ok ? (int)(r1 - r0) : 0;
+            const bool solve = nL > 0 && nR > 0;
+            s.numRow[f] = solve ? nL + nR : 0; s.numCol[f] = solve ? nL : 0;
+            s.nLeft[f] = nL;
+            s.firstL[f] = ok ? l0 : 0; s.firstR[f] = ok ? r0 : 0;
+            s.costOff[f] = f * maxBoxes * maxNL; s.r4cOff[f] = f * maxNL;
+            status[f] = ok ? 0 : 2;
+        }
+        __syncthreads();  // every thread has read carry and warpMax
+        if (t == SHAPE_THREADS - 1) carry = runMax;
+    }
+}
+
 }  // namespace
 }  // namespace pda
 
 using namespace pda;
 
-extern "C" int pda_asgn_bb_batch_host(const double* boxesL, const int64_t* offL, const double* boxesR, const int64_t* offR,
-                                      int64_t nFrames, double nonassign, int32_t* assignment, int32_t device) {
+extern "C" {
+
+// Frame f owns [offL[f], offL[f+1]) of boxesL / assignment and [offR[f], offR[f+1]) of boxesR: only [offL[0], offL[n])
+// and [offR[0], offR[n]) are read, staged and written back, so a call on a slice of a larger batch (a shard of
+// pda_asgn_bb_batch_host_multi) leaves the other frames' entries alone.
+int pda_asgn_bb_batch_host(const double* boxesL, const int64_t* offL, const double* boxesR, const int64_t* offR,
+                           int64_t nFrames, double nonassign, int32_t* assignment, int32_t device) {
     if (nFrames < 0) return fail(PDA_ERR_INVALID, "asgn_bb: nFrames < 0");
     if (nFrames == 0) return PDA_OK;
     if (!offL || !offR || !assignment) return fail(PDA_ERR_INVALID, "asgn_bb: NULL argument");
-    const int64_t totalL = offL[nFrames], totalR = offR[nFrames];
-    for (int64_t i = 0; i < totalL; ++i) assignment[i] = -1;  // frames with an empty side: every left box unmatched (:730-732)
+    if (offL[0] < 0 || offR[0] < 0) return fail(PDA_ERR_INVALID, "asgn_bb: negative offset");
+    const int64_t baseL = offL[0], baseR = offR[0];
     std::vector<int64_t> firstL, firstR, costOff, r4cOff;
     std::vector<int32_t> numRow, numCol;
     size_t nCost = 0, nR4c = 0;
@@ -95,12 +197,15 @@ extern "C" int pda_asgn_bb_batch_host(const double* boxesL, const int64_t* offL,
         if (nL < 0 || nR < 0) return fail(PDA_ERR_INVALID, "asgn_bb: offsets must be non-decreasing");
         if (nL == 0 || nR == 0) continue;
         if (nL + nR > PDA_MAX_DIM) return fail(PDA_ERR_UNSUPPORTED, "asgn_bb: frame %lld has %lld boxes (limit %d)", (long long)f, (long long)(nL + nR), PDA_MAX_DIM);
-        firstL.push_back(offL[f]); firstR.push_back(offR[f]);
+        firstL.push_back(offL[f] - baseL); firstR.push_back(offR[f] - baseR);
         numRow.push_back((int32_t)(nL + nR)); numCol.push_back((int32_t)nL);
         costOff.push_back((int64_t)nCost); r4cOff.push_back((int64_t)nR4c);
         nCost += (size_t)((nL + nR) * nL); nR4c += (size_t)nL;
         maxR = std::max<int>(maxR, (int)(nL + nR)); maxC = std::max<int>(maxC, (int)nL);
     }
+    const int64_t totalL = offL[nFrames] - baseL, totalR = offR[nFrames] - baseR;
+    int32_t* const asg = assignment + baseL;
+    for (int64_t i = 0; i < totalL; ++i) asg[i] = -1;  // frames with an empty side: every left box unmatched (:730-732)
     const size_t n = numRow.size();
     if (n == 0) return PDA_OK;
     if (!boxesL || !boxesR) return fail(PDA_ERR_INVALID, "asgn_bb: NULL boxes");
@@ -109,10 +214,10 @@ extern "C" int pda_asgn_bb_batch_host(const double* boxesL, const int64_t* offL,
     const int64_t wsBytes = pda_murty_workspace_bytes((int64_t)n, 1, maxR, maxC);
     if (wsBytes < 0) return (int)wsBytes;
     HostIO io(device);
-    const size_t oBL = io.in(boxesL, (size_t)totalL * 40), oBR = io.in(boxesR, (size_t)totalR * 40);
+    const size_t oBL = io.in(boxesL + 5 * baseL, (size_t)totalL * 40), oBR = io.in(boxesR + 5 * baseR, (size_t)totalR * 40);
     const size_t oFL = io.in(firstL.data(), n * 8), oFR = io.in(firstR.data(), n * 8), oNR = io.in(numRow.data(), n * 4);
     const size_t oNC = io.in(numCol.data(), n * 4), oCO = io.in(costOff.data(), n * 8), oRO = io.in(r4cOff.data(), n * 8);
-    const size_t oAsg = io.inout(assignment, (size_t)totalL * 4);
+    const size_t oAsg = io.inout(asg, (size_t)totalL * 4);
     const size_t oC = io.scratch(nCost * 8), oR4c = io.scratch(nR4c * 8), oFound = io.scratch(n * 4), oWs = io.scratch((size_t)wsBytes);
     PDA_TRY(io.commit());
     const cudaStream_t s = io.stream();
@@ -127,7 +232,61 @@ extern "C" int pda_asgn_bb_batch_host(const double* boxesL, const int64_t* offL,
                             nullptr, io.at<int32_t>(oFound), PDA_WEIGHTS_NONE, nullptr, nullptr, nullptr,
                             io.at<unsigned char>(oWs), wsBytes, s));
     bb_finish_kernel<<<blocks, 32 * WARPS, 0, s>>>(io.at<int64_t>(oR4c), io.at<int64_t>(oRO), io.at<int32_t>(oFound), io.at<int32_t>(oNR),
-                                                   io.at<int32_t>(oNC), io.at<int64_t>(oFL), (int64_t)n, io.at<int32_t>(oAsg));
+                                                   io.at<int32_t>(oNC), io.at<int32_t>(oNC), io.at<int64_t>(oFL), (int64_t)n,
+                                                   io.at<int32_t>(oAsg));
     PDA_CUDA_TRY(cudaGetLastError());
     return io.download();
 }
+
+int64_t pda_asgn_bb_workspace_bytes(int64_t nFrames, int32_t maxNL, int32_t maxBoxes) {
+    if (nFrames < 0 || maxNL < 1 || maxBoxes < maxNL)
+        return fail(PDA_ERR_INVALID, "asgn_bb: nFrames %lld, maxNL %d, maxBoxes %d", (long long)nFrames, maxNL, maxBoxes);
+    if (maxBoxes > PDA_MAX_DIM) return fail(PDA_ERR_UNSUPPORTED, "asgn_bb: maxBoxes %d above %d", maxBoxes, PDA_MAX_DIM);
+    const int64_t murty = pda_murty_workspace_bytes(std::max<int64_t>(nFrames, 1), 1, maxBoxes, maxNL);
+    if (murty < 0) return murty;
+    return (int64_t)carve_bb(nullptr, nFrames, maxNL, maxBoxes).bytes + murty;
+}
+
+int pda_asgn_bb_batch(const double* boxesL, const int64_t* offL, int64_t capL, const double* boxesR, const int64_t* offR,
+                      int64_t capR, int64_t nFrames, int32_t maxNL, int32_t maxBoxes, double nonassign, int32_t* assignment,
+                      int32_t* status, void* workspace, int64_t workspaceBytes, void* stream) {
+    if (!offL || !offR || !assignment || !status || !workspace || (capL > 0 && !boxesL) || (capR > 0 && !boxesR))
+        return fail(PDA_ERR_INVALID, "asgn_bb: NULL argument");
+    if (capL < 0 || capR < 0) return fail(PDA_ERR_INVALID, "asgn_bb: negative capacity");
+    const int64_t wsBytes = pda_asgn_bb_workspace_bytes(nFrames, maxNL, maxBoxes);
+    if (wsBytes < 0) return (int)wsBytes;
+    if (workspaceBytes < wsBytes)
+        return fail(PDA_ERR_WORKSPACE, "asgn_bb: workspace of %lld B, %lld B needed", (long long)workspaceBytes, (long long)wsBytes);
+    if (nFrames == 0) return PDA_OK;
+    const cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+    const BBShapes sh = carve_bb(workspace, nFrames, maxNL, maxBoxes);
+    bb_shapes_kernel<<<1, SHAPE_THREADS, 0, s>>>(offL, capL, offR, capR, nFrames, maxNL, maxBoxes, sh, status);
+    PDA_CUDA_TRY(cudaGetLastError());
+    const unsigned blocks = (unsigned)((nFrames + WARPS - 1) / WARPS);
+    bb_costs_kernel<<<blocks, 32 * WARPS, 0, s>>>(boxesL, boxesR, sh.firstL, sh.firstR, sh.numRow, sh.numCol, sh.costOff, nFrames,
+                                                  nonassign, sh.costs);
+    PDA_CUDA_TRY(cudaGetLastError());
+    PDA_TRY(pda_murty_batch(sh.costs, sh.costOff, sh.numRow, sh.numCol, nFrames, maxBoxes, maxNL, 1, PDA_CUT_NONE, 0.0,
+                            1 /* maximize */, 0, sh.r4c, sh.r4cOff, nullptr, nullptr, nullptr, sh.nFound, PDA_WEIGHTS_NONE, nullptr,
+                            nullptr, nullptr, sh.murty, workspaceBytes - (int64_t)sh.bytes, stream));
+    bb_finish_kernel<<<blocks, 32 * WARPS, 0, s>>>(sh.r4c, sh.r4cOff, sh.nFound, sh.numRow, sh.numCol, sh.nLeft, sh.firstL, nFrames,
+                                                   assignment);
+    PDA_CUDA_TRY(cudaGetLastError());
+    return PDA_OK;
+}
+
+// contiguous slices of frames, one per device, each a pda_asgn_bb_batch_host call on the whole arrays and its own
+// offsets: the slices' ranges of boxesL / assignment do not overlap
+int pda_asgn_bb_batch_host_multi(const double* boxesL, const int64_t* offL, const double* boxesR, const int64_t* offR,
+                                 int64_t nFrames, double nonassign, int32_t* assignment, const int32_t* devices,
+                                 int32_t nDevices) {
+    if (!devices || nDevices < 1) return fail(PDA_ERR_INVALID, "asgn_bb (multi): need at least one device");
+    if (nFrames < 0) return fail(PDA_ERR_INVALID, "asgn_bb: nFrames < 0");
+    if (nFrames == 0) return PDA_OK;
+    if (!offL || !offR || !assignment) return fail(PDA_ERR_INVALID, "asgn_bb: NULL argument");
+    return run_sharded(nFrames, devices, nDevices, [&](int64_t p0, int64_t p1, int dev) {
+        return pda_asgn_bb_batch_host(boxesL, offL + p0, boxesR, offR + p0, p1 - p0, nonassign, assignment, dev);
+    });
+}
+
+}  // extern "C"

@@ -6,6 +6,7 @@
 #include <math.h>
 #include <stdint.h>
 
+#include <algorithm>
 #include <limits>
 #include <stdexcept>
 #include <string>
@@ -360,6 +361,32 @@ std::vector<std::vector<std::vector<double> > > getAssignmentProbsBatch(const st
              "getAssignmentProbsBatch");
     for (size_t p = 0; p < n; p++) permStatusCheck(status[p]);
     return fb.tables(nL, nM);
+}
+
+std::vector<std::vector<int> > asgnBBRawBatch(const std::vector<std::vector<double> >& boxesL,
+                                              const std::vector<std::vector<double> >& boxesR, double nonassign,
+                                              const std::vector<int>& devices) {
+    if (boxesL.size() != boxesR.size()) throw std::invalid_argument("asgnBBRawBatch: boxesL and boxesR differ in frame count");
+    const size_t n = boxesL.size();
+    std::vector<int64_t> offL(n + 1, 0), offR(n + 1, 0);
+    for (size_t f = 0; f < n; f++) {
+        offL[f + 1] = offL[f] + int64_t(boxesL[f].size() / 5);
+        offR[f + 1] = offR[f] + int64_t(boxesR[f].size() / 5);
+    }
+    std::vector<double> flatL(5 * size_t(offL[n]) + 1), flatR(5 * size_t(offR[n]) + 1);
+    for (size_t f = 0; f < n; f++) {
+        std::copy(boxesL[f].begin(), boxesL[f].begin() + 5 * (offL[f + 1] - offL[f]), flatL.begin() + 5 * offL[f]);
+        std::copy(boxesR[f].begin(), boxesR[f].begin() + 5 * (offR[f + 1] - offR[f]), flatR.begin() + 5 * offR[f]);
+    }
+    std::vector<int32_t> a(offL[n] + 1, -1);
+    const std::vector<int32_t> dev = deviceList(devices);
+    if (n)
+        pdaCheck(pda_asgn_bb_batch_host_multi(flatL.data(), offL.data(), flatR.data(), offR.data(), int64_t(n), nonassign, a.data(),
+                                              dev.data(), int32_t(dev.size())),
+                 "asgnBBRawBatch");
+    std::vector<std::vector<int> > out(n);
+    for (size_t f = 0; f < n; f++) out[f].assign(a.begin() + offL[f], a.begin() + offL[f + 1]);
+    return out;
 }
 
 double permanentExactShardedRaw(const double* A, size_t n, const int* devices, size_t nDevices) {
