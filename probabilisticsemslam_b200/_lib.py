@@ -111,3 +111,11 @@ def lib() -> C.CDLL:
 def check(code: int) -> None:
     if code != 0:
         raise PdaError(int(code), lib().pda_last_error().decode(errors="replace"))
+
+
+def alloc_workspace(nbytes: int, device):
+    """A device workspace of `nbytes` bytes, as a pda_*_workspace_bytes call returned it; raises on its error codes."""
+    import torch
+    nbytes = int(nbytes)
+    check(min(nbytes, 0))
+    return torch.empty(nbytes, dtype=torch.uint8, device=device)

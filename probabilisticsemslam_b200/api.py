@@ -18,7 +18,7 @@ from dataclasses import dataclass
 import numpy as np
 
 from . import _lib
-from ._lib import check, lib
+from ._lib import alloc_workspace, check, lib
 from .synth import ProblemBatch, pack
 
 CUT_NONE, CUT_RELATIVE, CUT_STICKY = 0, 1, 2
@@ -237,9 +237,8 @@ def permanent_prob_batch_device(costs, cost_off, nL, nM, prob_off, total_prob_el
     status = torch.empty(nL.shape[0], dtype=torch.int32, device=dev) if status is None else status
     n = int(nL.shape[0])
     if workspace is None:
-        ws = int(lib().pda_permanent_prob_workspace_bytes(n, int(costs.numel()), int(total_prob_elems), max_num_row, max_num_col, perm_opt))
-        check(min(ws, 0))
-        workspace = torch.empty(ws, dtype=torch.uint8, device=dev)
+        workspace = alloc_workspace(lib().pda_permanent_prob_workspace_bytes(n, int(costs.numel()), int(total_prob_elems),
+                                                                             max_num_row, max_num_col, perm_opt), dev)
     stream = _device_call_args(dict(costs=costs, cost_off=cost_off, nL=nL, nM=nM, prob_off=prob_off, probs=probs,
                                     status=status, workspace=workspace), "permanent_prob_batch_device")
     check(lib().pda_permanent_prob_batch(costs.data_ptr(), cost_off.data_ptr(), nL.data_ptr(), nM.data_ptr(), n,
@@ -259,9 +258,7 @@ def conditioned_permanent_batch_device(mats, mat_off, rows, cols, max_dim: int, 
     out = torch.zeros(n, dtype=torch.float64, device=dev) if out is None else out
     status = torch.empty(n, dtype=torch.int32, device=dev) if status is None else status
     if workspace is None:
-        ws = int(lib().pda_conditioned_permanent_workspace_bytes(n, max_dim, perm_opt))
-        check(min(ws, 0))
-        workspace = torch.empty(ws, dtype=torch.uint8, device=dev)
+        workspace = alloc_workspace(lib().pda_conditioned_permanent_workspace_bytes(n, max_dim, perm_opt), dev)
     stream = _device_call_args(dict(mats=mats, mat_off=mat_off, rows=rows, cols=cols, out=out, status=status,
                                     workspace=workspace), "conditioned_permanent_batch_device")
     check(lib().pda_conditioned_permanent_batch(mats.data_ptr(), mat_off.data_ptr(), rows.data_ptr(), cols.data_ptr(), n,
@@ -364,9 +361,7 @@ def _moments_device_call(name, land_mean, land_cov, land_off, meas_mean, meas_co
     prob_off = torch.empty(n + 1, dtype=torch.int64, device=dev) if prob_off is None else prob_off
     status = torch.empty(max(n, 1), dtype=torch.int32, device=dev) if status is None else status
     if workspace is None:
-        ws = int(getattr(lib(), name + "_workspace_bytes")(n, max_nL, max_nM, int(prob_capacity), *ws_args))
-        check(min(ws, 0))
-        workspace = torch.empty(ws, dtype=torch.uint8, device=dev)
+        workspace = alloc_workspace(getattr(lib(), name + "_workspace_bytes")(n, max_nL, max_nM, int(prob_capacity), *ws_args), dev)
     tensors = dict(land_mean=land_mean, land_cov=land_cov, land_off=land_off, meas_mean=meas_mean, meas_cov=meas_cov,
                    meas_off=meas_off, probs=probs, prob_off=prob_off, status=status, workspace=workspace)
     tensors.update({k: v for k, v in extra_out.items() if v is not None})
@@ -484,9 +479,7 @@ def asgn_bb_batch_device(boxes_l, off_l, boxes_r, off_r, max_nL: int, max_boxes:
     assignment = torch.full((max(cap_l, 1),), -1, dtype=torch.int32, device=dev) if assignment is None else assignment
     status = torch.empty(max(n, 1), dtype=torch.int32, device=dev) if status is None else status
     if workspace is None:
-        ws = int(lib().pda_asgn_bb_workspace_bytes(n, max_nL, max_boxes))
-        check(min(ws, 0))
-        workspace = torch.empty(ws, dtype=torch.uint8, device=dev)
+        workspace = alloc_workspace(lib().pda_asgn_bb_workspace_bytes(n, max_nL, max_boxes), dev)
     stream = _device_call_args(dict(boxes_l=boxes_l, off_l=off_l, boxes_r=boxes_r, off_r=off_r, assignment=assignment,
                                     status=status, workspace=workspace), "asgn_bb_batch_device")
     ptr = lambda t: t.data_ptr() if t.numel() else None

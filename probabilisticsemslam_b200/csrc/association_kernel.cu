@@ -39,7 +39,27 @@ __global__ void uncompact_probs_kernel(const double* __restrict__ cond, const in
     }
 }
 
-size_t align256(size_t x) { return (x + 255) / 256 * 256; }
+struct AssocWorkspace {
+    int32_t* goodRows; int32_t* condNL; int32_t* found;
+    double* condCosts; int64_t* rowIdx; double* condProbs;
+    unsigned char* murty;  // workspace of pda_murty_batch
+    size_t bytes;          // everything up to `murty`
+};
+
+AssocWorkspace carve(void* workspace, int64_t nProblems, int64_t totalCostElems, int64_t totalRows, int64_t totalProbElems) {
+    const size_t n = (size_t)std::max<int64_t>(nProblems, 1);
+    WorkspaceLayout w(workspace);
+    AssocWorkspace a;
+    a.goodRows = w.take<int32_t>(n);
+    a.condNL = w.take<int32_t>(n);
+    a.found = w.take<int32_t>(n);
+    a.condCosts = w.take<double>((size_t)totalCostElems);
+    a.rowIdx = w.take<int64_t>((size_t)totalRows);
+    a.condProbs = w.take<double>((size_t)totalProbElems);
+    a.murty = w.rest();
+    a.bytes = w.bytes();
+    return a;
+}
 
 }  // namespace
 }  // namespace pda
@@ -52,9 +72,7 @@ int64_t pda_association_workspace_bytes(int64_t nProblems, int64_t totalCostElem
                                         int64_t totalProbElems, int32_t k, int32_t maxNumRow, int32_t maxNumCol) {
     const int64_t murty = pda_murty_workspace_bytes(nProblems, k, maxNumRow, maxNumCol);
     if (murty < 0) return murty;
-    const size_t n = (size_t)std::max<int64_t>(nProblems, 1);
-    return (int64_t)(4 * align256(n * 4) + align256((size_t)totalCostElems * 8) + align256((size_t)totalRows * 8) +
-                     align256((size_t)totalProbElems * 8) + 256) + murty;
+    return (int64_t)carve(nullptr, nProblems, totalCostElems, totalRows, totalProbElems).bytes + murty;
 }
 
 int pda_association_probs_batch(const double* costs, const int64_t* costOff, const int32_t* nL, const int32_t* nM,
@@ -73,27 +91,17 @@ int pda_association_probs_batch(const double* costs, const int64_t* costOff, con
     if (maxNumRow > PDA_MAX_DIM)
         return fail(PDA_ERR_UNSUPPORTED, "association: maxNumRow %d exceeds PDA_MAX_DIM %d", maxNumRow, PDA_MAX_DIM);
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-    const size_t n = (size_t)nProblems;
-    unsigned char* w = reinterpret_cast<unsigned char*>(workspace);
-    size_t o = 0;
-    int32_t* numRow = reinterpret_cast<int32_t*>(w + o); o += align256(n * 4);
-    int32_t* goodRows = reinterpret_cast<int32_t*>(w + o); o += align256(n * 4);
-    int32_t* condNL = reinterpret_cast<int32_t*>(w + o); o += align256(n * 4);
-    int32_t* found = reinterpret_cast<int32_t*>(w + o); o += align256(n * 4);
-    double* condCosts = reinterpret_cast<double*>(w + o); o += align256((size_t)totalCostElems * 8);
-    int64_t* rowIdx = reinterpret_cast<int64_t*>(w + o); o += align256((size_t)totalRows * 8);
-    double* condProbs = reinterpret_cast<double*>(w + o); o += align256((size_t)totalProbElems * 8);
-    if ((int64_t)o + 256 > workspaceBytes) return fail(PDA_ERR_WORKSPACE, "association: workspace too small");
+    const AssocWorkspace w = carve(workspace, nProblems, totalCostElems, totalRows, totalProbElems);
+    if ((int64_t)w.bytes > workspaceBytes) return fail(PDA_ERR_WORKSPACE, "association: workspace too small");
     // (numRow = nL + nM and condL = goodRows - nM are formed inside the conditioning kernel: two launches fewer)
-    (void)numRow;
-    PDA_TRY(launch_condition_costs(costs, costOff, nullptr, nM, nProblems, rowOff, condCosts, rowIdx, goodRows, s, nL, condNL,
-                                   maxNumRow, maxNumCol));
+    PDA_TRY(launch_condition_costs(costs, costOff, nullptr, nM, nProblems, rowOff, w.condCosts, w.rowIdx, w.goodRows, s, nL,
+                                   w.condNL, maxNumRow, maxNumCol));
     // conditioned problems live at the original cost offsets (they only shrink) and use the original probability offsets
-    PDA_TRY(pda_murty_batch(condCosts, costOff, goodRows, nM, nProblems, maxNumRow, maxNumCol, k, PDA_CUT_RELATIVE, 42.0, 0, 0,
-                            nullptr, nullptr, nullptr, nullptr, nullptr, nFound ? nFound : found, PDA_WEIGHTS_GATED, condProbs,
-                            probOff, condNL, w + o, workspaceBytes - (int64_t)o, stream));
-    uncompact_probs_kernel<<<(unsigned)((n + WARPS - 1) / WARPS), 32 * WARPS, 0, s>>>(condProbs, probOff, nL, nM, condNL, rowIdx,
-                                                                                   rowOff, nProblems, probs);
+    PDA_TRY(pda_murty_batch(w.condCosts, costOff, w.goodRows, nM, nProblems, maxNumRow, maxNumCol, k, PDA_CUT_RELATIVE, 42.0, 0, 0,
+                            nullptr, nullptr, nullptr, nullptr, nullptr, nFound ? nFound : w.found, PDA_WEIGHTS_GATED, w.condProbs,
+                            probOff, w.condNL, w.murty, workspaceBytes - (int64_t)w.bytes, stream));
+    uncompact_probs_kernel<<<(unsigned)((nProblems + WARPS - 1) / WARPS), 32 * WARPS, 0, s>>>(
+        w.condProbs, probOff, nL, nM, w.condNL, w.rowIdx, rowOff, nProblems, probs);
     PDA_CUDA_TRY(cudaGetLastError());
     return PDA_OK;
 }

@@ -37,8 +37,6 @@ constexpr int SMEM_BUDGET = 48 * 1024;         // dynamic shared memory per CTA:
 // the column scales, then the kept column (16) and row (PDA_MAX_DIM) indices as shorts
 __host__ __device__ constexpr int warp_doubles(int cap) { return 2 * cap + 16 + SUB_ROWS * SUB_COLS + 16 + (16 + PDA_MAX_DIM) / 4; }
 
-size_t align256(size_t x) { return (x + 255) / 256 * 256; }
-
 struct CondPermArgs {
     const double* P; const int64_t* costOff; const int32_t* nL; const int32_t* nM; const int32_t* condNL;
     const int64_t* probOff; double* perm; int32_t* slotStatus;
@@ -163,16 +161,15 @@ struct PermWorkspace {
 };
 PermWorkspace carve(void* workspace, int64_t nProblems, int64_t totalCostElems, int64_t totalRows, int64_t totalProbElems) {
     const size_t n = (size_t)std::max<int64_t>(nProblems, 1);
-    unsigned char* w = reinterpret_cast<unsigned char*>(workspace);
+    WorkspaceLayout w(workspace);
     PermWorkspace ws;
-    size_t o = 0;
-    ws.goodRows = reinterpret_cast<int32_t*>(w + o); o += align256(n * 4);
-    ws.condNL = reinterpret_cast<int32_t*>(w + o); o += align256(n * 4);
-    ws.condCosts = reinterpret_cast<double*>(w + o); o += align256((size_t)totalCostElems * 8);
-    ws.rowIdx = reinterpret_cast<int64_t*>(w + o); o += align256((size_t)totalRows * 8);
-    ws.perm = reinterpret_cast<double*>(w + o); o += align256((size_t)totalProbElems * 8);
-    ws.slotStatus = reinterpret_cast<int32_t*>(w + o); o += align256((size_t)totalProbElems * 4);
-    ws.bytes = o + 256;
+    ws.goodRows = w.take<int32_t>(n);
+    ws.condNL = w.take<int32_t>(n);
+    ws.condCosts = w.take<double>((size_t)totalCostElems);
+    ws.rowIdx = w.take<int64_t>((size_t)totalRows);
+    ws.perm = w.take<double>((size_t)totalProbElems);
+    ws.slotStatus = w.take<int32_t>((size_t)totalProbElems);
+    ws.bytes = w.bytes();
     return ws;
 }
 

@@ -9,6 +9,7 @@
 // host, so a CUDA graph captured once with fixed bounds serves frames of any shape (DESIGN.md 3.6b).
 #include "pda_internal.h"
 #include "pda_host_stage.h"
+#include "cta_scan.cuh"
 
 #include <math_constants.h>
 
@@ -80,9 +81,6 @@ __global__ void bb_finish_kernel(const int64_t* __restrict__ row4col, const int6
 }
 
 // ---- device-pointer form: frame shapes are read on the device, never on the host ----
-constexpr unsigned FULL = 0xffffffffu;
-constexpr int SHAPE_THREADS = 1024;  // one CTA; 32 warps, so the warp maxima are scanned by one warp
-
 struct BBShapes {
     int32_t* numRow; int32_t* numCol;  // nL + nR and nL; 0 x 0 for a frame with an empty side or a rejected one
     int32_t* nLeft;                    // left boxes the finish step writes: nL of a computed frame, else 0
@@ -95,65 +93,41 @@ struct BBShapes {
     size_t bytes;                      // everything up to `murty`
 };
 
-size_t align256(size_t x) { return (x + 255) / 256 * 256; }
-
 BBShapes carve_bb(void* workspace, int64_t nFrames, int32_t maxNL, int32_t maxBoxes) {
     const size_t n = (size_t)std::max<int64_t>(nFrames, 1);
-    unsigned char* w = reinterpret_cast<unsigned char*>(workspace);
+    WorkspaceLayout w(workspace);
     BBShapes s;
-    size_t o = 0;
-    s.numRow = reinterpret_cast<int32_t*>(w + o); o += align256(n * 4);
-    s.numCol = reinterpret_cast<int32_t*>(w + o); o += align256(n * 4);
-    s.nLeft = reinterpret_cast<int32_t*>(w + o); o += align256(n * 4);
-    s.nFound = reinterpret_cast<int32_t*>(w + o); o += align256(n * 4);
-    s.firstL = reinterpret_cast<int64_t*>(w + o); o += align256(n * 8);
-    s.firstR = reinterpret_cast<int64_t*>(w + o); o += align256(n * 8);
-    s.costOff = reinterpret_cast<int64_t*>(w + o); o += align256(n * 8);
-    s.r4cOff = reinterpret_cast<int64_t*>(w + o); o += align256(n * 8);
-    s.costs = reinterpret_cast<double*>(w + o); o += align256(n * (size_t)maxBoxes * (size_t)maxNL * 8);
-    s.r4c = reinterpret_cast<int64_t*>(w + o); o += align256(n * (size_t)maxNL * 8);
-    s.murty = w + o;
-    s.bytes = o;
+    s.numRow = w.take<int32_t>(n);
+    s.numCol = w.take<int32_t>(n);
+    s.nLeft = w.take<int32_t>(n);
+    s.nFound = w.take<int32_t>(n);
+    s.firstL = w.take<int64_t>(n);
+    s.firstR = w.take<int64_t>(n);
+    s.costOff = w.take<int64_t>(n);
+    s.r4cOff = w.take<int64_t>(n);
+    s.costs = w.take<double>(n * (size_t)maxBoxes * (size_t)maxNL);
+    s.r4c = w.take<int64_t>(n * (size_t)maxNL);
+    s.murty = w.rest();
+    s.bytes = w.bytes();
     return s;
 }
 
-// One CTA walks the frames in blocks of SHAPE_THREADS.  Results are addressed by offL directly, so a frame is computed
+// One CTA walks the frames in blocks of CTA_SCAN_THREADS.  Results are addressed by offL directly, so a frame is computed
 // only if no other computed frame can write its left entries: offL[f] must be the largest of offL[0..f] (a running
 // maximum carried across blocks) and its own ranges must ascend.  Then every earlier frame ends at some offL[g+1] <=
 // offL[f] and every later computed frame starts at or after offL[f+1].  Both ranges must also lie within capL / capR,
 // and nL <= maxNL, nL + nR <= maxBoxes.  Right boxes are only read, so they need the bounds checks alone.  Frames with
 // an empty side go on as 0 x 0 (the solver reports nFound -1 and touches nothing), with their nL left boxes still
 // written -1 by the finish step when computed; status 2 frames write nothing.
-__global__ void __launch_bounds__(SHAPE_THREADS) bb_shapes_kernel(
+__global__ void __launch_bounds__(CTA_SCAN_THREADS) bb_shapes_kernel(
     const int64_t* __restrict__ offL, const int64_t capL, const int64_t* __restrict__ offR, const int64_t capR,
     const long long nFrames, const int32_t maxNL, const int32_t maxBoxes, const BBShapes s, int32_t* __restrict__ status) {
-    __shared__ long long warpMax[SHAPE_THREADS / 32];
-    __shared__ long long carry;
-    const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
-    if (t == 0) carry = LLONG_MIN;
-    __syncthreads();
-    for (long long base = 0; base < nFrames; base += SHAPE_THREADS) {
-        const long long f = base + t;
+    __shared__ long long warpMax[32];
+    long long carry = LLONG_MIN;
+    for (long long base = 0; base < nFrames; base += CTA_SCAN_THREADS) {
+        const long long f = base + threadIdx.x;
         const long long l0 = f < nFrames ? offL[f] : LLONG_MIN;
-        long long x = l0;  // inclusive max-scan: warp, then the warp maxima, then the carry of earlier blocks
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const long long y = __shfl_up_sync(FULL, x, o);
-            if (lane >= o) x = max(x, y);
-        }
-        if (lane == 31) warpMax[warp] = x;
-        __syncthreads();
-        if (warp == 0) {
-            long long w = warpMax[lane];
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                const long long y = __shfl_up_sync(FULL, w, o);
-                if (lane >= o) w = max(w, y);
-            }
-            warpMax[lane] = w;
-        }
-        __syncthreads();
-        const long long runMax = max(carry, max(warp ? warpMax[warp - 1] : LLONG_MIN, x));
+        const long long runMax = cta_scan(l0, carry, warpMax, ScanMax());
         if (f < nFrames) {
             const long long l1 = offL[f + 1], r0 = offR[f], r1 = offR[f + 1];
             const bool ok = l0 == runMax && l0 >= 0 && l1 >= l0 && l1 <= capL && r0 >= 0 && r1 >= r0 && r1 <= capR &&
@@ -166,8 +140,6 @@ __global__ void __launch_bounds__(SHAPE_THREADS) bb_shapes_kernel(
             s.costOff[f] = f * maxBoxes * maxNL; s.r4cOff[f] = f * maxNL;
             status[f] = ok ? 0 : 2;
         }
-        __syncthreads();  // every thread has read carry and warpMax
-        if (t == SHAPE_THREADS - 1) carry = runMax;
     }
 }
 
@@ -255,12 +227,11 @@ int pda_asgn_bb_batch(const double* boxesL, const int64_t* offL, int64_t capL, c
     if (capL < 0 || capR < 0) return fail(PDA_ERR_INVALID, "asgn_bb: negative capacity");
     const int64_t wsBytes = pda_asgn_bb_workspace_bytes(nFrames, maxNL, maxBoxes);
     if (wsBytes < 0) return (int)wsBytes;
-    if (workspaceBytes < wsBytes)
-        return fail(PDA_ERR_WORKSPACE, "asgn_bb: workspace of %lld B, %lld B needed", (long long)workspaceBytes, (long long)wsBytes);
+    PDA_TRY(check_workspace("asgn_bb", workspaceBytes, wsBytes));
     if (nFrames == 0) return PDA_OK;
     const cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     const BBShapes sh = carve_bb(workspace, nFrames, maxNL, maxBoxes);
-    bb_shapes_kernel<<<1, SHAPE_THREADS, 0, s>>>(offL, capL, offR, capR, nFrames, maxNL, maxBoxes, sh, status);
+    bb_shapes_kernel<<<1, CTA_SCAN_THREADS, 0, s>>>(offL, capL, offR, capR, nFrames, maxNL, maxBoxes, sh, status);
     PDA_CUDA_TRY(cudaGetLastError());
     const unsigned blocks = (unsigned)((nFrames + WARPS - 1) / WARPS);
     bb_costs_kernel<<<blocks, 32 * WARPS, 0, s>>>(boxesL, boxesR, sh.firstL, sh.firstR, sh.numRow, sh.numCol, sh.costOff, nFrames,

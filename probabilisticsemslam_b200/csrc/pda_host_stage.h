@@ -138,7 +138,7 @@ public:
     int commit() {
         size_t declared = 0;
         for (const Item& it : items_)
-            if (it.dir != SCRATCH) declared += rounded(it.bytes);
+            if (it.dir != SCRATCH) declared += WorkspaceLayout::round(it.bytes);
         packed_ = declared <= PDA_PACKED_LIMIT;
         // in | inout | out | scratch, each in declaration order; an array used in place takes no room
         size_t used = 0;
@@ -149,7 +149,7 @@ public:
                 void* const alias = !packed_ && it.use == IN_PLACE ? mapped_alias(it.host, device_) : nullptr;
                 if (alias) { it.dev = static_cast<unsigned char*>(alias); it.host = nullptr; continue; }  // nothing to copy
                 it.off = used;
-                used += rounded(it.bytes);
+                used += WorkspaceLayout::round(it.bytes);
             }
             *ends[d] = used;
         }
@@ -212,7 +212,6 @@ private:
         size_t off; unsigned char* dev;
         bool copied() const { return host && bytes; }
     };
-    static size_t rounded(size_t bytes) { return (bytes + 255) / 256 * 256; }
     size_t add(void* host, size_t bytes, Dir dir, Use use) {
         items_.push_back({host, bytes, dir, use, 0, nullptr});
         return items_.size() - 1;

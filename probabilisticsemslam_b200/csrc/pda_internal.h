@@ -26,6 +26,32 @@ struct DeviceInfo {
 };
 int current_device_info(DeviceInfo* out);
 
+// ---- device workspaces -------------------------------------------------------------------------
+// A workspace is laid out as consecutive regions, each starting on a 256-byte boundary.  Every pipeline writes its
+// layout once, as a function that takes its regions in order from one of these: over the caller's workspace it hands out
+// the pointers, over a null base it only counts, and that count is what the pipeline's *_workspace_bytes returns.
+class WorkspaceLayout {
+public:
+    explicit WorkspaceLayout(void* base) : base_(reinterpret_cast<uintptr_t>(base)) {}
+    static size_t round(size_t bytes) { return (bytes + 255) / 256 * 256; }
+    template <class T> T* take(size_t count) {
+        T* const p = reinterpret_cast<T*>(at());
+        off_ += round(count * sizeof(T));
+        return p;
+    }
+    unsigned char* rest() const { return reinterpret_cast<unsigned char*>(at()); }  // where a chained pipeline's workspace starts
+    size_t bytes() const { return off_; }
+private:
+    uintptr_t at() const { return base_ ? base_ + off_ : 0; }
+    uintptr_t base_;
+    size_t off_ = 0;
+};
+
+inline int check_workspace(const char* who, int64_t have, int64_t need) {
+    if (have >= need) return PDA_OK;
+    return fail(PDA_ERR_WORKSPACE, "%s: workspace of %lld B, %lld B needed", who, (long long)have, (long long)need);
+}
+
 // ---- Murty k-best (murty_kernel.cu) ----------------------------------------------------------
 struct MurtyGeometry {
     int R;              // row slots per lane: numRow <= 32*R

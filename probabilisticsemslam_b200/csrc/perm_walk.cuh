@@ -334,5 +334,10 @@ __host__ __device__ inline PermShape perm_shape(int64_t nMats, int maxDim, int s
     return sh;
 }
 
+// Bytes of per-CTA partial sums that pda_permanent_workspace_bytes(nMats) provides (its arrival counters come on top).
+// launch_permanent_batch cuts perm_shape's CTAs per matrix to what fits in them; permprob_device_kernel.cu's plan_shapes
+// makes the same cut, so that it walks with the shape launch_permanent_batch would pick.
+__host__ __device__ inline long long perm_partial_bytes(long long nMats) { return 64 + 16 * ((nMats > 1 ? nMats : 1) + 8192); }
+
 }  // namespace pda
 #endif

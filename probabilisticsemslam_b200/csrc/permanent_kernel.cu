@@ -334,7 +334,7 @@ extern "C" {
 
 int64_t pda_permanent_workspace_bytes(int64_t nMats) {
     const int64_t n = std::max<int64_t>(nMats, 1);
-    return 64 + 16 * (n + 8192) + (n * 4 + 15) / 16 * 16;  // per-CTA partials + arrival counters
+    return perm_partial_bytes(n) + (n * 4 + 15) / 16 * 16;  // per-CTA partials + arrival counters
 }
 
 int pda_permanent_batch(const double* mats, const int64_t* matOff, const int32_t* rows, const int32_t* cols,

@@ -25,6 +25,7 @@
 #include "pda_host_stage.h"
 #include "perm_device.cuh"
 #include "perm_walk.cuh"
+#include "cta_scan.cuh"
 
 #include <algorithm>
 #include <vector>
@@ -37,11 +38,8 @@ constexpr int DP_MAX = 10;            // short sides the subset DP takes (PERM_D
 constexpr int SUB_DOUBLES = PDA_MAX_PERM_DIM * DP_MAX;
 constexpr int GATHER_WARPS = 4;
 constexpr int FINISH_WARPS = 4;
-constexpr int PREP_THREADS = 1024;
 constexpr int SMEM_BUDGET = 48 * 1024;
 constexpr int APPROX_TRIALS = 300;    // apprxIter (assignment.cpp:10)
-
-size_t align256(size_t x) { return (x + 255) / 256 * 256; }
 
 // Written by prep_kernel at the head of the workspace; the host never reads it.
 struct Ctrl {
@@ -77,33 +75,31 @@ Work carve(void* workspace, int mode, int64_t nUnits, int64_t totalCostElems, in
     w.slotDoubles = keptA * keptB;
     w.cpmCap = perm_shape(1, PDA_MAX_PERM_DIM, smCount, 0).ctasPerMat;  // no launch shape has more CTAs per matrix
     const size_t n = (size_t)std::max<int64_t>(nUnits, 1), c = (size_t)std::max<int64_t>(cap, 1);
-    unsigned char* b = reinterpret_cast<unsigned char*>(workspace);
-    size_t o = 0;
-    auto take = [&](size_t bytes) { unsigned char* p = b + o; o += align256(bytes); return p; };
-    w.ctrl = reinterpret_cast<Ctrl*>(take(sizeof(Ctrl)));
+    WorkspaceLayout L(workspace);
+    w.ctrl = L.take<Ctrl>(1);
     if (mode == 0) {
-        w.P = reinterpret_cast<double*>(take((size_t)totalCostElems * 8));
-        w.rowsLen = reinterpret_cast<int32_t*>(take(n * 4));
-        w.itemOff = reinterpret_cast<int64_t*>(take(n * 8));
+        w.P = L.take<double>((size_t)totalCostElems);
+        w.rowsLen = L.take<int32_t>(n);
+        w.itemOff = L.take<int64_t>(n);
     }
-    w.perm = reinterpret_cast<double*>(take(c * 8));
-    w.scale = reinterpret_cast<double*>(take(c * 8));
-    w.istat = reinterpret_cast<int32_t*>(take(c * 4));
+    w.perm = L.take<double>(c);
+    w.scale = L.take<double>(c);
+    w.istat = L.take<int32_t>(c);
     if (w.materialise) {
-        w.mRows = reinterpret_cast<int32_t*>(take(c * 4));
-        w.mCols = reinterpret_cast<int32_t*>(take(c * 4));
-        w.matOff = reinterpret_cast<int64_t*>(take(c * 8));
-        w.owner = reinterpret_cast<int32_t*>(take(c * 4));
-        w.list = reinterpret_cast<int32_t*>(take(c * 4));
-        w.negList = reinterpret_cast<int32_t*>(take(c * 4));
-        w.apStat = reinterpret_cast<int32_t*>(take(c * 4));
-        w.mats = reinterpret_cast<double*>(take(c * (size_t)w.slotDoubles * 8));
+        w.mRows = L.take<int32_t>(c);
+        w.mCols = L.take<int32_t>(c);
+        w.matOff = L.take<int64_t>(c);
+        w.owner = L.take<int32_t>(c);
+        w.list = L.take<int32_t>(c);
+        w.negList = L.take<int32_t>(c);
+        w.apStat = L.take<int32_t>(c);
+        w.mats = L.take<double>(c * (size_t)w.slotDoubles);
     }
     if (w.nw) {
-        w.partial = reinterpret_cast<dd*>(take(c * (size_t)w.cpmCap * sizeof(dd)));
-        w.done = reinterpret_cast<unsigned*>(take(c * 4));
+        w.partial = L.take<dd>(c * (size_t)w.cpmCap);
+        w.done = L.take<unsigned>(c);
     }
-    w.bytes = o;
+    w.bytes = L.bytes();
     return w;
 }
 
@@ -118,7 +114,7 @@ __device__ __forceinline__ bool out_of_scope1(int r, int c, int maxDim) { return
 __device__ void plan_shapes(Ctrl* c, long long nItems, int effDim, int smCount) {
     const long long nIt = nItems > 1 ? nItems : 1;  // a call without items walks nothing
     PermShape sh = perm_shape(nIt, effDim, smCount, 0);
-    const long long partBytes = 64 + 16 * (nIt + 8192);
+    const long long partBytes = perm_partial_bytes(nIt);
     while (sh.ctasPerMat > 1 && (long long)sh.ctasPerMat * nIt * (long long)sizeof(dd) > partBytes) sh.ctasPerMat >>= 1;
     c->mainShape = sh;
     c->retryShape = perm_shape(1, effDim, smCount, 0);
@@ -130,52 +126,30 @@ __device__ void plan_shapes(Ctrl* c, long long nItems, int effDim, int smCount) 
 
 // mode 0: itemOff[p] = sub-permanents of the problems before p (nM * (nL + 1) for nM > 1, counted for every problem in
 // scope or not), rowsLen[p] = nL + nM (0 out of scope: to_probs leaves it alone).  mode 1: only the largest dimension.
-__global__ void __launch_bounds__(PREP_THREADS) prep_kernel(int mode, const int32_t* __restrict__ a, const int32_t* __restrict__ b,
-                                                           int64_t n, int32_t maxA, int32_t maxB, int32_t* __restrict__ rowsLen,
-                                                           int64_t* __restrict__ itemOff, Ctrl* ctrl, int smCount) {
-    __shared__ long long sWarp[PREP_THREADS / 32];
-    __shared__ int sEff[PREP_THREADS / 32];
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    long long carry = 0;
-    int eff = 1;
-    for (int64_t base = 0; base < n; base += PREP_THREADS) {
-        const int64_t p = base + tid;
+__global__ void __launch_bounds__(CTA_SCAN_THREADS) prep_kernel(int mode, const int32_t* __restrict__ a, const int32_t* __restrict__ b,
+                                                               int64_t n, int32_t maxA, int32_t maxB, int32_t* __restrict__ rowsLen,
+                                                               int64_t* __restrict__ itemOff, Ctrl* ctrl, int smCount) {
+    __shared__ long long sWarp[32];
+    long long carry = 0, eff = 1;
+    for (int64_t base = 0; base < n; base += CTA_SCAN_THREADS) {
+        const int64_t p = base + threadIdx.x;
         long long add = 0;
         if (p < n) {
             const int x = a[p], y = b[p];
             if (mode == 0) {  // x = nL, y = nM
                 rowsLen[p] = out_of_scope0(x, y, maxA, maxB) ? 0 : x + y;
-                if (y > 1 && x >= 0) { add = (long long)y * (x + 1); eff = max(eff, min(PDA_MAX_PERM_DIM, x + y - 1)); }
+                if (y > 1 && x >= 0) { add = (long long)y * (x + 1); eff = max(eff, (long long)min(PDA_MAX_PERM_DIM, x + y - 1)); }
             } else {          // x = rows, y = cols
                 add = 1;
-                eff = max(eff, min(PDA_MAX_PERM_DIM, max(max(x, y), 0)));
+                eff = max(eff, (long long)min(PDA_MAX_PERM_DIM, max(max(x, y), 0)));
             }
         }
-        long long s = add;  // inclusive warp scan, then across the warps
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) { const long long v = __shfl_up_sync(FULLMASK, s, o); if (lane >= o) s += v; }
-        if (lane == 31) sWarp[warp] = s;
-        __syncthreads();
-        if (warp == 0) {
-            long long t = sWarp[lane];
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) { const long long v = __shfl_up_sync(FULLMASK, t, o); if (lane >= o) t += v; }
-            sWarp[lane] = t;
-        }
-        __syncthreads();
-        const long long before = carry + (warp ? sWarp[warp - 1] : 0) + s - add;
+        const long long before = cta_scan(add, carry, sWarp, ScanSum()) - add;
         if (mode == 0 && p < n) itemOff[p] = before;
-        carry += sWarp[PREP_THREADS / 32 - 1];
-        __syncthreads();
     }
-#pragma unroll
-    for (int o = 16; o; o >>= 1) eff = max(eff, __shfl_xor_sync(FULLMASK, eff, o));
-    if (lane == 0) sEff[warp] = eff;
-    __syncthreads();
-    if (tid == 0) {
-        for (int w = 1; w < PREP_THREADS / 32; ++w) eff = max(eff, sEff[w]);
-        plan_shapes(ctrl, carry, eff, smCount);
-    }
+    long long effMax = 1;
+    cta_scan(eff, effMax, sWarp, ScanMax());
+    if (threadIdx.x == 0) plan_shapes(ctrl, carry, (int)effMax, smCount);
 }
 
 struct GatherArgs {
@@ -518,7 +492,7 @@ int run(int mode, const double* src, const int64_t* srcOff, const int32_t* a, co
         return fail(PDA_ERR_WORKSPACE, "%s: workspace of %lld B too small (need %lld)", who, (long long)workspaceBytes, (long long)w.bytes);
     *out = w;
     const bool valid = permOpt >= 0 && permOpt <= 2;
-    prep_kernel<<<1, PREP_THREADS, 0, s>>>(mode, a, b, nUnits, maxA, maxB, w.rowsLen, w.itemOff, w.ctrl, dev.smCount);
+    prep_kernel<<<1, CTA_SCAN_THREADS, 0, s>>>(mode, a, b, nUnits, maxA, maxB, w.rowsLen, w.itemOff, w.ctrl, dev.smCount);
     PDA_CUDA_TRY(cudaGetLastError());
     GatherArgs g;
     g.mode = mode; g.permOpt = permOpt; g.a = a; g.b = b; g.itemOff = w.itemOff; g.nUnits = nUnits; g.maxA = maxA; g.maxB = maxB;

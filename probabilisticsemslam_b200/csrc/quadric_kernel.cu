@@ -16,6 +16,7 @@
 // north_star's 1e-9 relative, checked against the C restatement in oracle/ and against numpy.linalg.solve.
 #include "pda_internal.h"
 #include "pda_host_stage.h"
+#include "cta_scan.cuh"
 
 #include <algorithm>
 #include <cfloat>
@@ -124,9 +125,6 @@ __global__ void quadric_cost_kernel(const double* __restrict__ landMean, const d
 }
 
 // ---- device-pointer moments entries: frame shapes are read on the device, never on the host ----
-constexpr unsigned FULL = 0xffffffffu;
-constexpr int SHAPE_THREADS = 1024;  // one CTA; 32 warps, so the warp totals are scanned by one warp
-
 struct MomentShapes {
     int32_t* nL; int32_t* nM;            // sanitised counts: 0 / 0 for a rejected frame
     int64_t* landStart; int64_t* measStart;
@@ -137,42 +135,38 @@ struct MomentShapes {
     size_t bytes;                        // everything up to `inner`
 };
 
-size_t align256(size_t x) { return (x + 255) / 256 * 256; }
-
 MomentShapes carve_shapes(void* workspace, int64_t nFrames, int32_t maxNL, int32_t maxNM) {
     const size_t n = (size_t)std::max<int64_t>(nFrames, 1), rows = (size_t)(maxNL + maxNM);
-    unsigned char* w = reinterpret_cast<unsigned char*>(workspace);
+    WorkspaceLayout w(workspace);
     MomentShapes s;
-    size_t o = 0;
-    s.nL = reinterpret_cast<int32_t*>(w + o); o += align256(n * 4);
-    s.nM = reinterpret_cast<int32_t*>(w + o); o += align256(n * 4);
-    s.innerStatus = reinterpret_cast<int32_t*>(w + o); o += align256(n * 4);
-    s.landStart = reinterpret_cast<int64_t*>(w + o); o += align256(n * 8);
-    s.measStart = reinterpret_cast<int64_t*>(w + o); o += align256(n * 8);
-    s.costOff = reinterpret_cast<int64_t*>(w + o); o += align256(n * 8);
-    s.rowOff = reinterpret_cast<int64_t*>(w + o); o += align256(n * 8);
-    s.costs = reinterpret_cast<double*>(w + o); o += align256(n * rows * (size_t)maxNM * 8);
-    s.inner = w + o;
-    s.bytes = o;
+    s.nL = w.take<int32_t>(n);
+    s.nM = w.take<int32_t>(n);
+    s.innerStatus = w.take<int32_t>(n);
+    s.landStart = w.take<int64_t>(n);
+    s.measStart = w.take<int64_t>(n);
+    s.costOff = w.take<int64_t>(n);
+    s.rowOff = w.take<int64_t>(n);
+    s.costs = w.take<double>(n * rows * (size_t)maxNM);
+    s.inner = w.rest();
+    s.bytes = w.bytes();
     return s;
 }
 
-// One CTA walks the frames in blocks of SHAPE_THREADS.  A frame passes when its offsets are non-negative and ascending,
+// One CTA walks the frames in blocks of CTA_SCAN_THREADS.  A frame passes when its offsets are non-negative and ascending,
 // lie within landCap / measCap, and its counts are within maxNL / maxNM; probOff is the running sum of nM * (nL+1) over
 // passing frames.  A passing non-empty frame whose span ends past probCap keeps its span but is not computed (status
 // 2), so probOff stays a plain prefix sum.  Rejected frames go on as 0 x 0: the chained pipelines then touch nothing of
 // theirs.
-__global__ void __launch_bounds__(SHAPE_THREADS) moment_shapes_kernel(
+__global__ void __launch_bounds__(CTA_SCAN_THREADS) moment_shapes_kernel(
     const int64_t* __restrict__ landOff, const int64_t landCap, const int64_t* __restrict__ measOff, const int64_t measCap,
     const long long nFrames, const int32_t maxNL, const int32_t maxNM, const int64_t probCap, const MomentShapes s,
     int64_t* __restrict__ probOff, int32_t* __restrict__ status) {
-    __shared__ long long warpSum[SHAPE_THREADS / 32];
-    __shared__ long long carry;
-    const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+    __shared__ long long warpSum[32];
     const long long rows = maxNL + maxNM;
-    if (t == 0) { carry = 0; probOff[0] = 0; }
-    for (long long base = 0; base < nFrames; base += SHAPE_THREADS) {
-        const long long f = base + t;
+    long long carry = 0;
+    if (threadIdx.x == 0) probOff[0] = 0;
+    for (long long base = 0; base < nFrames; base += CTA_SCAN_THREADS) {
+        const long long f = base + threadIdx.x;
         int L = 0, M = 0;
         long long l0 = 0, m0 = 0;
         bool ok = false;
@@ -184,25 +178,7 @@ __global__ void __launch_bounds__(SHAPE_THREADS) moment_shapes_kernel(
             if (ok) { L = (int)(l1 - l0); M = (int)(m1 - m0); }
         }
         const long long span = (long long)M * (L + 1);
-        long long x = span;  // inclusive scan: warp, then the warp totals, then the carry of earlier blocks
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const long long y = __shfl_up_sync(FULL, x, o);
-            if (lane >= o) x += y;
-        }
-        if (lane == 31) warpSum[warp] = x;
-        __syncthreads();
-        if (warp == 0) {
-            long long w = warpSum[lane];
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                const long long y = __shfl_up_sync(FULL, w, o);
-                if (lane >= o) w += y;
-            }
-            warpSum[lane] = w;
-        }
-        __syncthreads();
-        const long long end = carry + (warp ? warpSum[warp - 1] : 0) + x;
+        const long long end = cta_scan(span, carry, warpSum, ScanSum());
         if (f < nFrames) {
             if (span > 0 && end > probCap) { ok = false; L = M = 0; }
             s.nL[f] = L; s.nM[f] = M;
@@ -211,8 +187,6 @@ __global__ void __launch_bounds__(SHAPE_THREADS) moment_shapes_kernel(
             probOff[f + 1] = end;
             status[f] = ok ? 0 : 2;
         }
-        __syncthreads();  // every thread has read carry and warpSum
-        if (t == SHAPE_THREADS - 1) carry = end;
     }
 }
 
@@ -401,8 +375,8 @@ static int launch_moment_costs(const double* landMean, const double* landCov, co
                                const double* measMean, const double* measCov, const int64_t* measOff, int64_t measCapacity,
                                int64_t nFrames, int32_t maxNL, int32_t maxNM, double nonassign, int64_t probCapacity,
                                const MomentShapes& sh, int64_t* probOff, int32_t* status, cudaStream_t s) {
-    moment_shapes_kernel<<<1, SHAPE_THREADS, 0, s>>>(landOff, landCapacity, measOff, measCapacity, nFrames, maxNL, maxNM,
-                                                    probCapacity, sh, probOff, status);
+    moment_shapes_kernel<<<1, CTA_SCAN_THREADS, 0, s>>>(landOff, landCapacity, measOff, measCapacity, nFrames, maxNL, maxNM,
+                                                       probCapacity, sh, probOff, status);
     PDA_CUDA_TRY(cudaGetLastError());
     if (nFrames == 0) return PDA_OK;
     quadric_cost_shaped_kernel<<<(unsigned)((nFrames + QWARPS - 1) / QWARPS), 32 * QWARPS, 0, s>>>(
@@ -436,9 +410,7 @@ int pda_association_from_moments_batch(const double* landMean, const double* lan
     if (landCapacity < 0 || measCapacity < 0) return fail(PDA_ERR_INVALID, "association_from_moments: negative capacity");
     const int64_t wsBytes = pda_association_from_moments_workspace_bytes(nFrames, maxNL, maxNM, probCapacity, k);
     if (wsBytes < 0) return (int)wsBytes;
-    if (workspaceBytes < wsBytes)
-        return fail(PDA_ERR_WORKSPACE, "association_from_moments: workspace of %lld B, %lld B needed", (long long)workspaceBytes,
-                    (long long)wsBytes);
+    PDA_TRY(check_workspace("association_from_moments", workspaceBytes, wsBytes));
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     const MomentShapes sh = carve_shapes(workspace, nFrames, maxNL, maxNM);
     PDA_TRY(launch_moment_costs(landMean, landCov, landOff, landCapacity, measMean, measCov, measOff, measCapacity, nFrames, maxNL,
@@ -470,9 +442,7 @@ int pda_association_perm_from_moments_batch(const double* landMean, const double
     if (landCapacity < 0 || measCapacity < 0) return fail(PDA_ERR_INVALID, "association_perm_from_moments: negative capacity");
     const int64_t wsBytes = pda_association_perm_from_moments_workspace_bytes(nFrames, maxNL, maxNM, probCapacity);
     if (wsBytes < 0) return (int)wsBytes;
-    if (workspaceBytes < wsBytes)
-        return fail(PDA_ERR_WORKSPACE, "association_perm_from_moments: workspace of %lld B, %lld B needed",
-                    (long long)workspaceBytes, (long long)wsBytes);
+    PDA_TRY(check_workspace("association_perm_from_moments", workspaceBytes, wsBytes));
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     const MomentShapes sh = carve_shapes(workspace, nFrames, maxNL, maxNM);
     PDA_TRY(launch_moment_costs(landMean, landCov, landOff, landCapacity, measMean, measCov, measOff, measCapacity, nFrames, maxNL,

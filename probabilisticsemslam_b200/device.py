@@ -11,7 +11,7 @@ import numpy as np
 import torch
 
 from . import api
-from ._lib import check, lib
+from ._lib import alloc_workspace, check, lib
 from .synth import ProblemBatch
 
 
@@ -166,10 +166,8 @@ class PermanentProbPlan:
         self.cost_off, self.nL, self.nM, self.prob_off = up(pb.cost_off.astype(np.int64)), up(self.nL_h), up(self.nM_h), up(self.prob_off_h)
         self.probs = torch.zeros(max(self.total_prob, 1), dtype=torch.float64, device=dev)
         self.status = torch.empty(self.n, dtype=torch.int32, device=dev)
-        ws = int(lib().pda_permanent_prob_workspace_bytes(self.n, int(self.costs.numel()), self.total_prob, self.max_row,
-                                                          self.max_col, self.perm_opt))
-        check(min(ws, 0))
-        self.workspace = torch.empty(ws, dtype=torch.uint8, device=dev)
+        self.workspace = alloc_workspace(lib().pda_permanent_prob_workspace_bytes(self.n, int(self.costs.numel()), self.total_prob,
+                                                                                  self.max_row, self.max_col, self.perm_opt), dev)
 
     def run(self):
         api.permanent_prob_batch_device(self.costs, self.cost_off, self.nL, self.nM, self.prob_off, self.total_prob,
@@ -198,9 +196,7 @@ class ConditionedPermanentPlan:
         self.rows, self.cols = up(rows), up(cols)
         self.out = torch.zeros(self.n, dtype=torch.float64, device=dev)
         self.status = torch.empty(self.n, dtype=torch.int32, device=dev)
-        ws = int(lib().pda_conditioned_permanent_workspace_bytes(self.n, self.max_dim, self.perm_opt))
-        check(min(ws, 0))
-        self.workspace = torch.empty(ws, dtype=torch.uint8, device=dev)
+        self.workspace = alloc_workspace(lib().pda_conditioned_permanent_workspace_bytes(self.n, self.max_dim, self.perm_opt), dev)
 
     def run(self):
         api.conditioned_permanent_batch_device(self.mats, self.mat_off, self.rows, self.cols, self.max_dim, self.perm_opt,
