@@ -416,7 +416,10 @@ int pda_permanent_sharded_host(const double* A, int32_t n, const int32_t* device
 /* Huber's randomised approximation of the permanent: permanentApproximation / permanentApproximationSquare with their
  * sinkhorn / hl_factor / pickRowFromProbs helpers (nwPerm.h:27-35, nwPerm.cpp:36-211), `iterations` acceptance /
  * rejection trials per matrix (the reference uses apprxIter = 300, assignment.cpp:10).  Rectangular input is padded with
- * ones and divided by (|rows-cols|)!; status[i] = 1 above dimension 32.  The reference draws from an unseeded global
+ * ones and divided by (|rows-cols|)!; status[i] = 1 (estimate 0) above dimension 32 or where a dimension is negative
+ * (the _host form returns PDA_ERR_INVALID for a negative dimension instead).  A matrix that Sinkhorn cannot balance -- a
+ * zero row or column, an inf or NaN entry, a column of subnormals only -- runs the full 100 000 Sinkhorn iterations, as
+ * the reference does, and gives NaN with status 0.  The reference draws from an unseeded global
  * rand(); here every draw is a counter-based value keyed by (seed, matrix index, trial, column), so results are
  * reproducible and independent of batch order -- agreement with the reference is statistical (same estimator, same
  * trial count), not sample for sample.  pda_set_approx_seed sets the seed used where the reference signature has no

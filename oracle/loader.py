@@ -48,6 +48,9 @@ class CpuChecker:
         f("asgn_bb", None, [_ptr, C.c_long, _ptr, C.c_long, _dbl, _ptr])
         if prefix == "orc":  # restatement only: needs Eigen on the reference side (oracle_quadric.c)
             f("permanent_approx", _dbl, [_ptr, _i64, _i64, _i64, C.c_uint64, _i64, _ptr])
+            f("approx_near_ties_reset", None, [])
+            f("approx_near_ties", _i64, [])
+            f("set_approx_stream", None, [C.c_uint64, _i64])
             f("kbest2d_cutoff_pruned", _i64, [_i64, _i64, _i64, _int, _ptr, _ptr, _ptr, _ptr, _dbl, _i64, _ptr])
             f("quadric_covs", None, [_ptr, _i64, _ptr])
             f("quadric_cost_matrix", None, [_ptr, _ptr, _i64, _ptr, _ptr, _i64, _dbl, _ptr])
@@ -192,11 +195,29 @@ class CpuChecker:
         return out[:bl.shape[0]]
 
     # ---- Huber's approximate permanent (restatement only; counter-based draws shared with the CUDA kernel) ----
-    def permanent_approx(self, a, iterations=300, seed=20260217, mat_index=0):
+    def permanent_approx(self, a, iterations=300, seed=20260217, mat_index=0, near_ties=False):
+        """-> (estimate, successes), or with near_ties=True (estimate, successes, near ties): the number of draws that lay
+        within 1e-12 of a partial sum they were compared with, i.e. how many trials the CUDA kernel may decide the other
+        way (oracle_perm_approx.c)."""
         a = np.asfortranarray(a, dtype=np.float64)
         succ = C.c_int64(0)
+        self._approx_near_ties_reset()
         est = self._permanent_approx(_p(a), a.shape[0], a.shape[1], int(iterations), int(seed), int(mat_index), C.byref(succ))
+        if near_ties:
+            return float(est), int(succ.value), int(self._approx_near_ties())
         return float(est), int(succ.value)
+
+    def approx_near_ties_reset(self):
+        """Zero this thread's near-tie counter (it also counts the draws of permanent_prob / conditioned_permanent with
+        perm_opt 0)."""
+        self._approx_near_ties_reset()
+
+    def approx_near_ties(self) -> int:
+        return int(self._approx_near_ties())
+
+    def set_approx_stream(self, seed=20260217, index=0):
+        """The stream (seed, matrix index) the next conditioned_permanent(.., 0) on this thread draws from."""
+        self._set_approx_stream(int(seed), int(index))
 
     # ---- cost matrices from quadric moments (restatement only) ---------------------------
     def quadric_covs(self, quadrics):

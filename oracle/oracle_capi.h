@@ -68,6 +68,10 @@ int orc_association_probs(const double* costs, int64_t nL, int64_t nM, int64_t k
  * in place of the reference's unseeded rand().  No `ref_` twin. */
 double orc_permanent_approx(const double* A, int64_t rows, int64_t cols, int64_t iterations, uint64_t seed, int64_t matIndex,
                             int64_t* successesOut);
+/* draws of orc_permanent_approx on this thread (conditionedPermanent / permanentProb with permOpt 0 included) that lay
+ * within 1e-12 of a partial sum they were compared with: where the kernel may pick differently (oracle_perm_approx.c) */
+void orc_approx_near_ties_reset(void);
+int64_t orc_approx_near_ties(void);
 /* which stream the next conditionedPermanent(.., permOpt = 0) draws from (thread-local index) */
 void orc_set_approx_stream(uint64_t seed, int64_t index);
 

@@ -8,6 +8,12 @@
  * depends on everything called before, so there is no reference sample to reproduce.  The draw of (matrix, trial,
  * column) is the same counter-based splitmix64 value the CUDA kernel uses (permanent_approx_kernel.cu: draw01), which
  * makes the two comparable trial for trial; agreement with the reference itself is statistical (same estimator).
+ *
+ * Near ties.  The kernel forms the same partial sums in another association (a warp prefix sum), and its products over
+ * rows and its log() differ from these by a few ulp, so a trial can go the other way only where a draw lies within
+ * rounding of a partial sum it was compared with.  Every such draw -- within NEAR_TIE of the sum that reached it or of the
+ * one before it, or of the total when no row was picked -- is counted in a thread-local counter
+ * (orc_approx_near_ties); a success count that differs from the kernel's by more than that count is a real difference.
  */
 #include <math.h>
 #include <stdint.h>
@@ -28,6 +34,11 @@ static double draw01(uint64_t seed, int64_t mat, int trial, int col) {
     const uint64_t x = mix64(key + 0x9E3779B97F4A7C15ULL * ((uint64_t)trial * 64ULL + (uint64_t)col + 1ULL));
     return (double)(x >> 11) * (1.0 / 9007199254740992.0);
 }
+static const double NEAR_TIE = 1e-12;
+static __thread int64_t g_nearTies = 0;
+void orc_approx_near_ties_reset(void) { g_nearTies = 0; }
+int64_t orc_approx_near_ties(void) { return g_nearTies; }
+
 static double hl(double x) { return (x > 1.0) ? x + 0.5 * log(x) + EE - 1.0 : 1.0 + (EE - 1.0) * x; }
 
 /* A: rows x cols column-major.  successesOut (optional) receives the number of accepted trials. */
@@ -91,8 +102,9 @@ double orc_permanent_approx(const double* A, int64_t rows, int64_t cols, int64_t
                 prob[j] = (hl2All / hlAll) * EE * (ccol / h2[j]);
             }
             const double u = draw01(seed, matIndex, (int)trial, column);
-            double sum = 0; int pick;
-            for (pick = 0; pick < n; pick++) { sum += prob[pick]; if (sum >= u) break; }
+            double sum = 0, before = 0; int pick;
+            for (pick = 0; pick < n; pick++) { before = sum; sum += prob[pick]; if (sum >= u) break; }
+            if (fabs(sum - u) <= NEAR_TIE || (pick < n && fabs(before - u) <= NEAR_TIE)) g_nearTies++;
             if (pick >= n) { column = n + 1; break; }
             for (int j = 0; j < n; j++) rowSum[j] = rowSum[j] - (alive[j] ? C[j + (size_t)column * n] : 0.0);
             alive[pick] = 0; rowSum[pick] = 0;

@@ -16,7 +16,7 @@
 // batch order, and the CPU restatement in oracle/oracle_perm_approx.c uses the same stream.  What is checked: against the
 // restatement (same draws; the two differ only when a pick falls within rounding of a cumulative sum), and against
 // the exact permanent within the estimator's own binomial standard error.  Matrices above dimension 32 get status 1
-// (the reference has no such limit; the exact path has, nwPerm.cpp:329).
+// (the reference has no such limit; the exact path has, nwPerm.cpp:329), and so do matrices with a negative dimension.
 #include "pda_internal.h"
 #include "pda_host_stage.h"
 
@@ -35,11 +35,6 @@ constexpr double EE = 2.71828182846;  // the reference's constant (nwPerm.cpp:88
 __device__ __forceinline__ double warp_prod(double x) {
 #pragma unroll
     for (int o = 16; o; o >>= 1) x *= __shfl_xor_sync(FULL, x, o);
-    return x;
-}
-__device__ __forceinline__ double warp_maxd(double x) {
-#pragma unroll
-    for (int o = 16; o; o >>= 1) { const double y = __shfl_xor_sync(FULL, x, o); x = (x < y) ? y : x; }
     return x;
 }
 // hl_factor (nwPerm.cpp:80-97)
@@ -73,7 +68,7 @@ __global__ void __launch_bounds__(32 * AW) permanent_approx_kernel(const ApproxA
     if (m >= a.nMats) return;
     const int rows = a.rows[m], cols = a.cols[m];
     const int n = rows > cols ? rows : cols;
-    if (n > PDA_MAX_PERM_DIM || n < 0) {
+    if (rows < 0 || cols < 0 || n > PDA_MAX_PERM_DIM) {
         if (lane == 0) { a.out[m] = 0.0; if (a.status) a.status[m] = 1; }
         return;
     }
@@ -101,8 +96,10 @@ __global__ void __launch_bounds__(32 * AW) permanent_approx_kernel(const ApproxA
         for (int iter = 0; iter < 100000; ++iter) {
             double cinv = 0.0;
             for (int j = 0; j < n; ++j) { const double rj = __shfl_sync(FULL, r, j); if (live) cinv += rj * C[j + lane * LD]; }
-            const double err = warp_maxd(live ? fabs(cinv * c - 1.0) : 0.0);
-            if (err <= 1e-4) break;  // NaN compares false and keeps iterating, like the reference
+            // One decision for the whole warp: stop only when every live column is within 1e-4 and none is NaN, like the
+            // restatement.  A degenerate matrix (zero line, inf or NaN entry) therefore runs all 100 000 iterations.
+            const double e = fabs(cinv * c - 1.0);
+            if (!__any_sync(FULL, live && !(e <= 1e-4))) break;
             c = live ? 1.0 / cinv : 1.0;
             s = 0.0;
             for (int k = 0; k < n; ++k) { const double ck = __shfl_sync(FULL, c, k); if (live) s += C[lane + k * LD] * ck; }

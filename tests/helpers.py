@@ -22,6 +22,27 @@ def kbest_cases(z):
         yield z[f"C{i}"], int(z[f"n{i}"]), z[f"r{i}"].astype(np.int64), z[f"c{i}"].astype(np.int64), z[f"g{i}"]
 
 
+def check_approx_rule(g, restated, iterations, what="", shape=None):
+    """Holds the CUDA approximate permanent's estimate g to its CPU restatement's (estimate, successes, near ties) with
+    the same draws.  K = estimate * iterations / successes; the kernel's successes round(g * iterations / K) must equal
+    the restatement's give or take its near ties (draws within 1e-12 of a partial sum they were compared with, where
+    the kernel's reassociated sums may decide the other way), and where they are equal, |g / estimate - 1| <= 1e-12."""
+    est, succ, ties = restated
+    what = f"{what} {shape}: kernel {g!r}, restatement {est!r} ({succ} of {iterations}, {ties} near ties)"
+    assert np.isnan(g) == np.isnan(est), what
+    if np.isnan(est):
+        return
+    if shape == (0, 0):
+        assert g == est == 1.0, what
+    elif succ == 0:
+        assert g == 0.0 or ties > 0, what
+    else:
+        s = round(g * iterations / (est * iterations / succ))
+        assert abs(s - succ) <= ties, what
+        if s == succ:
+            assert abs(g / est - 1.0) <= 1e-12, what
+
+
 def bits(a):
     return np.ascontiguousarray(a, dtype=np.float64).view(np.int64)
 
