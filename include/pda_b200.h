@@ -207,7 +207,24 @@ int pda_to_probs_batch_host(double* values, const int64_t* off, const int64_t* l
  * per detection (:51-53).  rowOff = prefix sums of (nL+nM); the total* arguments size the intermediates.
  * The bounds must satisfy 1 <= maxNumCol <= maxNumRow <= PDA_MAX_DIM (else PDA_ERR_INVALID / PDA_ERR_UNSUPPORTED before
  * anything is launched); a problem with nL+nM > maxNumRow or nM > maxNumCol is skipped: nFound[p] = -1 and its table
- * is zeros (ones where nL == 0).
+ * is zeros (ones where nL == 0).  A problem in which conditioning keeps fewer rows than there are detections
+ * (goodRows < nM: the usePerm form's status 3) is not solved either: nFound[p] = -1 and its table is all zero.  A
+ * solved row sums to 1, and a conditioned problem with no feasible assignment (nFound = 0; possible with goodRows >= nM
+ * once dummy rows are gated away) gives NaN in its rows' non-assignment entries, as the reference's 0/0 does; so an
+ * all-zero row marks the goodRows < nM case and no other.  The single-frame entries (api.getAssignmentProbs /
+ * getAssignmentProbsFromCosts and the C++ shim's getAssignmentProbsFromCosts / getAssignmentProbsFromMoments, usePerm
+ * false) raise for it as their usePerm forms do; they return the infeasible case's table as the reference does.
+ * Shape domain: nL >= 0, 1 <= nM, nL + nM <= PDA_MAX_DIM, and the Murty kernel must take the call's bounds with weights
+ * (on a B200, 227 KB of shared memory per block: (nL+nM) * nM <= 14352, so 128 x 112 runs and 128 x 113 does not).
+ * The _host forms (and pda_association_from_moments_batch_host and the _multi forms, which run them per slice) take
+ * those bounds as the largest nL+nM and the largest nM over the frames with nL >= 1: frames with no landmarks never
+ * reach the kernel and may have any nM up to PDA_MAX_DIM.  When the kernel cannot take the bounds, the call returns
+ * PDA_ERR_UNSUPPORTED before any launch, naming the first frame it cannot take alone by its index in the caller's batch
+ * (the _multi form too), or, when each frame fits alone, the two bounds that do not fit together (in the _multi form,
+ * those of one device's slice).
+ * A dummy row gated away (nonassign > colMin + 42) with goodRows >= nM is computed as the reference does; the two
+ * weight paths then differ (the reference's gates differ), so the k-best and usePerm tables agree, and equal the exact
+ * association marginals, only where no dummy row is gated away.
  */
 int64_t pda_association_workspace_bytes(int64_t nProblems, int64_t totalCostElems, int64_t totalRows,
                                         int64_t totalProbElems, int32_t k, int32_t maxNumRow, int32_t maxNumCol);

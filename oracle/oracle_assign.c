@@ -202,9 +202,12 @@ int orc_association_probs(const double* costs, int64_t nL, int64_t nM, int64_t k
     int64_t* rowIdx = (int64_t*)malloc((size_t)nR * sizeof(int64_t));
     const int64_t good = orc_condition_costs(costs, nR, nM, cond, rowIdx);
     const int64_t condL = good - nM; /* (conditionedCosts.size()/nM) - nM (:60) */
+    for (int64_t i = 0; i < nM * W; i++) probs[i] = 0;
+    /* fewer kept rows than detections: the reference's size_t subtraction underflows; status 3 and a zero table, as
+     * the device pipelines report it */
+    if (condL < 0) { free(cond); free(rowIdx); return 3; }
     double* cp = (double*)malloc((size_t)(nM * (condL + 1)) * sizeof(double));
     int status = usePerm ? orc_permanent_prob(cond, condL, nM, 1, cp) : orc_assignment_prob(cond, condL, nM, k, cp);
-    for (int64_t i = 0; i < nM * W; i++) probs[i] = 0;
     if (!status)
         for (int64_t m = 0; m < nM; m++) {
             for (int64_t l = 0; l < condL; l++) probs[m * W + rowIdx[l]] = cp[m * (condL + 1) + l];

@@ -430,13 +430,21 @@ def getCovs(quadrics: np.ndarray, device: int = 0) -> np.ndarray:
     return out.reshape(-1, 3, 3)
 
 
+def _kbest_table_or_raise(tab: np.ndarray, who: str) -> np.ndarray:
+    """A k-best table whose frame was computed has every row summing to 1; an all-zero row is the frame in which
+    conditioning kept fewer rows than detections (nFound = -1), which the usePerm form reports as status 3."""
+    if tab.size and not np.any(tab, axis=1).all():
+        raise RuntimeError(f"{who}: the reference throws for this input (status 3)")
+    return tab
+
+
 def getAssignmentProbs(land_mean, land_cov, meas_mean, meas_cov, nonassign: float, k: int, device: int = 0,
                        usePerm: bool = False) -> np.ndarray:
     """The reference's SLAM entry point (assignment.cpp:38-74) on the moments getMeans/getCovs return; usePerm selects
     the permanent-based weights (:64) over the k-best ones.  Raises where the reference throws."""
     frame = [(land_mean, land_cov, meas_mean, meas_cov)]
     if not usePerm:
-        return association_from_moments_batch(frame, nonassign, k, device)[0]
+        return _kbest_table_or_raise(association_from_moments_batch(frame, nonassign, k, device)[0], "getAssignmentProbs")
     tabs, st = association_perm_from_moments_batch(frame, nonassign, device)
     if st[0]:
         raise RuntimeError(f"getAssignmentProbs: the reference throws for this input (status {int(st[0])})")
@@ -605,7 +613,7 @@ def getAssignmentProbsFromCosts(C: np.ndarray, nL: int, k: int, usePerm: bool = 
     """assignment.cpp:57-74: what getAssignmentProbs does once computeQuadricCostMatrix has produced C."""
     C = np.asarray(C, np.float64)
     if not usePerm:
-        return association_probs_batch(_one(C, nL), k, device)[0].copy()
+        return _kbest_table_or_raise(association_probs_batch(_one(C, nL), k, device)[0].copy(), "getAssignmentProbsFromCosts")
     tabs, st = association_perm_probs_batch(_one(C, nL), device)
     if st[0]:
         raise RuntimeError(f"getAssignmentProbsFromCosts: the reference throws for this input (status {int(st[0])})")

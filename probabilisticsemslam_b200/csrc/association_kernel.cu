@@ -62,6 +62,29 @@ AssocWorkspace carve(void* workspace, int64_t nProblems, int64_t totalCostElems,
 }
 
 }  // namespace
+
+// The k-best _host forms size the Murty kernel once for the whole batch: the largest nL+nM and the largest nM over the
+// frames that reach it (nL >= 1; frames with no landmarks are {1} per detection and never see a LAP).  When the kernel
+// cannot take that geometry, the call fails with the first frame it cannot take on its own, or, when every frame fits
+// alone, with the two largest dimensions that do not fit together.
+int check_association_geometry(const int32_t* nL, const int32_t* nM, size_t n, int32_t k, int maxR, int maxC,
+                               int64_t frameBase) {
+    DeviceInfo dev;
+    PDA_TRY(current_device_info(&dev));
+    MurtyGeometry g;
+    const int rc = murty_geometry(k, maxR, maxC, true, dev, &g);
+    if (rc != PDA_ERR_UNSUPPORTED) return rc;
+    for (size_t p = 0; p < n; ++p) {
+        const int L = nL[p], M = nM[p];
+        if (L < 1 || M < 1) continue;
+        if (murty_geometry(k, L + M, M, true, dev, &g) == PDA_ERR_UNSUPPORTED)
+            return fail(PDA_ERR_UNSUPPORTED, "association: frame %lld (nL=%d, nM=%d) is beyond the Murty kernel at k=%d "
+                        "(a %d x %d problem with weights)", (long long)(frameBase + (int64_t)p), L, M, k, L + M, M);
+    }
+    return fail(PDA_ERR_UNSUPPORTED, "association: every frame fits the Murty kernel alone, but the batch's largest nL+nM "
+                "(%d) and largest nM (%d) at k=%d do not fit together; split the batch", maxR, maxC, k);
+}
+
 }  // namespace pda
 
 using namespace pda;
@@ -109,6 +132,16 @@ int pda_association_probs_batch(const double* costs, const int64_t* costOff, con
 int pda_association_probs_batch_host(const double* costs, const int64_t* costOff, const int32_t* nL, const int32_t* nM,
                                      int64_t nProblems, int32_t k, double* probs, const int64_t* probOff,
                                      int32_t device) {
+    return association_probs_host(costs, costOff, nL, nM, nProblems, k, probs, probOff, device, 0);
+}
+
+}  // extern "C"
+
+// pda_association_probs_batch_host on a slice of a caller's batch that starts at frame frameBase (the _multi form):
+// errors name frames by their index in the caller's batch
+int pda::association_probs_host(const double* costs, const int64_t* costOff, const int32_t* nL, const int32_t* nM,
+                                int64_t nProblems, int32_t k, double* probs, const int64_t* probOff, int32_t device,
+                                int64_t frameBase) {
     if (nProblems < 0) return fail(PDA_ERR_INVALID, "association: nProblems < 0");
     if (nProblems == 0) return PDA_OK;
     if (!costs || !costOff || !nL || !nM || !probs || !probOff) return fail(PDA_ERR_INVALID, "association: NULL argument");
@@ -124,10 +157,11 @@ int pda_association_probs_batch_host(const double* costs, const int64_t* costOff
         nRows += (size_t)(L + M);
         nCost = std::max(nCost, (size_t)costOff[p] + (size_t)(L + M) * M);
         nProb = std::max(nProb, (size_t)probOff[p] + (size_t)M * (L + 1));
-        maxR = std::max(maxR, L + M); maxC = std::max(maxC, M);
+        if (L > 0) { maxR = std::max(maxR, L + M); maxC = std::max(maxC, M); }
     }
     DeviceScope scope;
     PDA_TRY(scope.enter(device));
+    PDA_TRY(check_association_geometry(nL, nM, n, k, maxR, maxC, frameBase));
     const int64_t wsBytes = pda_association_workspace_bytes(nProblems, (int64_t)nCost, (int64_t)nRows, (int64_t)nProb, k, maxR, maxC);
     if (wsBytes < 0) return (int)wsBytes;
     HostIO io(device);
@@ -142,5 +176,3 @@ int pda_association_probs_batch_host(const double* costs, const int64_t* costOff
                                         io.stream()));
     return io.download();
 }
-
-}  // extern "C"

@@ -458,8 +458,8 @@ int pda_association_probs_batch_host_multi(const double* costs, const int64_t* c
     if (!costs || !costOff || !nL || !nM || !probs || !probOff) return fail(PDA_ERR_INVALID, "association: NULL argument");
     return run_slices(costOff, probOff, nProblems, devices, nDevices, "association (multi)",
                       [&](int64_t p0, int64_t p1, int dev, const int64_t* co, const int64_t* po) {
-                          return pda_association_probs_batch_host(costs + costOff[p0], co, nL + p0, nM + p0, p1 - p0, k,
-                                                                  probs + probOff[p0], po, dev);
+                          return association_probs_host(costs + costOff[p0], co, nL + p0, nM + p0, p1 - p0, k,
+                                                        probs + probOff[p0], po, dev, p0);
                       });
 }
 

@@ -78,6 +78,14 @@ struct MurtyGeometry {
 };
 int murty_geometry(int32_t k, int32_t maxNumRow, int32_t maxNumCol, bool weights, const DeviceInfo& dev,
                    MurtyGeometry* g);
+// PDA_OK when the k-best association pipeline can run frames nL[0..n) x nM[0..n) at the bounds maxR x maxC (taken over
+// the frames with nL >= 1); otherwise PDA_ERR_UNSUPPORTED naming a frame, numbered from frameBase (association_kernel.cu)
+int check_association_geometry(const int32_t* nL, const int32_t* nM, size_t n, int32_t k, int maxR, int maxC,
+                               int64_t frameBase);
+// pda_association_probs_batch_host on frames numbered from frameBase in its error messages (the _multi form's slices)
+int association_probs_host(const double* costs, const int64_t* costOff, const int32_t* nL, const int32_t* nM,
+                           int64_t nProblems, int32_t k, double* probs, const int64_t* probOff, int32_t device,
+                           int64_t frameBase);
 
 struct MurtyArgs {
     const double* costs; const int64_t* costOff; const int32_t* numRow; const int32_t* numCol;

@@ -288,7 +288,7 @@ static int quadric_shapes(const int64_t* landOff, const int64_t* measOff, int64_
                                              (long long)f, (long long)L, (long long)M, PDA_MAX_DIM);
         costOff[f] = (int64_t)nCost; probOff[f] = (int64_t)nProb; rowOff[f] = (int64_t)nRows;
         nCost += (size_t)((L + M) * M); nProb += (size_t)(M * (L + 1)); nRows += (size_t)(L + M);
-        maxR = std::max(maxR, (int)(L + M)); maxC = std::max(maxC, (int)M);
+        if (L > 0 && M > 0) { maxR = std::max(maxR, (int)(L + M)); maxC = std::max(maxC, (int)M); }  // the frames Murty sees
     }
     return PDA_OK;
 }
@@ -338,6 +338,9 @@ int pda_association_from_moments_batch_host(const double* landMean, const double
     if (nProb == 0) return PDA_OK;
     DeviceScope scope;
     PDA_TRY(scope.enter(device));
+    std::vector<int32_t> frameNL(n), frameNM(n);
+    for (size_t f = 0; f < n; ++f) { frameNL[f] = (int32_t)(landOff[f + 1] - landOff[f]); frameNM[f] = (int32_t)(measOff[f + 1] - measOff[f]); }
+    PDA_TRY(check_association_geometry(frameNL.data(), frameNM.data(), n, k, maxR, maxC, 0));
     const int64_t wsBytes = pda_association_workspace_bytes(nFrames, (int64_t)nCost, (int64_t)nRows, (int64_t)nProb, k, maxR, maxC);
     if (wsBytes < 0) return (int)wsBytes;
     HostIO io(device);

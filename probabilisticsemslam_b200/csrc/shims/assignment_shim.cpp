@@ -83,6 +83,16 @@ static void permStatusCheck(int32_t status) {
                                  "= goodRows - nM is negative (the reference's size_t subtraction underflows)");
 }
 
+// a k-best table with an all-zero row: conditioning kept fewer rows than detections (every computed row sums to 1), the
+// case the usePerm pipeline reports as status 3
+static void kbestZeroRowCheck(const std::vector<double>& probs, size_t nM, size_t width) {
+    for (size_t m = 0; m < nM; m++) {
+        bool zero = true;
+        for (size_t l = 0; l < width && zero; l++) zero = probs[m * width + l] == 0.0;
+        if (zero) permStatusCheck(3);
+    }
+}
+
 std::vector<std::vector<double> > getAssignmentProbsFromCosts(const std::vector<double>& costMatrix, size_t nL, size_t nM,
                                                               size_t k, bool usePerm) {
     if (nM == 0) return std::vector<std::vector<double> >();
@@ -93,6 +103,7 @@ std::vector<std::vector<double> > getAssignmentProbsFromCosts(const std::vector<
         pdaCheck(pda_association_probs_batch_host(costMatrix.data(), &costOff, &nl, &nm, 1, int32_t(k), probs.data(), &probOff,
                                                   pdaShimDevice()),
                  "getAssignmentProbsFromCosts");
+        kbestZeroRowCheck(probs, nM, nL + 1);
         return unflatten(probs, nM, nL + 1);
     }
     const int64_t costOff = 0, probOff = 0;  // usePerm: the fused permanent pipeline
@@ -132,6 +143,7 @@ std::vector<std::vector<double> > getAssignmentProbsFromMoments(const std::vecto
     pdaCheck(pda_association_from_moments_batch_host(landMeans.data(), landCovs.data(), offL, measMeans.data(), measCovs.data(), offM, 1,
                                                      nonassign, int32_t(k), probs.data(), pdaShimDevice()),
              "getAssignmentProbsFromMoments");
+    kbestZeroRowCheck(probs, nM, nL + 1);
     return unflatten(probs, nM, nL + 1);
 }
 

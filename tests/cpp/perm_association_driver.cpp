@@ -1,10 +1,11 @@
 // perm_association_driver.cpp -- the usePerm forms of the C++ drop-in layer (include/assignment.h) from a C++ caller:
 // getAssignmentProbsFromMoments(.., usePerm = true), getAssignmentProbsFromCosts(.., usePerm = true) and the batch form
-// getAssignmentProbsBatch.  Reads "nFrames nonassign" and then, per frame, "nL nM" and the flattened moments (landmark
+// getAssignmentProbsBatch; with the argument "kbest", the same calls with usePerm = false.  Reads "nFrames nonassign" and then, per frame, "nL nM" and the flattened moments (landmark
 // means, landmark covariances, detection means, detection covariances; covariances column-major) from stdin, and prints
 // every table at full precision; tests/test_gpu_association_perm.py compares them with the Python face of the library.
 #include <cstdio>
 #include <exception>
+#include <string>
 #include <vector>
 
 #include "assignment.h"
@@ -17,7 +18,8 @@ static void print_table(const char* kind, size_t f, const std::vector<std::vecto
     }
 }
 
-int main() {
+int main(int argc, char** argv) {
+    const bool usePerm = !(argc > 1 && std::string(argv[1]) == "kbest");
     size_t nFrames;
     double nonassign;
     if (scanf("%zu %lf", &nFrames, &nonassign) != 2) return 2;
@@ -33,13 +35,13 @@ int main() {
             for (double& x : lc) if (scanf("%lf", &x) != 1) return 2;
             for (double& x : mm) if (scanf("%lf", &x) != 1) return 2;
             for (double& x : mc) if (scanf("%lf", &x) != 1) return 2;
-            print_table("moments", f, getAssignmentProbsFromMoments(lm, lc, mm, mc, nonassign, k, true));
+            print_table("moments", f, getAssignmentProbsFromMoments(lm, lc, mm, mc, nonassign, k, usePerm));
             costs[f] = computeQuadricCostMatrixRaw(lm, lc, mm, mc, nonassign);
             nLs[f] = nL;
             nMs[f] = nM;
-            print_table("costs", f, getAssignmentProbsFromCosts(costs[f], nL, nM, k, true));
+            print_table("costs", f, getAssignmentProbsFromCosts(costs[f], nL, nM, k, usePerm));
         }
-        const std::vector<std::vector<std::vector<double> > > batch = getAssignmentProbsBatch(costs, nLs, nMs, k, true);
+        const std::vector<std::vector<std::vector<double> > > batch = getAssignmentProbsBatch(costs, nLs, nMs, k, usePerm);
         for (size_t f = 0; f < nFrames; f++) print_table("batch", f, batch[f]);
     } catch (const std::exception& e) {
         printf("throw %s\n", e.what());
