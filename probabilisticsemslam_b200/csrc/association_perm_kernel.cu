@@ -8,8 +8,8 @@
 //                              and runs the subset DP there -- nothing is materialised in global memory.  A batch too
 //                              small to fill the chip (a single SLAM frame) spreads each problem over blockIdx.y too
 //   4. finish_scatter_kernel   one warp per problem: |P(l,m) * perm|, column sums, normalisation by the largest column
-//                              sum (finish_kernel of permprob_device_kernel.cu), written straight into the caller's
-//                              nM x (nL+1) table through rowIdx
+//                              sum (perm_prob_table, as finish_kernel of permprob_device_kernel.cu), written straight
+//                              into the caller's nM x (nL+1) table through rowIdx
 // The sub-permanents live in slots sized from the UNconditioned dimensions, nM * (nL+1) per problem at probOff[p]
 // (slot (m, l): landmark item l for l < condL, the non-assignment item for l == nL), so the host never needs condL.
 // Scope: nM <= 11.  Every sub-permanent then has a short side <= 10, which the subset DP takes, and no permanent can
@@ -65,17 +65,10 @@ __global__ void __launch_bounds__(32 * PERM_WARPS) cond_perm_kernel(const CondPe
         const int64_t slot = slot0 + (int64_t)m * (L + 1) + (l < cL ? l : L);
         Gather g;
         if (!item_gather(Pp, cL, M, m, l, g)) continue;  // zero likelihood: the finish never reads this slot
-        __syncwarp();  // the previous item's reads of the shared buffers are done
+        // the short side is at most nM - 1 <= PERM_DP_MAX: always the subset DP
         int nKR, nKC;
-        condition_warp(g, scale, keepC, keepR, lane, nKR, nKC);
-        if ((nKR > nKC ? nKR : nKC) > PDA_MAX_PERM_DIM) {  // permanentExactSquare throws (nwPerm.cpp:327-330): 1 and
-            if (lane == 0) { a.perm[slot] = 1.0; a.slotStatus[slot] = 1; }  // status 1, as permanentProb leaves them
-            continue;
-        }
-        write_scaled(g, scale, keepC, keepR, nKR, nKC, 1, sub, lane);
-        __syncwarp();
-        const double r = perm_dp_subsets(sub, nKC, nKR, buf, a.cap, lane);
-        if (lane == 0) { a.perm[slot] = r / scale_product(scale, nKC); a.slotStatus[slot] = 0; }
+        perm_item_warp(g, true, buf, a.cap, sub, scale, keepC, keepR, lane, nKR, nKC,
+                       [&](double v, int st) { a.perm[slot] = v; a.slotStatus[slot] = st; });
     }
 }
 
@@ -108,50 +101,18 @@ __global__ void finish_scatter_kernel(const double* __restrict__ P, const int64_
     }
     __syncwarp();
     const double* Pp = P + costOff[p];
-    if (M == 1) {  // permanentProb with one detection (:166-171): normalise by std::reduce, which sums in blocks of four
-        double norm = 0.0;
-        if (lane == 0) {
-            const int n = cL + 1;
-            double acc = 0.0;
-            int i = 0;
-            for (; n - i >= 4; i += 4) acc = acc + ((Pp[i] + Pp[i + 1]) + (Pp[i + 2] + Pp[i + 3]));
-            for (; i < n; ++i) acc = acc + Pp[i];
-            norm = 1.0 / acc;
-            status[p] = 0;
-        }
-        norm = __shfl_sync(0xffffffffu, norm, 0);
-        for (int i = lane; i <= cL; i += 32) out[i < cL ? (int)idx[i] : L] = Pp[i] * norm;
+    // permprob_device_kernel.cu's finish_kernel on the conditioned problem (nL = cL): the terms go back into the slots,
+    // the table entries through rowIdx (:68-74)
+    const auto put = [&](int m, int l, int, double v) { out[(size_t)m * (L + 1) + (l < cL ? (int)idx[l] : L)] = v; };
+    if (M == 1) {
+        perm_prob_one(Pp, cL, put, lane);
+        if (lane == 0) status[p] = 0;
         return;
     }
-    // permprob_device_kernel.cu's finish_kernel on the conditioned problem (nL = cL); the terms go back into the slots
-    const int good = cL + M;
     const int64_t slot0 = probOff[p];
-    double best = 0.0;
-    int bad = 0;
-    for (int m = lane; m < M; m += 32) {
-        double colPerm = 0.0;
-        for (int l = 0; l <= cL; ++l) {
-            const int64_t s = slot0 + (int64_t)m * (L + 1) + (l < cL ? l : L);
-            const double e = (l < cL) ? Pp[l + (size_t)m * good] : Pp[(cL + m) + (size_t)m * good];
-            double t = 0.0;
-            if (l == cL || e != 0.0) {
-                bad |= slotStatus[s];
-                t = fabs(e * perm[s]);
-                colPerm += t;
-            }
-            perm[s] = t;
-        }
-        best = (best < colPerm) ? colPerm : best;  // std::max over columns (:255)
-    }
-    best = warp_max(best);
-    bad = __any_sync(0xffffffffu, bad != 0);
-    __syncwarp();
-    const double norm = 1.0 / best;
-    for (int e = lane; e < M * (cL + 1); e += 32) {  // scatter through rowIdx (:68-74)
-        const int m = e / (cL + 1), l = e % (cL + 1);
-        const int dst = (l < cL) ? (int)idx[l] : L;
-        out[(size_t)m * (L + 1) + dst] = perm[slot0 + (int64_t)m * (L + 1) + (l < cL ? l : L)] * norm;
-    }
+    const auto slot = [&](int m, int l, int) { return slot0 + (int64_t)m * (L + 1) + (l < cL ? l : L); };
+    const bool bad = perm_prob_table(Pp, cL, M, perm, slotStatus, slot,
+                                     [&](int m, int l, int e) -> double& { return perm[slot(m, l, e)]; }, put, lane);
     if (lane == 0) status[p] = bad ? 1 : 0;
 }
 

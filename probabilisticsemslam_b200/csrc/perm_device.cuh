@@ -1,6 +1,7 @@
 // perm_device.cuh -- device pieces of permanentProb shared by permanentProb / conditionedPermanent
 // (permprob_device_kernel.cu), the permanent kernel's subset DP (permanent_kernel.cu) and the fused conditioned-permanent
-// pipeline (association_perm_kernel.cu).  All of them run the SAME code here, so their results agree bit for bit.
+// pipeline (association_perm_kernel.cu): the conditioning, the subset DP, one item and the table.  All of them run the
+// SAME code here, so their results agree bit for bit.
 #ifndef PDA_PERM_DEVICE_CUH
 #define PDA_PERM_DEVICE_CUH
 
@@ -104,6 +105,10 @@ __device__ __forceinline__ double scale_product(const double* scale, const int n
     return sf;
 }
 
+// Short sides the subset DP takes: matrices and permanentProb items with a short side up to this run perm_dp_subsets
+// rather than the NW walk.
+constexpr int PERM_DP_MAX = 10;
+
 // Sum over injective maps of the short side of the rows x cols matrix A (column-major) into its long side, by the subset
 // dynamic programme over the short side (see perm_dp_warp in permanent_kernel.cu):
 //     f_j[S] = f_{j-1}[S] + sum_{i in S} B[i, j] * f_{j-1}[S \ {i}],        perm = f_n[all].
@@ -136,6 +141,84 @@ __device__ __forceinline__ double perm_dp_subsets(const double* A, const int row
     }
     __syncwarp();
     return cur[states - 1];
+}
+
+// One permanentProb item by one warp (assignment.cpp:355-402): conditions g into scale / keepC / keepR (condition_warp)
+// and nKR x nKC.  More than 32 kept rows or columns is where permanentExactSquare throws (nwPerm.cpp:327-330): lane 0
+// stores status 1 with 1 (an empty permanent over scale 1) as the value.  Else, when `dp` is set and the short side is
+// at most PERM_DP_MAX, the scaled transposed sub-matrix goes to `sub` and through the subset DP in buf (cap states), and
+// lane 0 stores perm / scale with status 0.  store(value, status) is called by lane 0 only.  Returns false when nothing
+// was stored: the caller takes the conditioned item on.
+template <class Store>
+__device__ __forceinline__ bool perm_item_warp(const Gather& g, const bool dp, double* buf, const int cap, double* sub,
+                                               double* scale, short* keepC, short* keepR, const int lane, int& nKR, int& nKC,
+                                               Store store) {
+    __syncwarp();  // the previous item's reads of the shared buffers are done
+    condition_warp(g, scale, keepC, keepR, lane, nKR, nKC);
+    if ((nKR > nKC ? nKR : nKC) > PDA_MAX_PERM_DIM) {
+        if (lane == 0) store(1.0, 1);
+        return true;
+    }
+    if (!dp || (nKR < nKC ? nKR : nKC) > PERM_DP_MAX) return false;
+    write_scaled(g, scale, keepC, keepR, nKR, nKC, 1, sub, lane);
+    __syncwarp();
+    const double r = perm_dp_subsets(sub, nKC, nKR, buf, cap, lane);
+    if (lane == 0) store(r / scale_product(scale, nKC), 0);
+    return true;
+}
+
+// permanentProb's table with one detection (assignment.cpp:166-171): the likelihoods P[0, nL] over their sum, which
+// std::reduce adds in blocks of four.  One warp; put(0, l, l, v) writes table entry l.
+template <class Put>
+__device__ __forceinline__ void perm_prob_one(const double* P, const int nL, Put put, const int lane) {
+    double norm = 0.0;
+    if (lane == 0) {
+        const int n = nL + 1;
+        double acc = 0.0;
+        int i = 0;
+        for (; n - i >= 4; i += 4) acc = acc + ((P[i] + P[i + 1]) + (P[i + 2] + P[i + 3]));
+        for (; i < n; ++i) acc = acc + P[i];
+        norm = 1.0 / acc;
+    }
+    norm = __shfl_sync(0xffffffffu, norm, 0);
+    for (int i = lane; i <= nL; i += 32) put(0, i, i, P[i] * norm);
+}
+
+// permanentProb's table with nM >= 2 (assignment.cpp:248-262) on the (nL + nM) x nM likelihoods P.  Item (m, l), number
+// e = m (nL + 1) + l of the problem, has its value at perm[slot(m, l, e)] and its status at istat[slot(m, l, e)].  The
+// terms |P(l, m) * perm| (0 for an item a zero likelihood skipped, :217) go to term(m, l, e), then each term over the
+// largest column sum to put(m, l, e, v).  One warp.  Returns whether an item had a non-zero status.
+template <class Slot, class Term, class Put>
+__device__ __forceinline__ bool perm_prob_table(const double* P, const int nL, const int nM, const double* perm,
+                                                const int32_t* istat, Slot slot, Term term, Put put, const int lane) {
+    const int nR = nL + nM;
+    double best = 0.0;
+    int bad = 0;
+    for (int m = lane; m < nM; m += 32) {
+        double colPerm = 0.0;
+        for (int l = 0; l <= nL; ++l) {
+            const int e = m * (nL + 1) + l;
+            const int64_t s = slot(m, l, e);
+            const double p = (l < nL) ? P[l + (size_t)m * nR] : P[(nL + m) + (size_t)m * nR];
+            double t = 0.0;
+            if (l == nL || p != 0.0) {
+                bad |= istat[s];
+                t = fabs(p * perm[s]);
+                colPerm += t;
+            }
+            term(m, l, e) = t;
+        }
+        best = (best < colPerm) ? colPerm : best;  // std::max over columns (:255)
+    }
+    best = warp_max(best);
+    const bool anyBad = __any_sync(0xffffffffu, bad != 0);
+    __syncwarp();
+    const double norm = 1.0 / best;
+    for (int e = lane; e < nM * (nL + 1); e += 32) {
+        const int m = e / (nL + 1), l = e % (nL + 1);
+        put(m, l, e, term(m, l, e) * norm);
+    }
+    return anyBad;
 }
 
 }  // namespace pda

@@ -1,8 +1,11 @@
 // perm_walk.cuh -- the Nijenhuis-Wilf walk of permanent_kernel.cu (see there): error-free double-double sums, the
-// three walk variants, the shared-memory layout, the register budget and the launch shape.  permprob_device_kernel.cu
-// walks its materialised sub-permanents with the same code and the same shape, so both give the same bits.
+// three walk variants, one (matrix, CTA) unit of the walk with its reduction, the last CTA's sum, the shared-memory
+// layout, the register budget, the tile dispatch and the launch shape.  permprob_device_kernel.cu walks its materialised
+// sub-permanents with the same code and the same shape, so both give the same bits.
 #ifndef PDA_PERM_WALK_CUH
 #define PDA_PERM_WALK_CUH
+
+#include <type_traits>
 
 #include "pda_internal.h"
 
@@ -26,6 +29,17 @@ __device__ __forceinline__ dd dd_add(dd a, dd b) {
     r.hi = s + e;
     r.lo = e - (r.hi - s);
     return r;
+}
+// lane 0 gets the sum of the warp's values, in a fixed shuffle tree
+__device__ __forceinline__ dd dd_warp_sum(dd x) {
+#pragma unroll
+    for (int o = 16; o; o >>= 1) {
+        dd other;
+        other.hi = __shfl_down_sync(0xffffffffu, x.hi, o);
+        other.lo = __shfl_down_sync(0xffffffffu, x.lo, o);
+        x = dd_add(x, other);
+    }
+    return x;
 }
 
 // n! for n = 0..32, correctly rounded (tgamma(n+1) of nwPerm.cpp:223)
@@ -295,6 +309,122 @@ __host__ __device__ constexpr bool perm_cache0(int np) { return np <= PERM_C0_MA
 __host__ __device__ constexpr int perm_min_blocks(int np) {
     if (perm_cache01(np)) return np <= 8 ? 4 : 2;
     return perm_cache0(np) ? (np <= 12 ? 4 : (np <= 16 ? 3 : 2)) : (np <= 16 ? 4 : (np <= 24 ? 3 : 2));
+}
+
+// One unit of an NW launch: CTA `cta` of the cpm CTAs that share the matrix of this thread's slot (the tpm threads
+// threadIdx.x / tpm).  Stages the rows x cols matrix A (column-major) ones-padded to n = max(rows, cols) in sA (NP rows of
+// perm_ld(NP)), its base row in sBase, walks this thread's chunk-aligned share of the Gray indices -- [begin, end) in range
+// mode, all of [0, 2^(n-1)) otherwise -- and adds up lanes, then the slot's warps, into partial[m * stride + cta].
+// `live`: the slot has matrix m; `ok`: walk it (otherwise its partial is 0).  The whole CTA calls this (it synchronises
+// the CTA).  Returns true on the first 32 threads of the slot when this CTA is the last of the matrix's CTAs to arrive,
+// counted in done[m]: that warp then adds up the partials (nw_partials_sum).
+template <int NP>
+__device__ __forceinline__ bool nw_unit(const double* __restrict__ A, const int rows, const int cols, const bool live,
+                                        const bool ok, const bool rangeMode, const unsigned long long begin,
+                                        const unsigned long long end, const int chunk, const int tpm, const int cpm,
+                                        const int cta, double* sA, double* sBase, const int64_t m, dd* partial,
+                                        const int stride, unsigned* done) {
+    __shared__ dd sWarp[PERM_THREADS / 32];
+    __shared__ int sLast[PERM_THREADS / 32];
+    constexpr int LD = perm_ld(NP);
+    const int tid = threadIdx.x, slot = tid / tpm, t = tid % tpm;
+    const int n = rows > cols ? rows : cols;
+    if (ok) {  // ones outside the given block (nwPerm.cpp:226-228), zero rows beyond n
+        for (int e = t; e < NP * n; e += tpm) {
+            const int j = e % NP, k = e / NP;
+            double val = 0.0;
+            if (j < n) val = (j < rows && k < cols) ? A[j + (size_t)k * rows] : 1.0;
+            sA[j + k * LD] = val;
+        }
+    }
+    __syncthreads();
+    if (ok && t < NP) {
+        double b = 1.0;  // padded rows keep x == 1 forever
+        if (t < n) {
+            double rs = 0.0;
+            for (int k = 0; k < n; ++k) rs += sA[t + k * LD];
+            b = sA[t + (n - 1) * LD] - rs / 2;  // nwPerm.cpp:289
+        }
+        sBase[t] = b;
+    }
+    __syncthreads();
+    dd acc;
+    acc.hi = 0.0;
+    acc.lo = 0.0;
+    if (ok) {
+        unsigned long long b0 = 0, b1 = 1ULL << (n - 1);
+        if (rangeMode) { b0 = begin; b1 = end; }
+        // contiguous, chunk-aligned share of [b0, b1) for this thread
+        const unsigned long long total = b1 - b0, ch = (unsigned long long)chunk;
+        const unsigned long long nChunks = (total + ch - 1) / ch;
+        const unsigned long long threads = (unsigned long long)cpm * tpm;
+        const unsigned long long per = (nChunks + threads - 1) / threads;
+        const unsigned long long g = (unsigned long long)cta * tpm + t;
+        unsigned long long lo = b0 + g * per * ch, hi = lo + per * ch;
+        if (hi > b1) hi = b1;
+        if (g * per < nChunks && lo < hi) {
+            if (perm_cache01(NP) && (lo & 3ULL) == 0 && ((hi - lo) & 3ULL) == 0) acc = walk_range_c01<NP>(sA, sBase, lo, hi);
+            else if (perm_cache0(NP) && (lo & 1ULL) == 0) acc = walk_range_c0<NP>(sA, sBase, lo, hi);
+            else acc = walk_range<NP>(sA, sBase, lo, hi);
+        }
+    }
+    // fixed-order reduction: lanes, then the warps that share the matrix
+    acc = dd_warp_sum(acc);
+    if ((tid & 31) == 0) sWarp[tid >> 5] = acc;
+    __syncthreads();
+    if (live && t == 0) {
+        const int w0 = tid >> 5, nw = tpm >> 5;
+        dd tot = sWarp[w0];
+        for (int w = 1; w < nw; ++w) tot = dd_add(tot, sWarp[w0 + w]);
+        partial[(size_t)m * stride + cta] = tot;
+        bool last = true;
+        if (cpm > 1) {
+            __threadfence();  // the partial above is visible before the arrival is counted
+            last = atomicAdd(&done[m], 1u) == (unsigned)cpm - 1u;
+        }
+        sLast[slot] = last ? 1 : 0;
+    }
+    __syncthreads();
+    return live && t < 32 && sLast[slot];
+}
+
+// The last CTA of a matrix adds up its cpm per-CTA partials, which other CTAs wrote: lane-strided, then a fixed shuffle
+// tree, so the order depends only on cpm and the result is reproducible.  One warp; lane 0 gets the sum.
+__device__ __forceinline__ dd nw_partials_sum(const dd* partial, const int cpm, const int lane) {
+    __threadfence();
+    dd s;
+    s.hi = 0.0;
+    s.lo = 0.0;
+    for (int c = lane; c < cpm; c += 32) {
+        const double2 v = __ldcg(reinterpret_cast<const double2*>(partial + c));
+        dd o;
+        o.hi = v.x; o.lo = v.y;
+        s = dd_add(s, o);
+    }
+    return dd_warp_sum(s);
+}
+
+// The permanent from the NW sum s of a rows x cols matrix: sign and factor 2 (nwPerm.cpp:326), and for a rectangular one
+// the division by (|rows - cols|)! of the ones-padding (nwPerm.cpp:223-230).
+__device__ __forceinline__ double nw_value(const dd s, const int rows, const int cols) {
+    const int n = rows > cols ? rows : cols;
+    double p = (double)(4 * (n & 1) - 2) * (s.hi + s.lo);
+    if (rows != cols) p = p / kFactorial[rows > cols ? rows - cols : cols - rows];
+    return p;
+}
+
+// Calls launch(std::integral_constant<int, NP>()) with the NW tile of dimension maxN: the even NP at or above it, and at
+// least MinNP (no smaller tile is instantiated).
+template <int MinNP, class Launch>
+int nw_dispatch(const int maxN, Launch&& launch) {
+    const int np = (maxN + 1) / 2 * 2;
+    switch (np < MinNP ? MinNP : np) {
+#define PDA_CASE(N) case N: if constexpr (N >= MinNP) return launch(std::integral_constant<int, N>()); break;
+        PDA_CASE(2) PDA_CASE(4) PDA_CASE(6) PDA_CASE(8) PDA_CASE(10) PDA_CASE(12) PDA_CASE(14) PDA_CASE(16)
+        PDA_CASE(18) PDA_CASE(20) PDA_CASE(22) PDA_CASE(24) PDA_CASE(26) PDA_CASE(28) PDA_CASE(30) PDA_CASE(32)
+#undef PDA_CASE
+    }
+    return fail(PDA_ERR_UNSUPPORTED, "permanent: dimension %d above %d", maxN, PDA_MAX_PERM_DIM);
 }
 
 }  // namespace

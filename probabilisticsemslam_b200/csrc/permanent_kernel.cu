@@ -8,8 +8,9 @@
 // flips the SAME column at the same step, so the column is read from shared memory as
 // a broadcast; x lives in registers (row count is a template parameter, rows padded
 // with x == 1); the running sum is kept as an error-free double-double and reduced in
-// a fixed order (lane, warp, CTA, then a finalize kernel over CTAs), so results are
-// reproducible and slightly MORE accurate than the reference's single running double.
+// a fixed order (lane, warp, CTA, then the CTAs of a matrix, added up by the last one
+// to finish), so results are reproducible and slightly MORE accurate than the
+// reference's single running double.
 // Bound: FP64 pipe (n DFMA + n DMUL per subset per thread); the matrix is <= 8 KB.
 //
 // Rectangular input follows permanentExact (nwPerm.cpp:217-231): pad with ones to
@@ -25,9 +26,7 @@
 namespace pda {
 namespace {
 
-constexpr unsigned FULL = 0xffffffffu;
-
-// dd, the walk variants, perm_ld, perm_min_blocks: perm_walk.cuh
+// dd, the walk variants, nw_unit, perm_ld, perm_min_blocks: perm_walk.cuh
 
 struct PermArgs {
     const double* mats; const int64_t* matOff; const int32_t* rows; const int32_t* cols;
@@ -42,148 +41,51 @@ struct PermArgs {
     int maxN;           // largest dimension in the batch (sizes the shared-memory slots)
     dd* partial;        // [nMats * ctasPerMat]
     int dpBits;         // matrices whose SMALLER side is <= dpBits go to perm_dp_kernel instead (-1: none)
-    // fused finalisation: the CTA that finishes a matrix last sums the per-CTA partials (same fixed order as
-    // perm_finalize_kernel) and writes the result, so a large single matrix costs ONE launch
-    int fuse;
     unsigned* done;     // [nMats] arrival counters (zero before the launch; the finishing CTA resets its counter)
     double* out; int32_t* status; double* rangePartial;
     int oneDim;         // > 0: a single oneDim x oneDim matrix at mats[0]; rows / cols / matOff are not read (range mode)
 };
 
-// Matrices with a small side are not walked by the NW kernel at all: see perm_dp_kernel.
-constexpr int PERM_DP_MAX = 10;
 __device__ __forceinline__ bool perm_uses_dp(const int rows, const int cols, const int dpBits) {
     return (rows < cols ? rows : cols) <= dpBits;
 }
 
-
-// Sums the per-CTA partials of matrix m (lane-strided, then a fixed shuffle tree: the order depends only on ctasPerMat,
-// so results are reproducible) and applies sign, factor 2 and the rectangular scale.  One warp.
-__device__ __forceinline__ void perm_finish_warp(const PermArgs& a, const int64_t m, double* __restrict__ out,
-                                                 int32_t* __restrict__ status, double* __restrict__ rangePartial, const int lane) {
-    dd t;
-    t.hi = 0.0;
-    t.lo = 0.0;
-    for (int c = lane; c < a.ctasPerMat; c += 32) {
-        const double2 v = __ldcg(reinterpret_cast<const double2*>(a.partial + (size_t)m * a.ctasPerMat + c));  // written by other CTAs
-        dd o;
-        o.hi = v.x; o.lo = v.y;
-        t = dd_add(t, o);
-    }
-#pragma unroll
-    for (int o = 16; o; o >>= 1) {
-        dd other;
-        other.hi = __shfl_down_sync(FULL, t.hi, o);
-        other.lo = __shfl_down_sync(FULL, t.lo, o);
-        t = dd_add(t, other);
-    }
-    if (lane != 0) return;
+// Lane 0 of the CTA that completes matrix m: the raw NW sum s in range mode, else the status and the permanent.
+__device__ __forceinline__ void perm_finish(const PermArgs& a, const int64_t m, const dd s) {
     if (a.rangeMode) {
-        rangePartial[0] = t.hi;
-        rangePartial[1] = t.lo;
+        a.rangePartial[0] = s.hi;
+        a.rangePartial[1] = s.lo;
         return;
     }
+    // read again rather than kept in registers over the walk
     const int rows = a.oneDim > 0 ? a.oneDim : a.rows[m], cols = a.oneDim > 0 ? a.oneDim : a.cols[m];
     const int n = rows > cols ? rows : cols;
-    if (n > PDA_MAX_PERM_DIM) { out[m] = 0.0; if (status) status[m] = 1; return; }  // nwPerm.cpp:327-330 throws
-    if (n > a.maxN) { out[m] = 0.0; if (status) status[m] = 2; return; }  // above the call's maxDim: perm_kernel skipped it
-    if (status) status[m] = 0;
-    if (n == 0) { out[m] = 1.0; return; }  // nwPerm.cpp:261-264
-    double p = (double)(4 * (n & 1) - 2) * (t.hi + t.lo);
-    if (rows != cols) p = p / kFactorial[rows > cols ? rows - cols : cols - rows];
-    out[m] = p;
+    if (n > PDA_MAX_PERM_DIM) { a.out[m] = 0.0; if (a.status) a.status[m] = 1; return; }  // nwPerm.cpp:327-330 throws
+    if (n > a.maxN) { a.out[m] = 0.0; if (a.status) a.status[m] = 2; return; }  // above the call's maxDim: not walked
+    if (a.status) a.status[m] = 0;
+    a.out[m] = n == 0 ? 1.0 : nw_value(s, rows, cols);  // nwPerm.cpp:261-264
 }
 
+// blockIdx.x is the CTA of a matrix, blockIdx.y the group of matrices.  The CTA that completes a matrix finishes it, so a
+// large single matrix costs one launch.
 template <int NP>
 __global__ void __launch_bounds__(PERM_THREADS, perm_min_blocks(NP)) perm_kernel(const PermArgs a) {
     extern __shared__ __align__(16) double smemD[];
-    __shared__ dd sWarp[PERM_THREADS / 32];
-    const int tid = threadIdx.x, tpm = a.threadsPerMat;
-    const int slot = tid / tpm, t = tid % tpm, slots = PERM_THREADS / tpm;
-    const int64_t m = (int64_t)blockIdx.y * slots + slot;
-    const int cta = blockIdx.x;
-    constexpr int LD = perm_ld(NP);
-    const int slotDoubles = LD * a.maxN + NP;
-    double* sA = smemD + (size_t)slot * slotDoubles;
-    double* sBase = sA + LD * a.maxN;
+    const int tid = threadIdx.x, tpm = a.threadsPerMat, slot = tid / tpm, t = tid % tpm;
+    const int64_t m = (int64_t)blockIdx.y * (PERM_THREADS / tpm) + slot;
+    double* sA = smemD + (size_t)slot * (perm_ld(NP) * a.maxN + NP);
     const bool live = m < a.nMats;
     const int rows = live ? (a.oneDim > 0 ? a.oneDim : a.rows[m]) : 0, cols = live ? (a.oneDim > 0 ? a.oneDim : a.cols[m]) : 0;
     const int n = rows > cols ? rows : cols;
     const bool ok = live && n >= 1 && n <= NP && n <= PDA_MAX_PERM_DIM && n <= a.maxN && !perm_uses_dp(rows, cols, a.dpBits);
-    if (ok) {
-        const double* A = a.mats + (a.oneDim > 0 ? 0 : a.matOff[m]);
-        // stage the matrix: ones outside the given block (nwPerm.cpp:226-228), zero rows beyond n
-        for (int e = t; e < NP * n; e += tpm) {
-            const int j = e % NP, k = e / NP;
-            double val = 0.0;
-            if (j < n) val = (j < rows && k < cols) ? A[j + (size_t)k * rows] : 1.0;
-            sA[j + k * LD] = val;
-        }
-    }
-    __syncthreads();
-    if (ok && t < NP) {
-        double b = 1.0;  // padded rows keep x == 1 forever
-        if (t < n) {
-            double rs = 0.0;
-            for (int k = 0; k < n; ++k) rs += sA[t + k * LD];
-            b = sA[t + (n - 1) * LD] - rs / 2;  // nwPerm.cpp:289
-        }
-        sBase[t] = b;
-    }
-    __syncthreads();
-    dd acc;
-    acc.hi = 0.0;
-    acc.lo = 0.0;
-    if (ok) {
-        unsigned long long begin = 0, end = 1ULL << (n - 1);
-        if (a.rangeMode) { begin = a.begin; end = a.end; }
-        // contiguous, chunk-aligned share of [begin, end) for this thread
-        const unsigned long long total = end - begin, chunk = (unsigned long long)a.chunk;
-        const unsigned long long nChunks = (total + chunk - 1) / chunk;
-        const unsigned long long threads = (unsigned long long)a.ctasPerMat * tpm;
-        const unsigned long long per = (nChunks + threads - 1) / threads;
-        const unsigned long long g = (unsigned long long)cta * tpm + t;
-        unsigned long long lo = begin + g * per * chunk, hi = lo + per * chunk;
-        if (hi > end) hi = end;
-        if (g * per < nChunks && lo < hi) {
-            if (perm_cache01(NP) && (lo & 3ULL) == 0 && ((hi - lo) & 3ULL) == 0) acc = walk_range_c01<NP>(sA, sBase, lo, hi);
-            else if (perm_cache0(NP) && (lo & 1ULL) == 0) acc = walk_range_c0<NP>(sA, sBase, lo, hi);
-            else acc = walk_range<NP>(sA, sBase, lo, hi);
-        }
-    }
-    // fixed-order reduction: lanes, then the warps that share the matrix
-#pragma unroll
-    for (int o = 16; o; o >>= 1) {
-        dd other;
-        other.hi = __shfl_down_sync(FULL, acc.hi, o);
-        other.lo = __shfl_down_sync(FULL, acc.lo, o);
-        acc = dd_add(acc, other);
-    }
-    if ((tid & 31) == 0) sWarp[tid >> 5] = acc;
-    __syncthreads();
-    if (live && t == 0) {
-        const int w0 = tid >> 5, nw = tpm >> 5;
-        dd tot = sWarp[w0];
-        for (int w = 1; w < nw; ++w) tot = dd_add(tot, sWarp[w0 + w]);
-        a.partial[(size_t)m * a.ctasPerMat + cta] = tot;
-    }
-    if (a.fuse) {  // the CTA that completes a matrix finalises it: no second launch
-        __shared__ int sLast[PERM_THREADS / 32];
-        if (live && t == 0) {
-            bool last = true;
-            if (a.ctasPerMat > 1) {
-                __threadfence();  // the partial above is visible before the arrival is counted
-                last = atomicAdd(&a.done[m], 1u) == (unsigned)a.ctasPerMat - 1u;
-            }
-            sLast[slot] = last ? 1 : 0;
-        }
-        __syncthreads();
-        if (live && t < 32 && sLast[slot] && !(a.dpBits >= 0 && perm_uses_dp(rows, cols, a.dpBits))) {
-            __threadfence();
-            perm_finish_warp(a, m, a.out, a.status, a.rangePartial, t);
-            if (t == 0 && a.ctasPerMat > 1) a.done[m] = 0u;  // ready for the next launch on this stream
-        }
-    }
+    const bool last = nw_unit<NP>(ok ? a.mats + (a.oneDim > 0 ? 0 : a.matOff[m]) : nullptr, rows, cols, live, ok, a.rangeMode,
+                                  a.begin, a.end, a.chunk, tpm, a.ctasPerMat, blockIdx.x, sA, sA + perm_ld(NP) * a.maxN, m,
+                                  a.partial, a.ctasPerMat, a.done);
+    if (!last || (a.dpBits >= 0 && perm_uses_dp(rows, cols, a.dpBits))) return;
+    const dd s = nw_partials_sum(a.partial + (size_t)m * a.ctasPerMat, a.ctasPerMat, t);
+    if (t != 0) return;
+    perm_finish(a, m, s);
+    if (a.ctasPerMat > 1) a.done[m] = 0u;  // ready for the next launch on this stream
 }
 
 // ---- matrices with a small side: subset dynamic programme ---------------------------------------------------------
@@ -200,31 +102,21 @@ __global__ void __launch_bounds__(PERM_THREADS, perm_min_blocks(NP)) perm_kernel
 // PERM_DP_MAX (square matrices included); the reference's n > 32 limit is kept (status 1) so callers see the same
 // "throws" behaviour.
 __device__ __forceinline__ void perm_dp_warp(const PermArgs& a, const int64_t it, const int rows, const int cols,
-                                             double* __restrict__ buf, double* __restrict__ out,
-                                             int32_t* __restrict__ status, const int lane) {
+                                             double* __restrict__ buf, const int lane) {
     const int n = rows < cols ? cols : rows;
-    if (n > PDA_MAX_PERM_DIM) { if (lane == 0) { out[it] = 0.0; if (status) status[it] = 1; } return; }  // nwPerm.cpp:327-330
+    if (n > PDA_MAX_PERM_DIM) { if (lane == 0) { a.out[it] = 0.0; if (a.status) a.status[it] = 1; } return; }  // nwPerm.cpp:327-330
     const double r = perm_dp_subsets(a.mats + a.matOff[it], rows, cols, buf, 1 << a.dpBits, lane);
-    if (lane == 0) { out[it] = r; if (status) status[it] = 0; }
+    if (lane == 0) { a.out[it] = r; if (a.status) a.status[it] = 0; }
 }
 
-// One warp per matrix: sums the per-CTA partials (lane-strided, then a fixed shuffle tree -- the order depends
-// only on ctasPerMat, so results are reproducible) and applies sign, factor 2 and the rectangular scale.
-__global__ void perm_finalize_kernel(const PermArgs a, double* __restrict__ out, int32_t* __restrict__ status,
-                                     double* __restrict__ rangePartial) {
+// One warp per matrix: the short-sided matrices, which perm_kernel leaves alone.
+__global__ void perm_dp_kernel(const PermArgs a) {
     extern __shared__ __align__(16) double smemD[];
-    const int lane = threadIdx.x & 31;
     const int64_t m = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (m >= a.nMats) return;
-    if (a.dpBits >= 0 && !a.rangeMode) {
-        const int rows = a.oneDim > 0 ? a.oneDim : a.rows[m], cols = a.oneDim > 0 ? a.oneDim : a.cols[m];
-        if (perm_uses_dp(rows, cols, a.dpBits)) {  // the NW kernel skipped this one
-            perm_dp_warp(a, m, rows, cols, smemD + (size_t)(threadIdx.x >> 5) * (2 * ((size_t)1 << a.dpBits) + 16), out, status, lane);
-            return;
-        }
-    }
-    if (a.fuse) return;  // perm_kernel finalised this one itself
-    perm_finish_warp(a, m, out, status, rangePartial, lane);
+    const int rows = a.rows[m], cols = a.cols[m];
+    if (!perm_uses_dp(rows, cols, a.dpBits)) return;
+    perm_dp_warp(a, m, rows, cols, smemD + (size_t)(threadIdx.x >> 5) * (2 * ((size_t)1 << a.dpBits) + 16), threadIdx.x & 31);
 }
 
 template <int NP>
@@ -239,14 +131,7 @@ int launch_np(const PermArgs& a, cudaStream_t stream) {
 }
 
 int dispatch(const PermArgs& a, cudaStream_t stream) {
-    const int np = std::max(2, (a.maxN + 1) / 2 * 2);
-    switch (np) {
-#define PDA_CASE(N) case N: return launch_np<N>(a, stream);
-        PDA_CASE(2) PDA_CASE(4) PDA_CASE(6) PDA_CASE(8) PDA_CASE(10) PDA_CASE(12) PDA_CASE(14) PDA_CASE(16)
-        PDA_CASE(18) PDA_CASE(20) PDA_CASE(22) PDA_CASE(24) PDA_CASE(26) PDA_CASE(28) PDA_CASE(30) PDA_CASE(32)
-#undef PDA_CASE
-    }
-    return fail(PDA_ERR_UNSUPPORTED, "permanent: dimension %d above %d", a.maxN, PDA_MAX_PERM_DIM);
+    return nw_dispatch<2>(a.maxN, [&](auto np) { return launch_np<decltype(np)::value>(a, stream); });
 }
 
 }  // namespace
@@ -258,22 +143,22 @@ int launch_permanent_batch(const double* mats, const int64_t* matOff, const int3
                            int64_t workspaceBytes, cudaStream_t stream, int32_t maxSmall, int32_t minSmall) {
     DeviceInfo dev;
     PDA_TRY(current_device_info(&dev));
-    // 0 when maxDim is 0: every matrix with a side then ends as status 2 (perm_finish_warp)
+    // 0 when maxDim is 0: every matrix with a side then ends as status 2 (perm_kernel)
     const int effDim = std::max(0, std::min<int>(maxDim, PDA_MAX_PERM_DIM));
     // maxSmall / minSmall: bounds on min(rows, cols) over the batch when the caller knows them (else maxDim / 0)
     const int dpBits = std::min(PERM_DP_MAX, std::max(0, std::min<int>(maxSmall < 0 ? maxDim : maxSmall, maxDim)));
     const bool noneDp = minSmall > dpBits;
     // nothing for the NW walk.  Never together with noneDp: the DP path then has no shared memory (dpSmem == 0)
     const bool allDp = !noneDp && (maxSmall >= 0 ? maxSmall : maxDim) <= dpBits;
-    const size_t dpSmem = noneDp ? 0 : (size_t)4 * (2 * ((size_t)1 << dpBits) + 16) * sizeof(double);  // 4 warps per finalize CTA
-    if (dpSmem > 48 * 1024) PDA_CUDA_TRY(cudaFuncSetAttribute(perm_finalize_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dpSmem));
+    const size_t dpSmem = noneDp ? 0 : (size_t)4 * (2 * ((size_t)1 << dpBits) + 16) * sizeof(double);  // 4 warps per DP CTA
+    if (dpSmem > 48 * 1024) PDA_CUDA_TRY(cudaFuncSetAttribute(perm_dp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dpSmem));
     if (allDp) {
-        PermArgs d = {mats, matOff, rows, cols, nMats, 0, 0, 0, 1, 32, 0, effDim, nullptr, dpBits, 0, nullptr, nullptr, nullptr, nullptr, 0};
-        perm_finalize_kernel<<<(unsigned)((nMats + 3) / 4), 128, dpSmem, stream>>>(d, out, status, nullptr);
+        PermArgs d = {mats, matOff, rows, cols, nMats, 0, 0, 0, 1, 32, 0, effDim, nullptr, dpBits, nullptr, out, status, nullptr, 0};
+        perm_dp_kernel<<<(unsigned)((nMats + 3) / 4), 128, dpSmem, stream>>>(d);
         PDA_CUDA_TRY(cudaGetLastError());
         return PDA_OK;
     }
-    // workspace: arrival counters of the fused finalisation, then the per-CTA partial sums
+    // workspace: arrival counters of the matrices, then the per-CTA partial sums
     const int64_t cntBytes = (nMats * 4 + 15) / 16 * 16;
     const int64_t partBytes = workspaceBytes - cntBytes;
     PermShape sh = perm_shape(nMats, effDim, dev.smCount, 0);
@@ -285,7 +170,7 @@ int launch_permanent_batch(const double* mats, const int64_t* matOff, const int3
     if (sh.ctasPerMat > 1) PDA_CUDA_TRY(cudaMemsetAsync(done, 0, (size_t)nMats * 4, stream));
     PermArgs a = {mats, matOff, rows, cols, nMats, 0, 0, 0, sh.chunk, sh.threadsPerMat, sh.ctasPerMat, effDim,
                   reinterpret_cast<dd*>(reinterpret_cast<unsigned char*>(workspace) + cntBytes), noneDp ? -1 : dpBits,
-                  1, done, out, status, nullptr, 0};
+                  done, out, status, nullptr, 0};
     // blockIdx.y is limited to 65535: slice the batch
     const int64_t slots = PERM_THREADS / sh.threadsPerMat, perLaunch = 65535 * slots;
     for (int64_t m0 = 0; m0 < nMats; m0 += perLaunch) {
@@ -298,8 +183,8 @@ int launch_permanent_batch(const double* mats, const int64_t* matOff, const int3
         s.status = status ? status + m0 : nullptr;
         PDA_TRY(dispatch(s, stream));
     }
-    if (!noneDp) {  // only the short-sided matrices are left for this kernel: everything else finalised itself
-        perm_finalize_kernel<<<(unsigned)((nMats + 3) / 4), 128, dpSmem, stream>>>(a, out, status, nullptr);
+    if (!noneDp) {  // the short-sided matrices
+        perm_dp_kernel<<<(unsigned)((nMats + 3) / 4), 128, dpSmem, stream>>>(a);
         PDA_CUDA_TRY(cudaGetLastError());
     }
     return PDA_OK;
@@ -322,7 +207,7 @@ int launch_permanent_range(const double* A, int32_t n, uint64_t begin, uint64_t 
     unsigned* done = reinterpret_cast<unsigned*>(ws);
     if (sh.ctasPerMat > 1) PDA_CUDA_TRY(cudaMemsetAsync(done, 0, 4, stream));
     PermArgs a = {A, nullptr, nullptr, nullptr, 1, begin, end, 1, sh.chunk, sh.threadsPerMat, sh.ctasPerMat, n,
-                  reinterpret_cast<dd*>(ws + 64), -1, 1, done, nullptr, nullptr, partial, n};
+                  reinterpret_cast<dd*>(ws + 64), -1, done, nullptr, nullptr, partial, n};
     return dispatch(a, stream);
 }
 
@@ -347,7 +232,7 @@ int pda_permanent_batch(const double* mats, const int64_t* matOff, const int32_t
     // the dimensions live on the device, so this entry cannot tell whether any matrix has a short side: it walks every
     // matrix the reference's way (NW on the ones-padded square), tiles 2..32 alike (minSmall above every dpBits keeps
     // perm_dp_warp out).  The *_host entries, which see the dimensions, send short-sided matrices to the
-    // cancellation-free subset programme (perm_dp_warp).  A matrix above maxDim ends as status 2 (perm_finish_warp).
+    // cancellation-free subset programme (perm_dp_warp).  A matrix above maxDim ends as status 2 (perm_kernel).
     return launch_permanent_batch(mats, matOff, rows, cols, nMats, maxDim, out, status, workspace, workspaceBytes,
                                   reinterpret_cast<cudaStream_t>(stream), -1, PDA_MAX_DIM + 1);
 }

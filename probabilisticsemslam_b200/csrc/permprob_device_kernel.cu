@@ -33,9 +33,7 @@
 namespace pda {
 namespace {
 
-constexpr unsigned FULLMASK = 0xffffffffu;
-constexpr int DP_MAX = 10;            // short sides the subset DP takes (PERM_DP_MAX of permanent_kernel.cu)
-constexpr int SUB_DOUBLES = PDA_MAX_PERM_DIM * DP_MAX;
+constexpr int SUB_DOUBLES = PDA_MAX_PERM_DIM * PERM_DP_MAX;
 constexpr int GATHER_WARPS = 4;
 constexpr int FINISH_WARPS = 4;
 constexpr int SMEM_BUDGET = 48 * 1024;
@@ -70,7 +68,7 @@ Work carve(void* workspace, int mode, int64_t nUnits, int64_t totalCostElems, in
     const int keptB = std::max(1, std::min(PDA_MAX_PERM_DIM, mode == 0 ? maxB - 1 : maxB));  // kept columns
     Work w{};
     w.cap = cap;
-    w.nw = valid && permOpt != 0 && std::min(keptA, keptB) > DP_MAX;
+    w.nw = valid && permOpt != 0 && std::min(keptA, keptB) > PERM_DP_MAX;
     w.materialise = valid && (permOpt == 0 || w.nw);
     w.slotDoubles = keptA * keptB;
     w.cpmCap = perm_shape(1, PDA_MAX_PERM_DIM, smCount, 0).ctasPerMat;  // no launch shape has more CTAs per matrix
@@ -167,7 +165,8 @@ struct GatherArgs {
 // scales, then the kept column and row indices as shorts
 __host__ __device__ constexpr int gather_doubles(int cap) { return 2 * cap + 16 + SUB_DOUBLES + PDA_MAX_DIM + 2 * PDA_MAX_DIM / 4; }
 
-// One sub-permanent by one warp: conditioned, then either the subset DP and perm / scale, or written to its slot
+// One sub-permanent by one warp: conditioned, then either the subset DP and perm / scale (perm_item_warp), or written
+// to its slot
 __device__ __forceinline__ void gather_item(const GatherArgs& a, const Gather& g, const int64_t it, const int32_t owner,
                                             double* buf, const int lane) {
     double* sub = buf + 2 * a.cap + 16;
@@ -175,20 +174,10 @@ __device__ __forceinline__ void gather_item(const GatherArgs& a, const Gather& g
     short* keepC = reinterpret_cast<short*>(scale + PDA_MAX_DIM);
     short* keepR = keepC + PDA_MAX_DIM;
     const Work& w = a.w;
-    __syncwarp();  // the previous item's reads of the shared buffers are done
     int nKR, nKC;
-    condition_warp(g, scale, keepC, keepR, lane, nKR, nKC);
-    if ((nKR > nKC ? nKR : nKC) > PDA_MAX_PERM_DIM) {  // permanentExactSquare throws (nwPerm.cpp:327-330): status 1,
-        if (lane == 0) { w.perm[it] = 1.0; w.istat[it] = 1; }  // and 1 (an empty permanent over scale 1) as the value
+    if (perm_item_warp(g, a.permOpt != 0, buf, a.cap, sub, scale, keepC, keepR, lane, nKR, nKC,
+                       [&](double v, int st) { w.perm[it] = v; w.istat[it] = st; }))
         return;
-    }
-    if (a.permOpt != 0 && (nKR < nKC ? nKR : nKC) <= DP_MAX) {
-        write_scaled(g, scale, keepC, keepR, nKR, nKC, 1, sub, lane);
-        __syncwarp();
-        const double r = perm_dp_subsets(sub, nKC, nKR, buf, a.cap, lane);
-        if (lane == 0) { w.perm[it] = r / scale_product(scale, nKC); w.istat[it] = 0; }
-        return;
-    }
     double* M = w.mats + (size_t)it * w.slotDoubles;
     write_scaled(g, scale, keepC, keepR, nKR, nKC, 1, M, lane);
     if (lane == 0) {
@@ -265,21 +254,17 @@ struct WalkArgs {
     dd* partial; int cpmCap; unsigned* done; double* out;
 };
 
-// perm_kernel's walk, reduction and fused finalisation for the listed items.  The grid is persistent: unit u is
-// (item group u / cpm, CTA u % cpm) of the launch perm_kernel would be, so every item gets the same per-thread ranges and
-// the same reduction order as in a perm_kernel launch of that shape.
+// perm_kernel's unit of the NW walk (nw_unit) for the listed items.  The grid is persistent: unit u is (item group
+// u / cpm, CTA u % cpm) of the launch perm_kernel would be, so every item gets the same per-thread ranges and the same
+// reduction order as in a perm_kernel launch of that shape.  The shape and the item count are read on the device.
 template <int NP>
 __global__ void __launch_bounds__(PERM_THREADS, perm_min_blocks(NP)) walk_list_kernel(const WalkArgs a) {
     extern __shared__ __align__(16) double smemD[];
-    __shared__ dd sWarp[PERM_THREADS / 32];
-    __shared__ int sLast[PERM_THREADS / 32];
     const PermShape sh = *a.shape;
     const unsigned count = *a.count;
     const int tid = threadIdx.x, tpm = sh.threadsPerMat, cpm = sh.ctasPerMat;
     const int slot = tid / tpm, t = tid % tpm, slots = PERM_THREADS / tpm;
-    constexpr int LD = perm_ld(NP);
-    double* sA = smemD + (size_t)slot * (LD * NP + NP);
-    double* sBase = sA + LD * NP;
+    double* sA = smemD + (size_t)slot * (perm_ld(NP) * NP + NP);
     const long long units = (long long)((count + slots - 1) / slots) * cpm;
     for (long long u = blockIdx.x; u < units; u += gridDim.x) {
         const long long k = (u / cpm) * slots + slot;
@@ -288,88 +273,12 @@ __global__ void __launch_bounds__(PERM_THREADS, perm_min_blocks(NP)) walk_list_k
         const int64_t m = live ? a.list[k] : 0;
         const int rows = live ? a.rows[m] : 0, cols = live ? a.cols[m] : 0;
         const int n = rows > cols ? rows : cols;
-        const bool ok = live && n >= 1 && n <= NP;
-        if (ok) {
-            const double* A = a.mats + (size_t)m * a.slotDoubles;
-            for (int e = t; e < NP * n; e += tpm) {
-                const int j = e % NP, kk = e / NP;
-                double val = 0.0;
-                if (j < n) val = (j < rows && kk < cols) ? A[j + (size_t)kk * rows] : 1.0;
-                sA[j + kk * LD] = val;
-            }
-        }
-        __syncthreads();
-        if (ok && t < NP) {
-            double b = 1.0;
-            if (t < n) {
-                double rs = 0.0;
-                for (int kk = 0; kk < n; ++kk) rs += sA[t + kk * LD];
-                b = sA[t + (n - 1) * LD] - rs / 2;  // nwPerm.cpp:289
-            }
-            sBase[t] = b;
-        }
-        __syncthreads();
-        dd acc;
-        acc.hi = 0.0;
-        acc.lo = 0.0;
-        if (ok) {
-            const unsigned long long end = 1ULL << (n - 1), chunk = (unsigned long long)sh.chunk;
-            const unsigned long long nChunks = (end + chunk - 1) / chunk;
-            const unsigned long long threads = (unsigned long long)cpm * tpm;
-            const unsigned long long per = (nChunks + threads - 1) / threads;
-            const unsigned long long g = (unsigned long long)cta * tpm + t;
-            unsigned long long lo = g * per * chunk, hi = lo + per * chunk;
-            if (hi > end) hi = end;
-            if (g * per < nChunks && lo < hi) {
-                if (perm_cache01(NP) && (lo & 3ULL) == 0 && ((hi - lo) & 3ULL) == 0) acc = walk_range_c01<NP>(sA, sBase, lo, hi);
-                else if (perm_cache0(NP) && (lo & 1ULL) == 0) acc = walk_range_c0<NP>(sA, sBase, lo, hi);
-                else acc = walk_range<NP>(sA, sBase, lo, hi);
-            }
-        }
-#pragma unroll
-        for (int o = 16; o; o >>= 1) {
-            dd other;
-            other.hi = __shfl_down_sync(FULLMASK, acc.hi, o);
-            other.lo = __shfl_down_sync(FULLMASK, acc.lo, o);
-            acc = dd_add(acc, other);
-        }
-        if ((tid & 31) == 0) sWarp[tid >> 5] = acc;
-        __syncthreads();
-        if (live && t == 0) {
-            const int w0 = tid >> 5, nw = tpm >> 5;
-            dd tot = sWarp[w0];
-            for (int w = 1; w < nw; ++w) tot = dd_add(tot, sWarp[w0 + w]);
-            a.partial[(size_t)m * a.cpmCap + cta] = tot;
-            bool last = true;
-            if (cpm > 1) {
-                __threadfence();
-                last = atomicAdd(&a.done[m], 1u) == (unsigned)cpm - 1u;
-            }
-            sLast[slot] = last ? 1 : 0;
-        }
-        __syncthreads();
-        if (live && t < 32 && sLast[slot]) {  // perm_finish_warp
-            __threadfence();
-            dd s;
-            s.hi = 0.0;
-            s.lo = 0.0;
-            for (int c = t; c < cpm; c += 32) {
-                const double2 v = __ldcg(reinterpret_cast<const double2*>(a.partial + (size_t)m * a.cpmCap + c));
-                dd o;
-                o.hi = v.x; o.lo = v.y;
-                s = dd_add(s, o);
-            }
-#pragma unroll
-            for (int o = 16; o; o >>= 1) {
-                dd other;
-                other.hi = __shfl_down_sync(FULLMASK, s.hi, o);
-                other.lo = __shfl_down_sync(FULLMASK, s.lo, o);
-                s = dd_add(s, other);
-            }
+        const bool last = nw_unit<NP>(a.mats + (size_t)m * a.slotDoubles, rows, cols, live, live && n >= 1 && n <= NP, false, 0,
+                                      0, sh.chunk, tpm, cpm, cta, sA, sA + perm_ld(NP) * NP, m, a.partial, a.cpmCap, a.done);
+        if (last) {
+            const dd s = nw_partials_sum(a.partial + (size_t)m * a.cpmCap, cpm, t);
             if (t == 0) {
-                double p = (double)(4 * (n & 1) - 2) * (s.hi + s.lo);
-                if (rows != cols) p = p / kFactorial[rows > cols ? rows - cols : cols - rows];
-                a.out[m] = p;
+                a.out[m] = nw_value(s, rows, cols);
                 if (cpm > 1) a.done[m] = 0u;
             }
         }
@@ -387,13 +296,7 @@ int launch_walk_np(const WalkArgs& a, int smCount, cudaStream_t s) {
 }
 
 int launch_walk(const WalkArgs& a, int maxN, int smCount, cudaStream_t s) {
-    switch (std::max(12, (maxN + 1) / 2 * 2)) {
-#define PDA_CASE(N) case N: return launch_walk_np<N>(a, smCount, s);
-        PDA_CASE(12) PDA_CASE(14) PDA_CASE(16) PDA_CASE(18) PDA_CASE(20) PDA_CASE(22) PDA_CASE(24) PDA_CASE(26)
-        PDA_CASE(28) PDA_CASE(30) PDA_CASE(32)
-#undef PDA_CASE
-    }
-    return fail(PDA_ERR_UNSUPPORTED, "permanent_prob: dimension %d above %d", maxN, PDA_MAX_PERM_DIM);
+    return nw_dispatch<12>(maxN, [&](auto np) { return launch_walk_np<decltype(np)::value>(a, smCount, s); });
 }
 
 // perm[it] /= scale[it] over a device list (:402); negatives go to negList when it is given
@@ -416,23 +319,15 @@ __global__ void finish_kernel(const double* __restrict__ P, const int64_t* __res
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int64_t p = (int64_t)blockIdx.x * FINISH_WARPS + warp;
     if (p >= nProblems) return;
-    const int L = nL[p], M = nM[p], nR = L + M;
+    const int L = nL[p], M = nM[p];
     if (out_of_scope0(L, M, maxRow, maxCol)) { if (lane == 0) status[p] = 2; return; }
     const double* Pp = P + pOff[p];
     double* out = probs + probOff[p];
-    if (M == 1) {  // permanentProb with one detection (:166-171): normalise by std::reduce, which sums in blocks of four
-        double norm = 0.0;
-        if (lane == 0) {
-            const int n = L + 1;
-            double acc = 0.0;
-            int i = 0;
-            for (; n - i >= 4; i += 4) acc = acc + ((Pp[i] + Pp[i + 1]) + (Pp[i + 2] + Pp[i + 3]));
-            for (; i < n; ++i) acc = acc + Pp[i];
-            norm = 1.0 / acc;
-            status[p] = 0;
-        }
-        norm = __shfl_sync(FULLMASK, norm, 0);
-        for (int i = lane; i <= L; i += 32) out[i] = Pp[i] * norm;
+    const auto entry = [&](int, int, int e) -> double& { return out[e]; };
+    const auto put = [&](int, int, int e, double v) { out[e] = v; };
+    if (M == 1) {
+        perm_prob_one(Pp, L, put, lane);
+        if (lane == 0) status[p] = 0;
         return;
     }
     const int64_t it0 = itemOff[p];
@@ -442,28 +337,7 @@ __global__ void finish_kernel(const double* __restrict__ P, const int64_t* __res
         return;
     }
     if (it0 + (int64_t)M * (L + 1) > cap) { if (lane == 0) status[p] = 2; return; }
-    double best = 0.0;
-    int bad = 0;
-    for (int m = lane; m < M; m += 32) {
-        double colPerm = 0.0;
-        for (int l = 0; l <= L; ++l) {
-            const int64_t it = it0 + (int64_t)m * (L + 1) + l;
-            const double e = (l < L) ? Pp[l + (size_t)m * nR] : Pp[(L + m) + (size_t)m * nR];
-            double t = 0.0;
-            if (l == L || e != 0.0) {
-                bad |= istat[it];
-                t = fabs(e * perm[it]);
-                colPerm += t;
-            }
-            out[(size_t)m * (L + 1) + l] = t;
-        }
-        best = (best < colPerm) ? colPerm : best;  // std::max over columns (:255)
-    }
-    best = warp_max(best);
-    bad = __any_sync(FULLMASK, bad != 0);
-    __syncwarp();
-    const double norm = 1.0 / best;
-    for (int e = lane; e < M * (L + 1); e += 32) out[e] *= norm;
+    const bool bad = perm_prob_table(Pp, L, M, perm, istat, [&](int, int, int e) { return it0 + e; }, entry, put, lane);
     if (lane == 0) status[p] = bad ? 1 : 0;
 }
 
@@ -505,7 +379,7 @@ int run(int mode, const double* src, const int64_t* srcOff, const int32_t* a, co
         g.P = src; g.pOff = srcOff;
     }
     if (!valid) return PDA_OK;
-    const int shortMax = std::max(0, std::min(DP_MAX, mode == 0 ? maxB - 1 : maxA));
+    const int shortMax = std::max(0, std::min(PERM_DP_MAX, mode == 0 ? maxB - 1 : maxA));
     g.cap = 1 << shortMax;
     const int perWarp = gather_doubles(g.cap) * (int)sizeof(double);
     g.warps = std::max(1, std::min(GATHER_WARPS, SMEM_BUDGET / perWarp));
